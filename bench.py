@@ -1,13 +1,13 @@
 #!/usr/bin/env python3
 """bench.py - decoded frames/s (48 kHz, 10 ms, mono, 150 B) per GPU, with HBM-roofline fraction and CPU baseline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
   (N > 1: launched by torchrun, one rank per GPU; streams are sharded, no collective on the data path)
 
 A "step" is one Lc3Decoder::decode_frame (or Lc3Encoder::encode_frame) for EVERY stream of the batch: the batched hot
 path, one frame per stream.  Default workload `decode48`: BASELINE.json config 5's 262,144 concurrent 48 kHz / 10 ms /
 150 B mono streams, all of them on one GPU at N = 1 (they fit: 2.9 GB of codec state) and the same count on every
-GPU at N > 1 (weak scaling).  Bitstreams: tests/golden/bench_c1_frames.npy - 1,024 distinct synthetic streams of the
+GPU at N > 1 (weak scaling).  Bitstreams: tests/golden/bench_c1_frames_{0,1}.npy - 1,024 distinct synthetic streams of the
 SURVEY 8d corpus (200-frame clips, oracle-encoded from frame 0 by tools/make_bench_corpus.py), 8 consecutive frames
 each at a per-stream offset in [10, 192], tiled over the batch.  `config.corpus` carries the statistics of what was
 decoded (mean lastnz, near-empty and lsb_mode fractions), measured on the GPU from the decoder's own side information.
@@ -21,6 +21,9 @@ Printed JSON (one line, rank 0):
   e2e          same metric through the host-buffer entry points: pinned host buffers in and out, every step
   roofline     dominant kernel vs the measured HBM copy bandwidth; achieved = algorithmic bytes per launch / kernel time
   cpu_baseline the oracle (C++ restatement of the reference) on the host cores, bounded sample, reported not targeted
+
+--dump-outputs DIR writes what the last timed step returned to its caller (PCM and / or bitstreams, rank 0's streams) as
+DIR/<name>.npy in float32, so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it
 
 WORKLOADS = {
     "decode48": dict(fs=48000, ms=10, nbytes=150, nf=480, streams=262144, mode="decode",
@@ -118,7 +122,25 @@ def algo_bytes(w):
 
 
 def load_frames() -> np.ndarray:
-    return np.load(ROOT / "tests" / "golden" / "bench_c1_frames.npy")          # [1024, 8, 150] u8
+    from tools.corpus import load_bench_c1_frames
+    return load_bench_c1_frames()                                               # [1024, 8, 150] u8
+
+
+DUMP_LIMIT = 60_000_000                 # bytes of float32 in all: a dump stays under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each CUDA tensor of `arrays` (name -> [rows, ...]) as out_dir/<name>.npy in float32.  An array larger than
+    its share of DUMP_LIMIT keeps a fixed, seeded sample of its rows, in order: the same rows on every run of a shape."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT // len(arrays)
+    for name, t in arrays.items():
+        row_bytes = 4 * t[0].numel()
+        if t.shape[0] * row_bytes > share:
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], max(1, share // row_bytes), replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        np.save(Path(out_dir) / f"{name}.npy", t.float().cpu().numpy())
 
 
 def gpu_corpus_stats(dev, sf, fd, frames_fsb):
@@ -371,7 +393,7 @@ def run_mixed(args, w, rank, local_rank, world, dev, dist, quick=False):
         frames[:, first:first + count, :nb] = fr_u[:, idx]
         lens[first:first + count] = nb
         algo += count * (nb + 2 * nf)
-    pcm = torch.empty((S, 480), dtype=torch.int16, device=dev)
+    pcm = torch.zeros((S, 480), dtype=torch.int16, device=dev)         # a bucket writes nf of the 480: the rest stays 0
     stream = torch.cuda.current_stream(dev)
 
     def barrier():
@@ -401,6 +423,8 @@ def run_mixed(args, w, rank, local_rank, world, dev, dist, quick=False):
 
     with ClockSampler(local_rank) as clk:
         ms_total = timed(lambda i: dec.decode_frames(16, frames[i % F], lens, pcm), args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pcm": pcm})
     ups = world * S * args.steps / (ms_total * 1e-3)
     if quick:
         return {"quick": True, "value": ups, "unit": "frames/s", "ms_per_step": ms_total / args.steps, "streams_per_gpu": S}
@@ -513,6 +537,8 @@ def run_file(args, w, rank, local_rank, world, dev, dist, quick=False):
 
     with ClockSampler(local_rank) as clk:
         ms_total = timed(lambda i: dec.decode_stream_frames(16, frames, pcm, scratch), args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"pcm": pcm})
     ups = world * S * F * args.steps / (ms_total * 1e-3)
     if quick:
         return {"quick": True, "value": ups, "unit": "frames/s", "ms_per_step": ms_total / args.steps, "streams_per_gpu": S,
@@ -617,8 +643,12 @@ def main():
     ap.add_argument("--distinct", type=int, default=1024, help="distinct synthetic streams the batch is tiled from (PCM workloads)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the small-batch workloads reported under `secondary`")
-    ap.add_argument("--quick", action="store_true", help="device-resident loop only (for ncu captures; not a bench value)")
+    ap.add_argument("--quick", action="store_true", help="device-resident loop only (for profiler captures; not a bench value)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32, a seeded row sample above 60 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path: use it with --impl ours")
     claim_stdout()
     args.warmup = max(args.warmup, 3)
     w = dict(WORKLOADS[args.workload])
@@ -659,7 +689,7 @@ def main():
         if world == 1 and args.workload == "decode48" and not args.no_secondary:
             sec = {}
             sargs = argparse.Namespace(**vars(args))
-            sargs.steps, sargs.warmup = 200, 10
+            sargs.steps, sargs.warmup, sargs.dump_outputs = 200, 10, None
             for name in ("decode16", "mixed", "encode48", "file16"):
                 ws = dict(WORKLOADS[name])
                 fn = {"mixed": run_mixed, "file": run_file}.get(ws["mode"], run_codec)
@@ -782,6 +812,8 @@ def run_codec(args, w, rank, local_rank, world, dev, dist, quick=False):
     # ---- device-resident throughput (value) with clocks sampled during the timed region
     with ClockSampler(local_rank) as clk:
         ms_total = timed(step_dev, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {k: v for k, v in (("frames", frames_out), ("pcm", pcm_out)) if v is not None})
     clocks = clk.summary()
     ups = world * S * args.steps / (ms_total * 1e-3)
     if quick:

@@ -10,12 +10,12 @@ import numpy as np
 
 from conftest import GOLDEN
 from oracle import pyoracle as O
-from tools.corpus import CLIP_FRAMES, clip_offsets, make_pcm, take_window
+from tools.corpus import CLIP_FRAMES, clip_offsets, load_bench_c1_frames, make_pcm, take_window
 from tools.make_bench_corpus import N_FRAMES, stats_of
 
 
 def test_fixture_statistics():
-    frames = np.load(GOLDEN / "bench_c1_frames.npy")
+    frames = load_bench_c1_frames()
     assert frames.shape == (1024, N_FRAMES, 150) and frames.dtype == np.uint8
     doc = json.loads((GOLDEN / "bench_c1_stats.json").read_text())
     st = stats_of(frames, 48000, 10)
@@ -28,7 +28,7 @@ def test_fixture_statistics():
 
 
 def test_fixture_is_reproducible():
-    frames = np.load(GOLDEN / "bench_c1_frames.npy")
+    frames = load_bench_c1_frames()
     n = 24
     full = O.encode_streams(make_pcm(n, CLIP_FRAMES, 48000, 480), 48000, 10, 150)
     off = clip_offsets(n, N_FRAMES)

@@ -10,7 +10,7 @@ For every GPU count G it reports
   strong  BASELINE config 5 as written: 262,144 streams in total, split over the G GPUs
 as frames/s, timed on the host around `steps` calls + wait() after 3 warm-up calls (the copies are the work here, so the
 host clock is the honest one), next to the box's copy ceiling from tools/host_copy_ceiling.py when that file is present.
-Bitstreams: the bench corpus (tests/golden/bench_c1_frames.npy), tiled.
+Bitstreams: the bench corpus (tests/golden/bench_c1_frames_{0,1}.npy), tiled.
 """
 import argparse
 import json
@@ -24,6 +24,7 @@ import torch
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
 import lc3_codec_b200 as L  # noqa: E402
+from tools.corpus import load_bench_c1_frames  # noqa: E402
 
 
 def run(n_streams, devices, steps, corpus):
@@ -57,7 +58,7 @@ def main():
     a = ap.parse_args()
     have = torch.cuda.device_count()
     counts = [int(x) for x in a.gpus.split(",")] if a.gpus else [g for g in (1, 2, 4, 8) if g <= have]
-    corpus = np.load(ROOT / "tests" / "golden" / "bench_c1_frames.npy")
+    corpus = load_bench_c1_frames()
     ceiling = {}
     cf = ROOT / "profiles" / "r2_host_copy_ceiling.json"
     if cf.exists():

@@ -15,6 +15,8 @@ This is bench/test data, not part of the codec path.
 """
 from __future__ import annotations
 
+from pathlib import Path
+
 import numpy as np
 from scipy.signal import lfilter
 
@@ -178,3 +180,13 @@ def make_pcm_window(n_streams: int, n_frames: int, fs: int, nf: int, lead: int =
         clips = make_pcm(n, CLIP_FRAMES, fs, nf, first_stream + i)
         out[i:i + n] = take_window(clips, clip_offsets(n, n_frames, first_stream + i), n_frames, lead)
     return out
+
+
+# ---- the 48 kHz / 10 ms / 150 B bench fixture of tools/make_bench_corpus.py, [1024, 8, 150] u8: stored as two halves of
+# 512 streams so that every golden file stays under 1 MB
+GOLDEN = Path(__file__).resolve().parent.parent / "tests" / "golden"
+BENCH_C1_PARTS = ("bench_c1_frames_0.npy", "bench_c1_frames_1.npy")
+
+
+def load_bench_c1_frames() -> np.ndarray:
+    return np.concatenate([np.load(GOLDEN / p) for p in BENCH_C1_PARTS])

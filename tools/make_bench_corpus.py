@@ -8,7 +8,8 @@ keeps N_FRAMES consecutive frames of every stream starting at a per-stream offse
 offsets are spread over the whole clip, so the fixture samples every part of the sweep, the noise class's two silent
 gaps at their real 10 % duty and the voiced / unvoiced alternation of the speech class.
 
-  tests/golden/bench_c1_frames.npy      [1024, 8, 150] u8   48 kHz / 10 ms / 150 B   (BASELINE configs 1 and 5)
+  tests/golden/bench_c1_frames_{0,1}.npy  [1024, 8, 150] u8 in two halves of 512 streams (tools.corpus.load_bench_c1_frames)
+                                        48 kHz / 10 ms / 150 B   (BASELINE configs 1 and 5)
   tests/golden/bench_c1_stats.json      corpus statistics from the oracle decoder (mean lastnz, near-empty, lsb_mode ...)
   tests/golden/bench_mixed_8k_*.npy     8 kHz bitstreams for the mixed-rate bench (no 8 kHz encoder in the reference)
 
@@ -24,7 +25,8 @@ import numpy as np
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT))
 from oracle import pyoracle as O  # noqa: E402
-from tools.corpus import CLIP_FRAMES, CLIP_SKIP as SKIP, clip_offsets, make_pcm, take_window  # noqa: E402
+from tools.corpus import (BENCH_C1_PARTS, CLIP_FRAMES, CLIP_SKIP as SKIP, GOLDEN, clip_offsets, make_pcm,  # noqa: E402
+                          take_window)
 
 N_FRAMES = 8
 
@@ -49,15 +51,18 @@ def main():
     full = O.encode_streams(pcm, 48000, 10, 150)
     off = clip_offsets(n_streams, N_FRAMES)
     frames = take_window(full, off, N_FRAMES)
-    out = ROOT / "tests" / "golden" / "bench_c1_frames.npy"
-    np.save(out, frames)
+    half = n_streams // len(BENCH_C1_PARTS)
+    for k, name in enumerate(BENCH_C1_PARTS):
+        out = GOLDEN / name
+        np.save(out, frames[k * half:(k + 1) * half])
+        print(out, out.stat().st_size)
     st = stats_of(frames, 48000, 10)
     st.update({"clip_frames": CLIP_FRAMES, "first_frame_min": int(off.min()), "first_frame_max": int(off.max()),
                "whole_clip_frames_10_199": stats_of(full[:192, SKIP:], 48000, 10),
                "source": "tools/make_bench_corpus.py: 200-frame clips (SURVEY 8d), oracle encoder, 8 consecutive frames "
                          "per stream at a per-stream offset in [10, 192]"})
     (ROOT / "tests" / "golden" / "bench_c1_stats.json").write_text(json.dumps(st, indent=1) + "\n")
-    print(out, frames.shape, frames.dtype, out.stat().st_size)
+    print(frames.shape, frames.dtype)
     print(json.dumps(st, indent=1))
 
     # 8 kHz bitstreams for the mixed-rate bench (BASELINE config 4): the reference encoder (and therefore the GPU
