@@ -2,7 +2,8 @@
 //   lc3b_codec_file encode in.wav out.lc3 <fs> <ms> <nbytes_per_channel>     examples/encode.rs:37-116
 //   lc3b_codec_file decode in.lc3 out.wav <fs> <ms> <nbytes_per_channel> <channels>   examples/decode.rs:37-123
 //   lc3b_codec_file wavtest                                                  wav.rs:130-148 (no GPU needed)
-// Channels of the file are the streams of one batched handle; one call per frame period.
+// Channels of the file are the streams of one batched handle; each direction runs time-parallel calls over many frame
+// periods (lc3b_encode_stream_frames / lc3b_decode_stream_frames) instead of one call per period.
 #include <cuda_runtime.h>
 
 #include <cstdio>
@@ -68,21 +69,39 @@ static int encode(const char* wav_name, const char* lc3_name, int hz, const std:
     CUDA_OK(cudaMalloc(&ws, ws_bytes));
     Lc3BatchEncoder enc(nch, d, f, ws, ws_bytes, nbytes);
     const size_t nf = (size_t)enc.config.nf, bytes_per_frame = nf * nch * 2;
-    int16_t* samples = nullptr;
-    uint8_t* bits = nullptr;
-    CUDA_OK(cudaMallocHost((void**)&samples, nf * nch * sizeof(int16_t)));
-    CUDA_OK(cudaMallocHost((void**)&bits, nch * nbytes));
-    std::ofstream out(lc3_name, std::ios::binary);
-    size_t periods = 0;
-    for (size_t cur = wh.data_start_position; cur < in.size(); cur += bytes_per_frame, periods++) {   // encode.rs:73
-        const size_t avail = std::min(in.size() - cur, bytes_per_frame) / (2 * nch);
-        deinterleave(in.data() + cur, avail, nf, nch, samples);
-        enc.encode_frames(Residency::Host, samples, bits, nbytes, nbytes);
-        CUDA_OK(cudaStreamSynchronize(nullptr));
-        out.write((const char*)bits, (std::streamsize)(nch * nbytes));
+    const size_t data_bytes = in.size() > wh.data_start_position ? in.size() - wh.data_start_position : 0;
+    const size_t periods = (data_bytes + bytes_per_frame - 1) / bytes_per_frame;               // encode.rs:73
+    // up to CHUNK frame periods per time-parallel call, staged channel-major: [nch][F][nf] in, [nch][F][nbytes] out
+    constexpr size_t CHUNK = 4096;
+    const size_t max_f = std::min(periods, CHUNK);
+    std::vector<int16_t> period(nch * nf), staged(nch * max_f * nf);
+    std::vector<uint8_t> bits(nch * max_f * nbytes);
+    int16_t* d_pcm = nullptr;
+    uint8_t* d_bits = nullptr;
+    void* d_scratch = nullptr;
+    const size_t scratch_bytes = max_f ? enc.multi_scratch_bytes(max_f) : 0;
+    if (max_f) {
+        CUDA_OK(cudaMalloc((void**)&d_pcm, staged.size() * sizeof(int16_t)));
+        CUDA_OK(cudaMalloc((void**)&d_bits, bits.size()));
+        CUDA_OK(cudaMalloc(&d_scratch, scratch_bytes));
     }
-    std::printf("encoded %zu frame periods x %zu channels\n", periods, nch);
-    cudaFreeHost(samples); cudaFreeHost(bits); cudaFree(ws);
+    std::ofstream out(lc3_name, std::ios::binary);
+    for (size_t p0 = 0; p0 < periods; p0 += CHUNK) {
+        const size_t F = std::min(CHUNK, periods - p0);
+        for (size_t p = 0; p < F; p++) {
+            const size_t cur = wh.data_start_position + (p0 + p) * bytes_per_frame;
+            const size_t avail = std::min(in.size() - cur, bytes_per_frame) / (2 * nch);
+            deinterleave(in.data() + cur, avail, nf, nch, period.data());
+            for (size_t c = 0; c < nch; c++) std::memcpy(staged.data() + (c * F + p) * nf, period.data() + c * nf, nf * sizeof(int16_t));
+        }
+        CUDA_OK(cudaMemcpy(d_pcm, staged.data(), nch * F * nf * sizeof(int16_t), cudaMemcpyHostToDevice));
+        enc.encode_stream_frames(d_pcm, F, d_bits, nbytes, nbytes, d_scratch, scratch_bytes);
+        CUDA_OK(cudaMemcpy(bits.data(), d_bits, nch * F * nbytes, cudaMemcpyDeviceToHost));
+        for (size_t p = 0; p < F; p++)
+            for (size_t c = 0; c < nch; c++) out.write((const char*)bits.data() + (c * F + p) * nbytes, (std::streamsize)nbytes);
+    }
+    std::printf("encoded %zu frame periods x %zu channels in %zu calls\n", periods, nch, (periods + CHUNK - 1) / CHUNK);
+    cudaFree(d_pcm); cudaFree(d_bits); cudaFree(d_scratch); cudaFree(ws);
     return 0;
 }
 

@@ -224,6 +224,20 @@ int lc3b_encode_frames_host(lc3b_encoder* h, const int16_t* pcm_in, size_t pcm_s
  * overlaps the kernels of call i.  Results are ordered on `cuda_stream` as before (the bitstream copy stays on it);
  * the caller's PCM buffer must stay valid until the call's work has drained, as with any asynchronous copy. */
 int lc3b_encoder_set_host_pipelining(lc3b_encoder* h, int on);
+/* Time-parallel encode: `n_frames` consecutive frames of EVERY stream in one call - the whole-file workflow of
+ * examples/encode.rs:73-116 without one launch per frame period.  Equivalent to n_frames calls of lc3b_encode_frames
+ * with the same `nbytes` (same bytes, same per-stream state afterwards, so the two entry points can be mixed freely).
+ *   pcm_in      device int16 [n_streams][n_frames*nf]: every stream's audio is contiguous in time
+ *   frames_out  device; frame f of stream s at frames_out + (s*n_frames + f)*frame_stride, `nbytes` bytes each
+ *   scratch     device, at least lc3b_encoder_multi_scratch_bytes(h, n_frames) bytes, 256-byte aligned; caller-owned,
+ *               only used during the call
+ * Returns LC3B_ERR_INVALID_ARG as lc3b_encode_frames does, and for n_frames < 1 or n_streams*n_frames beyond an int;
+ * LC3B_ERR_WORKSPACE for scratch that is too small or misaligned.  The call follows lc3b_encoder_set_graph_mode (the
+ * whole call is one graph launch in graph mode); the stage mask does not apply to it, and lc3b_encoder_debug_read keeps
+ * reporting the last lc3b_encode_frames call (this call does not touch those buffers). */
+int lc3b_encoder_multi_scratch_bytes(const lc3b_encoder* h, int n_frames, size_t* device_bytes);
+int lc3b_encode_stream_frames(lc3b_encoder* h, const int16_t* pcm_in, int n_frames, uint8_t* frames_out, int nbytes,
+                              size_t frame_stride, void* scratch, size_t scratch_bytes, void* cuda_stream);
 int lc3b_encoder_set_graph_mode(lc3b_encoder* h, int mode);   /* as lc3b_decoder_set_graph_mode */
 /* Test hook: device copies of the last encode's intermediates (any pointer may be NULL): xf [S][ne] f32 (quantiser
  * input, after SNS and TNS), e_b [S][64] f32, hand [S][8] i32 (near_nyquist, attack, pitch_index, pitch_present,

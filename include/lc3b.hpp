@@ -158,6 +158,21 @@ class Lc3BatchEncoder {
         detail::check(fn(h_, samples_in, (size_t)config.nf, buf_out, (int)nbytes, frame_stride, stream_), "lc3b_encode_frames");
         return std::nullopt;
     }
+    // Time-parallel encode: n_frames consecutive frames of every stream in one call; equivalent to n_frames encode_frames
+    // calls (same bytes, same state afterwards).  Device buffers: samples_in [num_streams][n_frames * nf], buf_out frame f of
+    // stream s at (s * n_frames + f) * frame_stride, scratch >= multi_scratch_bytes(n_frames) bytes (caller-owned).
+    size_t multi_scratch_bytes(size_t n_frames) const {
+        size_t n = 0;
+        detail::check(lc3b_encoder_multi_scratch_bytes(h_, (int)n_frames, &n), "lc3b_encoder_multi_scratch_bytes");
+        return n;
+    }
+    Result<Lc3EncoderError> encode_stream_frames(const int16_t* samples_in, size_t n_frames, uint8_t* buf_out, size_t nbytes,
+                                                 size_t frame_stride, void* scratch, size_t scratch_bytes) {
+        detail::check(lc3b_encode_stream_frames(h_, samples_in, (int)n_frames, buf_out, (int)nbytes, frame_stride, scratch,
+                                                scratch_bytes, stream_),
+                      "lc3b_encode_stream_frames");
+        return std::nullopt;
+    }
     void set_host_pipelining(bool on) { detail::check(lc3b_encoder_set_host_pipelining(h_, on ? 1 : 0), "lc3b_encoder_set_host_pipelining"); }
 
     size_t num_streams() const { return num_streams_; }

@@ -31,6 +31,7 @@ struct AnalysisParams {
     size_t pcm_stride;
     int nbytes;
     int n_streams;
+    int n_frames;         // enc_ltpf_kernel: consecutive frames each warp walks; its frame f is unit s * n_frames + f
     int16_t* thist;
     int16_t* xs_hist;
     float* x12;
@@ -204,13 +205,11 @@ __global__ void __launch_bounds__(ANA_WARPS * 32) enc_mdct_kernel(AnalysisParams
     if (lane == 0) p.ehand[(size_t)stream * EH_WORDS + EH_NEAR_NYQUIST] = near_nyquist;
 }
 
-// Kernel 2: attack detector and LTPF analysis (runs after enc_mdct_kernel, whose near-Nyquist flag it reads).
-__global__ void __launch_bounds__(ANA_WARPS * 32) enc_ltpf_kernel(AnalysisParams p) {
-    extern __shared__ __align__(16) uint8_t smem[];
+// Kernel 2, one frame: attack detector and LTPF analysis of stream `stream` (per-stream state) on the input and
+// hand-off record of unit `unit` (runs after enc_mdct_kernel, whose near-Nyquist flag it reads).
+__device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* smem, int stream, size_t unit) {
     const EncConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int stream = blockIdx.x * ANA_WARPS + wid;
-    if (stream >= p.n_streams) return;
     const int nf = c.nf;
 
     uint8_t* base = smem + (size_t)wid * p.smem_per_warp;
@@ -222,10 +221,10 @@ __global__ void __launch_bounds__(ANA_WARPS * 32) enc_ltpf_kernel(AnalysisParams
     float* x6 = x12 + c.x12_len;                    // 178 floats
     float* xs = x6 + 178;                           // x_s_ext_len (<= 540) input samples as f32 (exact)
 
-    const int16_t* x = p.pcm + (size_t)stream * p.pcm_stride;     // this frame's input samples
+    const int16_t* x = p.pcm + unit * p.pcm_stride;               // this frame's input samples
     int32_t* es = p.estate + (size_t)stream * ES_WORDS;
     const int n_live_c = min(ANA_WARPS, p.n_streams - (int)blockIdx.x * ANA_WARPS);   // warps of this CTA that have a frame
-    const int near_nyquist = p.ehand[(size_t)stream * EH_WORDS + EH_NEAR_NYQUIST];
+    const int near_nyquist = p.ehand[unit * EH_WORDS + EH_NEAR_NYQUIST];
     const int up = c.up, ns_keep = 240 / up;
     {   // x_s_extended (long_term_post_filter.rs:217-224): last 240/up samples of the previous frame, then this frame
         int16_t* xh = p.xs_hist + (size_t)stream * 64;
@@ -602,12 +601,28 @@ __global__ void __launch_bounds__(ANA_WARPS * 32) enc_ltpf_kernel(AnalysisParams
             es[ES_MEM_LTPF_ACTIVE] = 0;
             es[ES_MEM_NC] = (int32_t)__float_as_uint(0.0f);
         }
-        int32_t* eh = p.ehand + (size_t)stream * EH_WORDS;
+        int32_t* eh = p.ehand + unit * EH_WORDS;
         eh[EH_ATTACK] = attack_detected;
         eh[EH_PITCH_INDEX] = pitch_index;
         eh[EH_PITCH_PRESENT] = pitch_present;
         eh[EH_LTPF_ACTIVE] = ltpf_active;
         eh[EH_NBITS_LTPF] = pitch_present ? 11 : 1;
+    }
+}
+
+// Kernel 2: a warp per stream walks p.n_frames frames in order (WALK), or encodes one frame (lc3b_encode_frames: a
+// separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a CTA walks the same count, so
+// the named barriers inside a frame stay matched.  The __syncwarp orders the state lane 0 (and warp 0, for the biquad)
+// wrote in frame f before the lanes read it in frame f + 1.
+template <bool WALK>
+__global__ void __launch_bounds__(ANA_WARPS * 32) enc_ltpf_kernel(AnalysisParams p) {
+    extern __shared__ __align__(16) uint8_t smem[];
+    const int stream = blockIdx.x * ANA_WARPS + (threadIdx.x >> 5);
+    if (stream >= p.n_streams) return;
+    const int F = WALK ? p.n_frames : 1;
+    for (int f = 0; f < F; f++) {
+        ltpf_frame(p, smem, stream, (size_t)stream * F + f);
+        if (WALK) __syncwarp();
     }
 }
 
@@ -628,11 +643,14 @@ cudaError_t prepare_enc_analysis(const EncoderState& st) {
     cudaError_t e = cudaFuncSetAttribute(enc_mdct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)(mdct_warp_bytes(st.cfg.nf) * ANA_WARPS));
     if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(enc_ltpf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ltpf_warp_bytes(st.cfg) * ANA_WARPS));
+        e = cudaFuncSetAttribute(enc_ltpf_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ltpf_warp_bytes(st.cfg) * ANA_WARPS));
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(enc_ltpf_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ltpf_warp_bytes(st.cfg) * ANA_WARPS));
     return e;
 }
 
-void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages) {
+void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
+                       int n_frames) {
     AnalysisParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
@@ -644,6 +662,7 @@ void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     p.pcm_stride = pcm_stride;
     p.nbytes = nbytes;
     p.n_streams = st.n_streams;
+    p.n_frames = 1;
     p.thist = st.thist;
     p.xs_hist = st.xs_hist;
     p.x12 = st.x12;
@@ -652,16 +671,18 @@ void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     p.xf = st.xf;
     p.e_b = st.e_b;
     p.ehand = st.ehand;
-    const int grid = (st.n_streams + ANA_WARPS - 1) / ANA_WARPS;
     if (stages & 1) {
         const size_t per_warp = mdct_warp_bytes(st.cfg.nf);
         p.smem_per_warp = (int)per_warp;
-        plan.add(enc_mdct_kernel, (unsigned)grid, ANA_WARPS * 32, per_warp * ANA_WARPS, p);
+        plan.add(enc_mdct_kernel, (unsigned)((st.n_streams + ANA_WARPS - 1) / ANA_WARPS), ANA_WARPS * 32, per_warp * ANA_WARPS, p);
     }
     if (stages & 2) {
         const size_t per_warp = ltpf_warp_bytes(st.cfg);
         p.smem_per_warp = (int)per_warp;
-        plan.add(enc_ltpf_kernel, (unsigned)grid, ANA_WARPS * 32, per_warp * ANA_WARPS, p);
+        p.n_streams = st.n_streams / n_frames;                   // one warp per stream, walking its frames
+        p.n_frames = n_frames;
+        plan.add(n_frames > 1 ? enc_ltpf_kernel<true> : enc_ltpf_kernel<false>, (unsigned)((p.n_streams + ANA_WARPS - 1) / ANA_WARPS),
+                 ANA_WARPS * 32, per_warp * ANA_WARPS, p);
     }
 }
 

@@ -293,6 +293,28 @@ int lc3b_encode_frames(lc3b_encoder* h, const int16_t* pcm_in, size_t pcm_stride
     return LC3B_OK;
 }
 
+int lc3b_encoder_multi_scratch_bytes(const lc3b_encoder* h, int n_frames, size_t* device_bytes) {
+    if (!h || !device_bytes || n_frames < 1 || (size_t)h->st.n_streams * (size_t)n_frames > (size_t)INT32_MAX)
+        return LC3B_ERR_INVALID_ARG;
+    *device_bytes = enc_multi_scratch_bytes(h->st, n_frames);
+    return LC3B_OK;
+}
+
+int lc3b_encode_stream_frames(lc3b_encoder* h, const int16_t* pcm_in, int n_frames, uint8_t* frames_out, int nbytes,
+                              size_t frame_stride, void* scratch, size_t scratch_bytes, void* cuda_stream) {
+    if (!h || !pcm_in || !frames_out || !scratch) return LC3B_ERR_INVALID_ARG;
+    const EncoderState& st = h->st;
+    if (nbytes < 20 || nbytes > st.max_nbytes || (size_t)nbytes > frame_stride || n_frames < 1 ||
+        (size_t)st.n_streams * (size_t)n_frames > (size_t)INT32_MAX)
+        return LC3B_ERR_INVALID_ARG;
+    if (scratch_bytes < enc_multi_scratch_bytes(st, n_frames) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
+    LaunchPlan plan;                                      // the whole call is one plan: one graph launch in graph mode
+    plan_enc_multi(plan, st, pcm_in, n_frames, frames_out, nbytes, frame_stride, scratch);
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    CU(h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream));
+    return LC3B_OK;
+}
+
 int lc3b_encode_frames_host(lc3b_encoder* h, const int16_t* pcm_in, size_t pcm_stride, uint8_t* frames_out, int nbytes,
                             size_t frame_stride, void* cuda_stream) {
     if (!h || !pcm_in || !frames_out) return LC3B_ERR_INVALID_ARG;

@@ -74,9 +74,18 @@ int enc_bitstream_scratch_words(int ne, int max_nbytes);   // per-stream size of
 cudaError_t launch_enc_analysis(const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages, cudaStream_t stream);
 // stages: bit 0 SNS kernel (with the bandwidth detector), bit 1 TNS kernel, bit 2 quantise kernel, bit 3 bitstream kernel
 cudaError_t launch_enc_quant(const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages, cudaStream_t stream);
-// the same launches written into a plan (lc3b_plan.cuh) instead of issued
+// the same launches written into a plan (lc3b_plan.cuh) instead of issued.  n_frames > 1: `st` is a view whose
+// st.n_streams = S * n_frames units (unit s * n_frames + f = frame f of stream s) and whose per-frame buffers have a row
+// per unit; its per-stream state (xs_hist, x12, x6, estate) keeps a row per stream.  The attack / LTPF kernel and the
+// quantise kernel then run a warp per stream that walks the stream's frames in order; every other kernel runs per unit.
 struct LaunchPlan;
-void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages);
-void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages);
+void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
+                       int n_frames = 1);
+void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
+                    int n_frames = 1);
+// time-parallel encode (lc3b_enc_multi.cu): n_frames consecutive frames of every stream as one plan
+size_t enc_multi_scratch_bytes(const EncoderState& st, int n_frames);
+void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_frames, uint8_t* frames_out, int nbytes,
+                    size_t frame_stride, void* scratch);
 
 }  // namespace lc3b

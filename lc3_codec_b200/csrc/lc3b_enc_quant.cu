@@ -37,6 +37,7 @@ namespace lc3b {
 struct QuantParams {
     const EncConfig* cfg;
     int n_streams, nbytes;
+    int n_frames;      // enc_quantize_kernel: consecutive frames each warp walks; its frame f is unit s * n_frames + f
     size_t frame_stride;
     float* xf;
     const float* e_b;
@@ -1506,7 +1507,11 @@ __global__ void __launch_bounds__(QNT_THREADS, 4) enc_tns_kernel(QuantParams p) 
     if (lane < 16) qh[QH_RC_I + lane] = tns.rc_i[lane];
 }
 
-// Kernel B: SpectralQuantization::run.  Shaped spectrum -> quantised spectrum + gain decisions.
+// Kernel B: SpectralQuantization::run.  Shaped spectrum -> quantised spectrum + gain decisions.  WALK: a warp per stream
+// walks p.n_frames frames in order, the rate loop's offsets (ES_Q_*) carrying from one frame to the next; otherwise one
+// frame (lc3b_encode_frames: a separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a
+// CTA walks the same count, so the named barriers inside a frame stay matched.
+template <bool WALK>
 __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const EncConfig& c = *p.cfg;
@@ -1519,21 +1524,26 @@ __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p
     float* e4 = xf + NE_MAX;                                      // [100]
     float* T = e4 + 100;                                          // [224]
     int16_t* xq = (int16_t*)(T + 224);                            // [NE_MAX]
-    const float4* gx = (const float4*)(p.xf + (size_t)stream * ne);
-    WARP_STRIDE(i, ne / 4) ((float4*)xf)[i] = gx[i];
-    __syncwarp();
-    const int32_t* eh = p.ehand + (size_t)stream * EH_WORDS;
     int32_t* es = p.estate + (size_t)stream * ES_WORDS;
-    int32_t* qh = p.qhand + (size_t)stream * QH_WORDS;
     const int n_live = min(QW, p.n_streams - blockIdx.x * QW);    // warps of this CTA that have a frame
-    const QRes q = spectral_quantization_w(c, es, xf, xq, e4, T, p.nbytes * 8, qh[QH_NBITS_BW], qh[QH_NBITS_TNS], eh[EH_NBITS_LTPF], lane,
-                                           wib, n_live, smem);
-    uint32_t* gq = (uint32_t*)(p.xq + (size_t)stream * ne);
-    WARP_STRIDE(i, ne / 2) gq[i] = ((const uint32_t*)xq)[i];
-    if (lane == 0) {
-        qh[QH_GG_IND] = q.gg_ind; qh[QH_NBITS_SPEC] = q.nbits_spec; qh[QH_NBITS_LSB] = q.nbits_lsb; qh[QH_NBITS_TRUNC] = q.nbits_trunc;
-        qh[QH_LSB_MODE] = q.lsb_mode; qh[QH_RATE_FLAG] = q.rate_flag; qh[QH_LASTNZ_TRUNC] = q.lastnz_trunc;
-        qh[QH_GG] = (int32_t)__float_as_uint(q.gg);
+    const int F = WALK ? p.n_frames : 1;
+    for (int f = 0; f < F; f++) {
+        const size_t unit = (size_t)stream * F + f;
+        const float4* gx = (const float4*)(p.xf + unit * ne);
+        WARP_STRIDE(i, ne / 4) ((float4*)xf)[i] = gx[i];
+        __syncwarp();
+        const int32_t* eh = p.ehand + unit * EH_WORDS;
+        int32_t* qh = p.qhand + unit * QH_WORDS;
+        const QRes q = spectral_quantization_w(c, es, xf, xq, e4, T, p.nbytes * 8, qh[QH_NBITS_BW], qh[QH_NBITS_TNS], eh[EH_NBITS_LTPF],
+                                               lane, wib, n_live, smem);
+        uint32_t* gq = (uint32_t*)(p.xq + unit * ne);
+        WARP_STRIDE(i, ne / 2) gq[i] = ((const uint32_t*)xq)[i];
+        if (lane == 0) {
+            qh[QH_GG_IND] = q.gg_ind; qh[QH_NBITS_SPEC] = q.nbits_spec; qh[QH_NBITS_LSB] = q.nbits_lsb; qh[QH_NBITS_TRUNC] = q.nbits_trunc;
+            qh[QH_LSB_MODE] = q.lsb_mode; qh[QH_RATE_FLAG] = q.rate_flag; qh[QH_LASTNZ_TRUNC] = q.lastnz_trunc;
+            qh[QH_GG] = (int32_t)__float_as_uint(q.gg);
+        }
+        if (WALK) __syncwarp();                                   // lane 0's state update before the next frame reads it
     }
 }
 
@@ -1714,18 +1724,21 @@ constexpr size_t QUANTIZE_SMEM = QW * QUANTIZE_WARP_BYTES;
 cudaError_t prepare_enc_quant(const EncoderState& st) {
     cudaError_t e = cudaFuncSetAttribute(enc_sns_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SHAPE_SMEM / QW * SNS_WARPS));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_tns_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SHAPE_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess)
         e = cudaFuncSetAttribute(enc_bs_prepare_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)(QW * bitstream_warp_bytes(st.cfg.ne, st.max_nbytes, nullptr)));
     return e;
 }
 
-void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages) {
+void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
+                    int n_frames) {
     QuantParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
     p.n_streams = st.n_streams;
+    p.n_frames = 1;
     p.nbytes = nbytes;
     p.frame_stride = frame_stride;
     p.xf = st.xf;
@@ -1743,7 +1756,13 @@ void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_ou
     const int grid = (p.n_streams + QW - 1) / QW;
     if (stages & 1) plan.add(enc_sns_kernel, (unsigned)((p.n_streams + SNS_WARPS - 1) / SNS_WARPS), SNS_WARPS * 32, SHAPE_SMEM / QW * SNS_WARPS, p);
     if (stages & 2) plan.add(enc_tns_kernel, (unsigned)grid, QNT_THREADS, SHAPE_SMEM, p);
-    if (stages & 4) plan.add(enc_quantize_kernel, (unsigned)grid, QNT_THREADS, QUANTIZE_SMEM, p);
+    if (stages & 4) {                                              // one warp per stream, walking its frames
+        QuantParams pw = p;
+        pw.n_streams = st.n_streams / n_frames;
+        pw.n_frames = n_frames;
+        plan.add(n_frames > 1 ? enc_quantize_kernel<true> : enc_quantize_kernel<false>, (unsigned)((pw.n_streams + QW - 1) / QW),
+                 QNT_THREADS, QUANTIZE_SMEM, pw);
+    }
     if (stages & 8) {
         plan.add(enc_bs_prepare_kernel, (unsigned)grid, QNT_THREADS, QW * wbytes, p);
         // a thread-per-frame kernel needs ~12 k frames before its serial latency (~80 us) is amortised

@@ -77,6 +77,35 @@ class Lc3BatchEncoder:
         if rc:
             raise Lc3bError(rc, fn.__name__)
 
+    # ------------------------------------------------------------------ time-parallel encode
+    def multi_scratch_bytes(self, n_frames: int) -> int:
+        """Bytes of caller-owned device scratch encode_stream_frames needs for n_frames frames per stream."""
+        n = C.c_size_t(0)
+        rc = native.lib().lc3b_encoder_multi_scratch_bytes(self._h, n_frames, C.byref(n))
+        if rc:
+            raise Lc3bError(rc, "lc3b_encoder_multi_scratch_bytes")
+        return int(n.value)
+
+    def encode_stream_frames(self, pcm_in: torch.Tensor, frames_out: torch.Tensor, scratch: torch.Tensor) -> None:
+        """Many consecutive frames of every stream in one call, equal to n_frames encode_frames calls.
+        pcm_in: CUDA int16 [num_streams, n_frames * nf] contiguous; frames_out: CUDA uint8 [num_streams, n_frames, nbytes]
+        contiguous; scratch: CUDA uint8, >= multi_scratch_bytes(n_frames)."""
+        if not (frames_out.is_cuda and frames_out.dtype == torch.uint8 and frames_out.dim() == 3
+                and frames_out.shape[0] == self.num_streams and frames_out.is_contiguous()):
+            raise Lc3bError(2, "frames_out: want contiguous CUDA uint8 [num_streams, n_frames, nbytes]")
+        F, nb = frames_out.shape[1], frames_out.shape[2]
+        if not (pcm_in.is_cuda and pcm_in.dtype == torch.int16 and pcm_in.dim() == 2 and pcm_in.shape[0] == self.num_streams
+                and pcm_in.shape[1] == F * self.nf and pcm_in.is_contiguous()):
+            raise Lc3bError(2, f"pcm_in: want contiguous CUDA int16 [num_streams, n_frames * nf = {F * self.nf}]")
+        if not (scratch.is_cuda and scratch.dtype == torch.uint8):
+            raise Lc3bError(2, "scratch must be a CUDA uint8 tensor")
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = native.lib().lc3b_encode_stream_frames(self._h, _ptr(pcm_in), F, _ptr(frames_out), nb, nb, _ptr(scratch),
+                                                        scratch.numel(), C.c_void_p(stream))
+        if rc:
+            raise Lc3bError(rc, "lc3b_encode_stream_frames")
+
     def set_host_pipelining(self, on: bool) -> None:
         """Let the PCM upload of encode_frames_host call i+1 overlap the kernels of call i (include/lc3b.h)."""
         rc = native.lib().lc3b_encoder_set_host_pipelining(self._h, 1 if on else 0)

@@ -56,7 +56,7 @@ EXPORTS = ["lc3b_config_new", "lc3b_last_cuda_error", "lc3b_version", "lc3b_deco
            "lc3b_decoder_host_fence", "lc3b_decoder_multi_scratch_bytes", "lc3b_decode_stream_frames", "lc3b_decoder_destroy",
            "lc3b_selftest_math_host",
            "lc3b_selftest_math_device", "lc3b_encoder_workspace_bytes", "lc3b_encoder_init", "lc3b_encode_frames",
-           "lc3b_encode_frames_host", "lc3b_encoder_set_host_pipelining", "lc3b_encoder_debug_read", "lc3b_encoder_set_stage_mask",
+           "lc3b_encode_frames_host", "lc3b_encoder_multi_scratch_bytes", "lc3b_encode_stream_frames", "lc3b_encoder_set_host_pipelining", "lc3b_encoder_debug_read", "lc3b_encoder_set_stage_mask",
            "lc3b_encoder_destroy", "lc3b_decoder_set_graph_mode", "lc3b_decoder_set_split", "lc3b_decoder_graph_stats", "lc3b_decoder_set_dequant_mode", "lc3b_mixed_decoder_set_dequant_mode", "lc3b_decoder_set_min_nbytes", "lc3b_decoder_set_synth_mode", "lc3b_encoder_set_graph_mode",
            "lc3b_mixed_decoder_layout", "lc3b_mixed_decoder_workspace_bytes", "lc3b_mixed_decoder_init", "lc3b_mixed_decode_frames",
            "lc3b_mixed_decode_frames_host", "lc3b_mixed_decoder_set_host_pipelining", "lc3b_mixed_decoder_host_fence",
@@ -106,6 +106,8 @@ def lib() -> C.CDLL:
         L.lc3b_encoder_init.argtypes = [C.POINTER(vp), i32, i32, i32, i32, i32, vp, sz, vp]
         L.lc3b_encode_frames.argtypes = [vp, vp, sz, vp, i32, sz, vp]
         L.lc3b_encode_frames_host.argtypes = [vp, vp, sz, vp, i32, sz, vp]
+        L.lc3b_encoder_multi_scratch_bytes.argtypes = [vp, i32, C.POINTER(sz)]
+        L.lc3b_encode_stream_frames.argtypes = [vp, vp, i32, vp, i32, sz, vp, sz, vp]
         L.lc3b_encoder_debug_read.argtypes = [vp, vp, vp, vp, vp, vp]
         L.lc3b_encoder_set_stage_mask.argtypes = [vp, i32]
         L.lc3b_encoder_set_host_pipelining.argtypes = [vp, i32]

@@ -165,6 +165,11 @@ extern "C" {
     pub fn lc3b_encode_frames_host(h: *mut lc3b_encoder, pcm_in: *const i16, pcm_stride: usize, frames_out: *mut u8,
                                    nbytes: c_int, frame_stride: usize, cuda_stream: *mut c_void) -> c_int;
     pub fn lc3b_encoder_set_host_pipelining(h: *mut lc3b_encoder, on: c_int) -> c_int;
+    /// the frame loop of examples/encode.rs:73-116 as one call: `n_frames` frames of every stream (time-parallel)
+    pub fn lc3b_encoder_multi_scratch_bytes(h: *const lc3b_encoder, n_frames: c_int, device_bytes: *mut usize) -> c_int;
+    pub fn lc3b_encode_stream_frames(h: *mut lc3b_encoder, pcm_in: *const i16, n_frames: c_int, frames_out: *mut u8,
+                                     nbytes: c_int, frame_stride: usize, scratch: *mut c_void, scratch_bytes: usize,
+                                     cuda_stream: *mut c_void) -> c_int;
     pub fn lc3b_encoder_set_graph_mode(h: *mut lc3b_encoder, mode: c_int) -> c_int;
     pub fn lc3b_encoder_destroy(h: *mut lc3b_encoder);
 }

@@ -225,6 +225,27 @@ impl<'a> Lc3BatchEncoder<'a> {
         check(f(self.h, samples_in, self.nf, buf_out, nbytes as i32, stride, self.stream), "lc3b_encode_frames");
         Ok(())
     }
+
+    /// Bytes of caller-owned device scratch `encode_stream_frames` needs for `n_frames` frames per stream.
+    pub fn multi_scratch_bytes(&self, n_frames: usize) -> usize {
+        let mut n = 0usize;
+        check(unsafe { sys::lc3b_encoder_multi_scratch_bytes(self.h, n_frames as i32, &mut n) }, "lc3b_encoder_multi_scratch_bytes");
+        n
+    }
+
+    /// The frame loop of examples/encode.rs:73-116 as ONE call: `n_frames` consecutive frames of every stream
+    /// (time-parallel).  Same bytes and same per-stream state afterwards as `n_frames` calls of `encode_frames`.
+    /// Device buffers: `samples_in` is `[num_streams][n_frames * nf]`; frame f of stream s goes to
+    /// `buf_out[(s * n_frames + f) * stride ..][.. nbytes]`.
+    ///
+    /// # Safety
+    /// Device pointers valid for the stated extents until the stream has drained.
+    pub unsafe fn encode_stream_frames(&mut self, samples_in: *const i16, n_frames: usize, buf_out: *mut u8, nbytes: usize,
+                                       stride: usize, scratch: DeviceBuf<'_>) -> Result<(), Lc3EncoderError> {
+        check(sys::lc3b_encode_stream_frames(self.h, samples_in, n_frames as i32, buf_out, nbytes as i32, stride, scratch.ptr,
+                                             scratch.bytes, self.stream), "lc3b_encode_stream_frames");
+        Ok(())
+    }
     pub fn num_streams(&self) -> usize { self.n_streams }
     pub fn samples_per_frame(&self) -> usize { self.nf }
 }
