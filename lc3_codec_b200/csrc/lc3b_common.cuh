@@ -177,9 +177,6 @@ int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_
 
 cudaError_t prepare_entropy(const DecoderState& st);   // shared-memory limits of the kernels, once per handle
 cudaError_t prepare_synth(const DecoderState& st);
-cudaError_t launch_entropy(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                           size_t frame_stride, int32_t* status_out, int stages, cudaStream_t stream);
-cudaError_t launch_synth(const DecoderState& st, int16_t* pcm_out, size_t pcm_stride, cudaStream_t stream);
 cudaError_t launch_init_state(const DecoderState& st, cudaStream_t stream);
 
 // time-parallel decode (SURVEY.md 8f-1), lc3b_dec_multi.cu

@@ -1525,13 +1525,6 @@ bool use_dequant_warp(int n_streams, int mode) {
 // (run_decode in lc3b_api.cu): measured at 48 kHz / 150 B, 65 536 streams gain 7 %, 131 072 18 %, 262 144 10 %, 32 768 nothing.
 int decode_split_min_streams() { return 65536; }
 
-cudaError_t launch_entropy(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                           size_t frame_stride, int32_t* status_out, int stages, cudaStream_t stream) {
-    LaunchPlan plan;
-    plan_entropy(plan, st, frames, frame_nbytes, nbytes, frame_stride, status_out, stages);
-    return plan_launch_direct(plan, stream);
-}
-
 // Mixed-rate call: one entropy launch over all buckets, one dequantisation launch per frame duration present.
 // Returns the node index of the 10 ms and of the 7.5 ms dequantisation launch (-1 if absent) for the synthesis nodes
 // to depend on.

@@ -21,6 +21,7 @@
 #include "lc3b_imdct.cuh"
 #include "lc3b_plan.cuh"
 #include "lc3b_math.cuh"
+#include "lc3b_synth.cuh"
 
 namespace lc3b {
 
@@ -69,6 +70,7 @@ struct MultiParams {
     int32_t* sstate;
     int16_t* pcm_out;
     int hist_len;
+    int smem_per_warp;    // ltpf_multi_kernel, bytes
 };
 
 constexpr int MW = 4;     // warps per CTA in the warp-per-unit kernels
@@ -86,8 +88,7 @@ __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
     float alpha = u2f((uint32_t)ss[SS_PLC_ALPHA]);
     uint32_t seed = (uint32_t)ss[SS_PLC_SEED];
     __syncwarp();
-    uint32_t A = 1, C = 0;                                        // ne steps of seed' = (16831 + seed * 12821) & 0xFFFF
-    for (int i = 0; i < ne; i++) { C = (16831u + C * 12821u) & 0xFFFFu; A = (A * 12821u) & 0xFFFFu; }
+    const PlcJump jump = plc_lcg_jump(ne);                         // a concealed frame takes ne steps of the LCG
     int last = -1;
     for (int f0 = 0; f0 < p.F; f0 += 32) {
         const int f = f0 + lane;
@@ -111,13 +112,13 @@ __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
                 last = s * p.F + f0 + j;
                 if (lane == j) sd[SD_SRC] = -2;
             } else {
-                if (lost >= 4) alpha = xm(alpha, lost < 8 ? 0.9f : 0.85f);
+                alpha = plc_fade(alpha, lost);
                 if (lane == j) {
                     sd[SD_SRC] = last;
                     sd[SD_PLC_ALPHA] = (int32_t)f2u(alpha);
                     sd[SD_PLC_SEED] = (int32_t)seed;
                 }
-                seed = (A * seed + C) & 0xFFFFu;
+                seed = jump.step(seed);
                 lost++;
             }
         }
@@ -156,21 +157,8 @@ __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
             if (k0 + 32 <= NF / 4 || k4 < NF / 4)
                 ((float4*)P)[k4] = 4 * k4 < NE ? ((const float4*)sp)[k4] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
         }
-    } else {                                                      // packet_loss_concealment.rs:63-85
-        const float alpha = u2f((uint32_t)sd[SD_PLC_ALPHA]);
-        uint32_t sgen = (uint32_t)sd[SD_PLC_SEED];
-        for (int i = 0; i <= lane; i++) sgen = (16831u + sgen * 12821u) & 0xFFFFu;
-        uint32_t a32 = 1, c32 = 0;
-        for (int i = 0; i < 32; i++) { c32 = (16831u + c32 * 12821u) & 0xFFFFu; a32 = (a32 * 12821u) & 0xFFFFu; }
-        for (int k = lane; k < NF; k += 32) {
-            float val = 0.0f;
-            if (k < NE) {
-                const float lg = sp[k];
-                val = sgen < 0x8000u ? xm(lg, alpha) : xm(lg, -alpha);
-                sgen = (a32 * sgen + c32) & 0xFFFFu;
-            }
-            P[k] = val;
-        }
+    } else {                                                      // concealed: the source spectrum, scrambled
+        plc_scramble<NF, NE>(P, sp, u2f((uint32_t)sd[SD_PLC_ALPHA]), (uint32_t)sd[SD_PLC_SEED], lane);
     }
     __syncwarp();
     const float* D = dct_iv_warp<NF>(P, Q, p.dtw, p.ftw, lane);
@@ -184,12 +172,6 @@ __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
 #pragma unroll
     for (int j = 0; j < NPT; j++)
         if (64 * j + 64 <= NF - Z || 64 * j + 2 * lane < NF - Z) tail[32 * j + lane] = make_float2(tl[2 * j], tl[2 * j + 1]);
-}
-
-__device__ __forceinline__ int16_t round_pcm(float v) {            // output_scaling.rs:13-26
-    int32_t q = v > 0.0f ? cast_i32(xa(v, 0.5f)) : cast_i32(xs(v, 0.5f));
-    q = q > 32767 ? 32767 : q < -32768 ? -32768 : q;
-    return (int16_t)q;
 }
 
 // ---------------------------------------------------------------- 4. overlap-add across units, PCM
@@ -208,51 +190,28 @@ __global__ void __launch_bounds__(MW * 32) ola_multi_kernel(MultiParams p) {
         float o = head[n];
         if (n < nf - z) o = xa(prev[n], o);
         xhat[n] = o;
-        out[n] = round_pcm(o);
+        out[n] = (int16_t)round_pcm_i32(o);
     }
 }
 
 // ---------------------------------------------------------------- 5. LTPF over its active spans + state hand-back
-struct LtpfPar { int active, p_int, p_fr, code; };
-__device__ __forceinline__ LtpfPar ltpf_params(const DevConfig& c, const int32_t* sd) {   // :142-190
-    LtpfPar r{sd[SD_LTPF_ACTIVE], 0, 0, 4};
-    if (r.active) {
-        const int pi = sd[SD_PITCH_INDEX], nbits = sd[SD_NBITS];
-        int pit;
-        double pfr;
-        if (pi >= 440) { pit = pi - 283; pfr = 0.0; }
-        else if (pi >= 380) { pit = pi / 2 - 63; pfr = (double)(2 * pi - 4 * pit - 252); }
-        else { pit = pi / 4 + 32; pfr = (double)(pi + 128 - 4 * pit); }
-        const double pitch = (double)pit + pfr / 4.0;
-        const double pitch_fs = pitch * (8000.0 * ceil((double)c.fs / 8000.0) / 12800.0);
-        const int p_up = (int)((pitch_fs * 4.0) + 0.5);
-        r.p_int = p_up / 4;
-        r.p_fr = p_up - 4 * r.p_int;
-        const int t_nbits = c.n_ms == LC3B_7P5MS ? (int)round((double)nbits * 10.0 / 7.5) : nbits;
-        const int sf = c.fs_ind * 80;
-        r.code = t_nbits < 320 + sf ? 0 : t_nbits < 400 + sf ? 1 : t_nbits < 480 + sf ? 2 : t_nbits < 560 + sf ? 3 : 4;
-    }
-    return r;
-}
-
-__global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p, int smem_per_warp) {
+__global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const DevConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int s = blockIdx.x * MW + wid;
     if (s >= p.S) return;
-    const int nf = c.nf, ne = c.ne, z = c.z, F = p.F;
-    const int blocks = c.ltpf_blocks, l_num = c.ltpf_l_num, l_den = c.ltpf_l_den, norm = c.ltpf_norm, s2p5 = c.ltpf_s2p5;
-    float* Y = (float*)(smem + (size_t)wid * smem_per_warp);       // hist_len
-    float* X = Y + p.hist_len;                                     // nf
-    float* xt = X + nf;                                            // 16: x_hat tail of the previous frame
-    float* scratch = xt + 16;                                      // l_num + norm
+    const LtpfGeo g = ltpf_geo(c, p.hist_len);
+    const int nf = g.nf, ne = c.ne, z = c.z, F = p.F, blocks = g.blocks;
+    float* Y = (float*)(smem + (size_t)wid * p.smem_per_warp);     // per-warp buffer, see ltpf_warp_bytes
+    float* X = Y + p.hist_len;
+    float* xt = X + nf;
+    float* scratch = xt + 16;
     int32_t* ss = p.sstate + (size_t)s * SS_WORDS;
     float* yhist = p.ltpf_y + (size_t)s * p.hist_len;
     float* xtail = p.ltpf_xtail + (size_t)s * XTAIL_FLOATS;      // [blocks][16], slot = ring block of the frame it closes
     const int blk0 = ss[SS_LTPF_BLK];
-    const int prevw = ss[SS_LTPF_PREV];
-    int prev_active = prevw & 1, prev_code = prevw >> 8, p_int_mem = ss[SS_LTPF_PINT], p_fr_mem = ss[SS_LTPF_PFR];
+    LtpfPar prev = ltpf_load_prev(ss);
     const int slot = ss[SS_SLOT];
     __syncwarp();
     for (int n = lane; n < p.hist_len; n += 32) Y[n] = yhist[n];
@@ -264,17 +223,16 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p, int 
         if ((f & 31) == 0) {                                       // fetch 32 frames' flags at once; skip idle chunks
             const int fl = f + lane;
             actm = __ballot_sync(0xffffffffu, fl < F && p.side_v[(v0 + fl) * SIDE_WORDS + SD_LTPF_ACTIVE] != 0);
-            if (actm == 0 && !prev_active) {
+            if (actm == 0 && !prev.active) {
                 span1 = span2 = span3 = false;
-                prev_code = 4; p_int_mem = 0; p_fr_mem = 0;
+                prev = LtpfPar{};
                 f += 31;
                 continue;
             }
         }
         const size_t v = v0 + f;
         const LtpfPar cur = ltpf_params(c, p.side_v + v * SIDE_WORDS);
-        const int active = cur.active, p_int = cur.p_int, p_fr = cur.p_fr, code = cur.code;
-        const bool in_span = active || prev_active;
+        const bool in_span = cur.active || prev.active;
         if (in_span) {
             const int blk = ((blk0 + f) % blocks) * nf;
             // history this frame may read: frames f-1 .. f-blocks (the oldest one sits in the block this frame is about
@@ -292,87 +250,15 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p, int 
             for (int n = lane; n < nf; n += 32) X[n] = xh[n];
             if (lane < 16) xt[lane] = f > 0 ? p.xhat[(v - 1) * nf + nf - 16 + lane] : xtail[((blk0 + blocks - 1) % blocks) * 16 + lane];
             __syncwarp();
-            // ---- long_term_post_filter.rs:252-343, as in synth_kernel
-            auto cnum = [&](int cd, int k) -> float { return cd < 4 ? c.ltpf_num[cd][k] : 0.0f; };
-            auto cden = [&](int cd, int fr, int k) -> float { return cd < 4 ? c.ltpf_den[cd][fr][k] : 0.0f; };
-            const int cur_code = active ? code : 4;
-            const int mem_code = prev_active ? prev_code : 4;
-            auto wrapi = [&](int idx) -> int { return idx < 0 ? idx + p.hist_len : idx; };
-            auto x_at = [&](int pos) -> float {
-                const int rel = pos - blk;
-                return rel >= 0 ? X[rel] : xt[16 + rel];
-            };
-            auto filt = [&](int start, int pint, int cd, int fr) -> float {
-                float out = 0.0f;
-                for (int k = 0; k <= l_num; k++) out = xa(out, xm(cnum(cd, k), x_at(start - k)));
-                const int sden = start - pint + l_den / 2;
-                for (int k = 0; k <= l_den; k++) out = xs(out, xm(cden(cd, fr, k), Y[wrapi(sden - k)]));
-                return out;
-            };
-            const float fnorm = (float)norm;
-            auto chunked = [&](int n0, int n1, int reach, auto body) {
-                const int C = reach < 32 ? reach : 32;
-                for (int st = n0; st < n1; st += C) {
-                    const int n = st + lane;
-                    if (lane < C && n < n1) body(n);
-                    __syncwarp();
-                }
-            };
-            const int reach_cur = active ? p_int - l_den / 2 : 32;
-            const int reach_mem = prev_active ? p_int_mem - l_den / 2 : 32;
-            auto deactivate_first = [&]() {
-                chunked(0, s2p5, reach_mem, [&](int n) {
-                    float fo = filt(blk + n, p_int_mem, mem_code, p_fr_mem);
-                    fo = xm(fo, xs(1.0f, xd((float)n, fnorm)));
-                    Y[blk + n] = xs(X[n], fo);
-                });
-            };
-            auto plain_from = [&](int n0) {
-                chunked(n0, nf, reach_cur, [&](int n) { Y[blk + n] = xs(X[n], filt(blk + n, p_int, cur_code, p_fr)); });
-            };
-            if (active && !prev_active) {                // case 2
-                chunked(0, s2p5, reach_cur, [&](int n) {
-                    float fo = filt(blk + n, p_int, cur_code, p_fr);
-                    fo = xm(fo, xd((float)n, fnorm));
-                    Y[blk + n] = xs(X[n], fo);
-                });
-                plain_from(s2p5);
-            } else if (!active && prev_active) {         // case 3
-                deactivate_first();
-                for (int n = s2p5 + lane; n < nf; n += 32) Y[blk + n] = X[n];
-            } else if (p_int == p_int_mem && p_fr == p_fr_mem) {   // case 4
-                plain_from(0);
-            } else {                                     // case 5
-                deactivate_first();
-                for (int i = lane; i < l_num + norm; i += 32) {
-                    int src;
-                    if (blk < l_num) src = i < l_num ? blocks * nf - l_num + i : i - l_num;
-                    else src = blk - l_num + i;
-                    scratch[i] = Y[src];
-                }
-                __syncwarp();
-                chunked(0, s2p5, reach_cur, [&](int n) {
-                    float fo = 0.0f;
-                    for (int k = 0; k <= l_num; k++) fo = xa(fo, xm(cnum(cur_code, k), scratch[l_num + n - k]));
-                    const int sden = blk + n - p_int + l_den / 2;
-                    for (int k = 0; k <= l_den; k++) fo = xs(fo, xm(cden(cur_code, p_fr, k), Y[wrapi(sden - k)]));
-                    fo = xm(fo, xd((float)n, fnorm));
-                    Y[blk + n] = xs(scratch[n + l_num], fo);
-                });
-                plain_from(s2p5);
-            }
-            __syncwarp();
+            ltpf_filter_frame(c, g, Y, X, xt, scratch, blk, cur, prev, lane);
             int16_t* out = p.pcm_out + v * nf;
-            for (int n = lane; n < nf; n += 32) out[n] = round_pcm(Y[blk + n]);
+            for (int n = lane; n < nf; n += 32) out[n] = (int16_t)round_pcm_i32(Y[blk + n]);
             __syncwarp();
         }
         span3 = span2;
         span2 = span1;
         span1 = in_span;
-        prev_active = active;
-        prev_code = active ? code : 4;
-        p_int_mem = p_int;
-        p_fr_mem = p_fr;
+        prev = cur;
     }
     if (F == 0) return;
     // ---- hand the per-stream state back as F frame-by-frame calls would have left it
@@ -397,18 +283,10 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p, int 
         for (int k = lane; k < ne; k += 32) dst[k] = src[k];
     }
     if (lane == 0) {
-        ss[SS_LTPF_PREV] = (prev_active ? 1 : 0) | (prev_code << 8);
-        ss[SS_LTPF_PINT] = p_int_mem;
-        ss[SS_LTPF_PFR] = p_fr_mem;
+        ltpf_store_prev(ss, prev);
         ss[SS_LTPF_BLK] = (blk0 + F) % blocks;
         if (lg >= 0) ss[SS_SLOT] = slot ^ 1;
     }
-}
-
-static size_t ltpf_multi_warp_bytes(const lc3b_config& c) {
-    const int blocks = c.n_ms == LC3B_10MS ? 2 : 3;
-    size_t b = (size_t)(blocks * c.nf + c.nf + 16 + 16 + c.nf / 3 + 16) * 4;
-    return (b + 15) & ~(size_t)15;
 }
 
 namespace {
@@ -418,19 +296,17 @@ struct PrepareImdct {
         e = cudaFuncSetAttribute(imdct_multi_kernel<NF, MS10>, cudaFuncAttributeMaxDynamicSharedMemorySize, MW * 2 * NF * 4);
     }
 };
-struct LaunchImdct {
+struct PlanImdct {
+    LaunchPlan& plan;
     const MultiParams& p;
     unsigned grid;
-    cudaStream_t stream;
-    template <int NF, bool MS10> void operator()() {
-        imdct_multi_kernel<NF, MS10><<<grid, MW * 32, MW * 2 * NF * 4, stream>>>(p);
-    }
+    template <int NF, bool MS10> void operator()() { plan.add(imdct_multi_kernel<NF, MS10>, grid, MW * 32, MW * 2 * NF * 4, p); }
 };
 }  // namespace
 
 cudaError_t prepare_multi(const DecoderState& st) {
     cudaError_t e = cudaFuncSetAttribute(ltpf_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)(ltpf_multi_warp_bytes(st.cfg) * MW));
+                                         (int)(ltpf_warp_bytes(st.cfg) * MW));
     if (e == cudaSuccess) {
         PrepareImdct pi;
         if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
@@ -476,6 +352,7 @@ cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, c
     }
     if (e != cudaSuccess) return e;
     MultiParams p;
+    memset(&p, 0, sizeof(p));
     p.cfg = st.dcfg; p.win = st.win; p.dtw = st.dtw; p.ftw = st.ftw;
     p.S = S; p.F = F;
     p.spec_v = vs.spec; p.side_v = vs.side;
@@ -484,14 +361,17 @@ cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, c
     p.spec = st.spec; p.ola = st.ola; p.ltpf_y = st.ltpf_y; p.ltpf_xtail = st.ltpf_xtail; p.sstate = st.sstate;
     p.pcm_out = pcm_out;
     p.hist_len = (st.cfg.n_ms == LC3B_10MS ? 2 : 3) * st.cfg.nf;
-    plc_scan_kernel<<<(S + MW - 1) / MW, MW * 32, 0, stream>>>(p);
-    const unsigned grid_v = (unsigned)((V + MW - 1) / MW);
-    LaunchImdct li{p, grid_v, stream};
-    if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, li)) return cudaErrorInvalidValue;
-    ola_multi_kernel<<<grid_v, MW * 32, 0, stream>>>(p);
-    const size_t lw = ltpf_multi_warp_bytes(st.cfg);
-    ltpf_multi_kernel<<<(S + MW - 1) / MW, MW * 32, lw * MW, stream>>>(p, (int)lw);
-    return cudaGetLastError();
+    p.smem_per_warp = (int)ltpf_warp_bytes(st.cfg);
+    // 2-5. a second plan on the caller's stream: plan_launch_direct joins the entropy plan's lanes back into the caller's
+    // stream only at the end of that plan, so lane-0 nodes added to it would not wait for lanes 1-3
+    LaunchPlan tail;
+    const unsigned grid_s = (unsigned)((S + MW - 1) / MW), grid_v = (unsigned)((V + MW - 1) / MW);
+    tail.add(plc_scan_kernel, grid_s, MW * 32, 0, p, -1);
+    PlanImdct pi{tail, p, grid_v};
+    if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
+    tail.add(ola_multi_kernel, grid_v, MW * 32, 0, p);
+    tail.add(ltpf_multi_kernel, grid_s, MW * 32, (size_t)p.smem_per_warp * MW, p);
+    return plan_launch_direct(tail, stream);
 }
 
 }  // namespace lc3b

@@ -6,17 +6,19 @@
 //                                             src/common/dct_iv.rs:49, src/common/kissfft.rs:78; window; overlap-add)
 //   LongTermPostFilter::run                   src/decoder/long_term_post_filter.rs:252 (five transition cases)
 //   output_scaling::scale_and_round           src/decoder/output_scaling.rs:13
+// Concealment, post filter and rounding are shared with the time-parallel path (lc3b_synth.cuh), the inverse MDCT too
+// (lc3b_imdct.cuh).
 //
-// synth_kernel<NF, MS10> (every stream): concealment, inverse MDCT (lc3b_imdct.cuh, frame length a template
-// constant), overlap-add, and the post filter's PASS-THROUGH case: x_hat goes to the LTPF history ring and, rounded,
-// to the PCM row.  Two consecutive samples per lane, so PCM leaves as 32-bit and f32 state as 64-bit accesses; all
-// global traffic is stream-major and coalesced (spectrum 4*ne B in, overlap memory 4*(nf-z) B in/out, LTPF history
-// 4*nf B out, PCM 2*nf B out).
+// synth_classic_kernel<NF, MS10> (every stream, the default): concealment, inverse MDCT (frame length a template
+// constant), overlap-add, and the post filter's PASS-THROUGH case: x_hat goes to the LTPF history ring and, rounded, to
+// the PCM row.  Two consecutive samples per lane, so PCM leaves as 32-bit and f32 state as 64-bit accesses; all global
+// traffic is stream-major and coalesced (spectrum 4*ne B in, overlap memory 4*(nf-z) B in/out, LTPF history 4*nf B
+// out, PCM 2*nf B out).  synth_kernel<NF, MS10> is the same work as a persistent kernel with TMA prefetch, the measured
+// alternative (lc3b_decoder_set_synth_mode).
 // ltpf_kernel (streams whose post filter is, or was in the previous frame, active): the IIR itself; for those streams
-// synth_kernel leaves x_hat in a side buffer (the ring block keeps the samples long pitch lags still reach), and this
-// kernel writes the filtered signal to the ring block and the PCM row.  The recursion only reaches back
-// p_int - l_den/2 >= 18 samples, so up to 32 consecutive outputs are computed in parallel per step.  Streams outside
-// such a span cost this kernel one flag load.
+// the synthesis kernel leaves x_hat in a side buffer (the ring block keeps the samples long pitch lags still reach), and
+// this kernel writes the filtered signal to the ring block and the PCM row.  Streams outside such a span cost this
+// kernel one flag load.
 #include <stdlib.h>
 #include <string.h>
 
@@ -24,6 +26,7 @@
 #include "lc3b_imdct.cuh"
 #include "lc3b_math.cuh"
 #include "lc3b_plan.cuh"
+#include "lc3b_synth.cuh"
 
 namespace lc3b {
 
@@ -36,7 +39,7 @@ struct SynthParams {
     float* ola;
     float* ltpf_y;
     float* ltpf_xtail;
-    float* ltpf_x;       // [n_streams][nf] x_hat of streams inside an active span (synth_kernel -> ltpf_kernel)
+    float* ltpf_x;       // [n_streams][nf] x_hat of streams inside an active span (synthesis kernel -> ltpf_kernel)
     int32_t* side;
     int32_t* sstate;
     int16_t* pcm_out;
@@ -55,11 +58,6 @@ constexpr int PIPE_WARPS = 8;    // warps per CTA of the persistent synthesis ke
 // per warp: two stage buffers + one pong buffer of nf floats and two mbarriers; per CTA: DCT-IV and FFT twiddles (nf/2 float2
 // each) and the window (2 nf floats reserved)
 static inline size_t synth_smem_bytes(int nf) { return (size_t)PIPE_WARPS * 3 * nf * 4 + (size_t)4 * nf * 4 + (size_t)PIPE_WARPS * 2 * 8; }
-
-__device__ __forceinline__ int32_t round_pcm_i32(float v) {          // output_scaling.rs:13-26
-    int32_t q = v > 0.0f ? cast_i32(xa(v, 0.5f)) : cast_i32(xs(v, 0.5f));
-    return q > 32767 ? 32767 : q < -32768 ? -32768 : q;
-}
 
 // synth_classic_kernel: one warp = one frame, spectrum through ordinary loads.  The default: at 262 144 streams it runs in
 // 0.50 ms against 0.525 ms for the persistent TMA-pipelined kernel below (profiles/r2_synth_ab.json).  What bounds it is
@@ -90,7 +88,7 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) synth_classic_kernel(const __g
     const int ok = sd_a.x;
     const int slot = sd_b.z;
     const int active = sd_a.y;
-    const int prev_active = ss_b.x & 1;
+    const int prev_active = ltpf_prev_active(ss_b.x);
     const int blk_idx = ss_b.w;
     const float* sp = p.spec + ((size_t)slot * p.slot_streams + stream) * NE;
 
@@ -111,26 +109,11 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) synth_classic_kernel(const __g
         }
         if (lane == 0 && (ss_a.y != 0 || ss_a.z != (int32_t)f2u(1.0f))) { ss[SS_PLC_LOST] = 0; ss[SS_PLC_ALPHA] = (int32_t)f2u(1.0f); }
     } else {
-        int lost = ss_a.y;
+        const int lost = ss_a.y;
         float alpha = u2f((uint32_t)ss_a.z);
-        uint32_t seed = (uint32_t)ss_a.w;
         __syncwarp();                                            // every lane has read the state before any lane updates it
-        if (lost >= 4) alpha = xm(alpha, lost < 8 ? 0.9f : 0.85f);
-        // lane's first line is k = lane: LCG advanced lane+1 times; then jump 32 steps at a time
-        uint32_t s = seed;
-        for (int i = 0; i <= lane; i++) s = (16831u + s * 12821u) & 0xFFFFu;
-        uint32_t a32 = 1, c32 = 0;                               // composition of 32 LCG steps
-        for (int i = 0; i < 32; i++) { c32 = (16831u + c32 * 12821u) & 0xFFFFu; a32 = (a32 * 12821u) & 0xFFFFu; }
-        for (int k = lane; k < NF; k += 32) {
-            float v = 0.0f;
-            if (k < NE) {
-                const float lg = sp[k];
-                v = s < 0x8000u ? xm(lg, alpha) : xm(lg, -alpha);
-                if (k == NE - 1) ss[SS_PLC_SEED] = (int32_t)s;
-                s = (a32 * s + c32) & 0xFFFFu;
-            }
-            P[k] = v;
-        }
+        alpha = plc_fade(alpha, lost);
+        plc_scramble<NF, NE>(P, sp, alpha, (uint32_t)ss_a.w, lane, ss + SS_PLC_SEED);
         if (lane == 0) { ss[SS_PLC_LOST] = lost + 1; ss[SS_PLC_ALPHA] = (int32_t)f2u(alpha); }
     }
     __syncwarp();
@@ -176,11 +159,7 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) synth_classic_kernel(const __g
         int nb = blk_idx + 1;                                    // :334-337
         if (nb > (MS10 ? 1 : 2)) nb = 0;
         ss[SS_LTPF_BLK] = nb;
-        if (!in_span) {                                          // otherwise ltpf_kernel carries the filter state on
-            ss[SS_LTPF_PREV] = 4 << 8;
-            ss[SS_LTPF_PINT] = 0;
-            ss[SS_LTPF_PFR] = 0;
-        }
+        if (!in_span) ltpf_store_prev(ss, LtpfPar{});            // otherwise ltpf_kernel carries the filter state on
     }
 }
 
@@ -225,7 +204,7 @@ __device__ __forceinline__ FrameHead load_head(const SynthParams& p, int stream)
     h.ok = sd[SD_OK];
     h.slot = sd[SD_SLOT];
     h.active = sd[SD_LTPF_ACTIVE];
-    h.prev_active = ss[SS_LTPF_PREV] & 1;
+    h.prev_active = ltpf_prev_active(ss[SS_LTPF_PREV]);
     h.blk_idx = ss[SS_LTPF_BLK];
     return h;
 }
@@ -315,17 +294,17 @@ __global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_
             float alpha = u2f((uint32_t)ss[SS_PLC_ALPHA]);
             uint32_t seed = (uint32_t)ss[SS_PLC_SEED];
             __syncwarp();                                            // every lane has read the state before any lane updates it
-            if (lost >= 4) alpha = xm(alpha, lost < 8 ? 0.9f : 0.85f);
-            // lane's first line is k = lane: LCG advanced lane+1 times; then jump 32 steps at a time
+            alpha = plc_fade(alpha, lost);
+            // plc_scramble's sequence, in place over the first NE lines (the rest of the stage buffer is zero already):
+            // plc_scramble itself, which also rewrites the zero lines, costs synth_kernel<360, 0> a register spill
             uint32_t s = seed;
-            for (int i = 0; i <= lane; i++) s = (16831u + s * 12821u) & 0xFFFFu;
-            uint32_t a32 = 1, c32 = 0;                               // composition of 32 LCG steps
-            for (int i = 0; i < 32; i++) { c32 = (16831u + c32 * 12821u) & 0xFFFFu; a32 = (a32 * 12821u) & 0xFFFFu; }
+            for (int i = 0; i <= lane; i++) s = plc_lcg(s);
+            const PlcJump j32 = plc_lcg_jump(32);
             for (int k = lane; k < NE; k += 32) {
                 const float lg = P[k];
                 P[k] = s < 0x8000u ? xm(lg, alpha) : xm(lg, -alpha);
                 if (k == NE - 1) ss[SS_PLC_SEED] = (int32_t)s;
-                s = (a32 * s + c32) & 0xFFFFu;
+                s = j32.step(s);
             }
             if (lane == 0) { ss[SS_PLC_LOST] = lost + 1; ss[SS_PLC_ALPHA] = (int32_t)f2u(alpha); }
             __syncwarp();
@@ -374,11 +353,7 @@ __global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_
             int nb = blk_idx + 1;                                    // :334-337
             if (nb > (MS10 ? 1 : 2)) nb = 0;
             ss[SS_LTPF_BLK] = nb;
-            if (!in_span) {                                          // otherwise ltpf_kernel carries the filter state on
-                ss[SS_LTPF_PREV] = 4 << 8;
-                ss[SS_LTPF_PINT] = 0;
-                ss[SS_LTPF_PFR] = 0;
-            }
+            if (!in_span) ltpf_store_prev(ss, LtpfPar{});            // otherwise ltpf_kernel carries the filter state on
         }
         stream = nstream;
         head = nhead;
@@ -400,146 +375,42 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) ltpf_kernel(SynthParams p) {
         const int s = first + lane;
         bool in_span = false;
         if (lane < p.group && s < p.n_streams)
-            in_span = p.side[(size_t)s * SIDE_WORDS + SD_LTPF_ACTIVE] != 0 || (p.sstate[(size_t)s * SS_WORDS + SS_LTPF_PREV] & 1) != 0;
+            in_span = p.side[(size_t)s * SIDE_WORDS + SD_LTPF_ACTIVE] != 0 || ltpf_prev_active(p.sstate[(size_t)s * SS_WORDS + SS_LTPF_PREV]);
         todo = __ballot_sync(0xffffffffu, in_span);
     }
     if (todo == 0) return;
-    const int nf = c.nf;
-    const int blocks = c.ltpf_blocks, l_num = c.ltpf_l_num, l_den = c.ltpf_l_den, norm = c.ltpf_norm, s2p5 = c.ltpf_s2p5;
-    float* Y = (float*)(smem + (size_t)wid * p.smem_per_warp);    // hist_len floats: LTPF circular history
-    float* X = Y + p.hist_len;                                    // nf floats: x_hat, the filter input
-    float* xt = X + nf;                                           // 16: x_hat tail of the previous frame
-    float* scratch = xt + 16;                                     // l_num + norm floats: frozen history for transition case 5
+    const LtpfGeo g = ltpf_geo(c, p.hist_len);
+    const int nf = g.nf, blocks = g.blocks;
+    float* Y = (float*)(smem + (size_t)wid * p.smem_per_warp);    // per-warp buffer, see ltpf_warp_bytes
+    float* X = Y + p.hist_len;
+    float* xt = X + nf;
+    float* scratch = xt + 16;
 
     while (todo) {
         const int stream = first + (__ffs(todo) - 1);
         todo &= todo - 1;
         const int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
         int32_t* ss = p.sstate + (size_t)stream * SS_WORDS;
-        const int active = sd[SD_LTPF_ACTIVE];
-        const int nbits = sd[SD_NBITS];
+        const LtpfPar cur = ltpf_params(c, sd), prev = ltpf_load_prev(ss);
         const int blk_idx = sd[SD_BLK];
         const int blk = blk_idx * nf;
-        const int prev = ss[SS_LTPF_PREV];
-        const int prev_active = prev & 1, prev_code = prev >> 8;
-        const int p_int_mem = ss[SS_LTPF_PINT], p_fr_mem = ss[SS_LTPF_PFR];
-        int p_int = 0, p_fr = 0, code = 4;
-        if (active) {                                  // compute_filter_parameters :164-190, compute_gains_params :142-161
-            const int pi = sd[SD_PITCH_INDEX];
-            int pit;
-            double pfr;
-            if (pi >= 440) { pit = pi - 283; pfr = 0.0; }
-            else if (pi >= 380) { pit = pi / 2 - 63; pfr = (double)(2 * pi - 4 * pit - 252); }
-            else { pit = pi / 4 + 32; pfr = (double)(pi + 128 - 4 * pit); }
-            const double pitch = (double)pit + pfr / 4.0;
-            const double pitch_fs = pitch * (8000.0 * ceil((double)c.fs / 8000.0) / 12800.0);
-            const int p_up = (int)((pitch_fs * 4.0) + 0.5);
-            p_int = p_up / 4;
-            p_fr = p_up - 4 * p_int;
-            const int t_nbits = c.n_ms == LC3B_7P5MS ? (int)round((double)nbits * 10.0 / 7.5) : nbits;
-            const int sf = c.fs_ind * 80;
-            code = t_nbits < 320 + sf ? 0 : t_nbits < 400 + sf ? 1 : t_nbits < 480 + sf ? 2 : t_nbits < 560 + sf ? 3 : 4;
-        }
         float* yhist = p.ltpf_y + (size_t)stream * p.hist_len;
         const float* xtail_prev = p.ltpf_xtail + (size_t)stream * XTAIL_FLOATS + (blk_idx == 0 ? blocks - 1 : blk_idx - 1) * 16;
         __syncwarp();                                  // the previous stream's reads of the shared buffers are done
         for (int n = lane; n < p.hist_len; n += 32) Y[n] = yhist[n];
         if (lane < 16) xt[lane] = xtail_prev[lane];
         __syncwarp();
-        for (int n = lane; n < nf; n += 32) X[n] = p.ltpf_x[(size_t)stream * nf + n];   // x_hat left by synth_kernel
+        for (int n = lane; n < nf; n += 32) X[n] = p.ltpf_x[(size_t)stream * nf + n];   // x_hat left by the synthesis kernel
         __syncwarp();
-
-        // coefficient sets: current (c_num, c_den) and previous (c_num_mem, c_den_mem); code 4 = all zero
-        auto cnum = [&](int cd, int k) -> float { return cd < 4 ? c.ltpf_num[cd][k] : 0.0f; };
-        auto cden = [&](int cd, int fr, int k) -> float { return cd < 4 ? c.ltpf_den[cd][fr][k] : 0.0f; };
-        const int cur_code = active ? code : 4;     // inactive: zeroed coefficients (:196-201)
-        const int mem_code = prev_active ? prev_code : 4;
-        auto wrapi = [&](int idx) -> int { return idx < 0 ? idx + p.hist_len : idx; };   // :244-250
-        auto x_at = [&](int pos) -> float {          // x_hat_mem[wrap(pos)], pos relative to buffer start
-            const int rel = pos - blk;               // >= -l_num
-            return rel >= 0 ? X[rel] : xt[16 + rel];
-        };
-        // compute_filter / compute_filter_mem :380-415
-        auto filt = [&](int start, int pint, int cd, int fr) -> float {
-            float out = 0.0f;
-            for (int k = 0; k <= l_num; k++) out = xa(out, xm(cnum(cd, k), x_at(start - k)));
-            const int sden = start - pint + l_den / 2;
-            for (int k = 0; k <= l_den; k++) out = xs(out, xm(cden(cd, fr, k), Y[wrapi(sden - k)]));
-            return out;
-        };
-        const float fnorm = (float)norm;
-        // run `body(n)` for n in [n0, n1) in dependency-safe chunks: outputs reach back at least `reach` samples
-        auto chunked = [&](int n0, int n1, int reach, auto body) {
-            const int C = reach < 32 ? reach : 32;
-            for (int s = n0; s < n1; s += C) {
-                const int n = s + lane;
-                if (lane < C && n < n1) body(n);
-                __syncwarp();
-            }
-        };
-        const int reach_cur = active ? p_int - l_den / 2 : 32;
-        const int reach_mem = prev_active ? p_int_mem - l_den / 2 : 32;
-        auto deactivate_first = [&]() {              // :417-424
-            chunked(0, s2p5, reach_mem, [&](int n) {
-                float fo = filt(blk + n, p_int_mem, mem_code, p_fr_mem);
-                fo = xm(fo, xs(1.0f, xd((float)n, fnorm)));
-                Y[blk + n] = xs(X[n], fo);
-            });
-        };
-        auto plain_from = [&](int n0) {
-            chunked(n0, nf, reach_cur, [&](int n) { Y[blk + n] = xs(X[n], filt(blk + n, p_int, cur_code, p_fr)); });
-        };
-        if (active && !prev_active) {                // case 2
-            chunked(0, s2p5, reach_cur, [&](int n) {
-                float fo = filt(blk + n, p_int, cur_code, p_fr);
-                fo = xm(fo, xd((float)n, fnorm));
-                Y[blk + n] = xs(X[n], fo);
-            });
-            plain_from(s2p5);
-        } else if (!active && prev_active) {         // case 3
-            deactivate_first();
-            for (int n = s2p5 + lane; n < nf; n += 32) Y[blk + n] = X[n];
-        } else if (p_int == p_int_mem && p_fr == p_fr_mem) {   // case 4
-            plain_from(0);
-        } else {                                     // case 5
-            deactivate_first();
-            // activate_first_2p5ms_from_mem :345-378: numerator taps read a frozen copy of y[blk-l_num .. blk+norm)
-            for (int i = lane; i < l_num + norm; i += 32) {
-                int src;
-                if (blk < l_num) src = i < l_num ? blocks * nf - l_num + i : i - l_num;
-                else src = blk - l_num + i;
-                scratch[i] = Y[src];
-            }
-            __syncwarp();
-            chunked(0, s2p5, reach_cur, [&](int n) {
-                float fo = 0.0f;
-                for (int k = 0; k <= l_num; k++) fo = xa(fo, xm(cnum(cur_code, k), scratch[l_num + n - k]));
-                const int sden = blk + n - p_int + l_den / 2;
-                for (int k = 0; k <= l_den; k++) fo = xs(fo, xm(cden(cur_code, p_fr, k), Y[wrapi(sden - k)]));
-                fo = xm(fo, xd((float)n, fnorm));
-                Y[blk + n] = xs(scratch[n + l_num], fo);
-            });
-            plain_from(s2p5);
-        }
-        __syncwarp();
+        ltpf_filter_frame(c, g, Y, X, xt, scratch, blk, cur, prev, lane);
         int16_t* out = p.pcm_out + (size_t)stream * p.pcm_stride;
         for (int n = lane; n < nf; n += 32) {
             const float v = Y[blk + n];
             yhist[blk + n] = v;
             out[n] = (int16_t)round_pcm_i32(v);
         }
-        if (lane == 0) {
-            ss[SS_LTPF_PREV] = (active ? 1 : 0) | ((active ? code : 4) << 8);
-            ss[SS_LTPF_PINT] = p_int;
-            ss[SS_LTPF_PFR] = p_fr;
-        }
+        if (lane == 0) ltpf_store_prev(ss, cur);
     }
-}
-
-static size_t ltpf_warp_bytes(const lc3b_config& c) {
-    const int blocks = c.n_ms == LC3B_10MS ? 2 : 3;
-    size_t b = (size_t)(blocks * c.nf + c.nf + 16 + 16 + c.nf / 3 + 16) * 4;
-    return (b + 15) & ~(size_t)15;
 }
 
 namespace {
@@ -620,12 +491,6 @@ int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_
     if (st.no_ltpf) return ps.node;                           // the post filter can never be active: nothing to launch
     const int n_warps = (n + group - 1) / group;
     return plan.add(ltpf_kernel, (unsigned)((n_warps + SYN_WARPS - 1) / SYN_WARPS), SYN_WARPS * 32, lw * SYN_WARPS, p, ps.node);
-}
-
-cudaError_t launch_synth(const DecoderState& st, int16_t* pcm_out, size_t pcm_stride, cudaStream_t stream) {
-    LaunchPlan plan;
-    if (plan_synth(plan, st, pcm_out, pcm_stride, -1) < 0) return cudaErrorInvalidValue;
-    return plan_launch_direct(plan, stream);
 }
 
 }  // namespace lc3b
