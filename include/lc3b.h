@@ -77,6 +77,26 @@ int lc3b_decode_frames(lc3b_decoder* h, int bits_per_sample, const uint8_t* fram
                        int nbytes, size_t frame_stride, int16_t* pcm_out, size_t pcm_stride, int32_t* status_out,
                        void* cuda_stream);
 
+/* One decode_frame (lc3_decoder.rs:217) for each listed stream; every other stream of the handle is untouched - the
+ * reference's addressing by channel_index, for streams that have nothing to decode in a period (paused, not started,
+ * finished, on another connection schedule: a lost frame would be concealed instead).
+ *   stream_ids  HOST int32[n_rows]: row i of frames / frame_nbytes / pcm_out / status_out belongs to stream stream_ids[i].
+ *               Any order; every id in [0, n_streams) and listed at most once, else LC3B_ERR_INVALID_ARG (the
+ *               reference's bad channel_index panic, :228) and nothing is enqueued.  Only read during the call.
+ *   n_rows      0 .. n_streams; 0 enqueues nothing and returns LC3B_OK.
+ * Every other argument is what lc3b_decode_frames takes, with n_rows rows in place of n_streams.  A stream's PCM, status
+ * and state are bit-identical to decoding its own frame sequence in a handle of its own, whatever mix of subset calls,
+ * full calls, time-parallel calls and resets it went through.  The call follows the graph mode, lc3b_decoder_set_split,
+ * set_dequant_mode (chosen by n_rows), set_synth_mode, set_min_nbytes and the stage mask, like lc3b_decode_frames; the
+ * trace (lc3b_decoder_set_trace) is written per call row, like `frames`.  The ids are copied into the workspace (4 bytes
+ * per stream, already counted by lc3b_decoder_workspace_bytes) with one cudaMemcpyAsync on `cuda_stream`. */
+int lc3b_decode_frames_subset(lc3b_decoder* h, int bits_per_sample, const int32_t* stream_ids, int n_rows,
+                              const uint8_t* frames, const int32_t* frame_nbytes, int nbytes, size_t frame_stride,
+                              int16_t* pcm_out, size_t pcm_stride, int32_t* status_out, void* cuda_stream);
+/* The listed streams get exactly the state lc3b_decoder_init gives a stream (a slot handed to a new call); no other
+ * stream is touched.  stream_ids / n as in lc3b_decode_frames_subset. */
+int lc3b_decoder_reset_streams(lc3b_decoder* h, const int32_t* stream_ids, int n, void* cuda_stream);
+
 /* Same call with HOST buffers (what a caller of the reference holds): copies frames host->device, decodes, copies
  * PCM device->host, all on `cuda_stream`, using staging areas inside the workspace.  Asynchronous when the host
  * buffers are pinned.  status_out (host, nullable) as above. */
@@ -107,7 +127,8 @@ int lc3b_decode_stream_frames(lc3b_decoder* h, int bits_per_sample, const uint8_
 
 /* Inspection (parity gate i, SURVEY.md 8d): when set, every decode also writes, per stream, a record of
  * LC3B_TRACE_WORDS int32 (layout below) and the entropy-decoded integer spectrum x[0..ne).  Device pointers,
- * NULL to disable.  trace: [n_streams][LC3B_TRACE_WORDS], x: [n_streams][ne]. */
+ * NULL to disable.  trace: [n_streams][LC3B_TRACE_WORDS], x: [n_streams][ne].  lc3b_decode_frames_subset writes
+ * rows 0 .. n_rows-1, one per call row. */
 int lc3b_decoder_set_trace(lc3b_decoder* h, int32_t* trace, int32_t* x);
 
 /* Spectrum handed to the IMDCT by the last decode (after SNS, or the concealed one): device f32 [n_streams][ne],
@@ -216,6 +237,18 @@ int lc3b_encoder_init(lc3b_encoder** out, int n_streams, int frame_duration, int
  * LC3B_ERR_INVALID_ARG here (nbytes < 20 underflows the bit budget, spectral_quantization.rs:133). */
 int lc3b_encode_frames(lc3b_encoder* h, const int16_t* pcm_in, size_t pcm_stride, uint8_t* frames_out, int nbytes,
                        size_t frame_stride, void* cuda_stream);
+/* One encode_frame (lc3_encoder.rs:175) for each listed stream; every other stream of the handle is untouched.
+ *   stream_ids  HOST int32[n_rows], as in lc3b_decode_frames_subset: row i of pcm_in / frames_out belongs to stream
+ *               stream_ids[i]; ids in [0, n_streams), none twice, else LC3B_ERR_INVALID_ARG and nothing is enqueued.
+ *   n_rows      0 .. n_streams; 0 enqueues nothing and returns LC3B_OK.
+ * Every other argument is what lc3b_encode_frames takes, with n_rows rows.  A stream's bytes and state are identical to
+ * encoding its own sequence in a handle of its own.  Follows the graph mode and the stage mask; lc3b_encoder_debug_read
+ * then reports per call row.  The ids are copied into the workspace (4 bytes per stream, already counted by
+ * lc3b_encoder_workspace_bytes) with one cudaMemcpyAsync on `cuda_stream`. */
+int lc3b_encode_frames_subset(lc3b_encoder* h, const int32_t* stream_ids, int n_rows, const int16_t* pcm_in,
+                              size_t pcm_stride, uint8_t* frames_out, int nbytes, size_t frame_stride, void* cuda_stream);
+/* The listed streams get exactly the state lc3b_encoder_init gives a stream; no other stream is touched. */
+int lc3b_encoder_reset_streams(lc3b_encoder* h, const int32_t* stream_ids, int n, void* cuda_stream);
 /* Same with HOST buffers (pinned => asynchronous). */
 int lc3b_encode_frames_host(lc3b_encoder* h, const int16_t* pcm_in, size_t pcm_stride, uint8_t* frames_out, int nbytes,
                             size_t frame_stride, void* cuda_stream);
@@ -241,7 +274,8 @@ int lc3b_encode_stream_frames(lc3b_encoder* h, const int16_t* pcm_in, int n_fram
 int lc3b_encoder_set_graph_mode(lc3b_encoder* h, int mode);   /* as lc3b_decoder_set_graph_mode */
 /* Test hook: device copies of the last encode's intermediates (any pointer may be NULL): xf [S][ne] f32 (quantiser
  * input, after SNS and TNS), e_b [S][64] f32, hand [S][8] i32 (near_nyquist, attack, pitch_index, pitch_present,
- * ltpf_active, nbits_ltpf), xq [S][ne] i16. */
+ * ltpf_active, nbits_ltpf), xq [S][ne] i16.  After lc3b_encode_frames_subset, row i is call row i (rows from n_rows on
+ * are left from earlier calls). */
 int lc3b_encoder_debug_read(lc3b_encoder* h, float* xf, float* e_b, int32_t* hand, int16_t* xq, void* cuda_stream);
 /* Profiling hook, like lc3b_decoder_set_stage_mask: bit 0 = MDCT kernel, bit 1 = attack/LTPF analysis kernel,
  * bit 2 = SNS kernel (with the bandwidth detector), bit 3 = TNS kernel, bit 4 = quantise kernel, bit 5 = the

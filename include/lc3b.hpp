@@ -96,6 +96,22 @@ class Lc3BatchDecoder {
         detail::check(rc, "lc3b_decode_frames");
         return std::nullopt;
     }
+    // decode_frame (lc3_decoder.rs:217) for the listed streams only, every other stream untouched.  Row i of the device
+    // buffers (frames, samples_out, frame_nbytes, status_out) belongs to stream stream_ids[i]; stream_ids is a host array of
+    // n_rows distinct ids in [0, num_streams), only read during the call (a bad list throws, like the reference's panic).
+    Result<Lc3DecoderError> decode_frames_subset(size_t num_bits_per_audio_sample, const int32_t* stream_ids, size_t n_rows,
+                                                 const uint8_t* frames, size_t nbytes, size_t frame_stride, int16_t* samples_out,
+                                                 const int32_t* frame_nbytes = nullptr, int32_t* status_out = nullptr) {
+        const int rc = lc3b_decode_frames_subset(h_, (int)num_bits_per_audio_sample, stream_ids, (int)n_rows, frames, frame_nbytes,
+                                                 (int)nbytes, frame_stride, samples_out, (size_t)config.nf, status_out, stream_);
+        if (rc == LC3B_ERR_BITS_PER_SAMPLE) return Lc3DecoderError::Only16BitsPerAudioSampleSupported;
+        detail::check(rc, "lc3b_decode_frames_subset");
+        return std::nullopt;
+    }
+    // the listed streams start over with the state Lc3Decoder::new gives a channel; no other stream is touched
+    void reset_streams(const int32_t* stream_ids, size_t n) {
+        detail::check(lc3b_decoder_reset_streams(h_, stream_ids, (int)n, stream_), "lc3b_decoder_reset_streams");
+    }
     // Time-parallel decode (SURVEY.md 8f-1): n_frames consecutive frames of every stream in one call; equivalent to
     // n_frames decode_frames calls (same PCM, same state afterwards).  Device buffers: frames [num_streams][n_frames][nbytes],
     // samples_out [num_streams][n_frames * nf], scratch >= multi_scratch_bytes(n_frames) bytes (caller-owned).
@@ -157,6 +173,19 @@ class Lc3BatchEncoder {
         auto fn = where == Residency::Device ? lc3b_encode_frames : lc3b_encode_frames_host;
         detail::check(fn(h_, samples_in, (size_t)config.nf, buf_out, (int)nbytes, frame_stride, stream_), "lc3b_encode_frames");
         return std::nullopt;
+    }
+    // encode_frame (lc3_encoder.rs:175) for the listed streams only: row i of the device buffers belongs to stream
+    // stream_ids[i] (host array of n_rows distinct ids, only read during the call)
+    Result<Lc3EncoderError> encode_frames_subset(const int32_t* stream_ids, size_t n_rows, const int16_t* samples_in, uint8_t* buf_out,
+                                                 size_t nbytes, size_t frame_stride) {
+        detail::check(lc3b_encode_frames_subset(h_, stream_ids, (int)n_rows, samples_in, (size_t)config.nf, buf_out, (int)nbytes,
+                                                frame_stride, stream_),
+                      "lc3b_encode_frames_subset");
+        return std::nullopt;
+    }
+    // the listed streams start over with the state Lc3Encoder::new gives a channel; no other stream is touched
+    void reset_streams(const int32_t* stream_ids, size_t n) {
+        detail::check(lc3b_encoder_reset_streams(h_, stream_ids, (int)n, stream_), "lc3b_encoder_reset_streams");
     }
     // Time-parallel encode: n_frames consecutive frames of every stream in one call; equivalent to n_frames encode_frames
     // calls (same bytes, same state afterwards).  Device buffers: samples_in [num_streams][n_frames * nf], buf_out frame f of

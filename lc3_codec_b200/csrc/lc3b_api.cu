@@ -63,7 +63,7 @@ struct Carve {
 
 struct Layout {
     size_t dcfg, win, dtw, ftw, sym_lut, spec, xq, handoff, gband, tns_list, nsym_prev, ola, ltpf_y, ltpf_xtail, ltpf_x, side, sstate, stage_in, stage_out, stage_len,
-        stage_status, total;
+        stage_status, ids, total;
 };
 
 static Layout make_layout(const lc3b_config& c, int n_streams, int max_nbytes, bool staging = true) {
@@ -93,6 +93,7 @@ static Layout make_layout(const lc3b_config& c, int n_streams, int max_nbytes, b
     L.stage_out = cv.take(staging ? sizeof(int16_t) * ns * c.nf * 2 : 0);   // double-buffered for the pipelined host path
     L.stage_len = cv.take(staging ? sizeof(int32_t) * ns : 0);
     L.stage_status = cv.take(staging ? sizeof(int32_t) * ns : 0);
+    L.ids = cv.take(staging ? sizeof(int32_t) * ns : 0);                 // id list of a subset call (lc3b_decode_frames_subset)
     L.total = cv.off;
     return L;
 }
@@ -173,10 +174,28 @@ __global__ void init_sym_lut_kernel(uint8_t* lut) {
     }
 }
 
-__global__ void init_streams_kernel(int32_t* sstate, int n_streams) {
-    const int s = blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    int32_t* ss = sstate + (size_t)s * SS_WORDS;
+// The state a stream starts from.  ids == nullptr: every stream, whose rows lc3b_decoder_init has just zeroed with the
+// rest of the workspace; otherwise the n listed streams (lc3b_decoder_reset_streams), whose persistent rows are zeroed
+// here first - one warp per stream.
+__global__ void init_streams_kernel(DecoderState st, const int32_t* ids, int n) {
+    const int lane = threadIdx.x & 31;
+    const int i = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    if (i >= n) return;
+    const int s = ids ? ids[i] : i;
+    const size_t S = (size_t)st.n_streams;
+    if (ids) {
+        const int ne = st.cfg.ne, nf = st.cfg.nf;
+        const int hist = (st.cfg.n_ms == LC3B_10MS ? 2 : 3) * nf;
+        for (int k = lane; k < ne; k += 32) { st.spec[(size_t)s * ne + k] = 0.0f; st.spec[(S + s) * ne + k] = 0.0f; }
+        for (int k = lane; k < nf - st.cfg.z; k += 32) st.ola[(size_t)s * (nf - st.cfg.z) + k] = 0.0f;
+        for (int k = lane; k < hist; k += 32) st.ltpf_y[(size_t)s * hist + k] = 0.0f;
+        for (int k = lane; k < XTAIL_FLOATS; k += 32) st.ltpf_xtail[(size_t)s * XTAIL_FLOATS + k] = 0.0f;
+        for (int k = lane; k < nf; k += 32) st.ltpf_x[(size_t)s * nf + k] = 0.0f;
+        if (lane < SIDE_WORDS) st.side[(size_t)s * SIDE_WORDS + lane] = 0;
+        if (lane == 0) st.nsym_prev[s] = 0;
+    }
+    if (lane != 0) return;
+    int32_t* ss = st.sstate + (size_t)s * SS_WORDS;
     ss[SS_SLOT] = 0;
     ss[SS_PLC_LOST] = 0;
     ss[SS_PLC_ALPHA] = (int32_t)f2u(1.0f);     // packet_loss_concealment.rs:31-33
@@ -185,6 +204,11 @@ __global__ void init_streams_kernel(int32_t* sstate, int n_streams) {
     ss[SS_LTPF_PINT] = 0;
     ss[SS_LTPF_PFR] = 0;
     ss[SS_LTPF_BLK] = 0;
+}
+
+static cudaError_t launch_init_streams(const DecoderState& st, const int32_t* ids, int n, cudaStream_t stream) {
+    init_streams_kernel<<<(unsigned)((n + 7) / 8), 256, 0, stream>>>(st, ids, n);
+    return cudaGetLastError();
 }
 
 static void fill_host_config(const lc3b_config& c, DevConfig* d) {
@@ -325,6 +349,7 @@ int decoder_init(lc3b_decoder** out, int n_streams, int frame_duration, int samp
     st.stage_out = (int16_t*)(base + L.stage_out);
     st.stage_len = (int32_t*)(base + L.stage_len);
     st.stage_status = (int32_t*)(base + L.stage_status);
+    st.ids = staging ? (int32_t*)(base + L.ids) : nullptr;
     st.trace = nullptr;
     st.trace_x = nullptr;
     st.fixed_slot = -1;
@@ -349,8 +374,8 @@ int decoder_init(lc3b_decoder** out, int n_streams, int frame_duration, int samp
     if (e == cudaSuccess) {
         init_tables_kernel<<<1, 256, 0, stream>>>(st.dcfg, st.win, st.dtw, st.ftw);
         init_sym_lut_kernel<<<64, 32, 0, stream>>>(st.sym_lut);
-        init_streams_kernel<<<(n_streams + 255) / 256, 256, 0, stream>>>(st.sstate, n_streams);
         e = cudaGetLastError();
+        if (e == cudaSuccess) e = launch_init_streams(st, nullptr, n_streams, stream);
     }
     if (e != cudaSuccess) {
         delete h;
@@ -475,9 +500,11 @@ int lc3b_decoder_set_trace(lc3b_decoder* h, int32_t* trace, int32_t* x) {
     return LC3B_OK;
 }
 
-// one decode_frame per stream: the call's kernels as a plan, issued directly or as a cached graph
+// one decode_frame per stream (ids == nullptr, n = every stream of the handle) or per row of a subset call (n rows, row u
+// = stream ids[u], ids in device memory): the call's kernels as a plan, issued directly or as a cached graph
 static cudaError_t run_decode(lc3b_decoder* h, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes, size_t frame_stride,
-                              int16_t* pcm_out, size_t pcm_stride, int32_t* status_out, int stage_mask, cudaStream_t stream) {
+                              int16_t* pcm_out, size_t pcm_stride, int32_t* status_out, int stage_mask, cudaStream_t stream,
+                              const int32_t* ids = nullptr, int n = 0) {
     LaunchPlan plan;
     // Sub-batches.  The three kernels are bound by different things (integer ALU / dependent-instruction latency / the
     // memory-instruction path) and each ends in a ragged last wave of CTAs that are serial chains as long as a full
@@ -486,7 +513,7 @@ static cudaError_t run_decode(lc3b_decoder* h, const uint8_t* frames, const int3
     // pipe.  Measured at 262 144 streams of 48 kHz / 150 B: 1.87 ms as one batch, 1.70 ms as two, 1.69 ms as four
     // (tools/exp_split_overlap.py); 131 072 streams 1.11 -> 0.91 ms, 65 536 streams 0.57 -> 0.53 ms, no difference at 32 768 and
     // below.  Streams are independent (lc3_decoder.rs:62-69), so any split computes the same bits.
-    const int n = h->st.n_streams;
+    if (!ids) n = h->st.n_streams;
     int k_sub = h->split;
     if (k_sub == 0) {
         static const int env = [] { const char* e = getenv("LC3B_SPLIT"); return e ? atoi(e) : 0; }();
@@ -497,12 +524,14 @@ static cudaError_t run_decode(lc3b_decoder* h, const uint8_t* frames, const int3
     int part = ((n + k_sub - 1) / k_sub + 127) & ~127;                // whole entropy CTAs
     if (k_sub <= 1 || part >= n) { k_sub = 1; part = n; }
     for (int k = 0, base = 0; k < k_sub && base < n; k++, base += part) {
-        const int count = k_sub == 1 ? -1 : (n - base < part ? n - base : part);
+        int count = k_sub == 1 ? -1 : (n - base < part ? n - base : part);
         plan.lane = k;
         const int first = plan.n;
-        if (stage_mask & 3) plan_entropy(plan, h->st, frames, frame_nbytes, nbytes, frame_stride, status_out, stage_mask & 3, base, count, -1);
+        if (ids && count < 0) count = n;                                // with an id list the launch size is the call's, not the handle's
+        if (stage_mask & 3)
+            plan_entropy(plan, h->st, frames, frame_nbytes, nbytes, frame_stride, status_out, stage_mask & 3, base, count, -1, ids, n);
         if (stage_mask & 4) {
-            if (plan_synth(plan, h->st, pcm_out, pcm_stride, plan.n > first ? plan.n - 1 : -1, base, count) < 0) return cudaErrorInvalidValue;
+            if (plan_synth(plan, h->st, pcm_out, pcm_stride, plan.n > first ? plan.n - 1 : -1, base, count, ids) < 0) return cudaErrorInvalidValue;
         }
     }
     return h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream, &h->lanes);
@@ -519,6 +548,41 @@ int lc3b_decode_frames(lc3b_decoder* h, int bits_per_sample, const uint8_t* fram
     if (!frame_nbytes && nbytes < st.min_nbytes) return LC3B_ERR_INVALID_ARG;       // lc3b_decoder_set_min_nbytes
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     CU(run_decode(h, frames, frame_nbytes, nbytes, frame_stride, pcm_out, pcm_stride, status_out, h->stage_mask, stream));
+    return LC3B_OK;
+}
+
+// Validates the id list on the host and copies it into the workspace's id area (one cudaMemcpyAsync).  Returns an
+// LC3B_* code; nothing is enqueued unless it is LC3B_OK.
+static int stage_ids(lc3b_decoder* h, const int32_t* stream_ids, int n, cudaStream_t stream) {
+    const DecoderState& st = h->st;
+    if (!stream_ids || n < 0 || n > st.n_streams || !st.ids) return LC3B_ERR_INVALID_ARG;
+    if (!h->id_list.take(stream_ids, n, st.n_streams)) return LC3B_ERR_INVALID_ARG;   // lc3_decoder.rs:228
+    if (n > 0) CU(cudaMemcpyAsync(st.ids, h->id_list.ids.data(), sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, stream));
+    return LC3B_OK;
+}
+
+int lc3b_decode_frames_subset(lc3b_decoder* h, int bits_per_sample, const int32_t* stream_ids, int n_rows, const uint8_t* frames,
+                              const int32_t* frame_nbytes, int nbytes, size_t frame_stride, int16_t* pcm_out, size_t pcm_stride,
+                              int32_t* status_out, void* cuda_stream) {
+    if (!h || !stream_ids || (n_rows > 0 && (!frames || !pcm_out))) return LC3B_ERR_INVALID_ARG;
+    if (bits_per_sample != 16) return LC3B_ERR_BITS_PER_SAMPLE;                       // lc3_decoder.rs:80
+    const DecoderState& st = h->st;
+    if (nbytes < 0 || nbytes > st.max_nbytes || (size_t)nbytes > frame_stride || pcm_stride < (size_t)st.cfg.nf)
+        return LC3B_ERR_INVALID_ARG;
+    if (!frame_nbytes && nbytes < st.min_nbytes) return LC3B_ERR_INVALID_ARG;       // lc3b_decoder_set_min_nbytes
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    const int r = stage_ids(h, stream_ids, n_rows, stream);
+    if (r != LC3B_OK || n_rows == 0) return r;
+    CU(run_decode(h, frames, frame_nbytes, nbytes, frame_stride, pcm_out, pcm_stride, status_out, h->stage_mask, stream, st.ids, n_rows));
+    return LC3B_OK;
+}
+
+int lc3b_decoder_reset_streams(lc3b_decoder* h, const int32_t* stream_ids, int n, void* cuda_stream) {
+    if (!h) return LC3B_ERR_INVALID_ARG;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    const int r = stage_ids(h, stream_ids, n, stream);
+    if (r != LC3B_OK || n == 0) return r;
+    CU(launch_init_streams(h->st, h->st.ids, n, stream));
     return LC3B_OK;
 }
 

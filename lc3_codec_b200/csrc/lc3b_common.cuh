@@ -43,6 +43,16 @@ enum {
 };
 constexpr int XTAIL_FLOATS = 3 * 16;   // per stream: last 16 samples of x_hat of the frame in each ring block
 
+// Subset calls (lc3b_decode_frames_subset, lc3b_encode_frames_subset) keep two indices apart: the ROW u of the call, which
+// indexes its I/O and every per-call buffer, and the STATE ROW, the handle stream ids[u] whose persistent buffers the row
+// reads and writes.  IDS is a template parameter of the kernels, so the dense instantiations (IDS = false) compile to
+// exactly the code they had before the indirection existed.
+template <bool IDS>
+__device__ __forceinline__ int state_row(const int32_t* ids, int u) {
+    if constexpr (IDS) return __ldg(ids + u);
+    else return u;
+}
+
 // Everything a kernel needs to know about the (fs, duration) configuration; lives in the workspace.
 struct DevConfig {
     int32_t fs_ind, fs, ne, nb, nf, z, n_ms;
@@ -94,6 +104,7 @@ struct DecoderState {
     int16_t* stage_out;  // [n_streams][nf]
     int32_t* stage_len;  // [n_streams]
     int32_t* stage_status;  // [n_streams]
+    int32_t* ids;        // [n_streams] id list of the current subset call (lc3b_decode_frames_subset, lc3b_decoder_reset_streams)
     // optional inspection outputs (caller-owned device memory)
     int32_t* trace;
     int32_t* trace_x;
@@ -136,6 +147,7 @@ struct EntropyParams {
     int fixed_slot;           // >= 0: spectrum always goes to this slot and sstate is left alone (time-parallel path)
     int min_nbytes;           // frames shorter than this (but not empty) break the handle's promise and are treated as lost
     int row_pitch;        // bytes per staged frame row in shared memory
+    const int32_t* ids;   // subset call: row u of this launch is handle stream ids[u] (the IDS instantiations only)
 };
 
 // Mixed-rate batches: one (fs, duration) bucket = a contiguous row range of the caller's buffers with its own state.
@@ -167,13 +179,19 @@ int entropy_row_pitch(int nbytes);
 bool use_dequant_warp(int n_streams, int mode);   // mode: 0 auto (by batch size), 1 warp-per-frame, 2 thread-per-frame
 // base / count: the sub-batch of the handle's streams the launches cover (base a multiple of 128; count < 0 = all);
 // first_dep: what the first node added waits for (-2 = the node added just before, -1 = nothing)
+// ids: a subset call's device id list (nullptr = a dense call, row u is stream u).  With ids, base / count cut the call's
+// rows and the state pointers stay at the handle's first stream; n_rows is the call's row count (the dequantisation
+// kernel is chosen by it).
 EntropyParams entropy_params(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                             size_t frame_stride, int32_t* status_out, int base = 0, int count = -1);
+                             size_t frame_stride, int32_t* status_out, int base = 0, int count = -1,
+                             const int32_t* ids = nullptr);
 void plan_entropy(LaunchPlan& plan, const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                  size_t frame_stride, int32_t* status_out, int stages, int base = 0, int count = -1, int first_dep = -2);
+                  size_t frame_stride, int32_t* status_out, int stages, int base = 0, int count = -1, int first_dep = -2,
+                  const int32_t* ids = nullptr, int n_rows = 0);
 void plan_entropy_mixed(LaunchPlan& plan, const MixedTables& t, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
                         size_t frame_stride, int32_t* status_out, int* node_d10, int* node_d75);
-int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_t pcm_stride, int dep, int base = 0, int count = -1);
+int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_t pcm_stride, int dep, int base = 0, int count = -1,
+               const int32_t* ids = nullptr);
 
 cudaError_t prepare_entropy(const DecoderState& st);   // shared-memory limits of the kernels, once per handle
 cudaError_t prepare_synth(const DecoderState& st);

@@ -329,6 +329,7 @@ __host__ __device__ inline size_t dequant_smem_bytes(int row_pitch) {
     return 16 * ENT_THREADS * 4 + 68 * 4 + (size_t)ENT_THREADS * row_pitch;
 }
 
+template <bool IDS>
 __device__ __forceinline__ void entropy_body(const EntropyParams& p, const int block) {
     // declared here, not handed in as a pointer: the compiler then addresses shared memory directly instead of rebuilding the
     // shared window base from a generic pointer inside the symbol loop
@@ -395,7 +396,7 @@ __device__ __forceinline__ void entropy_body(const EntropyParams& p, const int b
             if (good && pr.tail_uint(c.lastnz_bits, v)) {
                 int work = (int)((v + 1) << 1);
                 if (p.nsym_prev) {
-                    const int prev = p.nsym_prev[s_me];
+                    const int prev = p.nsym_prev[state_row<IDS>(p.ids, s_me)];
                     if (prev > 0) work = prev;
                 }
                 work = min(work, 0xffff);
@@ -565,7 +566,7 @@ __device__ __forceinline__ void entropy_body(const EntropyParams& p, const int b
             lev = fin ? 0 : lev2;
         }
         ok = !bad;
-        if (ok && p.nsym_prev) p.nsym_prev[stream] = nsym;              // next frame's sort key
+        if (ok && p.nsym_prev) p.nsym_prev[state_row<IDS>(p.ids, stream)] = nsym;   // next frame's sort key
         ac.low = low;
         ac.range = range;
         rd.head = head;
@@ -672,8 +673,9 @@ __device__ __forceinline__ void entropy_body(const EntropyParams& p, const int b
 }
 
 
+template <bool IDS>
 __global__ void __launch_bounds__(ENT_THREADS, 6) entropy_kernel(const __grid_constant__ EntropyParams p) {
-    entropy_body(p, blockIdx.x);
+    entropy_body<IDS>(p, blockIdx.x);
 }
 
 // Mixed-rate batches (BASELINE config 4; lc3b_mixed_*): ONE launch covers every (fs, duration) bucket.  A CTA finds its
@@ -701,13 +703,13 @@ __global__ void __launch_bounds__(ENT_THREADS, 6) entropy_mixed_kernel(const __g
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
     mixed_select(m, &s_p, &s_block);
-    entropy_body(s_p, s_block);
+    entropy_body<false>(s_p, s_block);
 }
 
 // ---------------------------------------------------------------- kernel 1b: integers -> shaped spectrum
 // Dequantisation, residual refinement, noise filling, global gain, TNS lattice, SNS gains (reference D4-D8); one
 // thread per frame, every thread walks all ne lines, so the warp stays converged without any work sorting.
-template <int W /* noise-filling half width: 3 at 10 ms, 2 at 7.5 ms */>
+template <int W /* noise-filling half width: 3 at 10 ms, 2 at 7.5 ms */, bool IDS>
 __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int block) {
     extern __shared__ __align__(16) uint8_t smem[];
     float* s_scf = (float*)smem;
@@ -724,6 +726,7 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
     const int fid = ho[HO_FID];
     const int stream = stream0 + fid;
     const bool live = stream < p.n_streams;
+    const int srow = live ? state_row<IDS>(p.ids, stream) : stream;   // the stream's persistent rows
     const bool ok = ho[HO_OK] != 0;
     SideInfoD si;
     si.lastnz = ho[HO_LASTNZ]; si.lsb_mode = ho[HO_LSB_MODE]; si.gg_ind = ho[HO_GG_IND]; si.bw = ho[HO_BW];
@@ -762,7 +765,7 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
 
     // ---- pass 2: dequantise, noise fill, gain, TNS, SNS; spectrum -> inactive slot
     int slot = 0;
-    if (live && p.fixed_slot < 0) slot = p.sstate[(size_t)stream * SS_WORDS + SS_SLOT];
+    if (live && p.fixed_slot < 0) slot = p.sstate[(size_t)srow * SS_WORDS + SS_SLOT];
     const int new_slot = p.fixed_slot >= 0 ? p.fixed_slot : slot ^ 1;
     float* s_y = s_scf + tid;                                          // PVQ vector / scale factors, stride T
     bool is_zero_frame = false;
@@ -852,7 +855,7 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
     // rows of one warp belong to arbitrary streams of the CTA (work sorting) and may sit in different slots
     // (a slot only flips on a good frame): every row is addressed through its own stream id and slot
     const size_t slot_stride = (size_t)p.slot_streams * ne;
-    const long long my_row_off_ll = (long long)((size_t)new_slot * slot_stride + (size_t)stream * ne);
+    const long long my_row_off_ll = (long long)((size_t)new_slot * slot_stride + (size_t)srow * ne);
 
     const bool any_ok = __any_sync(0xffffffffu, ok);
     if (any_ok) {
@@ -1036,20 +1039,20 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
 
     // ---- hand-off record for the synthesis kernel, slot flip
     if (live) {
-        int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
+        int32_t* sd = p.side + (size_t)srow * SIDE_WORDS;
         sd[SD_OK] = ok;
         sd[SD_LTPF_ACTIVE] = ok ? si.ltpf_active : 0;
         sd[SD_PITCH_INDEX] = ok ? si.pitch_index : 0;
         sd[SD_NBITS] = nbits;
         sd[SD_SLOT] = ok ? new_slot : slot;
-        if (ok && p.fixed_slot < 0) p.sstate[(size_t)stream * SS_WORDS + SS_SLOT] = new_slot;
+        if (ok && p.fixed_slot < 0) p.sstate[(size_t)srow * SS_WORDS + SS_SLOT] = new_slot;
     }
 }
 
 // 5 CTAs per SM (96 registers): measured against 4 (119 registers, 0.80 ms), 6 (80, 0.74 ms) and 7 (72, spills, 0.82 ms): 0.667 ms
-template <int W>
+template <int W, bool IDS>
 __global__ void __launch_bounds__(ENT_THREADS, 5) dequant_kernel(const __grid_constant__ EntropyParams p) {
-    dequant_body<W>(p, blockIdx.x);
+    dequant_body<W, IDS>(p, blockIdx.x);
 }
 
 template <int W>
@@ -1057,7 +1060,7 @@ __global__ void __launch_bounds__(ENT_THREADS, 5) dequant_mixed_kernel(const __g
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
     mixed_select(m, &s_p, &s_block);
-    dequant_body<W>(s_p, s_block);
+    dequant_body<W, false>(s_p, s_block);
 }
 
 // ---------------------------------------------------------------- kernels 1b' / 1b'': the small-batch dequantisation
@@ -1093,6 +1096,7 @@ __device__ __forceinline__ float sns_interp64(const float* scf, int j) {        
     return xa(fn, xm(w, d));
 }
 
+template <bool IDS>
 __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const int block) {
     extern __shared__ __align__(16) uint8_t smem[];
     float* s_gband = (float*)smem;                                     // [DQW_WARPS][64]
@@ -1131,6 +1135,7 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
     const int fid = field(HO_FID);
     const int stream = (slot / ENT_THREADS) * ENT_THREADS + fid;
     const bool live = stream < p.n_streams;
+    const int srow = live ? state_row<IDS>(p.ids, stream) : stream;   // the stream's persistent rows
     const bool ok = live && field(HO_OK) != 0;
     const int lastnz = field(HO_LASTNZ), lsb_mode = field(HO_LSB_MODE), gg_ind = field(HO_GG_IND), bw = field(HO_BW);
     const int num_tns = field(HO_NUM_TNS), noise_factor = field(HO_NOISE_FACTOR);
@@ -1141,7 +1146,7 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
     const int nbits = len * 8;
 
     int slot_cur = 0;
-    if (live && p.fixed_slot < 0) slot_cur = p.sstate[(size_t)stream * SS_WORDS + SS_SLOT];
+    if (live && p.fixed_slot < 0) slot_cur = p.sstate[(size_t)srow * SS_WORDS + SS_SLOT];
     const int new_slot = p.fixed_slot >= 0 ? p.fixed_slot : slot_cur ^ 1;
     constexpr int NR = (MAX_NE + 31) / 32;                             // rows of 32 lines
     if (ok) {                                                          // warp-uniform
@@ -1222,7 +1227,7 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
         }
         const bool is_zero_frame = lastnz == 2 && (__ballot_sync(0xffffffffu, x[0] != 0) & 3u) == 0 && gg_ind == 0;
         const uint8_t* fr = p.frames + (size_t)stream * p.frame_stride;
-        float* dst = p.spec + ((size_t)new_slot * p.slot_streams + stream) * ne;
+        float* dst = p.spec + ((size_t)new_slot * p.slot_streams + srow) * ne;
         int res_base = 0, fill_base = 0;
 #pragma unroll
         for (int j = 0; j < NR; j++) {
@@ -1266,18 +1271,19 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
         }
     }
     if (live && lane == 0) {
-        int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
+        int32_t* sd = p.side + (size_t)srow * SIDE_WORDS;
         sd[SD_OK] = ok;
         sd[SD_LTPF_ACTIVE] = ok ? ltpf_active : 0;
         sd[SD_PITCH_INDEX] = ok ? pitch_index : 0;
         sd[SD_NBITS] = nbits;
         sd[SD_SLOT] = ok ? new_slot : slot_cur;
-        if (ok && p.fixed_slot < 0) p.sstate[(size_t)stream * SS_WORDS + SS_SLOT] = new_slot;
+        if (ok && p.fixed_slot < 0) p.sstate[(size_t)srow * SS_WORDS + SS_SLOT] = new_slot;
     }
 }
 
 // The listed frames' lattices, one thread each: temporal_noise_shaping.rs:24-74 then the SNS gains, four lines at a time
 // in place on the frame's row (the row is the slot dequant_warp_kernel just wrote and made current).
+template <bool IDS>
 __device__ __forceinline__ void tns_list_body(const EntropyParams& p, const int block) {
     // band gains of the CTA's frames, [band][thread] (a thread walks its own column: no bank conflicts), and the band edges:
     // the walk along the bands must not wait for global memory at every band change
@@ -1315,7 +1321,7 @@ __device__ __forceinline__ void tns_list_body(const EntropyParams& p, const int 
     float rc0[8] = {0, 0, 0, 0, 0, 0, 0, 0}, rc1[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     float* row = p.spec;
     if (mine) {
-        const int stream = (slot / ENT_THREADS) * ENT_THREADS + ho[HO_FID];
+        const int stream = state_row<IDS>(p.ids, (slot / ENT_THREADS) * ENT_THREADS + ho[HO_FID]);   // listed frames are live
         const int bw = ho[HO_BW];
         const bool d10 = c.n_ms == LC3B_10MS;
         const int bw_stop = d10 ? 80 * (bw + 1) : 60 * (bw + 1);
@@ -1394,11 +1400,13 @@ __device__ __forceinline__ void tns_list_body(const EntropyParams& p, const int 
     report_done();
 }
 
+template <bool IDS>
 __global__ void __launch_bounds__(DQW_WARPS * 32) dequant_warp_kernel(const __grid_constant__ EntropyParams p) {
-    dequant_warp_body(p, blockIdx.x);
+    dequant_warp_body<IDS>(p, blockIdx.x);
 }
+template <bool IDS>
 __global__ void __launch_bounds__(ENT_THREADS) tns_list_kernel(const __grid_constant__ EntropyParams p) {
-    tns_list_body(p, blockIdx.x);
+    tns_list_body<IDS>(p, blockIdx.x);
 }
 
 // mixed-rate variants.  per_cta_slots: thread slots one CTA covers (DQW_WARPS for the warp kernel, ENT_THREADS for the list
@@ -1424,13 +1432,13 @@ __global__ void __launch_bounds__(DQW_WARPS * 32) dequant_warp_mixed_kernel(cons
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
     mixed_select_scaled(m, &s_p, &s_block, ENT_THREADS / DQW_WARPS);
-    dequant_warp_body(s_p, s_block);
+    dequant_warp_body<false>(s_p, s_block);
 }
 __global__ void __launch_bounds__(ENT_THREADS) tns_list_mixed_kernel(const __grid_constant__ MixedParams m) {
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
     mixed_select_scaled(m, &s_p, &s_block, 1);
-    tns_list_body(s_p, s_block);
+    tns_list_body<false>(s_p, s_block);
 }
 
 int entropy_row_pitch(int nbytes) {
@@ -1443,25 +1451,30 @@ int entropy_row_pitch(int nbytes) {
 cudaError_t prepare_entropy(const DecoderState& st) {
     const int pitch = entropy_row_pitch(st.max_nbytes);
     const int es = (int)entropy_smem_bytes(pitch), ds = (int)dequant_smem_bytes(pitch);
-    cudaError_t e = cudaFuncSetAttribute(entropy_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, es);
+    cudaError_t e = cudaFuncSetAttribute(entropy_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, es);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(entropy_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, es);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(entropy_mixed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, es);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_kernel<3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_mixed_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_mixed_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, ds);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dequant_warp_smem_bytes());
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_warp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dequant_warp_smem_bytes());
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_warp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dequant_warp_smem_bytes());
     if (e == cudaSuccess) e = cudaFuncSetAttribute(dequant_warp_mixed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dequant_warp_smem_bytes());
     return e;
 }
 
 EntropyParams entropy_params(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                             size_t frame_stride, int32_t* status_out, int base, int count) {
+                             size_t frame_stride, int32_t* status_out, int base, int count, const int32_t* ids) {
     EntropyParams p;
     memset(&p, 0, sizeof(p));                      // padding bytes are part of the graph cache key
     // a sub-batch is the same launch with every per-stream pointer moved to its first stream (base is a multiple of the
     // CTA's 128 thread slots, so the lane-interleaved scratch moves by whole blocks); only the stride between the two
-    // spectrum slots still belongs to the whole handle
-    const size_t b = (size_t)base;
+    // spectrum slots still belongs to the whole handle.  A subset call's rows reach the state through the id list:
+    // only the row-indexed pointers and the id list move, the state pointers (sb) stay at the handle's first stream.
+    const size_t b = (size_t)base, sb = ids ? 0 : b;
     const int ne = st.cfg.ne;
     p.cfg = st.dcfg;
     p.frames = frames ? frames + b * frame_stride : nullptr;
@@ -1470,41 +1483,51 @@ EntropyParams entropy_params(const DecoderState& st, const uint8_t* frames, cons
     p.frame_stride = frame_stride;
     p.n_streams = count < 0 ? st.n_streams : count;
     p.slot_streams = st.n_streams;
-    p.spec = st.spec + b * ne;
+    p.spec = st.spec + sb * ne;
     p.xq = st.xq + b * ne;                         // [block32][ne][32]: 32 streams are ne * 32 integers
     p.handoff = st.handoff + b * HO_WORDS;
-    p.side = st.side + b * SIDE_WORDS;
-    p.sstate = st.sstate + b * SS_WORDS;
+    p.side = st.side + sb * SIDE_WORDS;
+    p.sstate = st.sstate + sb * SS_WORDS;
     p.status_out = status_out ? status_out + b : nullptr;
     p.trace = st.trace ? st.trace + b * LC3B_TRACE_WORDS : nullptr;
     p.trace_x = st.trace_x ? st.trace_x + b * ne : nullptr;
     p.sym_lut = st.sym_lut;
     p.gband = st.gband;                            // small-batch path only (never split)
     p.tns_list = st.tns_list;
-    p.nsym_prev = st.nsym_prev ? st.nsym_prev + b : nullptr;
+    p.nsym_prev = st.nsym_prev ? st.nsym_prev + sb : nullptr;
     p.fixed_slot = st.fixed_slot;
     p.min_nbytes = st.min_nbytes;
     p.row_pitch = entropy_row_pitch(nbytes);
+    p.ids = ids ? ids + b : nullptr;
     return p;
+}
+
+// n_call: rows of the whole call (not of this sub-batch): the small-batch kernels share one list per handle, so the choice
+// between them and dequant_kernel is made once per call
+template <bool IDS>
+static void plan_entropy_kernels(LaunchPlan& plan, const DecoderState& st, const EntropyParams& p, int stages, int first_dep, int n_call) {
+    const unsigned grid = (unsigned)((p.n_streams + ENT_THREADS - 1) / ENT_THREADS);
+    int dep = first_dep;
+    if (stages & 1) { plan.add(entropy_kernel<IDS>, grid, ENT_THREADS, entropy_smem_bytes(p.row_pitch), p, dep); dep = -2; }
+    if (stages & 2) {
+        if (use_dequant_warp(n_call, st.dequant_mode)) {               // never split (its list is per handle)
+            plan.add(dequant_warp_kernel<IDS>, grid * (ENT_THREADS / DQW_WARPS), DQW_WARPS * 32, dequant_warp_smem_bytes(), p, dep);
+            plan.add(tns_list_kernel<IDS>, grid, ENT_THREADS, 0, p);
+        } else {
+            const size_t smem = dequant_smem_bytes(p.row_pitch);
+            if (st.cfg.n_ms == LC3B_10MS) plan.add(dequant_kernel<3, IDS>, grid, ENT_THREADS, smem, p, dep);
+            else plan.add(dequant_kernel<2, IDS>, grid, ENT_THREADS, smem, p, dep);
+        }
+    }
 }
 
 // stages: bit 0 entropy_kernel (bitstream -> integers), bit 1 dequant_kernel (integers -> shaped spectrum)
 void plan_entropy(LaunchPlan& plan, const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                  size_t frame_stride, int32_t* status_out, int stages, int base, int count, int first_dep) {
-    const EntropyParams p = entropy_params(st, frames, frame_nbytes, nbytes, frame_stride, status_out, base, count);
-    const unsigned grid = (unsigned)((p.n_streams + ENT_THREADS - 1) / ENT_THREADS);
-    int dep = first_dep;
-    if (stages & 1) { plan.add(entropy_kernel, grid, ENT_THREADS, entropy_smem_bytes(p.row_pitch), p, dep); dep = -2; }
-    if (stages & 2) {
-        if (use_dequant_warp(st.n_streams, st.dequant_mode)) {         // whole handle only (its list is per handle)
-            plan.add(dequant_warp_kernel, grid * (ENT_THREADS / DQW_WARPS), DQW_WARPS * 32, dequant_warp_smem_bytes(), p, dep);
-            plan.add(tns_list_kernel, grid, ENT_THREADS, 0, p);
-        } else {
-            const size_t smem = dequant_smem_bytes(p.row_pitch);
-            if (st.cfg.n_ms == LC3B_10MS) plan.add(dequant_kernel<3>, grid, ENT_THREADS, smem, p, dep);
-            else plan.add(dequant_kernel<2>, grid, ENT_THREADS, smem, p, dep);
-        }
-    }
+                  size_t frame_stride, int32_t* status_out, int stages, int base, int count, int first_dep,
+                  const int32_t* ids, int n_rows) {
+    const EntropyParams p = entropy_params(st, frames, frame_nbytes, nbytes, frame_stride, status_out, base, count, ids);
+    if (ids) plan_entropy_kernels<true>(plan, st, p, stages, first_dep, n_rows);
+    else plan_entropy_kernels<false>(plan, st, p, stages, first_dep, st.n_streams);
 }
 
 // Which dequantisation kernel a batch of n streams gets: warp-per-frame below DQW_MAX_STREAMS (it finishes a small batch

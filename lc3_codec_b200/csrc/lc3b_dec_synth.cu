@@ -51,6 +51,7 @@ struct SynthParams {
     int group;           // ltpf_kernel: streams looked after by one warp
     int smem_per_warp;   // ltpf_kernel, bytes
     int no_ltpf;         // the handle's minimum frame length rules the post filter out: no history is kept (lc3b_decoder_set_min_nbytes)
+    const int32_t* ids;  // subset call: row u of this launch is handle stream ids[u] (the IDS instantiations only)
 };
 
 constexpr int SYN_WARPS = 4;
@@ -66,14 +67,15 @@ static inline size_t synth_smem_bytes(int nf) { return (size_t)PIPE_WARPS * 3 * 
 // 262 144, and MORE resident warps make it slower (8 / 10 / 12 CTAs per SM: 0.502 / 0.516 / 0.529 ms - the twiddle and
 // window tables share L1 with the shared-memory carve-out).  The per-frame streams (spectrum, overlap memory, PCM)
 // therefore use evict-first loads and stores, which leaves L1 to the tables (0.517 -> 0.500 ms).
-template <int NF, bool MS10>
+template <int NF, bool MS10, bool IDS>
 __global__ void __launch_bounds__(SYN_WARPS * 32) synth_classic_kernel(const __grid_constant__ SynthParams p) {
     using G = FrameGeo<NF, MS10>;
     constexpr int NE = G::NE, Z = G::Z, NP = G::NP, NPT = G::NPT;
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int stream = blockIdx.x * SYN_WARPS + wid;
-    if (stream >= p.n_streams) return;                            // warps are independent: no CTA-wide barrier below
+    const int row = blockIdx.x * SYN_WARPS + wid;
+    if (row >= p.n_streams) return;                               // warps are independent: no CTA-wide barrier below
+    const int stream = state_row<IDS>(p.ids, row);                // persistent rows; PCM goes to the call's row
 
     float* P = (float*)smem + (size_t)wid * 2 * NF;               // spectrum in; FFT ping
     float* Q = P + NF;                                            // FFT pong
@@ -139,7 +141,7 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) synth_classic_kernel(const __g
     const bool in_span = active || prev_active;
     float* yblk = in_span ? p.ltpf_x + (size_t)stream * NF : p.ltpf_y + (size_t)stream * p.hist_len + blk_idx * NF;
     float* xtail = p.ltpf_xtail + (size_t)stream * XTAIL_FLOATS + blk_idx * 16;
-    int16_t* out = p.pcm_out + (size_t)stream * p.pcm_stride;
+    int16_t* out = p.pcm_out + (size_t)row * p.pcm_stride;
 #pragma unroll
     for (int j = 0; j < NP; j++) {
         const int n = 64 * j + 2 * lane;
@@ -197,7 +199,9 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 struct FrameHead {
     int ok, slot, active, prev_active, blk_idx;
 };
-__device__ __forceinline__ FrameHead load_head(const SynthParams& p, int stream) {
+template <bool IDS>
+__device__ __forceinline__ FrameHead load_head(const SynthParams& p, int row) {
+    const int stream = state_row<IDS>(p.ids, row);
     const int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
     const int32_t* ss = p.sstate + (size_t)stream * SS_WORDS;
     FrameHead h;
@@ -215,7 +219,8 @@ __device__ __forceinline__ FrameHead load_head(const SynthParams& p, int stream)
 // their way, so a warp never waits for HBM latency once it is running.  Per warp: two stage buffers of nf floats (the
 // spectrum arrives in the first ne, the rest stays zero; the stage buffer then serves as the FFT's ping buffer) and
 // one pong buffer.
-template <int NF, bool MS10>
+// Subset calls (IDS): `stream` walks the call's rows; the state and the spectrum are read at the row's handle stream.
+template <int NF, bool MS10, bool IDS>
 __global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_constant__ SynthParams p) {
     using G = FrameGeo<NF, MS10>;
     constexpr int NE = G::NE, Z = G::Z, NP = G::NP, NPT = G::NPT, N = NF / 2;
@@ -248,11 +253,11 @@ __global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_
             bulk_g2s(S0 + st * NF, sp, NE * 4, &bars[st]);
         }
     };
-    FrameHead head = load_head(p, stream);
-    fetch(0, stream, head);
+    FrameHead head = load_head<IDS>(p, stream);
+    fetch(0, state_row<IDS>(p.ids, stream), head);
     int nstream = stream + n_warps;
     FrameHead nhead = head;
-    if (nstream < p.n_streams) nhead = load_head(p, nstream);
+    if (nstream < p.n_streams) nhead = load_head<IDS>(p, nstream);
     uint32_t phase0 = 0, phase1 = 0;
 
     for (int it = 0; stream < p.n_streams; it++) {
@@ -269,16 +274,17 @@ __global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_
                 __syncwarp();
                 fence_proxy_async();
             }
-            fetch(st ^ 1, nstream, nhead);
-            if (n2stream < p.n_streams) n2head = load_head(p, n2stream);
+            fetch(st ^ 1, state_row<IDS>(p.ids, nstream), nhead);
+            if (n2stream < p.n_streams) n2head = load_head<IDS>(p, n2stream);
         }
 
-        int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
-        int32_t* ss = p.sstate + (size_t)stream * SS_WORDS;
+        const int srow = state_row<IDS>(p.ids, stream);
+        int32_t* sd = p.side + (size_t)srow * SIDE_WORDS;
+        int32_t* ss = p.sstate + (size_t)srow * SS_WORDS;
         const int ok = head.ok, active = head.active, prev_active = head.prev_active, blk_idx = head.blk_idx;
 
         // overlap memory: requested now, consumed after the FFT
-        float* ola = p.ola + (size_t)stream * (NF - Z);
+        float* ola = p.ola + (size_t)srow * (NF - Z);
         float2 ola_r[NPT];
 #pragma unroll
         for (int j = 0; j < NPT; j++)
@@ -331,8 +337,8 @@ __global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_
         // around the ring into it), so x_hat waits in a side buffer for ltpf_kernel instead.  When the handle's promised
         // minimum frame length rules the filter out for good (p.no_ltpf), the history is never read and is not kept.
         const bool in_span = active || prev_active;
-        float* yblk = in_span ? p.ltpf_x + (size_t)stream * NF : p.ltpf_y + (size_t)stream * p.hist_len + blk_idx * NF;
-        float* xtail = p.ltpf_xtail + (size_t)stream * XTAIL_FLOATS + blk_idx * 16;
+        float* yblk = in_span ? p.ltpf_x + (size_t)srow * NF : p.ltpf_y + (size_t)srow * p.hist_len + blk_idx * NF;
+        float* xtail = p.ltpf_xtail + (size_t)srow * XTAIL_FLOATS + blk_idx * 16;
         int16_t* out = p.pcm_out + (size_t)stream * p.pcm_stride;
 #pragma unroll
         for (int j = 0; j < NP; j++) {
@@ -363,6 +369,7 @@ __global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_
 }
 
 // ---------------------------------------------------------------- kernel 3: the post filter where it is not idle
+template <bool IDS>
 __global__ void __launch_bounds__(SYN_WARPS * 32) ltpf_kernel(SynthParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const DevConfig& c = *p.cfg;
@@ -372,10 +379,12 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) ltpf_kernel(SynthParams p) {
     // which streams of this warp's group are inside an active span
     uint32_t todo;
     {
-        const int s = first + lane;
+        const int r = first + lane;
         bool in_span = false;
-        if (lane < p.group && s < p.n_streams)
+        if (lane < p.group && r < p.n_streams) {
+            const int s = state_row<IDS>(p.ids, r);
             in_span = p.side[(size_t)s * SIDE_WORDS + SD_LTPF_ACTIVE] != 0 || ltpf_prev_active(p.sstate[(size_t)s * SS_WORDS + SS_LTPF_PREV]);
+        }
         todo = __ballot_sync(0xffffffffu, in_span);
     }
     if (todo == 0) return;
@@ -387,7 +396,8 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) ltpf_kernel(SynthParams p) {
     float* scratch = xt + 16;
 
     while (todo) {
-        const int stream = first + (__ffs(todo) - 1);
+        const int row = first + (__ffs(todo) - 1);
+        const int stream = state_row<IDS>(p.ids, row);
         todo &= todo - 1;
         const int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
         int32_t* ss = p.sstate + (size_t)stream * SS_WORDS;
@@ -403,7 +413,7 @@ __global__ void __launch_bounds__(SYN_WARPS * 32) ltpf_kernel(SynthParams p) {
         for (int n = lane; n < nf; n += 32) X[n] = p.ltpf_x[(size_t)stream * nf + n];   // x_hat left by the synthesis kernel
         __syncwarp();
         ltpf_filter_frame(c, g, Y, X, xt, scratch, blk, cur, prev, lane);
-        int16_t* out = p.pcm_out + (size_t)stream * p.pcm_stride;
+        int16_t* out = p.pcm_out + (size_t)row * p.pcm_stride;
         for (int n = lane; n < nf; n += 32) {
             const float v = Y[blk + n];
             yhist[blk + n] = v;
@@ -417,8 +427,10 @@ namespace {
 struct PrepareSynth {
     cudaError_t e = cudaSuccess;
     template <int NF, bool MS10> void operator()() {
-        e = cudaFuncSetAttribute(synth_kernel<NF, MS10>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)synth_smem_bytes(NF));
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYN_WARPS * 2 * NF * 4);
+        e = cudaFuncSetAttribute(synth_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)synth_smem_bytes(NF));
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)synth_smem_bytes(NF));
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYN_WARPS * 2 * NF * 4);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYN_WARPS * 2 * NF * 4);
     }
 };
 struct PlanSynth {
@@ -427,10 +439,14 @@ struct PlanSynth {
     int dep, node, sm_count;
     bool pipelined;
     template <int NF, bool MS10> void operator()() {
+        if (p.ids) add<NF, MS10, true>();
+        else add<NF, MS10, false>();
+    }
+    template <int NF, bool MS10, bool IDS> void add() {
         // persistent: at most as many CTAs as fit on the device at once (4 of 8 warps per SM by registers; shared memory may allow fewer)
         const int full = (p.n_streams + SYN_WARPS - 1) / SYN_WARPS;
         if (!pipelined) {
-            node = plan.add(synth_classic_kernel<NF, MS10>, (unsigned)full, SYN_WARPS * 32, SYN_WARPS * 2 * NF * 4, p, dep);
+            node = plan.add(synth_classic_kernel<NF, MS10, IDS>, (unsigned)full, SYN_WARPS * 32, SYN_WARPS * 2 * NF * 4, p, dep);
             return;
         }
         const size_t smem = synth_smem_bytes(NF);
@@ -439,7 +455,7 @@ struct PlanSynth {
         if (per_sm < 1) per_sm = 1;
         const int resident = sm_count * per_sm;
         const int ctas = (p.n_streams + PIPE_WARPS - 1) / PIPE_WARPS;
-        node = plan.add(synth_kernel<NF, MS10>, (unsigned)(ctas < resident ? ctas : resident), PIPE_WARPS * 32, smem, p, dep);
+        node = plan.add(synth_kernel<NF, MS10, IDS>, (unsigned)(ctas < resident ? ctas : resident), PIPE_WARPS * 32, smem, p, dep);
     }
 };
 }  // namespace
@@ -448,29 +464,33 @@ cudaError_t prepare_synth(const DecoderState& st) {
     PrepareSynth ps;
     if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, ps)) return cudaErrorInvalidValue;
     if (ps.e != cudaSuccess) return ps.e;
-    return cudaFuncSetAttribute(ltpf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ltpf_warp_bytes(st.cfg) * SYN_WARPS));
+    const int lb = (int)(ltpf_warp_bytes(st.cfg) * SYN_WARPS);
+    const cudaError_t e = cudaFuncSetAttribute(ltpf_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
+    return e != cudaSuccess ? e : cudaFuncSetAttribute(ltpf_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
 }
 
 // Adds the synthesis kernel (after node `dep`, -1 = none) and the post-filter kernel behind it; returns the last node.
-int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_t pcm_stride, int dep, int base, int count) {
+int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_t pcm_stride, int dep, int base, int count,
+               const int32_t* ids) {
     SynthParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.dcfg;
     p.win = st.win;
     p.dtw = st.dtw;
     p.ftw = st.ftw;
-    // a sub-batch: every per-stream pointer moved to its first stream (see entropy_params)
-    const size_t b = (size_t)base;
+    // a sub-batch: every per-stream pointer moved to its first stream, or with an id list only the rows (see entropy_params)
+    const size_t b = (size_t)base, sb = ids ? 0 : b;
     const int n = count < 0 ? st.n_streams : count;
     p.hist_len = (st.cfg.n_ms == LC3B_10MS ? 2 : 3) * st.cfg.nf;
-    p.spec = st.spec + b * st.cfg.ne;
-    p.ola = st.ola + b * (size_t)(st.cfg.nf - st.cfg.z);
-    p.ltpf_y = st.ltpf_y + b * (size_t)p.hist_len;
-    p.ltpf_xtail = st.ltpf_xtail + b * XTAIL_FLOATS;
-    p.ltpf_x = st.ltpf_x + b * (size_t)st.cfg.nf;
-    p.side = st.side + b * SIDE_WORDS;
-    p.sstate = st.sstate + b * SS_WORDS;
+    p.spec = st.spec + sb * st.cfg.ne;
+    p.ola = st.ola + sb * (size_t)(st.cfg.nf - st.cfg.z);
+    p.ltpf_y = st.ltpf_y + sb * (size_t)p.hist_len;
+    p.ltpf_xtail = st.ltpf_xtail + sb * XTAIL_FLOATS;
+    p.ltpf_x = st.ltpf_x + sb * (size_t)st.cfg.nf;
+    p.side = st.side + sb * SIDE_WORDS;
+    p.sstate = st.sstate + sb * SS_WORDS;
     p.pcm_out = pcm_out + b * pcm_stride;
+    p.ids = ids ? ids + b : nullptr;
     p.pcm_stride = pcm_stride;
     p.n_streams = n;
     p.slot_streams = st.n_streams;
@@ -490,7 +510,8 @@ int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_
     if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, ps)) return -1;
     if (st.no_ltpf) return ps.node;                           // the post filter can never be active: nothing to launch
     const int n_warps = (n + group - 1) / group;
-    return plan.add(ltpf_kernel, (unsigned)((n_warps + SYN_WARPS - 1) / SYN_WARPS), SYN_WARPS * 32, lw * SYN_WARPS, p, ps.node);
+    return plan.add(ids ? ltpf_kernel<true> : ltpf_kernel<false>, (unsigned)((n_warps + SYN_WARPS - 1) / SYN_WARPS), SYN_WARPS * 32,
+                    lw * SYN_WARPS, p, ps.node);
 }
 
 }  // namespace lc3b

@@ -41,6 +41,7 @@ struct AnalysisParams {
     float* e_b;
     int32_t* ehand;
     int smem_per_warp;
+    const int32_t* ids;   // subset call: row u is handle stream ids[u] (the IDS instantiations only)
 };
 
 constexpr int ANA_WARPS = 4;
@@ -110,11 +111,12 @@ __device__ __forceinline__ void bfly5(C2* f, const float2* tw, int fs, int m, in
     f[u + m3] = csub(s11, s12);
 }
 
+template <bool IDS>
 __global__ void __launch_bounds__(ANA_WARPS * 32) enc_mdct_kernel(AnalysisParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const EncConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int stream = blockIdx.x * ANA_WARPS + wid;
+    const int stream = blockIdx.x * ANA_WARPS + wid;             // the call's row; only the time history is per stream
     if (stream >= p.n_streams) return;
     const int nf = c.nf, ne = c.ne, z = c.z, N = c.n_fft, half = nf / 2;
 
@@ -124,7 +126,7 @@ __global__ void __launch_bounds__(ANA_WARPS * 32) enc_mdct_kernel(AnalysisParams
     int16_t* tb = (int16_t*)(cx + N);               // 2*nf
 
     const int16_t* in = p.pcm + (size_t)stream * p.pcm_stride;
-    int16_t* thist = p.thist + (size_t)stream * (nf - z);
+    int16_t* thist = p.thist + (size_t)state_row<IDS>(p.ids, stream) * (nf - z);
 
     // ---- update_time_buffer (modified_dct.rs:126-138)
     // samples move two at a time: nf, z and nf - z are even, the history rows are 4-byte aligned, the input row usually is
@@ -206,7 +208,9 @@ __global__ void __launch_bounds__(ANA_WARPS * 32) enc_mdct_kernel(AnalysisParams
 }
 
 // Kernel 2, one frame: attack detector and LTPF analysis of stream `stream` (per-stream state) on the input and
-// hand-off record of unit `unit` (runs after enc_mdct_kernel, whose near-Nyquist flag it reads).
+// hand-off record of unit `unit` (runs after enc_mdct_kernel, whose near-Nyquist flag it reads).  IDS: the CTA's warps hold
+// rows stream0 .. stream0 + 3 of a subset call, whose states the shared biquad reaches through the id list.
+template <bool IDS>
 __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* smem, int stream, size_t unit) {
     const EncConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -379,7 +383,7 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
             uint8_t* ob = smem + (size_t)lane * p.smem_per_warp;      // warp `lane`'s slice: same carve-up as above
             float* o_wk = (float*)ob;
             const float* o_x12n = o_wk + 320 + 98 + 98 + 236 + c.delay + NMEM;
-            int32_t* o_es = p.estate + (size_t)(stream0 + lane) * ES_WORDS;
+            int32_t* o_es = p.estate + (size_t)state_row<IDS>(p.ids, stream0 + lane) * ES_WORDS;
             float m1 = __uint_as_float((uint32_t)o_es[ES_H50_M1]), m2 = __uint_as_float((uint32_t)o_es[ES_H50_M2]);
             for (int n = 0; n < len12; n++) {
                 const float h50 = o_x12n[n] - -1.9652933726226904f * m1 - 0.9658854605688177f * m2;
@@ -614,14 +618,14 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
 // separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a CTA walks the same count, so
 // the named barriers inside a frame stay matched.  The __syncwarp orders the state lane 0 (and warp 0, for the biquad)
 // wrote in frame f before the lanes read it in frame f + 1.
-template <bool WALK>
+template <bool WALK, bool IDS>
 __global__ void __launch_bounds__(ANA_WARPS * 32) enc_ltpf_kernel(AnalysisParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int stream = blockIdx.x * ANA_WARPS + (threadIdx.x >> 5);
     if (stream >= p.n_streams) return;
     const int F = WALK ? p.n_frames : 1;
     for (int f = 0; f < F; f++) {
-        ltpf_frame(p, smem, stream, (size_t)stream * F + f);
+        ltpf_frame<IDS>(p, smem, state_row<IDS>(p.ids, stream), (size_t)stream * F + f);
         if (WALK) __syncwarp();
     }
 }
@@ -640,17 +644,17 @@ static size_t ltpf_warp_bytes(const lc3b_config& c) {
 
 // dynamic shared memory limits, once per handle (lc3b_encoder_init)
 cudaError_t prepare_enc_analysis(const EncoderState& st) {
-    cudaError_t e = cudaFuncSetAttribute(enc_mdct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)(mdct_warp_bytes(st.cfg.nf) * ANA_WARPS));
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(enc_ltpf_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ltpf_warp_bytes(st.cfg) * ANA_WARPS));
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(enc_ltpf_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(ltpf_warp_bytes(st.cfg) * ANA_WARPS));
+    const int mb = (int)(mdct_warp_bytes(st.cfg.nf) * ANA_WARPS), lb = (int)(ltpf_warp_bytes(st.cfg) * ANA_WARPS);
+    cudaError_t e = cudaFuncSetAttribute(enc_mdct_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mb);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_mdct_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mb);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     return e;
 }
 
 void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
-                       int n_frames) {
+                       int n_frames, const int32_t* ids) {
     AnalysisParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
@@ -671,18 +675,20 @@ void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     p.xf = st.xf;
     p.e_b = st.e_b;
     p.ehand = st.ehand;
+    p.ids = ids;
     if (stages & 1) {
         const size_t per_warp = mdct_warp_bytes(st.cfg.nf);
         p.smem_per_warp = (int)per_warp;
-        plan.add(enc_mdct_kernel, (unsigned)((st.n_streams + ANA_WARPS - 1) / ANA_WARPS), ANA_WARPS * 32, per_warp * ANA_WARPS, p);
+        plan.add(ids ? enc_mdct_kernel<true> : enc_mdct_kernel<false>, (unsigned)((st.n_streams + ANA_WARPS - 1) / ANA_WARPS),
+                 ANA_WARPS * 32, per_warp * ANA_WARPS, p);
     }
     if (stages & 2) {
         const size_t per_warp = ltpf_warp_bytes(st.cfg);
         p.smem_per_warp = (int)per_warp;
         p.n_streams = st.n_streams / n_frames;                   // one warp per stream, walking its frames
         p.n_frames = n_frames;
-        plan.add(n_frames > 1 ? enc_ltpf_kernel<true> : enc_ltpf_kernel<false>, (unsigned)((p.n_streams + ANA_WARPS - 1) / ANA_WARPS),
-                 ANA_WARPS * 32, per_warp * ANA_WARPS, p);
+        plan.add(n_frames > 1 ? enc_ltpf_kernel<true, false> : ids ? enc_ltpf_kernel<false, true> : enc_ltpf_kernel<false, false>,
+                 (unsigned)((p.n_streams + ANA_WARPS - 1) / ANA_WARPS), ANA_WARPS * 32, per_warp * ANA_WARPS, p);
     }
 }
 

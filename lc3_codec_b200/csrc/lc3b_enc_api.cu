@@ -17,7 +17,7 @@ namespace lc3b {
 
 struct EncLayout {
     size_t ecfg, win, dtw, ftw, perm, thist, xs_hist, x12, x6, estate, xf, e_b, ehand, xq, qhand, lsbs, bs_scratch, stage_in,
-        stage_out, total;
+        stage_out, ids, total;
 };
 
 static size_t take(size_t& off, size_t bytes) {
@@ -26,7 +26,7 @@ static size_t take(size_t& off, size_t bytes) {
     return o;
 }
 
-static int x12_len_of(const lc3b_config& c) { return (c.n_ms == LC3B_10MS ? 128 + 24 : 96 + 44) + 232; }
+__host__ __device__ static int x12_len_of(const lc3b_config& c) { return (c.n_ms == LC3B_10MS ? 128 + 24 : 96 + 44) + 232; }
 
 static EncLayout make_enc_layout(const lc3b_config& c, int n_streams, int max_nbytes) {
     EncLayout L;
@@ -51,6 +51,7 @@ static EncLayout make_enc_layout(const lc3b_config& c, int n_streams, int max_nb
     L.bs_scratch = take(off, ns * sizeof(uint32_t) * (size_t)enc_bitstream_scratch_words(c.ne, max_nbytes));
     L.stage_in = take(off, sizeof(int16_t) * ns * c.nf * 2);   // double-buffered for the pipelined host path
     L.stage_out = take(off, ns * (size_t)max_nbytes);
+    L.ids = take(off, sizeof(int32_t) * ns);                    // id list of a subset call (lc3b_encode_frames_subset)
     L.total = off;
     return L;
 }
@@ -94,13 +95,31 @@ __global__ void enc_init_band_kernel(EncConfig* cfg) {
     }
 }
 
-__global__ void enc_init_streams_kernel(int32_t* estate, int n_streams) {
-    const int s = blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    int32_t* es = estate + (size_t)s * ES_WORDS;
-    for (int i = 0; i < ES_WORDS; i++) es[i] = 0;
+// The state a stream starts from.  ids == nullptr: every stream, whose rows lc3b_encoder_init has just zeroed with the
+// rest of the workspace; otherwise the n listed streams (lc3b_encoder_reset_streams), whose persistent rows are zeroed
+// here first - one warp per stream.
+__global__ void enc_init_streams_kernel(EncoderState st, const int32_t* ids, int n) {
+    const int lane = threadIdx.x & 31;
+    const int i = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    if (i >= n) return;
+    const int s = ids ? ids[i] : i;
+    if (ids) {
+        const int nz = st.cfg.nf - st.cfg.z, x12_len = x12_len_of(st.cfg);
+        for (int k = lane; k < nz; k += 32) st.thist[(size_t)s * nz + k] = 0;
+        for (int k = lane; k < 64; k += 32) st.xs_hist[(size_t)s * 64 + k] = 0;
+        for (int k = lane; k < x12_len; k += 32) st.x12[(size_t)s * x12_len + k] = 0.0f;
+        for (int k = lane; k < 178; k += 32) st.x6[(size_t)s * 178 + k] = 0.0f;
+    }
+    if (lane != 0) return;
+    int32_t* es = st.estate + (size_t)s * ES_WORDS;
+    for (int k = 0; k < ES_WORDS; k++) es[k] = 0;
     es[ES_ATT_POS_LAST] = -1;      // attack_detector.rs:38
     es[ES_T_PREV] = 17;            // long_term_post_filter.rs:85 (K_MIN)
+}
+
+static cudaError_t launch_enc_init_streams(const EncoderState& st, const int32_t* ids, int n, cudaStream_t stream) {
+    enc_init_streams_kernel<<<(unsigned)((n + 7) / 8), 256, 0, stream>>>(st, ids, n);
+    return cudaGetLastError();
 }
 
 // host-side construction of everything that does not need the device tables
@@ -173,6 +192,7 @@ struct lc3b_encoder {
     int stage_mask = 63;
     int graph_mode = 0;                 // 0 = one launch per kernel, 1 = one cached CUDA graph per call (lc3b_plan.cuh)
     GraphCache graphs;
+    IdList id_list;                     // subset calls and resets (lc3b_encode_frames_subset, lc3b_encoder_reset_streams)
     // optional pipelining of the host entry point: PCM arrives on an internal copy stream into a double-buffered
     // staging area, so the upload of call i+1 overlaps the kernels of call i
     int pipelined = 0, buf = 0;
@@ -181,13 +201,26 @@ struct lc3b_encoder {
     bool consumed_valid[2] = {false, false};
 };
 
-// the kernels of one encode_frame per stream as a plan: stage mask bits 0-1 analysis, bits 2-5 quantisation / bitstream
+// the kernels of one encode_frame per stream (ids == nullptr) or per row of a subset call (n rows, row u = stream ids[u],
+// ids in device memory) as a plan: stage mask bits 0-1 analysis, bits 2-5 quantisation / bitstream
 static cudaError_t run_encode(lc3b_encoder* h, const int16_t* pcm, size_t pcm_stride, uint8_t* frames_out, int nbytes,
-                              size_t frame_stride, int mask, cudaStream_t stream) {
+                              size_t frame_stride, int mask, cudaStream_t stream, const int32_t* ids = nullptr, int n = 0) {
     LaunchPlan plan;
-    if (mask & 3) plan_enc_analysis(plan, h->st, pcm, pcm_stride, nbytes, mask & 3);
-    if (mask & 60) plan_enc_quant(plan, h->st, frames_out, nbytes, frame_stride, mask >> 2);
+    EncoderState v = h->st;                                 // a subset call: a view of n rows
+    if (ids) v.n_streams = n;
+    if (mask & 3) plan_enc_analysis(plan, v, pcm, pcm_stride, nbytes, mask & 3, 1, ids);
+    if (mask & 60) plan_enc_quant(plan, v, frames_out, nbytes, frame_stride, mask >> 2, 1, ids);
     return h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream);
+}
+
+// Validates the id list on the host and copies it into the workspace's id area (one cudaMemcpyAsync).  Returns an
+// LC3B_* code; nothing is enqueued unless it is LC3B_OK.
+static int stage_ids(lc3b_encoder* h, const int32_t* stream_ids, int n, cudaStream_t stream) {
+    const EncoderState& st = h->st;
+    if (!stream_ids || n < 0 || n > st.n_streams) return LC3B_ERR_INVALID_ARG;
+    if (!h->id_list.take(stream_ids, n, st.n_streams)) return LC3B_ERR_INVALID_ARG;   // lc3_encoder.rs:175 (channel_index)
+    if (n > 0) CU(cudaMemcpyAsync(st.ids, h->id_list.ids.data(), sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, stream));
+    return LC3B_OK;
 }
 
 extern bool lc3b_make_config(int sf, int fd, lc3b_config* c);
@@ -244,6 +277,7 @@ int lc3b_encoder_init(lc3b_encoder** out, int n_streams, int frame_duration, int
     st.bs_words = enc_bitstream_scratch_words(c.ne, max_nbytes);
     st.stage_in = (int16_t*)(base + L.stage_in);
     st.stage_out = base + L.stage_out;
+    st.ids = (int32_t*)(base + L.ids);
 
     const int N = c.nf / 2;
     EncConfig* hc = (EncConfig*)malloc(sizeof(EncConfig));
@@ -263,8 +297,8 @@ int lc3b_encoder_init(lc3b_encoder** out, int n_streams, int frame_duration, int
     if (e == cudaSuccess) {
         enc_init_band_kernel<<<1, 128, 0, stream>>>(st.ecfg);
         enc_init_tables_kernel<<<1, 256, 0, stream>>>(st.ecfg, st.win);
-        enc_init_streams_kernel<<<(n_streams + 255) / 256, 256, 0, stream>>>(st.estate, n_streams);
         e = cudaGetLastError();
+        if (e == cudaSuccess) e = launch_enc_init_streams(st, nullptr, n_streams, stream);
     }
     if (e != cudaSuccess) {
         delete h;
@@ -290,6 +324,28 @@ int lc3b_encode_frames(lc3b_encoder* h, const int16_t* pcm_in, size_t pcm_stride
     if (nbytes < 20 || nbytes > st.max_nbytes || (size_t)nbytes > frame_stride || pcm_stride < (size_t)st.cfg.nf)
         return LC3B_ERR_INVALID_ARG;
     CU(run_encode(h, pcm_in, pcm_stride, frames_out, nbytes, frame_stride, h->stage_mask, (cudaStream_t)cuda_stream));
+    return LC3B_OK;
+}
+
+int lc3b_encode_frames_subset(lc3b_encoder* h, const int32_t* stream_ids, int n_rows, const int16_t* pcm_in, size_t pcm_stride,
+                              uint8_t* frames_out, int nbytes, size_t frame_stride, void* cuda_stream) {
+    if (!h || !stream_ids || (n_rows > 0 && (!pcm_in || !frames_out))) return LC3B_ERR_INVALID_ARG;
+    const EncoderState& st = h->st;
+    if (nbytes < 20 || nbytes > st.max_nbytes || (size_t)nbytes > frame_stride || pcm_stride < (size_t)st.cfg.nf)
+        return LC3B_ERR_INVALID_ARG;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    const int r = stage_ids(h, stream_ids, n_rows, stream);
+    if (r != LC3B_OK || n_rows == 0) return r;
+    CU(run_encode(h, pcm_in, pcm_stride, frames_out, nbytes, frame_stride, h->stage_mask, stream, st.ids, n_rows));
+    return LC3B_OK;
+}
+
+int lc3b_encoder_reset_streams(lc3b_encoder* h, const int32_t* stream_ids, int n, void* cuda_stream) {
+    if (!h) return LC3B_ERR_INVALID_ARG;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    const int r = stage_ids(h, stream_ids, n, stream);
+    if (r != LC3B_OK || n == 0) return r;
+    CU(launch_enc_init_streams(h->st, h->st.ids, n, stream));
     return LC3B_OK;
 }
 

@@ -65,6 +65,7 @@ struct EncoderState {
     int bs_words;          //               32-bit words per stream of bs_scratch (for max_nbytes)
     int16_t* stage_in;     // [S][nf]       staging for the host entry point
     uint8_t* stage_out;    // [S][max_nbytes]
+    int32_t* ids;          // [S]           id list of the current subset call (lc3b_encode_frames_subset, lc3b_encoder_reset_streams)
 };
 
 cudaError_t prepare_enc_analysis(const EncoderState& st);   // shared-memory limits of the kernels, once per handle
@@ -78,11 +79,13 @@ cudaError_t launch_enc_quant(const EncoderState& st, uint8_t* frames_out, int nb
 // st.n_streams = S * n_frames units (unit s * n_frames + f = frame f of stream s) and whose per-frame buffers have a row
 // per unit; its per-stream state (xs_hist, x12, x6, estate) keeps a row per stream.  The attack / LTPF kernel and the
 // quantise kernel then run a warp per stream that walks the stream's frames in order; every other kernel runs per unit.
+// ids (n_frames == 1 only): a subset call, `st` a view whose st.n_streams is the call's row count; row u's persistent state
+// (thist, xs_hist, x12, x6, estate) is that of handle stream ids[u] (device memory), every other buffer has a row per call row.
 struct LaunchPlan;
 void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
-                       int n_frames = 1);
+                       int n_frames = 1, const int32_t* ids = nullptr);
 void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
-                    int n_frames = 1);
+                    int n_frames = 1, const int32_t* ids = nullptr);
 // time-parallel encode (lc3b_enc_multi.cu): n_frames consecutive frames of every stream as one plan
 size_t enc_multi_scratch_bytes(const EncoderState& st, int n_frames);
 void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_frames, uint8_t* frames_out, int nbytes,

@@ -51,6 +51,7 @@ struct QuantParams {
     uint8_t* frames_out;
     int w_bytes, w_bytes_fin, side_words, sym_cap, out_words;     // per-warp shared-memory slices (prepare / finish kernels)
     int inline_ac;     // small batches: the finish kernel runs the range coder itself (all lanes, same chain) and C2 is skipped
+    const int32_t* ids;   // subset call: row u's rate-loop state is that of handle stream ids[u] (enc_quantize_kernel<false, true>)
 };
 
 constexpr int QW = 8;                       // frames (warps) per CTA
@@ -1511,7 +1512,7 @@ __global__ void __launch_bounds__(QNT_THREADS, 4) enc_tns_kernel(QuantParams p) 
 // walks p.n_frames frames in order, the rate loop's offsets (ES_Q_*) carrying from one frame to the next; otherwise one
 // frame (lc3b_encode_frames: a separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a
 // CTA walks the same count, so the named barriers inside a frame stay matched.
-template <bool WALK>
+template <bool WALK, bool IDS>
 __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const EncConfig& c = *p.cfg;
@@ -1524,7 +1525,7 @@ __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p
     float* e4 = xf + NE_MAX;                                      // [100]
     float* T = e4 + 100;                                          // [224]
     int16_t* xq = (int16_t*)(T + 224);                            // [NE_MAX]
-    int32_t* es = p.estate + (size_t)stream * ES_WORDS;
+    int32_t* es = p.estate + (size_t)state_row<IDS>(p.ids, stream) * ES_WORDS;
     const int n_live = min(QW, p.n_streams - blockIdx.x * QW);    // warps of this CTA that have a frame
     const int F = WALK ? p.n_frames : 1;
     for (int f = 0; f < F; f++) {
@@ -1724,8 +1725,9 @@ constexpr size_t QUANTIZE_SMEM = QW * QUANTIZE_WARP_BYTES;
 cudaError_t prepare_enc_quant(const EncoderState& st) {
     cudaError_t e = cudaFuncSetAttribute(enc_sns_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SHAPE_SMEM / QW * SNS_WARPS));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_tns_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SHAPE_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess)
         e = cudaFuncSetAttribute(enc_bs_prepare_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)(QW * bitstream_warp_bytes(st.cfg.ne, st.max_nbytes, nullptr)));
@@ -1733,7 +1735,7 @@ cudaError_t prepare_enc_quant(const EncoderState& st) {
 }
 
 void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
-                    int n_frames) {
+                    int n_frames, const int32_t* ids) {
     QuantParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
@@ -1752,6 +1754,7 @@ void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_ou
     p.bs_words = st.bs_words;
     p.inline_ac = 0;
     p.frames_out = frames_out;
+    p.ids = ids;
     const size_t wbytes = bitstream_warp_bytes(st.cfg.ne, nbytes, &p);
     const int grid = (p.n_streams + QW - 1) / QW;
     if (stages & 1) plan.add(enc_sns_kernel, (unsigned)((p.n_streams + SNS_WARPS - 1) / SNS_WARPS), SNS_WARPS * 32, SHAPE_SMEM / QW * SNS_WARPS, p);
@@ -1760,8 +1763,8 @@ void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_ou
         QuantParams pw = p;
         pw.n_streams = st.n_streams / n_frames;
         pw.n_frames = n_frames;
-        plan.add(n_frames > 1 ? enc_quantize_kernel<true> : enc_quantize_kernel<false>, (unsigned)((pw.n_streams + QW - 1) / QW),
-                 QNT_THREADS, QUANTIZE_SMEM, pw);
+        plan.add(n_frames > 1 ? enc_quantize_kernel<true, false> : ids ? enc_quantize_kernel<false, true> : enc_quantize_kernel<false, false>,
+                 (unsigned)((pw.n_streams + QW - 1) / QW), QNT_THREADS, QUANTIZE_SMEM, pw);
     }
     if (stages & 8) {
         plan.add(enc_bs_prepare_kernel, (unsigned)grid, QNT_THREADS, QW * wbytes, p);

@@ -1,7 +1,33 @@
 // lc3b engine: the opaque handle types of the C ABI (include/lc3b.h), shared by the translation units that implement it.
 #pragma once
+#include <vector>
+
 #include "lc3b_common.cuh"
 #include "lc3b_plan.cuh"
+
+namespace lc3b {
+// The host-side id list of a subset call (lc3b_decode_frames_subset and friends): every id in [0, n_streams) and none
+// listed twice.  A stream is marked with the call's epoch, so a check is O(n) and the marks are never cleared (except
+// when the epoch wraps).  The accepted list is kept in `ids`, a pageable copy: cudaMemcpyAsync has consumed a pageable
+// source by the time it returns, so the caller's array is only read during the call even when it is pinned.
+struct IdList {
+    std::vector<uint32_t> mark;
+    std::vector<int32_t> ids;
+    uint32_t epoch = 0;
+    bool take(const int32_t* in, int n, int n_streams) {
+        if ((int)mark.size() != n_streams) mark.assign((size_t)n_streams, 0u);
+        if (++epoch == 0) { mark.assign((size_t)n_streams, 0u); epoch = 1; }
+        ids.resize((size_t)n);
+        for (int i = 0; i < n; i++) {
+            const int32_t s = in[i];
+            if (s < 0 || s >= n_streams || mark[(size_t)s] == epoch) return false;
+            mark[(size_t)s] = epoch;
+            ids[(size_t)i] = s;
+        }
+        return true;
+    }
+};
+}  // namespace lc3b
 
 struct lc3b_decoder {
     lc3b::DecoderState st{};
@@ -19,6 +45,7 @@ struct lc3b_decoder {
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t compute_done[2] = {nullptr, nullptr}, d2h_done[2] = {nullptr, nullptr};
     bool d2h_pending[2] = {false, false};
+    lc3b::IdList id_list;                 // subset calls and resets (lc3b_decode_frames_subset, lc3b_decoder_reset_streams)
 };
 
 namespace lc3b {

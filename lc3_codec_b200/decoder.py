@@ -5,6 +5,8 @@ Reference                                   here
 Lc3Decoder::calc_working_buffer_lengths     Lc3BatchDecoder.calc_working_buffer_lengths  (bytes of device workspace)
 Lc3Decoder::new(num_channels, ..bufs)       Lc3BatchDecoder(num_streams, .., workspace)  (caller-owned torch buffer)
 decode_frame(bits, channel, buf_in, out)    decode_frames(bits, frames, pcm_out, ..)     one frame for EVERY stream
+  the same for some channels only           decode_frames_subset(bits, stream_ids, ..)   one frame for each listed stream
+fresh channel state (Lc3Decoder::new)       reset_streams(stream_ids)                    for the listed streams only
 Err(Only16BitsPerAudioSampleSupported)      raises Lc3DecoderError("Only16BitsPerAudioSampleSupported")
 panic on bad channel index / slice length   raises Lc3bError(LC3B_ERR_INVALID_ARG)
 bitstream errors -> concealment, Ok(())     same; optional `status_out` exposes which streams were concealed
@@ -79,22 +81,42 @@ class Lc3BatchDecoder:
         self._call(native.lib().lc3b_decode_frames_host, False, num_bits_per_audio_sample, frames, pcm_out,
                    frame_nbytes, nbytes, status_out)
 
-    def _call(self, fn, want_cuda, bits, frames, pcm_out, frame_nbytes, nbytes, status_out):
+    def decode_frames_subset(self, num_bits_per_audio_sample: int, stream_ids, frames: torch.Tensor, pcm_out: torch.Tensor,
+                             frame_nbytes: torch.Tensor | None = None, nbytes: int | None = None,
+                             status_out: torch.Tensor | None = None) -> None:
+        """decode_frame for the listed streams only; every other stream is untouched (include/lc3b.h).
+        stream_ids: host ids (sequence, numpy array or CPU int32 tensor), any order, each at most once; row i of frames,
+        pcm_out, frame_nbytes and status_out (CUDA tensors with n_rows = len(stream_ids) rows) belongs to stream_ids[i]."""
+        self._call(native.lib().lc3b_decode_frames_subset, True, num_bits_per_audio_sample, frames, pcm_out, frame_nbytes,
+                   nbytes, status_out, native.host_ids(stream_ids))
+
+    def reset_streams(self, stream_ids) -> None:
+        """Give the listed streams the state a freshly initialised decoder has; no other stream is touched."""
+        ids = native.host_ids(stream_ids)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = native.lib().lc3b_decoder_reset_streams(self._h, C.c_void_p(ids.ctypes.data), ids.size, C.c_void_p(stream))
+        if rc:
+            raise Lc3bError(rc, "lc3b_decoder_reset_streams")
+
+    def _call(self, fn, want_cuda, bits, frames, pcm_out, frame_nbytes, nbytes, status_out, ids=None):
         if bits != 16:
             raise Lc3DecoderError("Only16BitsPerAudioSampleSupported")
+        rows = self.num_streams if ids is None else ids.size
         for t, dt, what in ((frames, torch.uint8, "frames"), (pcm_out, torch.int16, "pcm_out")):
-            if t.is_cuda != want_cuda or t.dtype != dt or t.dim() != 2 or t.shape[0] != self.num_streams or t.stride(1) != 1:
+            if t.is_cuda != want_cuda or t.dtype != dt or t.dim() != 2 or t.shape[0] != rows or t.stride(1) != 1:
                 raise Lc3bError(2, f"{what}: wrong device/dtype/shape")
         if pcm_out.shape[1] < self.nf:
             raise Lc3bError(2, f"pcm_out: {pcm_out.shape[1]} samples per stream, need nf = {self.nf}")
         for t, what in ((frame_nbytes, "frame_nbytes"), (status_out, "status_out")):
-            if t is not None and (t.is_cuda != want_cuda or t.dtype != torch.int32 or t.numel() != self.num_streams
+            if t is not None and (t.is_cuda != want_cuda or t.dtype != torch.int32 or t.numel() != rows
                                   or not t.is_contiguous()):
                 raise Lc3bError(2, f"{what}: wrong device/dtype/shape")
         nb = frames.shape[1] if nbytes is None else nbytes
+        head = () if ids is None else (C.c_void_p(ids.ctypes.data), ids.size)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         with torch.cuda.device(self.device):
-            rc = fn(self._h, bits, _ptr(frames), _ptr(frame_nbytes), nb, frames.stride(0), _ptr(pcm_out),
+            rc = fn(self._h, bits, *head, _ptr(frames), _ptr(frame_nbytes), nb, frames.stride(0), _ptr(pcm_out),
                     pcm_out.stride(0), _ptr(status_out), C.c_void_p(stream))
         if rc == 1:
             raise Lc3DecoderError("Only16BitsPerAudioSampleSupported")

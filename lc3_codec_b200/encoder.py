@@ -5,6 +5,8 @@ Reference                                   here
 Lc3Encoder::calc_working_buffer_lengths     Lc3BatchEncoder.calc_working_buffer_lengths  (bytes of device workspace)
 Lc3Encoder::new(num_channels, ..bufs)       Lc3BatchEncoder(num_streams, .., workspace)
 encode_frame(channel, samples_in, buf_out)  encode_frames(pcm_in, frames_out)            one frame for EVERY stream
+  the same for some channels only           encode_frames_subset(stream_ids, ..)         one frame for each listed stream
+fresh channel state (Lc3Encoder::new)       reset_streams(stream_ids)                    for the listed streams only
 Result<(), Lc3EncoderError> (empty enum)    returns None; cannot fail for valid shapes
 assert_eq!(samples_in.len(), nf) panics     raises Lc3bError(LC3B_ERR_INVALID_ARG)
 Lc3Encoder::new panics at 8 kHz             raises Lc3bError(LC3B_ERR_INVALID_ARG)
@@ -64,15 +66,32 @@ class Lc3BatchEncoder:
     def encode_frames_host(self, pcm_in: torch.Tensor, frames_out: torch.Tensor) -> None:
         self._call(native.lib().lc3b_encode_frames_host, False, pcm_in, frames_out)
 
-    def _call(self, fn, want_cuda, pcm_in, frames_out):
+    def encode_frames_subset(self, stream_ids, pcm_in: torch.Tensor, frames_out: torch.Tensor) -> None:
+        """encode_frame for the listed streams only; every other stream is untouched (include/lc3b.h).
+        stream_ids: host ids (sequence, numpy array or CPU int32 tensor), any order, each at most once; row i of pcm_in
+        and frames_out (CUDA tensors with n_rows = len(stream_ids) rows) belongs to stream_ids[i]."""
+        self._call(native.lib().lc3b_encode_frames_subset, True, pcm_in, frames_out, native.host_ids(stream_ids))
+
+    def reset_streams(self, stream_ids) -> None:
+        """Give the listed streams the state a freshly initialised encoder has; no other stream is touched."""
+        ids = native.host_ids(stream_ids)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = native.lib().lc3b_encoder_reset_streams(self._h, C.c_void_p(ids.ctypes.data), ids.size, C.c_void_p(stream))
+        if rc:
+            raise Lc3bError(rc, "lc3b_encoder_reset_streams")
+
+    def _call(self, fn, want_cuda, pcm_in, frames_out, ids=None):
+        rows = self.num_streams if ids is None else ids.size
         for t, dt, what in ((pcm_in, torch.int16, "pcm_in"), (frames_out, torch.uint8, "frames_out")):
-            if t.is_cuda != want_cuda or t.dtype != dt or t.dim() != 2 or t.shape[0] != self.num_streams or t.stride(1) != 1:
+            if t.is_cuda != want_cuda or t.dtype != dt or t.dim() != 2 or t.shape[0] != rows or t.stride(1) != 1:
                 raise Lc3bError(2, f"{what}: wrong device/dtype/shape")
         if pcm_in.shape[1] != self.nf:
             raise Lc3bError(2, f"pcm_in: {pcm_in.shape[1]} samples per stream, need nf = {self.nf}")
+        head = () if ids is None else (C.c_void_p(ids.ctypes.data), ids.size)
         stream = torch.cuda.current_stream(self.device).cuda_stream
         with torch.cuda.device(self.device):
-            rc = fn(self._h, _ptr(pcm_in), pcm_in.stride(0), _ptr(frames_out), frames_out.shape[1], frames_out.stride(0),
+            rc = fn(self._h, *head, _ptr(pcm_in), pcm_in.stride(0), _ptr(frames_out), frames_out.shape[1], frames_out.stride(0),
                     C.c_void_p(stream))
         if rc:
             raise Lc3bError(rc, fn.__name__)

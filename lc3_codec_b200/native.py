@@ -5,6 +5,8 @@ import ctypes as C
 import enum
 from pathlib import Path
 
+import numpy as np
+
 _HERE = Path(__file__).resolve().parent
 _SO = _HERE / "liblc3b.so"
 
@@ -65,7 +67,8 @@ EXPORTS = ["lc3b_config_new", "lc3b_last_cuda_error", "lc3b_version", "lc3b_deco
            "lc3b_sharded_decode_frames_host", "lc3b_sharded_decoder_wait", "lc3b_sharded_decoder_set_min_nbytes", "lc3b_sharded_decoder_destroy",
            "lc3b_sharded_encoder_create", "lc3b_sharded_encoder_n_shards", "lc3b_sharded_encoder_shard",
            "lc3b_sharded_encode_frames_host", "lc3b_sharded_encoder_wait", "lc3b_sharded_encoder_destroy",
-           "lc3b_host_alloc", "lc3b_host_free"]
+           "lc3b_host_alloc", "lc3b_host_free",
+           "lc3b_decode_frames_subset", "lc3b_decoder_reset_streams", "lc3b_encode_frames_subset", "lc3b_encoder_reset_streams"]
 
 
 class MixedBucket(C.Structure):             # lc3b_mixed_bucket
@@ -100,6 +103,8 @@ def lib() -> C.CDLL:
         L.lc3b_decoder_host_fence.argtypes = [vp, vp]
         L.lc3b_decoder_multi_scratch_bytes.argtypes = [vp, i32, C.POINTER(C.c_size_t)]
         L.lc3b_decode_stream_frames.argtypes = [vp, i32, vp, vp, i32, sz, i32, vp, vp, vp, sz, vp]
+        L.lc3b_decode_frames_subset.argtypes = [vp, i32, vp, i32, vp, vp, i32, sz, vp, sz, vp, vp]
+        L.lc3b_decoder_reset_streams.argtypes = [vp, vp, i32, vp]
         L.lc3b_decoder_destroy.argtypes = [vp]
         L.lc3b_decoder_destroy.restype = None
         L.lc3b_encoder_workspace_bytes.argtypes = [i32, i32, i32, i32, C.POINTER(sz)]
@@ -108,6 +113,8 @@ def lib() -> C.CDLL:
         L.lc3b_encode_frames_host.argtypes = [vp, vp, sz, vp, i32, sz, vp]
         L.lc3b_encoder_multi_scratch_bytes.argtypes = [vp, i32, C.POINTER(sz)]
         L.lc3b_encode_stream_frames.argtypes = [vp, vp, i32, vp, i32, sz, vp, sz, vp]
+        L.lc3b_encode_frames_subset.argtypes = [vp, vp, i32, vp, sz, vp, i32, sz, vp]
+        L.lc3b_encoder_reset_streams.argtypes = [vp, vp, i32, vp]
         L.lc3b_encoder_debug_read.argtypes = [vp, vp, vp, vp, vp, vp]
         L.lc3b_encoder_set_stage_mask.argtypes = [vp, i32]
         L.lc3b_encoder_set_host_pipelining.argtypes = [vp, i32]
@@ -149,6 +156,21 @@ def lib() -> C.CDLL:
         L.lc3b_selftest_math_device.argtypes = [i32, vp, vp, vp, i32, vp]
         _lib = L
     return _lib
+
+
+def host_ids(stream_ids) -> np.ndarray:
+    """A subset call's id list (a sequence, a numpy array or a CPU int32 tensor) as a contiguous host int32 array.
+    Range and uniqueness are checked by the library."""
+    if hasattr(stream_ids, "is_cuda"):                 # a torch tensor
+        if stream_ids.is_cuda or str(stream_ids.dtype) != "torch.int32" or stream_ids.dim() != 1:
+            raise Lc3bError(2, "stream_ids: want a 1-D CPU int32 tensor")
+        stream_ids = stream_ids.contiguous().numpy()
+    a = np.asarray(stream_ids)
+    if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
+        raise Lc3bError(2, "stream_ids: want a 1-D sequence of integers")
+    if a.size and (int(a.min()) < -2**31 or int(a.max()) >= 2**31):
+        raise Lc3bError(2, "stream_ids: ids beyond int32")
+    return np.ascontiguousarray(a, dtype=np.int32)
 
 
 def config(sampling_frequency: int, frame_duration: int) -> Config:

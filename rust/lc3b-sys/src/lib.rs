@@ -80,6 +80,13 @@ extern "C" {
     pub fn lc3b_decode_frames_host(h: *mut lc3b_decoder, bits_per_sample: c_int, frames: *const u8,
                                    frame_nbytes: *const i32, nbytes: c_int, frame_stride: usize, pcm_out: *mut i16,
                                    pcm_stride: usize, status_out: *mut i32, cuda_stream: *mut c_void) -> c_int;
+    /// one `decode_frame` for each listed stream (`stream_ids`: host, `n_rows` distinct ids), device buffers by call row
+    pub fn lc3b_decode_frames_subset(h: *mut lc3b_decoder, bits_per_sample: c_int, stream_ids: *const i32, n_rows: c_int,
+                                     frames: *const u8, frame_nbytes: *const i32, nbytes: c_int, frame_stride: usize,
+                                     pcm_out: *mut i16, pcm_stride: usize, status_out: *mut i32,
+                                     cuda_stream: *mut c_void) -> c_int;
+    /// the listed streams get the state `lc3b_decoder_init` gives a stream
+    pub fn lc3b_decoder_reset_streams(h: *mut lc3b_decoder, stream_ids: *const i32, n: c_int, cuda_stream: *mut c_void) -> c_int;
     pub fn lc3b_decoder_set_host_pipelining(h: *mut lc3b_decoder, on: c_int) -> c_int;
     pub fn lc3b_decoder_host_fence(h: *mut lc3b_decoder, cuda_stream: *mut c_void) -> c_int;
     /// the frame loop of examples/decode.rs:85-123 as one call: `n_frames` frames of every stream (time-parallel)
@@ -164,6 +171,12 @@ extern "C" {
     /// same, host buffers
     pub fn lc3b_encode_frames_host(h: *mut lc3b_encoder, pcm_in: *const i16, pcm_stride: usize, frames_out: *mut u8,
                                    nbytes: c_int, frame_stride: usize, cuda_stream: *mut c_void) -> c_int;
+    /// one `encode_frame` for each listed stream (`stream_ids`: host, `n_rows` distinct ids), device buffers by call row
+    pub fn lc3b_encode_frames_subset(h: *mut lc3b_encoder, stream_ids: *const i32, n_rows: c_int, pcm_in: *const i16,
+                                     pcm_stride: usize, frames_out: *mut u8, nbytes: c_int, frame_stride: usize,
+                                     cuda_stream: *mut c_void) -> c_int;
+    /// the listed streams get the state `lc3b_encoder_init` gives a stream
+    pub fn lc3b_encoder_reset_streams(h: *mut lc3b_encoder, stream_ids: *const i32, n: c_int, cuda_stream: *mut c_void) -> c_int;
     pub fn lc3b_encoder_set_host_pipelining(h: *mut lc3b_encoder, on: c_int) -> c_int;
     /// the frame loop of examples/encode.rs:73-116 as one call: `n_frames` frames of every stream (time-parallel)
     pub fn lc3b_encoder_multi_scratch_bytes(h: *const lc3b_encoder, n_frames: c_int, device_bytes: *mut usize) -> c_int;

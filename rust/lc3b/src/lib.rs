@@ -130,6 +130,30 @@ impl<'a> Lc3BatchDecoder<'a> {
         }
     }
 
+    /// `decode_frame` (:217) for the listed streams only; every other stream is untouched.  Row i of the device buffers
+    /// (`frames`, `samples_out`, `frame_nbytes`) belongs to stream `stream_ids[i]`: ids in `0..num_streams`, none twice
+    /// (a bad list panics, like the reference's bad `channel_index`, :228).  `stream_ids` is only read during the call.
+    ///
+    /// # Safety
+    /// As for `decode_frames`, with `stream_ids.len()` rows in device memory.
+    pub unsafe fn decode_frames_subset(&mut self, num_bits_per_audio_sample: usize, stream_ids: &[i32], frames: *const u8,
+                                       frame_nbytes: *const i32, nbytes: usize, stride: usize, samples_out: *mut i16)
+                                       -> Result<(), Lc3DecoderError> {
+        match sys::lc3b_decode_frames_subset(self.h, num_bits_per_audio_sample as i32, stream_ids.as_ptr(), stream_ids.len() as i32,
+                                             frames, frame_nbytes, nbytes as i32, stride, samples_out, self.nf, ptr::null_mut(),
+                                             self.stream) {
+            sys::LC3B_OK => Ok(()),
+            sys::LC3B_ERR_BITS_PER_SAMPLE => Err(Lc3DecoderError::Only16BitsPerAudioSampleSupported),
+            rc => { check(rc, "lc3b_decode_frames_subset"); unreachable!() }
+        }
+    }
+
+    /// The listed streams start over with the state `Lc3Decoder::new` gives a channel; no other stream is touched.
+    pub fn reset_streams(&mut self, stream_ids: &[i32]) {
+        check(unsafe { sys::lc3b_decoder_reset_streams(self.h, stream_ids.as_ptr(), stream_ids.len() as i32, self.stream) },
+              "lc3b_decoder_reset_streams");
+    }
+
     /// Bytes of caller-owned device scratch `decode_stream_frames` needs for `n_frames` frames per stream.
     pub fn multi_scratch_bytes(&self, n_frames: usize) -> usize {
         let mut n = 0usize;
@@ -224,6 +248,24 @@ impl<'a> Lc3BatchEncoder<'a> {
         };
         check(f(self.h, samples_in, self.nf, buf_out, nbytes as i32, stride, self.stream), "lc3b_encode_frames");
         Ok(())
+    }
+
+    /// `encode_frame` (:175) for the listed streams only: row i of the device buffers belongs to stream `stream_ids[i]`
+    /// (ids in `0..num_streams`, none twice; only read during the call).
+    ///
+    /// # Safety
+    /// As for `encode_frames`, with `stream_ids.len()` rows in device memory.
+    pub unsafe fn encode_frames_subset(&mut self, stream_ids: &[i32], samples_in: *const i16, buf_out: *mut u8, nbytes: usize,
+                                       stride: usize) -> Result<(), Lc3EncoderError> {
+        check(sys::lc3b_encode_frames_subset(self.h, stream_ids.as_ptr(), stream_ids.len() as i32, samples_in, self.nf, buf_out,
+                                             nbytes as i32, stride, self.stream), "lc3b_encode_frames_subset");
+        Ok(())
+    }
+
+    /// The listed streams start over with the state `Lc3Encoder::new` gives a channel; no other stream is touched.
+    pub fn reset_streams(&mut self, stream_ids: &[i32]) {
+        check(unsafe { sys::lc3b_encoder_reset_streams(self.h, stream_ids.as_ptr(), stream_ids.len() as i32, self.stream) },
+              "lc3b_encoder_reset_streams");
     }
 
     /// Bytes of caller-owned device scratch `encode_stream_frames` needs for `n_frames` frames per stream.
