@@ -1,4 +1,4 @@
-// lc3b engine, decoder kernels 2 and 3: shaped spectrum -> PCM, one WARP per frame.
+// lc3b engine, decoder kernels 2 and 3: shaped spectrum -> PCM, one WARP per frame (two at nf = 480, large batches).
 //
 // Replaces, per stream, the second half of DecoderChannel::decode (src/decoder/lc3_decoder.rs:134-153):
 //   PacketLossConcealment::save / load_into   src/decoder/packet_loss_concealment.rs:50,63
@@ -13,8 +13,9 @@
 // constant), overlap-add, and the post filter's PASS-THROUGH case: x_hat goes to the LTPF history ring and, rounded, to
 // the PCM row.  Two consecutive samples per lane, so PCM leaves as 32-bit and f32 state as 64-bit accesses; all global
 // traffic is stream-major and coalesced (spectrum 4*ne B in, overlap memory 4*(nf-z) B in/out, LTPF history 4*nf B
-// out, PCM 2*nf B out).  synth_kernel<NF, MS10> is the same work as a persistent kernel with TMA prefetch, the measured
-// alternative (lc3b_decoder_set_synth_mode).
+// out, PCM 2*nf B out).  synth_pair_kernel<480, true> is the same work with two frames per warp and the FFT in registers
+// (large batches at 48 / 44.1 kHz, 10 ms).  synth_kernel<NF, MS10> is the same work as a persistent kernel with TMA
+// prefetch, the measured alternative (lc3b_decoder_set_synth_mode).
 // ltpf_kernel (streams whose post filter is, or was in the previous frame, active): the IIR itself; for those streams
 // the synthesis kernel leaves x_hat in a side buffer (the ring block keeps the samples long pitch lags still reach), and
 // this kernel writes the filtered signal to the ring block and the PCM row.  Streams outside such a span cost this
@@ -67,103 +68,155 @@ static inline size_t synth_smem_bytes(int nf) { return (size_t)PIPE_WARPS * 3 * 
 // 262 144, and MORE resident warps make it slower (8 / 10 / 12 CTAs per SM: 0.502 / 0.516 / 0.529 ms - the twiddle and
 // window tables share L1 with the shared-memory carve-out).  The per-frame streams (spectrum, overlap memory, PCM)
 // therefore use evict-first loads and stores, which leaves L1 to the tables (0.517 -> 0.500 ms).
-template <int NF, bool MS10, bool IDS>
-__global__ void __launch_bounds__(SYN_WARPS * 32) synth_classic_kernel(const __grid_constant__ SynthParams p) {
+//
+// synth_pair_kernel: the same work with two frames per warp (rows 2w and 2w + 1), at 48 / 44.1 kHz, 10 ms (nf = 480)
+// only.  The two frames are transformed together by dct_iv_pair, one per half warp: the FFT stays in registers but for
+// one exchange through shared memory, and every table load and shared-memory instruction of the transform serves both
+// frames (per frame: 45 -> 23 shared loads, 43 -> 23.5 shared stores, 36 -> 26.5 table loads).  Everything else
+// (spectrum load, concealment, unfold, overlap-add, history, PCM) runs one frame at a time on the whole warp.  A pair
+// warp is a longer serial chain than a single-frame warp, so small launches, which are latency bound, keep
+// synth_classic_kernel (the row threshold is in PlanSynth::add).
+template <int NF>
+constexpr bool synth_pairs() { return NF == 480; }
+constexpr int SYN_PAIR_CTAS = 5;      // CTAs per SM the pair kernel is compiled for (96 registers; 4 CTAs at 104: 0.400 ms, 5: 0.358)
+
+// One warp's FPW frames: the body of both kernels.
+template <int NF, bool MS10, bool IDS, int FPW>
+__device__ __forceinline__ void synth_frames(const SynthParams& p) {
     using G = FrameGeo<NF, MS10>;
     constexpr int NE = G::NE, Z = G::Z, NP = G::NP, NPT = G::NPT;
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int row = blockIdx.x * SYN_WARPS + wid;
-    if (row >= p.n_streams) return;                               // warps are independent: no CTA-wide barrier below
-    const int stream = state_row<IDS>(p.ids, row);                // persistent rows; PCM goes to the call's row
+    const int row0 = (blockIdx.x * SYN_WARPS + wid) * FPW;
+    if (row0 >= p.n_streams) return;                              // warps are independent: no CTA-wide barrier below
 
-    float* P = (float*)smem + (size_t)wid * 2 * NF;               // spectrum in; FFT ping
-    float* Q = P + NF;                                            // FFT pong
+    // per frame f of the warp: P = spectrum in, FFT ping (and the output of dct_iv_pair); Q = FFT pong / exchange
+    float* const W = (float*)smem + (size_t)wid * FPW * 2 * NF;
+    auto P = [&](int f) { return W + f * NF; };
+    auto Q = [&](int f) { return W + (FPW + f) * NF; };
 
-    int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
-    int32_t* ss = p.sstate + (size_t)stream * SS_WORDS;
-    // the two records as 16-byte loads (every lane reads the same words; each load is one slot of the memory pipe)
-    static_assert(SD_OK == 0 && SD_LTPF_ACTIVE == 1 && SD_SLOT == 6 && SS_PLC_LOST == 1 && SS_PLC_ALPHA == 2 && SS_LTPF_PREV == 4 && SS_LTPF_BLK == 7,
-                  "record layout");
-    const int4 sd_a = ((const int4*)sd)[0], sd_b = ((const int4*)sd)[1];
-    const int4 ss_a = ((const int4*)ss)[0], ss_b = ((const int4*)ss)[1];
-    const int ok = sd_a.x;
-    const int slot = sd_b.z;
-    const int active = sd_a.y;
-    const int prev_active = ltpf_prev_active(ss_b.x);
-    const int blk_idx = ss_b.w;
-    const float* sp = p.spec + ((size_t)slot * p.slot_streams + stream) * NE;
-
-    // overlap memory: requested now, consumed after the FFT
-    float* ola = p.ola + (size_t)stream * (NF - Z);
-    float2 ola_r[NPT];
+    // what a frame needs after the transform
+    int stream[FPW], active[FPW], prev_active[FPW], blk_idx[FPW];
+    int32_t *sd[FPW], *ss[FPW];
+    float* ola[FPW];
+    float2 ola_r[FPW][NPT];
 #pragma unroll
-    for (int j = 0; j < NPT; j++)
-        ola_r[j] = (64 * j + 64 <= NF - Z || 64 * j + 2 * lane < NF - Z) ? __ldcs((const float2*)ola + 32 * j + lane) : make_float2(0.0f, 0.0f);
+    for (int f = 0; f < FPW; f++) {
+        if (f > 0 && row0 + f >= p.n_streams) break;              // an odd row count: the last warp has one frame
+        const int s = stream[f] = state_row<IDS>(p.ids, row0 + f);   // persistent rows; PCM goes to the call's row
+        sd[f] = p.side + (size_t)s * SIDE_WORDS;
+        ss[f] = p.sstate + (size_t)s * SS_WORDS;
+        // the two records as 16-byte loads (every lane reads the same words; each load is one slot of the memory pipe)
+        static_assert(SD_OK == 0 && SD_LTPF_ACTIVE == 1 && SD_SLOT == 6 && SS_PLC_LOST == 1 && SS_PLC_ALPHA == 2 && SS_LTPF_PREV == 4 &&
+                          SS_LTPF_BLK == 7,
+                      "record layout");
+        const int4 sd_a = ((const int4*)sd[f])[0], sd_b = ((const int4*)sd[f])[1];
+        const int4 ss_a = ((const int4*)ss[f])[0], ss_b = ((const int4*)ss[f])[1];
+        const int ok = sd_a.x;
+        const int slot = sd_b.z;
+        active[f] = sd_a.y;
+        prev_active[f] = ltpf_prev_active(ss_b.x);
+        blk_idx[f] = ss_b.w;
+        const float* sp = p.spec + ((size_t)slot * p.slot_streams + s) * NE;
 
-    // ---- spectrum load, with concealment (packet_loss_concealment.rs:63-85) when the frame was bad
-    if (ok) {
+        // overlap memory: requested now, consumed after the FFT
+        ola[f] = p.ola + (size_t)s * (NF - Z);
 #pragma unroll
-        for (int k0 = 0; k0 < NF / 4; k0 += 32) {
-            const int k4 = k0 + lane;
-            if (k0 + 32 <= NF / 4 || k4 < NF / 4)
-                ((float4*)P)[k4] = 4 * k4 < NE ? __ldcs((const float4*)sp + k4) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+        for (int j = 0; j < NPT; j++)
+            ola_r[f][j] = (64 * j + 64 <= NF - Z || 64 * j + 2 * lane < NF - Z) ? __ldcs((const float2*)ola[f] + 32 * j + lane) : make_float2(0.0f, 0.0f);
+
+        // ---- spectrum load, with concealment (packet_loss_concealment.rs:63-85) when the frame was bad
+        if (ok) {
+#pragma unroll
+            for (int k0 = 0; k0 < NF / 4; k0 += 32) {
+                const int k4 = k0 + lane;
+                if (k0 + 32 <= NF / 4 || k4 < NF / 4)
+                    ((float4*)P(f))[k4] = 4 * k4 < NE ? __ldcs((const float4*)sp + k4) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            }
+            if (lane == 0 && (ss_a.y != 0 || ss_a.z != (int32_t)f2u(1.0f))) { ss[f][SS_PLC_LOST] = 0; ss[f][SS_PLC_ALPHA] = (int32_t)f2u(1.0f); }
+        } else {
+            const int lost = ss_a.y;
+            float alpha = u2f((uint32_t)ss_a.z);
+            __syncwarp();                                        // every lane has read the state before any lane updates it
+            alpha = plc_fade(alpha, lost);
+            plc_scramble<NF, NE>(P(f), sp, alpha, (uint32_t)ss_a.w, lane, ss[f] + SS_PLC_SEED);
+            if (lane == 0) { ss[f][SS_PLC_LOST] = lost + 1; ss[f][SS_PLC_ALPHA] = (int32_t)f2u(alpha); }
         }
-        if (lane == 0 && (ss_a.y != 0 || ss_a.z != (int32_t)f2u(1.0f))) { ss[SS_PLC_LOST] = 0; ss[SS_PLC_ALPHA] = (int32_t)f2u(1.0f); }
-    } else {
-        const int lost = ss_a.y;
-        float alpha = u2f((uint32_t)ss_a.z);
-        __syncwarp();                                            // every lane has read the state before any lane updates it
-        alpha = plc_fade(alpha, lost);
-        plc_scramble<NF, NE>(P, sp, alpha, (uint32_t)ss_a.w, lane, ss + SS_PLC_SEED);
-        if (lane == 0) { ss[SS_PLC_LOST] = lost + 1; ss[SS_PLC_ALPHA] = (int32_t)f2u(alpha); }
     }
     __syncwarp();
 
-    // ---- DCT-IV, unfold, window (dct_iv.rs:49-67, modified_dct.rs:97-136)
-    const float* D = dct_iv_warp<NF>(P, Q, p.dtw, p.ftw, lane);
-    float head[2 * NP], tail[2 * NPT];
-    imdct_unfold<NF, MS10>(D, p.win, lane, head, tail);
+    // ---- DCT-IV (dct_iv.rs:49-67)
+    const float* D0;                                              // where frame 0's coefficients are (frame 1's: in P(1))
+    if constexpr (FPW == 2) {
+        const int h = lane >> 4;
+        dct_iv_pair<NF>(P(h), (float2*)Q(h), p.dtw, p.ftw, lane & 15, h == 1, row0 + h < p.n_streams);
+        D0 = P(0);
+    } else D0 = dct_iv_warp<NF>(P(0), Q(0), p.dtw, p.ftw, lane);
 
-    // ---- overlap-add (modified_dct.rs:138-151): two roundings, like the reference (and the time-parallel path)
 #pragma unroll
-    for (int j = 0; j < NPT; j++) {
-        if (64 * j + 64 <= NF - Z || 64 * j + 2 * lane < NF - Z) {
-            head[2 * j] = xa(ola_r[j].x, head[2 * j]);
-            head[2 * j + 1] = xa(ola_r[j].y, head[2 * j + 1]);
-            __stcs((float2*)ola + 32 * j + lane, make_float2(tail[2 * j], tail[2 * j + 1]));
-        }
-    }
+    for (int f = 0; f < FPW; f++) {
+        if (f > 0 && row0 + f >= p.n_streams) break;
+        const int s = stream[f];
+        // with two frames the per-stream pointers are derived again rather than held through the transform (registers)
+        float* const ola_f = FPW == 1 ? ola[f] : p.ola + (size_t)s * (NF - Z);
+        int32_t* const sd_f = FPW == 1 ? sd[f] : p.side + (size_t)s * SIDE_WORDS;
+        int32_t* const ss_f = FPW == 1 ? ss[f] : p.sstate + (size_t)s * SS_WORDS;
+        // ---- unfold, window (modified_dct.rs:97-136)
+        float head[2 * NP], tail[2 * NPT];
+        imdct_unfold<NF, MS10>(f == 0 ? D0 : P(f), p.win, lane, head, tail);
 
-    // ---- post filter, pass-through case (long_term_post_filter.rs:252-343 with zero coefficients): history + PCM
-    // Inside an active span the ring block must keep its old content until the filter has run (long pitch lags reach
-    // around the ring into it), so x_hat waits in a side buffer for ltpf_kernel instead.
-    const bool in_span = active || prev_active;
-    float* yblk = in_span ? p.ltpf_x + (size_t)stream * NF : p.ltpf_y + (size_t)stream * p.hist_len + blk_idx * NF;
-    float* xtail = p.ltpf_xtail + (size_t)stream * XTAIL_FLOATS + blk_idx * 16;
-    int16_t* out = p.pcm_out + (size_t)row * p.pcm_stride;
+        // ---- overlap-add (modified_dct.rs:138-151): two roundings, like the reference (and the time-parallel path)
 #pragma unroll
-    for (int j = 0; j < NP; j++) {
-        const int n = 64 * j + 2 * lane;
-        if (64 * j + 64 <= NF || n < NF) {
-            const float a = head[2 * j], b = head[2 * j + 1];
-            if (!p.no_ltpf) {
-                ((float2*)yblk)[32 * j + lane] = make_float2(a, b);
-                if (n >= NF - 16) ((float2*)xtail)[(n - (NF - 16)) >> 1] = make_float2(a, b);   // x_hat tail for the next frame's filter
+        for (int j = 0; j < NPT; j++) {
+            if (64 * j + 64 <= NF - Z || 64 * j + 2 * lane < NF - Z) {
+                head[2 * j] = xa(ola_r[f][j].x, head[2 * j]);
+                head[2 * j + 1] = xa(ola_r[f][j].y, head[2 * j + 1]);
+                __stcs((float2*)ola_f + 32 * j + lane, make_float2(tail[2 * j], tail[2 * j + 1]));
             }
-            const int32_t qa = round_pcm_i32(a), qb = round_pcm_i32(b);
-            if (p.pcm_pairs) __stcs((uint32_t*)out + 32 * j + lane, ((uint32_t)qa & 0xffffu) | ((uint32_t)qb << 16));
-            else { out[n] = (int16_t)qa; out[n + 1] = (int16_t)qb; }
         }
-    }
-    if (lane == 0 && !p.no_ltpf) {
-        sd[SD_BLK] = blk_idx;
-        int nb = blk_idx + 1;                                    // :334-337
-        if (nb > (MS10 ? 1 : 2)) nb = 0;
-        ss[SS_LTPF_BLK] = nb;
-        if (!in_span) ltpf_store_prev(ss, LtpfPar{});            // otherwise ltpf_kernel carries the filter state on
+
+        // ---- post filter, pass-through case (long_term_post_filter.rs:252-343 with zero coefficients): history + PCM
+        // Inside an active span the ring block must keep its old content until the filter has run (long pitch lags reach
+        // around the ring into it), so x_hat waits in a side buffer for ltpf_kernel instead.
+        const bool in_span = active[f] || prev_active[f];
+        const int blk = blk_idx[f];
+        float* yblk = in_span ? p.ltpf_x + (size_t)s * NF : p.ltpf_y + (size_t)s * p.hist_len + blk * NF;
+        float* xtail = p.ltpf_xtail + (size_t)s * XTAIL_FLOATS + blk * 16;
+        int16_t* out = p.pcm_out + (size_t)(row0 + f) * p.pcm_stride;
+#pragma unroll
+        for (int j = 0; j < NP; j++) {
+            const int n = 64 * j + 2 * lane;
+            if (64 * j + 64 <= NF || n < NF) {
+                const float a = head[2 * j], b = head[2 * j + 1];
+                if (!p.no_ltpf) {
+                    ((float2*)yblk)[32 * j + lane] = make_float2(a, b);
+                    if (n >= NF - 16) ((float2*)xtail)[(n - (NF - 16)) >> 1] = make_float2(a, b);   // x_hat tail for the next frame's filter
+                }
+                const int32_t qa = round_pcm_i32(a), qb = round_pcm_i32(b);
+                if (p.pcm_pairs) __stcs((uint32_t*)out + 32 * j + lane, ((uint32_t)qa & 0xffffu) | ((uint32_t)qb << 16));
+                else { out[n] = (int16_t)qa; out[n + 1] = (int16_t)qb; }
+            }
+        }
+        if (lane == 0 && !p.no_ltpf) {
+            sd_f[SD_BLK] = blk;
+            int nb = blk + 1;                                    // :334-337
+            if (nb > (MS10 ? 1 : 2)) nb = 0;
+            ss_f[SS_LTPF_BLK] = nb;
+            if (!in_span) ltpf_store_prev(ss_f, LtpfPar{});     // otherwise ltpf_kernel carries the filter state on
+        }
     }
 }
+
+template <int NF, bool MS10, bool IDS>
+__global__ void __launch_bounds__(SYN_WARPS * 32) synth_classic_kernel(const __grid_constant__ SynthParams p) {
+    synth_frames<NF, MS10, IDS, 1>(p);
+}
+template <int NF, bool MS10, bool IDS>
+__global__ void __launch_bounds__(SYN_WARPS * 32, SYN_PAIR_CTAS) synth_pair_kernel(const __grid_constant__ SynthParams p) {
+    synth_frames<NF, MS10, IDS, 2>(p);
+}
+// shared memory of both kernels: per warp two nf-float buffers per frame
+constexpr int synth_warp_smem_bytes(int nf, int fpw) { return SYN_WARPS * fpw * 2 * nf * 4; }
 
 
 // ---- 1-D bulk copies global -> shared through the TMA unit, completion on an mbarrier (PTX cp.async.bulk, sm_90+)
@@ -429,8 +482,12 @@ struct PrepareSynth {
     template <int NF, bool MS10> void operator()() {
         e = cudaFuncSetAttribute(synth_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)synth_smem_bytes(NF));
         if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)synth_smem_bytes(NF));
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYN_WARPS * 2 * NF * 4);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SYN_WARPS * 2 * NF * 4);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 1));
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 1));
+        if constexpr (synth_pairs<NF>()) {
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_pair_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 2));
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_pair_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 2));
+        }
     }
 };
 struct PlanSynth {
@@ -444,9 +501,18 @@ struct PlanSynth {
     }
     template <int NF, bool MS10, bool IDS> void add() {
         // persistent: at most as many CTAs as fit on the device at once (4 of 8 warps per SM by registers; shared memory may allow fewer)
-        const int full = (p.n_streams + SYN_WARPS - 1) / SYN_WARPS;
         if (!pipelined) {
-            node = plan.add(synth_classic_kernel<NF, MS10, IDS>, (unsigned)full, SYN_WARPS * 32, SYN_WARPS * 2 * NF * 4, p, dep);
+            if constexpr (synth_pairs<NF>()) {
+                // two frames per warp once the launch fills every SM with pair warps twice over; below that the launch is
+                // latency bound and one frame per warp, twice the warps, finishes sooner
+                if (p.n_streams >= 2 * sm_count * SYN_PAIR_CTAS * SYN_WARPS * 2) {
+                    node = plan.add(synth_pair_kernel<NF, MS10, IDS>, (unsigned)((p.n_streams + 2 * SYN_WARPS - 1) / (2 * SYN_WARPS)), SYN_WARPS * 32,
+                                    synth_warp_smem_bytes(NF, 2), p, dep);
+                    return;
+                }
+            }
+            node = plan.add(synth_classic_kernel<NF, MS10, IDS>, (unsigned)((p.n_streams + SYN_WARPS - 1) / SYN_WARPS), SYN_WARPS * 32,
+                            synth_warp_smem_bytes(NF, 1), p, dep);
             return;
         }
         const size_t smem = synth_smem_bytes(NF);

@@ -9,7 +9,8 @@
 // is straight-line code: the pre-twiddle is folded into the first stage (which needs no FFT twiddles) and the
 // post-twiddle into the last.  It uses another factor order than kissfft: the PCM contract is +-1 LSB, not bit
 // equality.  All products are written with explicit fma/mul intrinsics so that the frame-by-frame kernel and the
-// time-parallel kernel, which both instantiate this header, produce identical bits.
+// time-parallel kernel, which both instantiate this header, produce identical bits.  dct_iv_pair computes the same
+// butterflies for two frames per warp with all stages in registers and one shared-memory exchange (bit-identical too).
 //
 // The unfolded, windowed 2*nf samples leave in registers, two consecutive samples per lane and step:
 //   head[n] = t[z + n]      * w[z + n]        n in [0, nf)      (added to the overlap memory / output)
@@ -143,6 +144,57 @@ __device__ __forceinline__ void stages(float* P, float* Q, const float2* __restr
     }
 }
 
+// ---- The same FFT with every stage in registers but one exchange through shared memory (dct_iv_pair below).
+// With G = r0 * r1 and L = N / G, the Stockham index maps of stage<> split into two register-resident halves:
+//  * pass A, stages 0 and 1, lane a < L: stage 1's butterflies j = r0 * a + k (k < r0) read the outputs of stage 0's
+//    butterflies a + L * t (t < r1), so the lane runs those r1 butterflies, then the r0 butterflies of stage 1 on the
+//    values it holds; its G outputs are the contiguous positions G * a ... G * a + G - 1;
+//  * pass B, stages 2 .. n - 1, lane k < G: every later stage reads and writes only positions = k (mod G) (all its
+//    strides and butterfly counts are multiples of G), so the lane gathers "column" k (positions G * m + k, m < L) and
+//    runs the remaining stages on it as a Stockham FFT of L points whose twiddle index carries the column.
+// Every butterfly sees the inputs, twiddle and dft<R> / cmul sequence of stage<>: the output is bit-identical.
+template <int N>
+struct RegFftPlan {
+    using Plan = FftPlan<N>;
+    static constexpr int R0 = Plan::r(0), R1 = Plan::r(1), G = R0 * R1, L = N / G;
+    static constexpr bool half_warp = Plan::n >= 3 && G <= 16 && L <= 16;   // one frame fits half a warp in both passes
+};
+
+// Pass B from stage S on: x[m] is position G * m + k, NSM = (stage S's NS) / G.  The last stage applies the DCT-IV
+// post-twiddle and scatters into yr.  `odd` (the warp's second frame) swaps the order of the two scatter stores, so
+// that one store instruction writes even words for one frame and odd words for the other: no bank conflicts.
+template <int NF, int S, int NSM>
+__device__ __forceinline__ void column_stages(const float2 (&x)[RegFftPlan<NF / 2>::L], float* __restrict__ yr, const float2* __restrict__ dtw,
+                                              const float2* __restrict__ ftw, int k, bool odd) {
+    using Plan = FftPlan<NF / 2>;
+    constexpr int N = NF / 2, G = RegFftPlan<N>::G, L = RegFftPlan<N>::L, R = Plan::r(S), NBF = L / R, TW = N / (G * NSM * R);
+    constexpr bool last = S == Plan::n - 1;
+    float2 y[L];
+#pragma unroll
+    for (int jm = 0; jm < NBF; jm++) {
+        const int km = jm % NSM;
+        float2 v[R];
+#pragma unroll
+        for (int t = 0; t < R; t++) {
+            v[t] = x[jm + t * NBF];
+            if (t > 0) v[t] = cmul(v[t], ftw[(G * km + k) * t * TW]);
+        }
+        dft<R>(v);
+#pragma unroll
+        for (int t = 0; t < R; t++) {
+            const int m = (jm - km) * R + km + t * NSM;
+            if constexpr (last) {
+                const int o = G * m + k;
+                const float2 w = cmul(dtw[o], v[t]);
+                const float re = __fmul_rn(w.x, 2.0f), im = __fmul_rn(w.y, -2.0f);
+                yr[odd ? NF - 1 - 2 * o : 2 * o] = odd ? im : re;
+                yr[odd ? 2 * o : NF - 1 - 2 * o] = odd ? re : im;
+            } else y[m] = v[t];
+        }
+    }
+    if constexpr (!last) column_stages<NF, S + 1, NSM * R>(y, yr, dtw, ftw, k, odd);
+}
+
 }  // namespace imdct_detail
 
 // DCT-IV of the nf floats in P (spectrum, zero padded beyond ne); P and Q are nf floats each (8-byte aligned).
@@ -151,6 +203,58 @@ template <int NF>
 __device__ __forceinline__ float* dct_iv_warp(float* P, float* Q, const float2* __restrict__ dtw, const float2* __restrict__ ftw, int lane) {
     imdct_detail::stages<NF, 0, 1>(P, Q, dtw, ftw, lane);
     return (FftPlan<NF / 2>::n & 1) ? Q : P;
+}
+
+// DCT-IV of two frames per warp, one per half warp, bit-identical to dct_iv_warp: passes A and B above with a single
+// exchange through X in between.  Per half: P = the frame's nf floats (spectrum in, the nf output coefficients out, in
+// place), X = nf floats of exchange space, l = lane within the half, odd = second half, live = the half has a frame.
+// Every lane of the warp must call it (it synchronises the warp).  Per frame and pass A lane: 2 G shared loads, G
+// pre-twiddle loads, one shared store per position; per pass B lane: L shared loads, L post-twiddle loads, 2 L stores.
+template <int NF>
+__device__ __forceinline__ void dct_iv_pair(float* __restrict__ P, float2* __restrict__ X, const float2* __restrict__ dtw,
+                                            const float2* __restrict__ ftw, int l, bool odd, bool live) {
+    using namespace imdct_detail;
+    using RP = RegFftPlan<NF / 2>;
+    constexpr int N = NF / 2, R0 = RP::R0, R1 = RP::R1, G = RP::G, L = RP::L;
+    static_assert(RP::half_warp, "both passes must fit half a warp");
+    if (live && l < L) {
+        float2 u[G];                                                  // stage 0 outputs, u[R0 * t1 + t0]
+#pragma unroll
+        for (int t1 = 0; t1 < R1; t1++) {
+            float2 v[R0];
+#pragma unroll
+            for (int t0 = 0; t0 < R0; t0++) {
+                // stage 0 butterfly l + L * t1, input t0: z[n] = dtw[n] * (x[2n] + i x[nf-1-2n]); the second half
+                // loads the pair in the other order (even words for one frame, odd for the other: no bank conflicts)
+                const int n = l + L * t1 + (N / R0) * t0;
+                const float a = P[odd ? NF - 1 - 2 * n : 2 * n], b = P[odd ? 2 * n : NF - 1 - 2 * n];
+                v[t0] = cmul(dtw[n], make_float2(odd ? b : a, odd ? a : b));
+            }
+            dft<R0>(v);
+#pragma unroll
+            for (int t0 = 0; t0 < R0; t0++) u[R0 * t1 + t0] = v[t0];
+        }
+#pragma unroll
+        for (int k1 = 0; k1 < R0; k1++) {                             // stage 1 butterfly R0 * l + k1
+            float2 v[R1];
+#pragma unroll
+            for (int t1 = 0; t1 < R1; t1++) {
+                v[t1] = u[R0 * t1 + k1];
+                if (t1 > 0) v[t1] = cmul(v[t1], ftw[k1 * t1 * L]);
+            }
+            dft<R1>(v);
+#pragma unroll
+            for (int t1 = 0; t1 < R1; t1++) X[G * l + k1 + R0 * t1] = v[t1];
+        }
+    }
+    __syncwarp();
+    if (live && l < G) {
+        float2 x[L];
+#pragma unroll
+        for (int m = 0; m < L; m++) x[m] = X[G * m + l];
+        column_stages<NF, 2, 1>(x, P, dtw, ftw, l, odd);
+    }
+    __syncwarp();
 }
 
 // Unfold (modified_dct.rs:97-136) and window: D holds the DCT-IV output; win[m] = gain * w[2nf-1-m].
