@@ -156,9 +156,9 @@ int lc3b_decoder_set_split(lc3b_decoder* h, int k);
  * keeps the promise; a non-empty frame shorter than min_nbytes is treated as a lost frame (concealed), and a call whose
  * fixed `nbytes` is below it returns LC3B_ERR_INVALID_ARG.  Set it before the first decode. */
 int lc3b_decoder_set_min_nbytes(lc3b_decoder* h, int min_nbytes);
-/* Which synthesis (IMDCT + overlap-add) kernel runs: 0 = one warp per frame, ordinary loads (default); 1 = persistent
- * warps that fetch the next frame's spectrum with the TMA unit (cp.async.bulk + mbarrier) while transforming the current
- * one.  Bit-identical results; 0 measured 3.5 % faster at 262 144 streams (the kernel is issue bound, DESIGN.md). */
+/* Which synthesis (IMDCT + overlap-add) kernel runs: 0 = by launch size (default: two frames per warp for large
+ * 48 / 44.1 kHz 10 ms launches, one frame per warp otherwise); 1 = always one frame per warp.  Bit-identical results;
+ * the choice only matters for speed. */
 int lc3b_decoder_set_synth_mode(lc3b_decoder* h, int mode);
 /* Which dequantisation kernel runs: 0 = by batch size (default: one warp per frame up to 12 288 streams, one thread per
  * frame above), 1 = warp per frame, 2 = thread per frame.  Bit-identical results; the choice only matters for speed. */

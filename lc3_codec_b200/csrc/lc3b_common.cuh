@@ -39,7 +39,7 @@ enum {
     SD_PLC_ALPHA,       // f32 bits: alpha to apply (concealed frames)
     SD_SLOT,            // which of the two spectrum slots holds the spectrum to transform
     SD_SRC,             // time-parallel path: unit whose spectrum to transform (-2 own, -1 the handle's last good slot)
-    SD_BLK,             // LTPF ring block synth_kernel wrote this frame's x_hat to (synth_kernel -> ltpf_kernel)
+    SD_BLK,             // LTPF ring block of this frame's x_hat (synthesis kernel -> ltpf_kernel)
 };
 constexpr int XTAIL_FLOATS = 3 * 16;   // per stream: last 16 samples of x_hat of the frame in each ring block
 
@@ -79,8 +79,8 @@ struct DecoderState {
     int fixed_slot;      // -1: double-buffered spectrum slots tracked in sstate; >= 0: always write that slot (time-parallel path)
     int no_ltpf;         // 1: every frame the handle accepts is too long for the post filter to be active (gain row (0.0, 0))
     int min_nbytes;      // promised minimum frame length (0 = none), lc3b_decoder_set_min_nbytes
-    int sm_count;        // multiprocessors of the handle's device (persistent kernels size their grids with it)
-    int synth_mode;      // 0 one warp per frame with ordinary loads (default), 1 persistent warps + TMA prefetch (lc3b_decoder_set_synth_mode)
+    int sm_count;        // multiprocessors of the handle's device (the launch size from which synthesis takes two frames per warp)
+    int synth_mode;      // 0 synthesis kernel by launch size (default), 1 one frame per warp always (lc3b_decoder_set_synth_mode)
     int dequant_mode;    // 0 auto, 1 warp-per-frame dequantisation kernel, 2 thread-per-frame (lc3b_decoder_set_dequant_mode)
     // device pointers (carved from the caller's workspace)
     DevConfig* dcfg;

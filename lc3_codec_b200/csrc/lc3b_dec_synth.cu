@@ -14,13 +14,12 @@
 // the PCM row.  Two consecutive samples per lane, so PCM leaves as 32-bit and f32 state as 64-bit accesses; all global
 // traffic is stream-major and coalesced (spectrum 4*ne B in, overlap memory 4*(nf-z) B in/out, LTPF history 4*nf B
 // out, PCM 2*nf B out).  synth_pair_kernel<480, true> is the same work with two frames per warp and the FFT in registers
-// (large batches at 48 / 44.1 kHz, 10 ms).  synth_kernel<NF, MS10> is the same work as a persistent kernel with TMA
-// prefetch, the measured alternative (lc3b_decoder_set_synth_mode).
+// (large batches at 48 / 44.1 kHz, 10 ms); synth mode 1 (lc3b_decoder_set_synth_mode) keeps synth_classic_kernel there
+// too.  Both give the same bits.
 // ltpf_kernel (streams whose post filter is, or was in the previous frame, active): the IIR itself; for those streams
 // the synthesis kernel leaves x_hat in a side buffer (the ring block keeps the samples long pitch lags still reach), and
 // this kernel writes the filtered signal to the ring block and the PCM row.  Streams outside such a span cost this
 // kernel one flag load.
-#include <stdlib.h>
 #include <string.h>
 
 #include "lc3b_common.cuh"
@@ -56,18 +55,15 @@ struct SynthParams {
 };
 
 constexpr int SYN_WARPS = 4;
-constexpr int PIPE_WARPS = 8;    // warps per CTA of the persistent synthesis kernel (they share the CTA's copy of the tables)
-// per warp: two stage buffers + one pong buffer of nf floats and two mbarriers; per CTA: DCT-IV and FFT twiddles (nf/2 float2
-// each) and the window (2 nf floats reserved)
-static inline size_t synth_smem_bytes(int nf) { return (size_t)PIPE_WARPS * 3 * nf * 4 + (size_t)4 * nf * 4 + (size_t)PIPE_WARPS * 2 * 8; }
 
-// synth_classic_kernel: one warp = one frame, spectrum through ordinary loads.  The default: at 262 144 streams it runs in
-// 0.50 ms against 0.525 ms for the persistent TMA-pipelined kernel below (profiles/r2_synth_ab.json).  What bounds it is
-// the SM's L1 / shared-memory data path, not instruction issue, DRAM or latency: dropping a quarter of its instructions
-// (the float -> int casts) changed nothing, the time per frame is the same at 16 384 streams (everything in L2) as at
-// 262 144, and MORE resident warps make it slower (8 / 10 / 12 CTAs per SM: 0.502 / 0.516 / 0.529 ms - the twiddle and
-// window tables share L1 with the shared-memory carve-out).  The per-frame streams (spectrum, overlap memory, PCM)
-// therefore use evict-first loads and stores, which leaves L1 to the tables (0.517 -> 0.500 ms).
+// synth_classic_kernel: one warp = one frame, spectrum through ordinary loads.  What bounds it is the SM's L1 /
+// shared-memory data path, not instruction issue, DRAM or latency: dropping a quarter of its instructions (the float ->
+// int casts) changed nothing, the time per frame is the same at 16 384 streams (everything in L2) as at 262 144, MORE
+// resident warps make it slower (8 / 10 / 12 CTAs per SM: 0.502 / 0.516 / 0.529 ms - the twiddle and window tables share
+// L1 with the shared-memory carve-out), and a persistent variant that prefetched the next frame's spectrum with the TMA
+// unit was slower still (0.525 against 0.50 ms at 262 144 streams, profiles/r2_synth_ab.json, DESIGN.md §3).  The
+// per-frame streams (spectrum, overlap memory, PCM) therefore use evict-first loads and stores, which leaves L1 to the
+// tables (0.517 -> 0.500 ms).
 //
 // synth_pair_kernel: the same work with two frames per warp (rows 2w and 2w + 1), at 48 / 44.1 kHz, 10 ms (nf = 480)
 // only.  The two frames are transformed together by dct_iv_pair, one per half warp: the FFT stays in registers but for
@@ -218,209 +214,6 @@ __global__ void __launch_bounds__(SYN_WARPS * 32, SYN_PAIR_CTAS) synth_pair_kern
 // shared memory of both kernels: per warp two nf-float buffers per frame
 constexpr int synth_warp_smem_bytes(int nf, int fpw) { return SYN_WARPS * fpw * 2 * nf * 4; }
 
-
-// ---- 1-D bulk copies global -> shared through the TMA unit, completion on an mbarrier (PTX cp.async.bulk, sm_90+)
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, uint32_t bytes, uint64_t* bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(dst_smem)),
-                 "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "LC3B_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra LC3B_DONE;\n"
-        "bra LC3B_WAIT;\n"
-        "LC3B_DONE:\n"
-        "}\n" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-// generic-proxy accesses of a buffer are ordered before the async-proxy (TMA) writes issued afterwards
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-
-// What the kernel needs to know about a frame before it can fetch its spectrum: a handful of words per stream.
-struct FrameHead {
-    int ok, slot, active, prev_active, blk_idx;
-};
-template <bool IDS>
-__device__ __forceinline__ FrameHead load_head(const SynthParams& p, int row) {
-    const int stream = state_row<IDS>(p.ids, row);
-    const int32_t* sd = p.side + (size_t)stream * SIDE_WORDS;
-    const int32_t* ss = p.sstate + (size_t)stream * SS_WORDS;
-    FrameHead h;
-    h.ok = sd[SD_OK];
-    h.slot = sd[SD_SLOT];
-    h.active = sd[SD_LTPF_ACTIVE];
-    h.prev_active = ltpf_prev_active(ss[SS_LTPF_PREV]);
-    h.blk_idx = ss[SS_LTPF_BLK];
-    return h;
-}
-
-// synth_kernel: PERSISTENT, one warp per frame at a time.  A warp walks the frames w, w + W, w + 2W, ... (W = warps in
-// the grid); while it transforms frame i the TMA unit already fetches the spectrum of frame i + 1 into the warp's other
-// stage buffer (cp.async.bulk + mbarrier: no registers, no issue slots), and the side words of frame i + 2 are on
-// their way, so a warp never waits for HBM latency once it is running.  Per warp: two stage buffers of nf floats (the
-// spectrum arrives in the first ne, the rest stays zero; the stage buffer then serves as the FFT's ping buffer) and
-// one pong buffer.
-// Subset calls (IDS): `stream` walks the call's rows; the state and the spectrum are read at the row's handle stream.
-template <int NF, bool MS10, bool IDS>
-__global__ void __launch_bounds__(PIPE_WARPS * 32, 4) synth_kernel(const __grid_constant__ SynthParams p) {
-    using G = FrameGeo<NF, MS10>;
-    constexpr int NE = G::NE, Z = G::Z, NP = G::NP, NPT = G::NPT, N = NF / 2;
-    extern __shared__ __align__(16) uint8_t smem[];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int n_warps = gridDim.x * PIPE_WARPS;
-    int stream = blockIdx.x * PIPE_WARPS + wid;
-
-    // the CTA's copy of the transform tables: a persistent CTA pays for it once and every later access is a shared-memory load
-    float2* s_dtw = (float2*)((float*)smem + (size_t)PIPE_WARPS * 3 * NF);
-    float2* s_ftw = s_dtw + N;
-    float* s_win = (float*)(s_ftw + N);                           // win[Z .. 2 NF): the part the unfold reads, indexed from 0
-    for (int i = threadIdx.x; i < N; i += PIPE_WARPS * 32) { s_dtw[i] = p.dtw[i]; s_ftw[i] = p.ftw[i]; }
-    for (int i = threadIdx.x; i < 2 * NF - Z; i += PIPE_WARPS * 32) s_win[i] = p.win[Z + i];
-    __syncthreads();
-    if (stream >= p.n_streams) return;                            // warps are independent from here on: no CTA-wide barrier below
-
-    float* S0 = (float*)smem + (size_t)wid * 3 * NF;              // stage buffers (spectrum in; FFT ping)
-    float* Q = S0 + 2 * NF;                                       // FFT pong
-    uint64_t* bars = (uint64_t*)(s_win + 2 * NF) + 2 * wid;
-    if (lane == 0) { mbar_init(&bars[0], 1); mbar_init(&bars[1], 1); }
-    for (int k = lane; k < 2 * NF; k += 32) S0[k] = 0.0f;         // the zero padding beyond ne (both stages)
-    __syncwarp();
-    fence_proxy_async();
-
-    auto fetch = [&](int st, int s, const FrameHead& h) {         // spectrum of stream s -> stage st
-        if (lane == 0) {
-            const float* sp = p.spec + ((size_t)h.slot * p.slot_streams + s) * NE;
-            mbar_expect_tx(&bars[st], NE * 4);
-            bulk_g2s(S0 + st * NF, sp, NE * 4, &bars[st]);
-        }
-    };
-    FrameHead head = load_head<IDS>(p, stream);
-    fetch(0, state_row<IDS>(p.ids, stream), head);
-    int nstream = stream + n_warps;
-    FrameHead nhead = head;
-    if (nstream < p.n_streams) nhead = load_head<IDS>(p, nstream);
-    uint32_t phase0 = 0, phase1 = 0;
-
-    for (int it = 0; stream < p.n_streams; it++) {
-        const int st = it & 1;
-        float* P = S0 + st * NF;
-        // ---- next frame: its spectrum starts moving now, the side words of the one after are requested
-        const int n2stream = nstream + n_warps;
-        FrameHead n2head = nhead;
-        if (nstream < p.n_streams) {
-            // the other stage buffer was this warp's FFT ping buffer one frame ago: restore its zero tail, then hand it to the TMA
-            float* O = S0 + (st ^ 1) * NF;
-            if (it > 0) {
-                for (int k = NE + lane; k < NF; k += 32) O[k] = 0.0f;
-                __syncwarp();
-                fence_proxy_async();
-            }
-            fetch(st ^ 1, state_row<IDS>(p.ids, nstream), nhead);
-            if (n2stream < p.n_streams) n2head = load_head<IDS>(p, n2stream);
-        }
-
-        const int srow = state_row<IDS>(p.ids, stream);
-        int32_t* sd = p.side + (size_t)srow * SIDE_WORDS;
-        int32_t* ss = p.sstate + (size_t)srow * SS_WORDS;
-        const int ok = head.ok, active = head.active, prev_active = head.prev_active, blk_idx = head.blk_idx;
-
-        // overlap memory: requested now, consumed after the FFT
-        float* ola = p.ola + (size_t)srow * (NF - Z);
-        float2 ola_r[NPT];
-#pragma unroll
-        for (int j = 0; j < NPT; j++)
-            ola_r[j] = (64 * j + 64 <= NF - Z || 64 * j + 2 * lane < NF - Z) ? ((const float2*)ola)[32 * j + lane] : make_float2(0.0f, 0.0f);
-
-        // ---- the spectrum has landed in P; concealment (packet_loss_concealment.rs:63-85) when the frame was bad
-        mbar_wait(&bars[st], st ? phase1 : phase0);
-        if (st) phase1 ^= 1; else phase0 ^= 1;
-        if (ok) {
-            if (lane == 0) { ss[SS_PLC_LOST] = 0; ss[SS_PLC_ALPHA] = (int32_t)f2u(1.0f); }
-        } else {
-            int lost = ss[SS_PLC_LOST];
-            float alpha = u2f((uint32_t)ss[SS_PLC_ALPHA]);
-            uint32_t seed = (uint32_t)ss[SS_PLC_SEED];
-            __syncwarp();                                            // every lane has read the state before any lane updates it
-            alpha = plc_fade(alpha, lost);
-            // plc_scramble's sequence, in place over the first NE lines (the rest of the stage buffer is zero already):
-            // plc_scramble itself, which also rewrites the zero lines, costs synth_kernel<360, 0> a register spill
-            uint32_t s = seed;
-            for (int i = 0; i <= lane; i++) s = plc_lcg(s);
-            const PlcJump j32 = plc_lcg_jump(32);
-            for (int k = lane; k < NE; k += 32) {
-                const float lg = P[k];
-                P[k] = s < 0x8000u ? xm(lg, alpha) : xm(lg, -alpha);
-                if (k == NE - 1) ss[SS_PLC_SEED] = (int32_t)s;
-                s = j32.step(s);
-            }
-            if (lane == 0) { ss[SS_PLC_LOST] = lost + 1; ss[SS_PLC_ALPHA] = (int32_t)f2u(alpha); }
-            __syncwarp();
-        }
-
-        // ---- DCT-IV, unfold, window (dct_iv.rs:49-67, modified_dct.rs:97-136)
-        const float* D = dct_iv_warp<NF>(P, Q, s_dtw, s_ftw, lane);
-        float head_s[2 * NP], tail[2 * NPT];
-        imdct_unfold<NF, MS10>(D, s_win - Z, lane, head_s, tail);
-        __syncwarp();                                                // every lane is done reading P / Q before they are reused
-
-        // ---- overlap-add (modified_dct.rs:138-151): two roundings, like the reference (and the time-parallel path)
-#pragma unroll
-        for (int j = 0; j < NPT; j++) {
-            if (64 * j + 64 <= NF - Z || 64 * j + 2 * lane < NF - Z) {
-                head_s[2 * j] = xa(ola_r[j].x, head_s[2 * j]);
-                head_s[2 * j + 1] = xa(ola_r[j].y, head_s[2 * j + 1]);
-                ((float2*)ola)[32 * j + lane] = make_float2(tail[2 * j], tail[2 * j + 1]);
-            }
-        }
-
-        // ---- post filter, pass-through case (long_term_post_filter.rs:252-343 with zero coefficients): history + PCM
-        // Inside an active span the ring block must keep its old content until the filter has run (long pitch lags reach
-        // around the ring into it), so x_hat waits in a side buffer for ltpf_kernel instead.  When the handle's promised
-        // minimum frame length rules the filter out for good (p.no_ltpf), the history is never read and is not kept.
-        const bool in_span = active || prev_active;
-        float* yblk = in_span ? p.ltpf_x + (size_t)srow * NF : p.ltpf_y + (size_t)srow * p.hist_len + blk_idx * NF;
-        float* xtail = p.ltpf_xtail + (size_t)srow * XTAIL_FLOATS + blk_idx * 16;
-        int16_t* out = p.pcm_out + (size_t)stream * p.pcm_stride;
-#pragma unroll
-        for (int j = 0; j < NP; j++) {
-            const int n = 64 * j + 2 * lane;
-            if (64 * j + 64 <= NF || n < NF) {
-                const float a = head_s[2 * j], b = head_s[2 * j + 1];
-                if (!p.no_ltpf) {
-                    ((float2*)yblk)[32 * j + lane] = make_float2(a, b);
-                    if (n >= NF - 16) ((float2*)xtail)[(n - (NF - 16)) >> 1] = make_float2(a, b);   // x_hat tail for the next frame's filter
-                }
-                const int32_t qa = round_pcm_i32(a), qb = round_pcm_i32(b);
-                if (p.pcm_pairs) ((uint32_t*)out)[32 * j + lane] = ((uint32_t)qa & 0xffffu) | ((uint32_t)qb << 16);
-                else { out[n] = (int16_t)qa; out[n + 1] = (int16_t)qb; }
-            }
-        }
-        if (lane == 0 && !p.no_ltpf) {
-            sd[SD_BLK] = blk_idx;
-            int nb = blk_idx + 1;                                    // :334-337
-            if (nb > (MS10 ? 1 : 2)) nb = 0;
-            ss[SS_LTPF_BLK] = nb;
-            if (!in_span) ltpf_store_prev(ss, LtpfPar{});            // otherwise ltpf_kernel carries the filter state on
-        }
-        stream = nstream;
-        head = nhead;
-        nstream = n2stream;
-        nhead = n2head;
-    }
-}
-
 // ---------------------------------------------------------------- kernel 3: the post filter where it is not idle
 template <bool IDS>
 __global__ void __launch_bounds__(SYN_WARPS * 32) ltpf_kernel(SynthParams p) {
@@ -480,9 +273,7 @@ namespace {
 struct PrepareSynth {
     cudaError_t e = cudaSuccess;
     template <int NF, bool MS10> void operator()() {
-        e = cudaFuncSetAttribute(synth_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)synth_smem_bytes(NF));
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)synth_smem_bytes(NF));
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 1));
+        e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 1));
         if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_classic_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 1));
         if constexpr (synth_pairs<NF>()) {
             if (e == cudaSuccess) e = cudaFuncSetAttribute(synth_pair_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, synth_warp_smem_bytes(NF, 2));
@@ -494,34 +285,23 @@ struct PlanSynth {
     LaunchPlan& plan;
     const SynthParams& p;
     int dep, node, sm_count;
-    bool pipelined;
+    bool single;         // synth mode 1: one frame per warp at every size
     template <int NF, bool MS10> void operator()() {
         if (p.ids) add<NF, MS10, true>();
         else add<NF, MS10, false>();
     }
     template <int NF, bool MS10, bool IDS> void add() {
-        // persistent: at most as many CTAs as fit on the device at once (4 of 8 warps per SM by registers; shared memory may allow fewer)
-        if (!pipelined) {
-            if constexpr (synth_pairs<NF>()) {
-                // two frames per warp once the launch fills every SM with pair warps twice over; below that the launch is
-                // latency bound and one frame per warp, twice the warps, finishes sooner
-                if (p.n_streams >= 2 * sm_count * SYN_PAIR_CTAS * SYN_WARPS * 2) {
-                    node = plan.add(synth_pair_kernel<NF, MS10, IDS>, (unsigned)((p.n_streams + 2 * SYN_WARPS - 1) / (2 * SYN_WARPS)), SYN_WARPS * 32,
-                                    synth_warp_smem_bytes(NF, 2), p, dep);
-                    return;
-                }
+        if constexpr (synth_pairs<NF>()) {
+            // two frames per warp once the launch fills every SM with pair warps twice over; below that the launch is
+            // latency bound and one frame per warp, twice the warps, finishes sooner
+            if (!single && p.n_streams >= 2 * sm_count * SYN_PAIR_CTAS * SYN_WARPS * 2) {
+                node = plan.add(synth_pair_kernel<NF, MS10, IDS>, (unsigned)((p.n_streams + 2 * SYN_WARPS - 1) / (2 * SYN_WARPS)), SYN_WARPS * 32,
+                                synth_warp_smem_bytes(NF, 2), p, dep);
+                return;
             }
-            node = plan.add(synth_classic_kernel<NF, MS10, IDS>, (unsigned)((p.n_streams + SYN_WARPS - 1) / SYN_WARPS), SYN_WARPS * 32,
-                            synth_warp_smem_bytes(NF, 1), p, dep);
-            return;
         }
-        const size_t smem = synth_smem_bytes(NF);
-        int per_sm = (int)((227 * 1024) / (smem + 1024));
-        if (per_sm > 4) per_sm = 4;
-        if (per_sm < 1) per_sm = 1;
-        const int resident = sm_count * per_sm;
-        const int ctas = (p.n_streams + PIPE_WARPS - 1) / PIPE_WARPS;
-        node = plan.add(synth_kernel<NF, MS10, IDS>, (unsigned)(ctas < resident ? ctas : resident), PIPE_WARPS * 32, smem, p, dep);
+        node = plan.add(synth_classic_kernel<NF, MS10, IDS>, (unsigned)((p.n_streams + SYN_WARPS - 1) / SYN_WARPS), SYN_WARPS * 32,
+                        synth_warp_smem_bytes(NF, 1), p, dep);
     }
 };
 }  // namespace
@@ -568,11 +348,8 @@ int plan_synth(LaunchPlan& plan, const DecoderState& st, int16_t* pcm_out, size_
     const size_t lw = ltpf_warp_bytes(st.cfg);
     p.smem_per_warp = (int)lw;
     p.no_ltpf = st.no_ltpf;
-    // which synthesis kernel: 0 = one warp per frame, ordinary loads (default: measured faster, the kernel is issue bound);
-    // 1 = persistent warps with the next frame's spectrum prefetched by the TMA unit (lc3b_decoder_set_synth_mode / LC3B_SYNTH=pipe)
-    static const int env_mode = [] { const char* e = getenv("LC3B_SYNTH"); return !e ? -1 : (e[0] == 'p' ? 1 : 0); }();
-    const int mode = env_mode >= 0 ? env_mode : st.synth_mode;
-    PlanSynth ps{plan, p, dep, -1, st.sm_count > 0 ? st.sm_count : 148, mode == 1};
+    // which synthesis kernel (lc3b_decoder_set_synth_mode): 0 = by launch size (default), 1 = one frame per warp always
+    PlanSynth ps{plan, p, dep, -1, st.sm_count > 0 ? st.sm_count : 148, st.synth_mode == 1};
     if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, ps)) return -1;
     if (st.no_ltpf) return ps.node;                           // the post filter can never be active: nothing to launch
     const int n_warps = (n + group - 1) / group;

@@ -200,7 +200,7 @@ class Lc3BatchDecoder:
             raise Lc3bError(rc, "lc3b_decoder_set_min_nbytes")
 
     def set_synth_mode(self, mode: int) -> None:
-        """0 = synthesis kernel with one warp per frame (default), 1 = persistent warps + TMA prefetch (identical results)."""
+        """0 = synthesis kernel chosen by launch size (default), 1 = one frame per warp always (identical results)."""
         rc = native.lib().lc3b_decoder_set_synth_mode(self._h, mode)
         if rc:
             raise Lc3bError(rc, "lc3b_decoder_set_synth_mode")

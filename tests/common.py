@@ -55,7 +55,7 @@ def gpu_decode(fs, ms, frames, nbytes_per_frame=None, host=False, trace=True, de
     dec.set_dequant_mode(dequant_mode)                  # 0 auto, 1 warp-per-frame kernel, 2 thread-per-frame kernel
     if graph is not None:
         dec.set_graph_mode(graph)
-    dec.set_synth_mode(synth_mode)                      # 0 one warp per frame, 1 persistent + TMA prefetch
+    dec.set_synth_mode(synth_mode)                      # 0 kernel by launch size, 1 one frame per warp always
     if split is not None:
         dec.set_split(split)                            # sub-batches per call (include/lc3b.h)
     if min_nbytes:

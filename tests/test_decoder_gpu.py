@@ -448,27 +448,6 @@ def test_min_nbytes_promise_drops_the_post_filter_history_without_changing_resul
         dec.set_min_nbytes(151)
 
 
-def test_tma_pipelined_synthesis_kernel_is_bit_identical():
-    """lc3b_decoder_set_synth_mode(1): persistent warps, spectrum prefetched with cp.async.bulk + mbarrier.  Same PCM, bit for
-    bit, as the default kernel - small batches (one frame per warp), batches large enough that every warp loops (more than
-    148 x 32 frames), lost frames, LTPF-active streams, with and without the min_nbytes promise."""
-    rng = np.random.default_rng(23)
-    for fs, ms, nb, S, F, promise in ((48000, 10, 150, 61, 10, 0), (16000, 7.5, 30, 200, 16, 0), (48000, 10, 150, 6000, 3, 150),
-                                      (44100, 7.5, 60, 97, 12, 0), (8000, 10, 26, 33, 8, 0)):
-        _, base = corpus(fs, ms, nb, min(S, 128), F)
-        frames = np.tile(base, ((S + base.shape[0] - 1) // base.shape[0], 1, 1))[:S]
-        lens = np.where(rng.random((S, F)) < 0.05, 0, nb).astype(np.int32)
-        a = gpu_decode(fs, ms, frames, lens, trace=False, synth_mode=0, min_nbytes=promise)
-        b = gpu_decode(fs, ms, frames, lens, trace=False, synth_mode=1, min_nbytes=promise)
-        assert np.array_equal(a[0], b[0]) and np.array_equal(a[4], b[4]), (fs, ms, S)
-    _, frames = corpus(48000, 10, 60, 96, 30)
-    assert_parity(48000, 10, frames)            # default kernel vs oracle is covered everywhere; the pipelined one here:
-    g = gpu_decode(48000, 10, frames, trace=False, synth_mode=1)
-    from oracle import pyoracle as O
-    assert np.abs(g[0].astype(np.int32) - O.decode_streams(frames, 48000, 10).astype(np.int32)).max() <= PCM_TOL
-
-
-
 @pytest.mark.parametrize("fs,ms,nbytes,split,graph,host", [
     (48000, 10.0, 150, 4, False, False), (48000, 10.0, 150, 2, True, False), (16000, 7.5, 30, 4, False, True),
     (16000, 7.5, 30, 2, True, True)])

@@ -2,15 +2,16 @@
 
 At nf = 480 (48 and 44.1 kHz, 10 ms) synth mode 0 runs synth_pair_kernel for every launch of at least
 2 x SMs x 5 CTAs x 8 frames rows (80 x SMs; 11 840 on a 148-SM B200): two frames per warp, one per half warp, with the
-FFT's stages in registers.  Synth mode 1 (the persistent kernel) still runs the shared-memory Stockham stages of
-dct_iv_warp.  Both compute every butterfly with the same inputs, twiddles and instruction sequence, so their PCM must be
-identical bit for bit.  Every case below is sized above that threshold, from the device's SM count, and
-test_cases_reach_the_pair_kernel shows with the profiler that they launch synth_pair_kernel.  The cases aim at what the
-pairing can get wrong:
+FFT's stages in registers.  Synth mode 1 runs synth_classic_kernel at every size: one frame per warp, with the
+shared-memory Stockham stages of dct_iv_warp.  Both compute every butterfly with the same inputs, twiddles and
+instruction sequence, so their PCM must be identical bit for bit.  Every case below is sized above that threshold, from
+the device's SM count, and test_cases_reach_the_pair_kernel shows with the profiler that mode 0 launches
+synth_pair_kernel there and mode 1 synth_classic_kernel.  The cases aim at what the pairing can get wrong:
 - odd row counts: the last warp has one frame, and its second half warp has no frame to transform;
 - a good and a concealed frame in one warp;
 - subset calls, the IDS instantiation, whose rows map to streams in random order;
-- split calls: sub-batches of the pair kernel whose last one has an odd row count.
+- split calls: sub-batches of the pair kernel whose last one has an odd row count;
+- streams whose post filter is active (x_hat goes to ltpf_kernel), and the min_nbytes promise that keeps no history.
 """
 import numpy as np
 import pytest
@@ -53,9 +54,10 @@ def _tiled(fs, nb, S, F, seed, lossy=True):
     return frames, lens
 
 
-def _both_modes(fs, frames, lens, **kw):
-    a = gpu_decode(fs, 10, frames, lens, trace=False, synth_mode=0, **kw)
-    b = gpu_decode(fs, 10, frames, lens, trace=False, synth_mode=1, **kw)
+def _both_modes(fs, frames, lens, trace=False, **kw):
+    """Decode with the default kernel choice (pairs above the threshold) and with one frame per warp forced."""
+    a = gpu_decode(fs, 10, frames, lens, trace=trace, synth_mode=0, **kw)
+    b = gpu_decode(fs, 10, frames, lens, trace=trace, synth_mode=1, **kw)
     return a, b
 
 
@@ -86,7 +88,7 @@ def _subset_call(dec, ids, frames, lens):
 
 @pytest.mark.parametrize("fs,nb", GEOMETRIES)
 @pytest.mark.parametrize("extra", [1, 449])
-def test_odd_row_counts_equal_persistent_kernel(fs, nb, extra):
+def test_odd_row_counts_equal_single_frame_kernel(fs, nb, extra):
     """T + 1 and T + 449 rows (T = the pair threshold): the last warp has one frame."""
     S = _pair_min_rows() + extra
     frames, lens = _tiled(fs, nb, S, 4, seed=extra)
@@ -145,6 +147,19 @@ def test_full_size_batch():
     assert np.array_equal(a[4], b[4])
 
 
+@pytest.mark.parametrize("nb,promise", [(60, 0), (150, 150)])
+def test_post_filter_streams_and_the_min_nbytes_promise(nb, promise):
+    """60 B frames and no promise, so the post filter really filters (the synthesis kernel hands x_hat to ltpf_kernel);
+    150 B frames under min_nbytes = 150, where the synthesis kernel keeps no post-filter history."""
+    S = _pair_min_rows() + 1
+    frames, lens = _tiled(48000, nb, S, 8, seed=nb)
+    a, b = _both_modes(48000, frames, lens, trace=promise == 0, min_nbytes=promise)
+    assert np.array_equal(a[0], b[0]), (nb, promise)
+    assert np.array_equal(a[4], b[4])
+    if promise == 0:
+        assert a[1][..., 18].mean() > 0.1                      # LTPF-active frames (trace word 18, as assert_parity reads it)
+
+
 def _synth_kernels(fn):
     """Names of the synthesis kernels fn() launches (torch.profiler sees every kernel of the process)."""
     import torch
@@ -161,17 +176,18 @@ def _synth_kernels(fn):
 
 
 def test_cases_reach_the_pair_kernel():
-    """The sizes above launch synth_pair_kernel (full calls, split calls and subset calls), one row fewer does not."""
+    """The sizes above launch synth_pair_kernel (full calls, split calls and subset calls), one row fewer does not, and
+    synth mode 1 launches synth_classic_kernel at the same sizes: the reference really is the other kernel."""
     import torch
     t = _pair_min_rows()
     n_split, _, _ = _split4_rows(t)
-    for S, split, want in ((t + 1, None, "synth_pair_kernel<480, true, false>"), (n_split, 4, "synth_pair_kernel<480, true, false>"),
-                           (t - 1, None, "synth_classic_kernel")):
+    for S, split, mode, want in ((t + 1, None, 0, "synth_pair_kernel<480, true, false>"), (n_split, 4, 0, "synth_pair_kernel<480, true, false>"),
+                                 (t - 1, None, 0, "synth_classic_kernel"), (t + 1, None, 1, "synth_classic_kernel")):
         frames, lens = _tiled(48000, 150, S, 1, seed=1)
-        dec = _decoder(48000, S, 150, 0, split=split, graph=False)
+        dec = _decoder(48000, S, 150, mode, split=split, graph=False)
         fr, ln = torch.from_numpy(frames[:, 0].copy()).cuda(), torch.from_numpy(lens[:, 0].copy()).cuda()
         out = torch.zeros((S, 480), dtype=torch.int16, device="cuda:0")
-        assert _synth_kernels(lambda: dec.decode_frames(16, fr, out, ln)) == {want}, (S, split)
+        assert _synth_kernels(lambda: dec.decode_frames(16, fr, out, ln)) == {want}, (S, split, mode)
     S = t + 501
     frames, lens = _tiled(48000, 150, S, 1, seed=2)
     dec = _decoder(48000, S, 150, 0, graph=False)

@@ -27,12 +27,9 @@ LC3B_NCU_RANGE=1 LC3B_GRAPH=0 ncu --set full --clock-control none --import-sourc
     python bench.py --workload decode16 --streams 8192 --steps 2 --warmup 3 --quick --no-cpu-baseline > $OUT/${TAG}_small.log 2>&1
 LC3B_NCU_RANGE=1 ncu --set full --clock-control none --import-source on --profile-from-start off -c 6 -o $OUT/${TAG}_multi \
     python bench.py --workload file48 --steps 2 --warmup 3 --no-cpu-baseline > $OUT/${TAG}_multi.log 2>&1
-# the TMA-pipelined synthesis kernel, for the A/B table
-LC3B_NCU_RANGE=1 LC3B_SYNTH=pipe ncu --set full --clock-control none --import-source on --profile-from-start off -k regex:"synth_kernel" -c 1 -o $OUT/${TAG}_synth_pipe \
-    python bench.py --steps 2 --warmup 3 --quick --no-cpu-baseline > $OUT/${TAG}_synth_pipe.log 2>&1
 # summarise on the box and keep the reports out of gpurun_out (64 MiB limit for what travels back)
 mkdir -p /tmp/ncu_reps
-for r in all dec48 small multi synth_pipe; do
+for r in all dec48 small multi; do
   if [ -f $OUT/${TAG}_$r.ncu-rep ]; then
     python tools/ncu_summary.py $OUT/${TAG}_$r.ncu-rep $OUT/${TAG}_${r}_ncu_summary.md $OUT/${TAG}_${r}_ncu_summary.json > /dev/null 2>&1 || echo "summary $r failed"
     : > $OUT/${TAG}_${r}_source_hotspots.txt

@@ -2,14 +2,6 @@
 set -u
 OUT=gpurun_out; mkdir -p $OUT; T=${1:-r2_e}
 timeout 900 python -m pytest tests/test_decoder_gpu.py tests/test_clip200_gpu.py tests/test_multi_frame_gpu.py -m gpu -q -x > $OUT/${T}_pytest.log 2>&1; echo "pytest rc=$?"; tail -4 $OUT/${T}_pytest.log
-for v in pipe classic; do
-  LC3B_SYNTH=$v python bench.py --steps 100 --no-secondary --no-cpu-baseline > $OUT/${T}_bench_decode48_$v.json 2> $OUT/${T}_bench_decode48_$v.err
-  python - <<PY
-import json
-d = json.load(open("$OUT/${T}_bench_decode48_$v.json"))
-print("synth=$v decode48 value", round(d["value"]/1e6,2), "ms/step", round(d["ms_per_step"],4), "e2e", round(d["e2e"]["value"]/1e6,2), {k: round(x,4) for k,x in d["roofline"]["kernels_ms"].items()})
-PY
-done
 LC3B_DEQUANT=warp python bench.py --steps 100 --quick 2>/dev/null | sed 's/^/decode48 warp-dequant: /'
 for s in 2048 8192 16384 32768; do
   for m in warp thread; do
