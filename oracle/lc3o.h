@@ -183,11 +183,29 @@ struct Plc {                   // decoder/packet_loss_concealment.rs:7
     LtpfInfo load_into(float* spec, int n);
 };
 
+// The CUDA engine's inverse MDCT (lc3o_engine_imdct.cpp): its DCT-IV (lc3b_imdct.cuh's Stockham FFT, not kissfft), its
+// unfold and its folded window, tables as the engine builds them.  Opt-in per decoder (TRANSFORM_ENGINE below).
+struct EngineImdct {
+    int nf = 0, z = 0, n_stages = 0, radices[4] = {0, 0, 0, 0};
+    std::vector<Cpx> dtw, ftw;   // DCT-IV pre/post twiddles and FFT twiddles, nf / 2 each
+    std::vector<float> win;      // win[m] = gain * w[2 nf - 1 - m], 2 nf
+    std::vector<float> p, q;     // the two Stockham buffers
+    static bool plan(int n, int* radices, int* count);
+    void init(const Config& c);
+    void dct_iv(float* buf);     // nf floats in place
+    void unfold(const float* D, float* head /*nf*/, float* tail /*nf - z*/) const;
+};
+
+// which inverse transform a decoder runs: the reference's (kissfft DCT-IV, gain then window) or the engine's
+enum { TRANSFORM_REFERENCE = 0, TRANSFORM_ENGINE = 1 };
+
 struct DecMdct {               // decoder/modified_dct.rs:13
     Config cfg{};
     DctIv dct;
+    int transform = TRANSFORM_REFERENCE;
+    EngineImdct eng;
     std::vector<float> mem_ola_add, t_hat;
-    void init(const Config& c);
+    void init(const Config& c, int transform = TRANSFORM_REFERENCE);
     void run(const float* spec, float* freq);
 };
 
@@ -217,7 +235,7 @@ struct DecoderChannel {        // decoder/lc3_decoder.rs:62
     SideInfo last_si{};
     ArithmeticData last_ad{};
     int32_t last_x[400] = {0};
-    void init(SamplingFrequency sf, FrameDuration fd);
+    void init(SamplingFrequency sf, FrameDuration fd, int transform = TRANSFORM_REFERENCE);
     // returns 0, or 1 for Only16BitsPerAudioSampleSupported (lc3_decoder.rs:80)
     int decode(int bits_per_sample, const uint8_t* buf, int64_t len, int16_t* out, int n_out);
 };

@@ -100,6 +100,34 @@ void lc3o_dct_iv(int nf, float* buf) {
     d.run(buf);
 }
 
+// the decoder's MDCT window w_N (2 nf entries, decoder/modified_dct.rs:37-56)
+void lc3o_mdct_window(int sf, int fd, float* out) {
+    Config c = make_config((SamplingFrequency)sf, (FrameDuration)fd);
+    std::memcpy(out, mdct_window(c), sizeof(float) * 2 * c.nf);
+}
+
+// the engine's inverse MDCT pieces (lc3o_engine_imdct.cpp) for the configuration (sf, fd)
+void lc3o_engine_dct_iv(int sf, int fd, float* buf) {
+    EngineImdct e;
+    e.init(make_config((SamplingFrequency)sf, (FrameDuration)fd));
+    e.dct_iv(buf);
+}
+void lc3o_engine_unfold(int sf, int fd, const float* D, float* head, float* tail) {
+    EngineImdct e;
+    e.init(make_config((SamplingFrequency)sf, (FrameDuration)fd));
+    e.unfold(D, head, tail);
+}
+// win [2 nf], dtw and ftw [nf / 2][2]
+void lc3o_engine_tables(int sf, int fd, float* win, float* dtw, float* ftw) {
+    EngineImdct e;
+    e.init(make_config((SamplingFrequency)sf, (FrameDuration)fd));
+    for (int m = 0; m < 2 * e.nf; m++) win[m] = e.win[m];
+    for (int i = 0; i < e.nf / 2; i++) {
+        dtw[2 * i] = e.dtw[i].r; dtw[2 * i + 1] = e.dtw[i].i;
+        ftw[2 * i] = e.ftw[i].r; ftw[2 * i + 1] = e.ftw[i].i;
+    }
+}
+
 // ---------------------------------------------------------------- decoder stages
 int lc3o_read_tail_usize(const uint8_t* buf, int len, int head, int* tail_cursor, int nbits, uint64_t* out) {
     BufferReader r;
@@ -194,6 +222,11 @@ void lc3o_plc_free(void* h) { delete (Plc*)h; }
 
 // decoder MDCT object
 void* lc3o_decmdct_new(int sf, int fd) { DecMdct* m = new DecMdct; m->init(make_config((SamplingFrequency)sf, (FrameDuration)fd)); return m; }
+void* lc3o_decmdct_new_ex(int sf, int fd, int transform) {
+    DecMdct* m = new DecMdct;
+    m->init(make_config((SamplingFrequency)sf, (FrameDuration)fd), transform);
+    return m;
+}
 void lc3o_decmdct_run(void* h, const float* spec, float* freq) { ((DecMdct*)h)->run(spec, freq); }
 void lc3o_decmdct_free(void* h) { delete (DecMdct*)h; }
 
@@ -316,13 +349,15 @@ void lc3o_encode_streams(int nthreads, int n_streams, int n_frames, const int32_
     });
 }
 
-void lc3o_decode_streams(int nthreads, int n_streams, int n_frames, int sf, int fd, const uint8_t* bytes, int nbytes,
-                         const int32_t* nbytes_per_frame /*nullable*/, int16_t* pcm, int32_t* trace /*nullable*/,
-                         int32_t* x_out /*nullable*/, float* spec_out /*nullable: spectrum handed to the IMDCT*/) {
+// transform: TRANSFORM_REFERENCE (the reference's kissfft DCT-IV) or TRANSFORM_ENGINE (the CUDA engine's inverse MDCT)
+void lc3o_decode_streams_ex(int nthreads, int n_streams, int n_frames, int sf, int fd, const uint8_t* bytes, int nbytes,
+                            const int32_t* nbytes_per_frame /*nullable*/, int16_t* pcm, int32_t* trace /*nullable*/,
+                            int32_t* x_out /*nullable*/, float* spec_out /*nullable: spectrum handed to the IMDCT*/,
+                            int transform) {
     Config c = make_config((SamplingFrequency)sf, (FrameDuration)fd);
     parallel_for(nthreads, n_streams, [=](int s) {
         DecoderChannel d;
-        d.init((SamplingFrequency)sf, (FrameDuration)fd);
+        d.init((SamplingFrequency)sf, (FrameDuration)fd, transform);
         for (int f = 0; f < n_frames; f++) {
             size_t fi = (size_t)s * n_frames + f;
             int len = nbytes_per_frame ? nbytes_per_frame[fi] : nbytes;
@@ -331,6 +366,12 @@ void lc3o_decode_streams(int nthreads, int n_streams, int n_frames, int sf, int 
             if (spec_out) std::memcpy(spec_out + fi * c.ne, d.spec.data(), sizeof(float) * c.ne);
         }
     });
+}
+void lc3o_decode_streams(int nthreads, int n_streams, int n_frames, int sf, int fd, const uint8_t* bytes, int nbytes,
+                         const int32_t* nbytes_per_frame /*nullable*/, int16_t* pcm, int32_t* trace /*nullable*/,
+                         int32_t* x_out /*nullable*/, float* spec_out /*nullable: spectrum handed to the IMDCT*/) {
+    lc3o_decode_streams_ex(nthreads, n_streams, n_frames, sf, fd, bytes, nbytes, nbytes_per_frame, pcm, trace, x_out,
+                           spec_out, TRANSFORM_REFERENCE);
 }
 
 }  // extern "C"

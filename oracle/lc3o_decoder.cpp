@@ -546,9 +546,11 @@ LtpfInfo Plc::load_into(float* spec, int n) {                    // :63-85
 }
 
 // ================================================================== modified_dct.rs (decoder)
-void DecMdct::init(const Config& c) {                            // :24-74
+void DecMdct::init(const Config& c, int transform_) {            // :24-74
     cfg = c;
+    transform = transform_;
     dct.init(c.nf);
+    if (transform == TRANSFORM_ENGINE) eng.init(c);
     mem_ola_add.assign(c.nf - c.z, 0.0f);
     t_hat.assign(2 * c.nf, 0.0f);
 }
@@ -556,8 +558,17 @@ void DecMdct::run(const float* spec, float* freq) {              // :76-151
     int nf = cfg.nf, ne = cfg.ne, z = cfg.z, half = nf / 2;
     for (int k = 0; k < ne; k++) freq[k] = spec[k];
     for (int k = ne; k < nf; k++) freq[k] = 0.0f;
-    dct.run(freq);
     float* t = t_hat.data();
+    if (transform == TRANSFORM_ENGINE) {
+        // the engine's DCT-IV, unfold and window; its head / tail are t[z + n] and t[nf + z + n] below
+        eng.dct_iv(freq);
+        eng.unfold(freq, t + z, t + nf + z);
+        for (int n = 0; n < nf - z; n++) freq[n] = mem_ola_add[n] + t[z + n];
+        for (int n = 0; n < nf - z; n++) mem_ola_add[n] = t[nf + z + n];
+        for (int n = 0; n < z; n++) freq[nf - z + n] = t[nf + n];
+        return;
+    }
+    dct.run(freq);
     // apply_mdct_inverse :97-136: t = [y, -rev(y)] rotated left by nf/2, wrapped quarter negated
     for (int n = 0; n < nf; n++) t[n] = freq[n];
     for (int n = 0; n < nf; n++) t[nf + n] = -freq[nf - 1 - n];
@@ -737,12 +748,12 @@ void scale_and_round(const float* x, int n, int16_t* out) {
 }
 
 // ================================================================== lc3_decoder.rs
-void DecoderChannel::init(SamplingFrequency sf, FrameDuration fd) {   // :181-215 (zeroed buffers)
+void DecoderChannel::init(SamplingFrequency sf, FrameDuration fd, int transform) {   // :181-215 (zeroed buffers)
     cfg = make_config(sf, fd);
     spec.assign(cfg.ne, 0.0f);
     freq.assign(cfg.nf, 0.0f);
     plc.init(cfg.ne);
-    mdct.init(cfg);
+    mdct.init(cfg, transform);
     ltpf.init(cfg);
     frame_index = 0;
 }

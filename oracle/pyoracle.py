@@ -50,7 +50,7 @@ def lib() -> C.CDLL:
         _lib.lc3o_powi.restype = C.c_float
         _lib.lc3o_powi.argtypes = [C.c_float, C.c_int]
         for name in ("lc3o_plc_new", "lc3o_decmdct_new", "lc3o_decltpf_new", "lc3o_decoder_new", "lc3o_encmdct_new",
-                     "lc3o_attack_new", "lc3o_encltpf_new", "lc3o_quant_new", "lc3o_encoder_new"):
+                     "lc3o_attack_new", "lc3o_encltpf_new", "lc3o_quant_new", "lc3o_encoder_new", "lc3o_decmdct_new_ex"):
             getattr(_lib, name).restype = C.c_void_p
     return _lib
 
@@ -86,9 +86,16 @@ def encode_streams(pcm: np.ndarray, fs: int, ms: float, nbytes: int, nthreads: i
     return out
 
 
+TRANSFORMS = {"reference": 0, "engine": 1}
+
+
 def decode_streams(frames: np.ndarray, fs: int, ms: float, nbytes_per_frame: np.ndarray | None = None,
-                   nthreads: int | None = None, trace: bool = False):
-    """bytes [n_streams, n_frames, nbytes] u8 -> pcm [n_streams, n_frames, nf] i16 (+ trace, x, spectrum) via the oracle decoder."""
+                   nthreads: int | None = None, trace: bool = False, transform: str = "reference"):
+    """bytes [n_streams, n_frames, nbytes] u8 -> pcm [n_streams, n_frames, nf] i16 (+ trace, x, spectrum) via the oracle decoder.
+
+    transform = "reference": the reference's inverse MDCT (kissfft DCT-IV, then gain, then window).  "engine": the CUDA
+    engine's (its Stockham DCT-IV, unfold and folded window, oracle/lc3o_engine_imdct.cpp); everything else is the
+    oracle's own code, so the engine's PCM must equal this bit for bit."""
     frames = np.ascontiguousarray(frames, np.uint8)
     s, f, nb = frames.shape
     cfg = config(fs, ms)
@@ -97,6 +104,10 @@ def decode_streams(frames: np.ndarray, fs: int, ms: float, nbytes_per_frame: np.
     xo = np.zeros((s, f, cfg["ne"]), np.int32) if trace else None
     sp = np.zeros((s, f, cfg["ne"]), np.float32) if trace else None
     npf = None if nbytes_per_frame is None else np.ascontiguousarray(nbytes_per_frame, np.int32)
-    lib().lc3o_decode_streams(C.c_int(nthreads or ncores()), s, f, SF[fs], FD[ms], p(frames), nb, p(npf), p(pcm), p(tr),
-                              p(xo), p(sp))
+    if transform == "reference":
+        lib().lc3o_decode_streams(C.c_int(nthreads or ncores()), s, f, SF[fs], FD[ms], p(frames), nb, p(npf), p(pcm), p(tr),
+                                  p(xo), p(sp))
+    else:
+        lib().lc3o_decode_streams_ex(C.c_int(nthreads or ncores()), s, f, SF[fs], FD[ms], p(frames), nb, p(npf), p(pcm),
+                                     p(tr), p(xo), p(sp), TRANSFORMS[transform])
     return (pcm, tr, xo, sp) if trace else pcm

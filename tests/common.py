@@ -89,10 +89,27 @@ def gpu_decode(fs, ms, frames, nbytes_per_frame=None, host=False, trace=True, de
     return pcm, tr, xs, sp, status
 
 
+def assert_pcm_matches_oracle(g_pcm, fs, ms, frames, nbytes_per_frame=None, what=""):
+    """The decoder's PCM gates against the oracle on the same bytes: bit exact against the oracle run with the engine's
+    inverse MDCT (oracle/lc3o_engine_imdct.cpp; everything else is the oracle's own code), and within +-1 LSB against the
+    oracle run with the reference's (the two DCT-IVs differ in their last bits, tests/test_engine_transform_cpu.py).
+    g_pcm may be wider than nf.  Returns the reference-transform oracle's PCM."""
+    e_pcm = O.decode_streams(frames, fs, ms, nbytes_per_frame, transform="engine")
+    o_pcm = O.decode_streams(frames, fs, ms, nbytes_per_frame)
+    g = np.asarray(g_pcm)[..., :o_pcm.shape[-1]]
+    bad = np.argwhere(g != e_pcm)
+    assert bad.size == 0, f"{what}: PCM not bit exact against the engine-transform oracle in {len(bad)} samples, first " \
+                          f"(stream, frame, n) {bad[:4].tolist()}: gpu {g[tuple(bad[0])]} oracle {e_pcm[tuple(bad[0])]}"
+    d = np.abs(o_pcm.astype(np.int32) - g.astype(np.int32))
+    assert d.max() <= 1, f"{what}: PCM differs from the reference transform by {d.max()} LSB at {np.argwhere(d > 1)[:4].tolist()}"
+    return o_pcm
+
+
 def assert_parity(fs, ms, frames, nbytes_per_frame=None, host=False, exact_spectrum=True, dequant_mode=0, graph=None,
                   min_nbytes=0, split=None):
-    """The three decoder parity gates of SURVEY.md 8d against the oracle on the same bytes."""
+    """The decoder parity gates of SURVEY.md 8d against the oracle on the same bytes, PCM to the bit."""
     o_pcm, o_tr, o_x, o_sp = O.decode_streams(frames, fs, ms, nbytes_per_frame, trace=True)
+    e_pcm = O.decode_streams(frames, fs, ms, nbytes_per_frame, transform="engine")
     g_pcm, g_tr, g_x, g_sp, g_status = gpu_decode(fs, ms, frames, nbytes_per_frame, host=host, dequant_mode=dequant_mode, graph=graph,
                                                     min_nbytes=min_nbytes, split=split)
     # (i) side info, TNS data, integer spectrum, residual-bit count, seed, zero-frame flag: bit exact
@@ -106,7 +123,12 @@ def assert_parity(fs, ms, frames, nbytes_per_frame=None, host=False, exact_spect
     if exact_spectrum:
         ok = o_tr[..., 0] == 1
         assert np.array_equal(o_sp[ok].view(np.uint32), g_sp[ok].view(np.uint32)), "shaped spectrum not bit exact"
-    # (ii) PCM within +-1 LSB
+    # (ii) PCM bit exact against the oracle with the engine's inverse MDCT: concealment, overlap-add, post filter and
+    # rounding are the oracle's, so only the transform separates the two gates below
+    bad = np.argwhere(g_pcm != e_pcm)
+    assert bad.size == 0, f"PCM not bit exact against the engine-transform oracle in {len(bad)} samples, first (stream, " \
+                          f"frame, n) {bad[:4].tolist()}: gpu {g_pcm[tuple(bad[0])]} oracle {e_pcm[tuple(bad[0])]}"
+    # (iii) PCM within +-1 LSB against the reference's transform (kissfft DCT-IV)
     d = np.abs(o_pcm.astype(np.int32) - g_pcm.astype(np.int32))
     assert d.max() <= 1, f"PCM differs by {d.max()} LSB (streams {np.unique(np.argwhere(d > 1)[:, 0])[:8]})"
     return dict(pcm_exact=float((d == 0).mean()), concealed=float((o_tr[..., 0] == 0).mean()),

@@ -15,8 +15,7 @@ Run on the B200 box: python -m pytest tests -m gpu
 import numpy as np
 import pytest
 
-from common import assert_encoder_parity, assert_parity, corpus_clip
-from oracle import pyoracle as O
+from common import assert_encoder_parity, assert_parity, assert_pcm_matches_oracle, corpus_clip
 
 pytestmark = pytest.mark.gpu
 
@@ -67,6 +66,4 @@ def test_time_parallel_whole_clip(fs, ms, nbytes):
     out = torch.zeros((S, F * dec.nf), dtype=torch.int16, device="cuda:0")
     dec.decode_stream_frames(16, torch.from_numpy(np.ascontiguousarray(frames)).cuda(), out, scratch)
     torch.cuda.synchronize()
-    exp = O.decode_streams(frames, fs, ms)
-    d = np.abs(out.cpu().numpy().reshape(S, F, dec.nf).astype(np.int32) - exp.astype(np.int32))
-    assert d.max() <= 1
+    assert_pcm_matches_oracle(out.cpu().numpy().reshape(S, F, dec.nf), fs, ms, frames)

@@ -2,14 +2,17 @@
 
 Parity bar (BASELINE.json north_star / SURVEY.md 8d):
   * entropy-decoded integer spectrum and side info: bit exact;
-  * decoded i16 PCM: within +-1 LSB (PCM_TOL below);
-  * reference golden vector lc3_decode_channel: +-1 LSB (the engine's FFT factorisation differs from kissfft).
+  * decoded i16 PCM: bit exact against the oracle run with the engine's inverse MDCT (transform="engine",
+    oracle/lc3o_engine_imdct.cpp), whose concealment, overlap-add, post filter and rounding are the oracle's own;
+  * decoded i16 PCM: within +-1 LSB (PCM_TOL below) against the oracle run with the reference's inverse MDCT, and against
+    the reference golden vector lc3_decode_channel: the engine's FFT factorisation differs from kissfft, and
+    tests/test_engine_transform_cpu.py bounds both DCT-IVs against float64.
 Run on the B200 box: python -m pytest tests -m gpu
 """
 import numpy as np
 import pytest
 
-from common import ALL_CONFIGS, assert_parity, corpus, corpus_clip, gpu_decode
+from common import ALL_CONFIGS, assert_parity, assert_pcm_matches_oracle, corpus, corpus_clip, gpu_decode
 from conftest import load_golden
 from tools.corpus import MIXED_NBYTES
 
@@ -25,6 +28,7 @@ def test_golden_lc3_decode_channel():
     assert (st == 0).all()
     d = np.abs(pcm[:, 0].astype(np.int32) - exp[None, :].astype(np.int32))
     assert d.max() <= PCM_TOL
+    assert_pcm_matches_oracle(pcm, 48000, 10, frames)
     assert (pcm == pcm[:1]).all()                       # every lane decodes identically
     # arithmetic_codec.rs:458-473 scalars of the same frame
     assert tr[0, 0, 40] == 56909 and tr[0, 0, 21] == 8 and tr[0, 0, 22] == 0
@@ -109,10 +113,10 @@ def test_variable_frame_lengths():
     lens[sel] = 60
     # the oracle is handed each frame at its own length: compare against per-length decodes
     from oracle import pyoracle as O
-    o_pcm, o_tr, o_x, _ = O.decode_streams(frames, 48000, 10, lens, trace=True)
+    _, o_tr, o_x, _ = O.decode_streams(frames, 48000, 10, lens, trace=True)
     g_pcm, g_tr, g_x, _, _ = gpu_decode(48000, 10, frames, lens)
     assert np.array_equal(o_tr, g_tr) and np.array_equal(o_x, g_x)
-    assert np.abs(o_pcm.astype(np.int32) - g_pcm.astype(np.int32)).max() <= PCM_TOL
+    assert_pcm_matches_oracle(g_pcm, 48000, 10, frames, lens)
 
 
 def test_host_buffer_entry_point():
@@ -126,7 +130,6 @@ def test_pipelined_host_entry_point():
     import torch
 
     import lc3_codec_b200 as L
-    from oracle import pyoracle as O
     _, frames = corpus(48000, 10, 100, 70, 12)
     S, F, nb = frames.shape
     sf, fd = L.SamplingFrequency.Hz48000, L.FrameDuration.TenMs
@@ -139,9 +142,7 @@ def test_pipelined_host_entry_point():
         dec.decode_frames_host(16, host_in[f], host_out[f])
     dec.host_fence()
     torch.cuda.synchronize()
-    o_pcm = O.decode_streams(frames, 48000, 10)
-    d = np.abs(host_out.numpy().transpose(1, 0, 2).astype(np.int32) - o_pcm.astype(np.int32))
-    assert d.max() <= PCM_TOL
+    assert_pcm_matches_oracle(host_out.numpy().transpose(1, 0, 2), 48000, 10, frames)
 
 
 def test_odd_pcm_stride_and_unaligned_rows():
@@ -198,7 +199,7 @@ def test_mixed_rate_batch():
     for (fs, ms) in ALL_CONFIGS:
         _, fr = corpus(fs, ms, MIXED_NBYTES[(fs, ms)], per, F)
         frames_by[(fs, ms)] = fr
-        pcm_by[(fs, ms)] = O.decode_streams(fr, fs, ms)
+        pcm_by[(fs, ms)] = O.decode_streams(fr, fs, ms), O.decode_streams(fr, fs, ms, transform="engine")
     # interleave the configurations over stream ids like SURVEY.md 8d: stream s -> config s mod 12
     stream_cfg = [ALL_CONFIGS[s % 12] for s in range(12 * per)]
     dec = L.Lc3MixedBatchDecoder([(L.SamplingFrequency.from_hz(fs), L.FrameDuration.from_ms(ms)) for fs, ms in stream_cfg],
@@ -219,8 +220,9 @@ def test_mixed_rate_batch():
         got[:, f] = out.cpu().numpy()
     for pos, s in enumerate(dec.order):
         fs, ms = stream_cfg[s]
-        exp = pcm_by[(fs, ms)][s // 12]
+        exp, exact = (p[s // 12] for p in pcm_by[(fs, ms)])
         nf = exp.shape[-1]
+        assert np.array_equal(got[pos, :, :nf], exact), (fs, ms, s)
         assert np.abs(got[pos, :, :nf].astype(np.int32) - exp.astype(np.int32)).max() <= PCM_TOL, (fs, ms, s)
 
 
@@ -236,7 +238,7 @@ def test_mixed_rate_batch_host_entry():
     for (fs, ms) in ALL_CONFIGS:
         _, fr = corpus(fs, ms, MIXED_NBYTES[(fs, ms)], per, F)
         frames_by[(fs, ms)] = fr
-        pcm_by[(fs, ms)] = O.decode_streams(fr, fs, ms)
+        pcm_by[(fs, ms)] = O.decode_streams(fr, fs, ms), O.decode_streams(fr, fs, ms, transform="engine")
     stream_cfg = [ALL_CONFIGS[s % 12] for s in range(12 * per)]
     for graph in (True, False):
         dec = L.Lc3MixedBatchDecoder([(L.SamplingFrequency.from_hz(fs), L.FrameDuration.from_ms(ms)) for fs, ms in stream_cfg],
@@ -263,8 +265,9 @@ def test_mixed_rate_batch_host_entry():
             for r in range(count):
                 s = dec.order[first + r]
                 fs, ms = stream_cfg[s]
-                exp = pcm_by[(fs, ms)][s // 12]
+                exp, exact = (p[s // 12] for p in pcm_by[(fs, ms)])
                 got = np.stack([views[f][b][r].numpy() for f in range(F)])
+                assert np.array_equal(got, exact), (fs, ms, s, graph)
                 assert np.abs(got.astype(np.int32) - exp.astype(np.int32)).max() <= PCM_TOL, (fs, ms, s, graph)
 
 
@@ -366,9 +369,8 @@ def test_sharded_decoder_two_shards_on_one_gpu():
     for f in range(F):
         dec.decode_frames_host(16, host_in[f], host_out[f], frame_nbytes=host_len[f], status_out=status[f])
     dec.wait()
-    o_pcm, o_tr, _, _ = O.decode_streams(frames, 48000, 10, lens, trace=True)
-    d = np.abs(host_out.numpy().transpose(1, 0, 2).astype(np.int32) - o_pcm.astype(np.int32))
-    assert d.max() <= PCM_TOL
+    o_tr = O.decode_streams(frames, 48000, 10, lens, trace=True)[1]
+    assert_pcm_matches_oracle(host_out.numpy().transpose(1, 0, 2), 48000, 10, frames, lens)
     assert np.array_equal(status.numpy().T, 1 - o_tr[..., 0])
     with pytest.raises(L.Lc3DecoderError):
         dec.decode_frames_host(24, host_in[0], host_out[0])

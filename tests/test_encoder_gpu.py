@@ -101,14 +101,14 @@ def test_8k_rejected_like_the_reference():
 
 
 def test_round_trip_gpu_encode_gpu_decode():
-    """BASELINE config 5's shape at test size: GPU encode -> GPU decode equals oracle encode -> oracle decode (+-1 LSB)."""
-    from common import corpus, gpu_decode
+    """BASELINE config 5's shape at test size: GPU encode -> GPU decode equals oracle encode -> oracle decode (bit exact
+    with the engine's inverse MDCT in the oracle, +-1 LSB with the reference's)."""
+    from common import assert_pcm_matches_oracle, corpus, gpu_decode
     from oracle import pyoracle as O
     pcm, o_frames = corpus(48000, 10, 150, 64, 20)
     g_frames = gpu_encode(48000, 10, pcm, 150)
     g_pcm = gpu_decode(48000, 10, g_frames, trace=False)[0]
-    o_pcm = O.decode_streams(o_frames, 48000, 10)
-    assert np.abs(g_pcm.astype(np.int32) - o_pcm.astype(np.int32)).max() <= 1
+    assert_pcm_matches_oracle(g_pcm, 48000, 10, o_frames)
 
 
 def test_sharded_encoder_and_graph_executor():

@@ -7,8 +7,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from common import corpus
-from oracle import pyoracle as O
+from common import assert_pcm_matches_oracle, corpus
 
 pytestmark = pytest.mark.gpu
 ROOT = pathlib.Path(__file__).resolve().parent.parent
@@ -37,5 +36,4 @@ def test_wav_to_lc3_to_wav_stereo_48k(tmp_path):
     raw = wav_out.read_bytes()
     assert raw[:4] == b"RIFF" and raw[8:16] == b"WAVEfmt " and struct.unpack("<H", raw[22:24])[0] == 2
     out = np.frombuffer(raw[44:], "<i2").reshape(F * 480, 2).T.reshape(2, F, 480)
-    exp = O.decode_streams(o_frames, 48000, 10)
-    assert np.abs(out.astype(np.int32) - exp.astype(np.int32)).max() <= 1
+    assert_pcm_matches_oracle(out, 48000, 10, o_frames)

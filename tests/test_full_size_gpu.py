@@ -11,7 +11,7 @@ Run on the B200 box: python -m pytest tests -m gpu
 import numpy as np
 import pytest
 
-from common import corpus_clip
+from common import assert_pcm_matches_oracle, corpus_clip
 from oracle import pyoracle as O
 
 pytestmark = pytest.mark.gpu
@@ -45,16 +45,14 @@ def _decode_full(frames_base, S, fs=48000, ms=10):
 def test_decode_262144_streams_replication_invariance():
     _, frames = corpus_clip(48000, 10, 150, BASE, window=FRAMES)
     got = _decode_full(frames, FULL)
-    exp = O.decode_streams(frames, 48000, 10)
-    assert np.abs(got.astype(np.int32) - exp.astype(np.int32)).max() <= 1
+    assert_pcm_matches_oracle(got, 48000, 10, frames)
 
 
 def test_decode_65536_streams_16k_7p5ms():
     """BASELINE config 3's shape, four times its stream count (LTPF and TNS active)."""
     _, frames = corpus_clip(16000, 7.5, 30, BASE, window=FRAMES)
     got = _decode_full(frames, 65536, 16000, 7.5)
-    exp = O.decode_streams(frames, 16000, 7.5)
-    assert np.abs(got.astype(np.int32) - exp.astype(np.int32)).max() <= 1
+    assert_pcm_matches_oracle(got, 16000, 7.5, frames)
 
 
 def test_encode_262144_streams_byte_identity_and_round_trip():
@@ -72,6 +70,7 @@ def test_encode_262144_streams_byte_identity_and_round_trip():
     bits = torch.zeros((S, 150), dtype=torch.uint8, device="cuda:0")
     out = torch.zeros((S, 480), dtype=torch.int16, device="cuda:0")
     o_pcm = O.decode_streams(o_frames, 48000, 10)
+    e_pcm = O.decode_streams(o_frames, 48000, 10, transform="engine")
     for f in range(FRAMES):
         x = torch.from_numpy(np.ascontiguousarray(pcm[:, f])).cuda().repeat(reps, 1)
         enc.encode_frames(x, bits)
@@ -81,6 +80,7 @@ def test_encode_262144_streams_byte_identity_and_round_trip():
         assert np.array_equal(b[0].cpu().numpy(), o_frames[:, f]), f"frame {f}: bytes differ from the oracle encoder"
         y = out.view(reps, BASE, 480)
         assert bool((y == y[:1]).all()), f"frame {f}: decoded replicas differ"
+        assert np.array_equal(y[0].cpu().numpy(), e_pcm[:, f]), f"frame {f}: PCM not bit exact"
         d = np.abs(y[0].cpu().numpy().astype(np.int32) - o_pcm[:, f].astype(np.int32))
         assert d.max() <= 1
 

@@ -7,8 +7,7 @@ and (+-1 LSB) against the oracle, with LTPF transitions, lost and corrupted fram
 import numpy as np
 import pytest
 
-from common import corpus, gpu_decode
-from oracle import pyoracle as O
+from common import assert_pcm_matches_oracle, corpus, gpu_decode
 
 pytestmark = pytest.mark.gpu
 
@@ -54,8 +53,7 @@ def test_multi_equals_frame_by_frame_and_oracle(fs, ms, nbytes):
     got, status = _multi(dec, frames)
     ref = gpu_decode(fs, ms, frames, trace=False)[0]
     assert np.array_equal(got, ref), "time-parallel PCM differs from the frame-by-frame path"
-    exp = O.decode_streams(frames, fs, ms)
-    assert np.abs(got.astype(np.int32) - exp.astype(np.int32)).max() <= 1
+    assert_pcm_matches_oracle(got, fs, ms, frames)
     assert status.shape == (48, 40)
 
 
@@ -102,5 +100,4 @@ def test_multi_file_shape_few_streams_many_frames():
     _, frames = corpus(48000, 10, 150, 2, 600)
     dec, _ws = _decoder(48000, 10, 2, 150)
     got, _ = _multi(dec, frames)
-    exp = O.decode_streams(frames, 48000, 10)
-    assert np.abs(got.astype(np.int32) - exp.astype(np.int32)).max() <= 1
+    assert_pcm_matches_oracle(got, 48000, 10, frames)

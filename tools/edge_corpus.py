@@ -161,6 +161,20 @@ def make_edge_pcm(n_streams: int, n_frames: int, fs: int, ms: float, first_strea
     return make_edge_streams(range(first_stream, first_stream + n_streams), n_frames, fs, ms)
 
 
+def make_quiet_tone_pcm(n_streams: int, n_frames: int, fs: int, ms: float, dbfs: float = -90.0) -> np.ndarray:
+    """[n_streams, n_frames, nf] int16: sines at dbfs (-90 dBFS: amplitude 1.04 LSB, so the samples are -1, 0 and 1),
+    stream i at 100 Hz * (i + 1) with a phase drawn from its id.  Not an edge class: adding one would renumber the
+    classes of every edge stream."""
+    nf = frame_geometry(fs, ms)[0]
+    t = np.arange(n_frames * nf)
+    amp = 32768.0 * 10.0 ** (dbfs / 20.0)
+    out = np.empty((n_streams, n_frames * nf), np.int16)
+    for i in range(n_streams):
+        ph = 2 * np.pi * _draw(np.array([np.uint64(int(SEED_EDGE) ^ (0x51E7 + i))]), 0)[0]
+        out[i] = np.round(amp * np.sin(2 * np.pi * 100.0 * (i + 1) / fs * t + ph))
+    return out.reshape(n_streams, n_frames, nf)
+
+
 # ---- the reference's integer rate decisions, restated from its formulas (not from the engine) so that tests can put
 # frame lengths on either side of each.  fs_ind: 0..4 for 8 / 16 / 24 / 32 / 44.1 and 48 kHz.
 MIN_NBYTES, MAX_NBYTES = 20, 400

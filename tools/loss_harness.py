@@ -105,6 +105,8 @@ def run(fs: int, ms: float, nbytes: int, n_streams: int, n_frames: int, seed: in
     o_concealed = o_tr[..., 0] == 0
     assert np.array_equal(g_status != 0, o_concealed), "concealed flags differ from the oracle's"
     assert np.array_equal(o_tr, g_tr), "decoded side information differs on the frames that survived"
+    e_pcm = O.decode_streams(damaged, fs, ms, lens, transform="engine")
+    assert np.array_equal(g_pcm, e_pcm), "PCM not bit exact against the oracle with the engine's inverse MDCT"
     diff = np.abs(o_pcm.astype(np.int32) - g_pcm.astype(np.int32))
     assert diff.max() <= 1, f"PCM differs by {diff.max()} LSB"
     rep = {
