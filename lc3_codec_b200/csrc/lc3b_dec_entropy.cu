@@ -681,10 +681,12 @@ __global__ void __launch_bounds__(ENT_THREADS, 6) entropy_kernel(const __grid_co
 // Mixed-rate batches (BASELINE config 4; lc3b_mixed_*): ONE launch covers every (fs, duration) bucket.  A CTA finds its
 // bucket in a small device table, patches the per-call pointers into that bucket's parameter block (rows of the caller's
 // buffers are in bucket order, so a bucket is a contiguous row range) and runs the single-configuration body on it.
-__device__ __forceinline__ void mixed_select(const MixedParams& m, EntropyParams* s_p, int* s_block) {
+// per_entropy_cta: CTAs of the calling kernel per entropy CTA of ENT_THREADS thread slots (a bucket's first_cta counts
+// entropy CTAs): 1 but for the warp-per-frame kernel, whose CTAs cover DQW_WARPS slots.
+__device__ __forceinline__ void mixed_select(const MixedParams& m, EntropyParams* s_p, int* s_block, int per_entropy_cta) {
     if (threadIdx.x == 0) {
         int b = 0;
-        while (b + 1 < m.n_buckets && (int)blockIdx.x >= m.buckets[b + 1].first_cta) b++;
+        while (b + 1 < m.n_buckets && (int)blockIdx.x >= m.buckets[b + 1].first_cta * per_entropy_cta) b++;
         const MixedBucket& bk = m.buckets[b];
         EntropyParams q = bk.ep;
         q.frames = m.frames + (size_t)bk.first_row * m.frame_stride;
@@ -694,7 +696,7 @@ __device__ __forceinline__ void mixed_select(const MixedParams& m, EntropyParams
         q.status_out = m.status_out ? m.status_out + bk.first_row : nullptr;
         q.row_pitch = m.row_pitch;
         *s_p = q;
-        *s_block = (int)blockIdx.x - bk.first_cta;
+        *s_block = (int)blockIdx.x - bk.first_cta * per_entropy_cta;
     }
     __syncthreads();
 }
@@ -702,8 +704,170 @@ __device__ __forceinline__ void mixed_select(const MixedParams& m, EntropyParams
 __global__ void __launch_bounds__(ENT_THREADS, 6) entropy_mixed_kernel(const __grid_constant__ MixedParams m) {
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
-    mixed_select(m, &s_p, &s_block);
+    mixed_select(m, &s_p, &s_block, 1);
     entropy_body<false>(s_p, s_block);
+}
+
+// ---------------------------------------------------------------- reference steps D4-D8, one definition each
+// Shared by the thread-per-frame (dequant_body), warp-per-frame (dequant_warp_body) and lattice (tns_list_body) kernels,
+// so that the kernels' f32 operations are the same ones in the same order and their spectra are bit-identical.
+
+__device__ __forceinline__ int bw_stop_lines(const DevConfig& c, int bw) {
+    return c.n_ms == LC3B_10MS ? 80 * (bw + 1) : 60 * (bw + 1);
+}
+
+// Per-frame scalars: global gain (global_gain.rs:15-25), noise-filling level and the noise-filled line range.
+struct FrameScalars {
+    float gg, nf_level;
+    int bw_stop, nf_start;
+};
+__device__ __forceinline__ FrameScalars frame_scalars(const DevConfig& c, int nbits, int gg_ind, int noise_factor, int bw) {
+    FrameScalars f;
+    const int fs = c.fs_ind + 1;
+    const int gg_off = -min(nbits / (10 * fs), 115) - 105 - 5 * fs;
+    f.gg = c.gg_table[gg_ind + gg_off + 245];
+    f.nf_level = xd(xs(8.0f, (float)noise_factor), 16.0f);
+    f.bw_stop = bw_stop_lines(c, bw);
+    f.nf_start = c.n_ms == LC3B_10MS ? 24 : 18;
+    return f;
+}
+
+// residual_spectrum.rs:13-39: non-zero line x refined by one tail bit
+__device__ __forceinline__ float residual_refine(float v, int32_t xi, uint32_t bit) {
+    const float up = xi > 0 ? 0.3125f : 0.1875f, down = xi > 0 ? -0.1875f : -0.3125f;
+    return xa(v, bit ? up : down);
+}
+
+// noise_filling.rs:37-55: the level a filled line takes from the LCG state that filled it
+__device__ __forceinline__ float nf_fill_level(uint32_t state, float nf_level) {
+    return state < 0x8000u ? nf_level : -nf_level;
+}
+// one LCG step for a filled line; v passes through unchanged when the line is not filled
+__device__ __forceinline__ float noise_fill(bool fill, int& nf_state, float nf_level, float v) {
+    const int nxt = (13849 + nf_state * 31821) & 0xFFFF;
+    nf_state = fill ? nxt : nf_state;
+    return fill ? nf_fill_level((uint32_t)nxt, nf_level) : v;
+}
+
+// temporal_noise_shaping.rs:83-138: filter 0 runs over lines [s0, e0), filter 1 over [e0, e1) (empty below bw 3);
+// ord1 is 0 for a frame with one filter.  rc_i: the 16 coefficient indices (an array or a hand-off pointer).
+struct TnsPlan {
+    float rc0[8], rc1[8];
+    int ord0, ord1, s0, e0, e1;
+};
+template <typename RcIndices>
+__device__ __forceinline__ void tns_plan(TnsPlan& f, const DevConfig& c, int bw, int num_tns, int order0, int order1,
+                                         const RcIndices& rc_i) {
+    const int bw_stop = bw_stop_lines(c, bw);
+    f.s0 = c.n_ms == LC3B_10MS ? 12 : 9;
+    if (bw < 3) { f.e0 = bw_stop; f.e1 = bw_stop; }
+    else { f.e0 = bw_stop / 2; f.e1 = bw_stop; }
+    f.ord0 = order0;
+    f.ord1 = num_tns == 2 ? order1 : 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {                                       // QUIRK: index 0 -> rc = 0.0
+        const int a = rc_i[i], b = rc_i[8 + i];
+        f.rc0[i] = a != 0 ? c.tns_sin[a] : 0.0f;
+        f.rc1[i] = b != 0 ? c.tns_sin[b] : 0.0f;
+    }
+}
+
+// The filter change at line `next`: phase 0 -> 1 enters filter 0, 1 -> 2 filter 1 when it covers any line, and the end
+// of the last filter sets the order to 0.  QUIRK: st is not reset, the lattice state carries across filters.
+__device__ __forceinline__ void tns_switch(const TnsPlan& f, float (&rc)[8], int& ord, int& phase, int& next) {
+    if (phase == 0) {
+#pragma unroll
+        for (int i = 0; i < 8; i++) rc[i] = f.rc0[i];
+        ord = f.ord0;
+        phase = 1;
+        next = f.e0;
+    } else if (phase == 1 && f.e0 < f.e1) {
+#pragma unroll
+        for (int i = 0; i < 8; i++) rc[i] = f.rc1[i];
+        ord = f.ord1;
+        phase = 2;
+        next = f.e1;
+    } else {
+        ord = 0;
+        next = 0x7fffffff;
+    }
+}
+
+// temporal_noise_shaping.rs:24-74: one line through the all-pole lattice of order ord.  Lanes of a warp sit in different
+// filters with different orders: the lattice runs `depth` stages (warp-uniform, at least the warp's largest order; a
+// compile-time constant where the caller has one) and the stages at or above the lane's own order are selects that keep
+// its value and state, so the warp never splits over it.
+__device__ __forceinline__ float tns_lattice_line(float v, const float (&rc)[8], float (&st)[8], int ord, int depth) {
+    if (depth <= 0) return v;
+    float t = v;
+#pragma unroll
+    for (int j = 7; j >= 0; j--) {
+        if (j < depth) {
+            const float t2 = xs(t, xm(rc[j], st[j]));
+            t = j < ord ? t2 : t;
+            if (j + 1 < 8) {
+                const float s2 = xa(xm(rc[j], t), st[j]);
+                st[j + 1 < 8 ? j + 1 : 7] = j + 1 < ord ? s2 : st[j + 1 < 8 ? j + 1 : 7];
+            }
+        }
+    }
+    st[0] = ord > 0 ? t : st[0];
+    return t;
+}
+
+// spectral_noise_shaping.rs:61-84: the shape vector (stride ys) into y and its gain divided by the vector's norm
+__device__ __forceinline__ float sns_norm_gain(const float* yv, int ys, const float* gains, int g_ind, float (&y)[16]) {
+    float sum = 0.0f;
+#pragma unroll
+    for (int i = 0; i < 16; i++) { y[i] = yv[i * ys]; sum = xa(sum, xm(y[i], y[i])); }
+    const float y_norm = sqrtf(sum);
+    float g = gains[g_ind];
+    if (y_norm != 0.0f) g = xd(g, y_norm);
+    return g;
+}
+// scale factor n: stage-1 codebook entry plus the gain times row n of the DCT rotation
+__device__ __forceinline__ float sns_scale_factor(const float (&y)[16], float g, int n, int ind_lf, int ind_hf) {
+    float factor = 0.0f;
+#pragma unroll
+    for (int col = 0; col < 16; col++) factor = xa(factor, xm(y[col], LC3T_D[n][col]));
+    const float st1 = n < 8 ? LC3T_LFCB[ind_lf][n] : LC3T_HFCB[ind_hf][n - 8];
+    return xa(st1, xm(g, factor));
+}
+
+// spectral_noise_shaping.rs:85-98: interpolated scale factor j of 64 from the 16 at scf[n * STRIDE]
+template <int STRIDE>
+__device__ __forceinline__ float sns_interp64(const float* scf, int j) {
+    if (j < 2) return scf[0];
+    if (j >= 62) {
+        const float d = xs(scf[15 * STRIDE], scf[14 * STRIDE]);
+        return xa(scf[15 * STRIDE], xm(j == 62 ? 0.125f : 0.375f, d));
+    }
+    const int n = (j - 2) >> 2, r = (j - 2) & 3;
+    const float fn = scf[n * STRIDE], d = xs(scf[(n + 1) * STRIDE], fn);
+    const float w = r == 0 ? 0.125f : r == 1 ? 0.375f : r == 2 ? 0.625f : 0.875f;
+    return xa(fn, xm(w, d));
+}
+// :100-123: the gain of band b, the 64 interpolated values folded onto nb < 64 bands
+template <int STRIDE>
+__device__ __forceinline__ float sns_band_gain(const float* scf, int b, int nb) {
+    const int n2 = 64 - nb;
+    float s;
+    if (n2 != 0) s = b < n2 ? xd(xa(sns_interp64<STRIDE>(scf, 2 * b), sns_interp64<STRIDE>(scf, 2 * b + 1)), 2.0f)
+                            : sns_interp64<STRIDE>(scf, b + n2);
+    else s = sns_interp64<STRIDE>(scf, b);
+    return exp2_raw_fm(s);
+}
+
+// Side record for the synthesis kernel; a good frame makes the slot just written the stream's current one.
+__device__ __forceinline__ void write_side(const EntropyParams& p, int srow, bool ok, int ltpf_active, int pitch_index,
+                                           int nbits, int slot, int new_slot) {
+    int32_t* sd = p.side + (size_t)srow * SIDE_WORDS;
+    sd[SD_OK] = ok;
+    sd[SD_LTPF_ACTIVE] = ok ? ltpf_active : 0;
+    sd[SD_PITCH_INDEX] = ok ? pitch_index : 0;
+    sd[SD_NBITS] = nbits;
+    sd[SD_SLOT] = ok ? new_slot : slot;
+    if (ok && p.fixed_slot < 0) p.sstate[(size_t)srow * SS_WORDS + SS_SLOT] = new_slot;
 }
 
 // ---------------------------------------------------------------- kernel 1b: integers -> shaped spectrum
@@ -769,37 +933,20 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
     const int new_slot = p.fixed_slot >= 0 ? p.fixed_slot : slot ^ 1;
     float* s_y = s_scf + tid;                                          // PVQ vector / scale factors, stride T
     bool is_zero_frame = false;
-    float gg = 0.0f, nf_level = 0.0f;
-    float rc0[8] = {0, 0, 0, 0, 0, 0, 0, 0}, rc1[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    int bw_stop = 0, nf_start = 0, tns_s0 = 0, tns_e0 = 0, tns_e1 = 0;
+    FrameScalars fs{};
+    TnsPlan tf{};
     int lastnz = 0;
     if (ok) {
         lastnz = si.lastnz;
         const int x0 = xq[0], x1 = xq[1];
         is_zero_frame = si.lastnz == 2 && x0 == 0 && x1 == 0 && si.gg_ind == 0;
-        {                                                              // global_gain.rs:15-25
-            const int fs = c.fs_ind + 1;
-            const int gg_off = -min(nbits / (10 * fs), 115) - 105 - 5 * fs;
-            gg = c.gg_table[si.gg_ind + gg_off + 245];
-        }
-        nf_level = xd(xs(8.0f, (float)si.noise_factor), 16.0f);
-        const bool d10 = c.n_ms == LC3B_10MS;
-        bw_stop = d10 ? 80 * (si.bw + 1) : 60 * (si.bw + 1);
-        nf_start = d10 ? 24 : 18;
-        // temporal_noise_shaping.rs:83-138 band split
-        tns_s0 = d10 ? 12 : 9;
-        if (si.bw < 3) { tns_e0 = bw_stop; tns_e1 = bw_stop; }
-        else { tns_e0 = bw_stop / 2; tns_e1 = bw_stop; }
-#pragma unroll
-        for (int i = 0; i < 8; i++) {                                   // QUIRK: index 0 -> rc = 0.0
-            rc0[i] = rc_i[i] != 0 ? c.tns_sin[rc_i[i]] : 0.0f;
-            rc1[i] = rc_i[8 + i] != 0 ? c.tns_sin[rc_i[8 + i]] : 0.0f;
-        }
-        // spectral_noise_shaping.rs:21-98: stage 1 + PVQ shape + DCT rotation -> 16 scale factors in s_y
+        fs = frame_scalars(c, nbits, si.gg_ind, si.noise_factor, si.bw);
+        tns_plan(tf, c, si.bw, si.num_tns, rc_order0, rc_order1, rc_i);
+        // SNS: stage 1 + PVQ shape + DCT rotation -> 16 scale factors in s_y, evaluated per band on demand below
         const int shape_j = (si.submode_msb << 1) + si.submode_lsb;
         const float* gains;
         constexpr int YS = ENT_THREADS;
-        switch (shape_j) {
+        switch (shape_j) {                                             // spectral_noise_shaping.rs:21-60
             case 0: {
                 mpvq_deenum(10, 10, si.ls_inda, (uint32_t)si.idx_a, s_y, YS);
                 // second call writes z[0..6) which the reference copies to y[10..16)
@@ -816,41 +963,10 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
             default: mpvq_deenum(16, 6, si.ls_inda, (uint32_t)si.idx_a, s_y, YS); gains = LC3T_SNS_VQ_FAR_ADJ_GAINS; break;
         }
         float y[16];
-        float sum = 0.0f;
-#pragma unroll
-        for (int i = 0; i < 16; i++) { y[i] = s_y[i * YS]; sum = xa(sum, xm(y[i], y[i])); }
-        const float y_norm = sqrtf(sum);
-        float g = gains[si.g_ind];
-        if (y_norm != 0.0f) g = xd(g, y_norm);
-        for (int n = 0; n < 16; n++) {
-            float factor = 0.0f;
-#pragma unroll
-            for (int col = 0; col < 16; col++) factor = xa(factor, xm(y[col], LC3T_D[n][col]));
-            const float st1 = n < 8 ? LC3T_LFCB[si.ind_lf][n] : LC3T_HFCB[si.ind_hf][n - 8];
-            s_y[n * YS] = xa(st1, xm(g, factor));
-        }
+        const float g = sns_norm_gain(s_y, ENT_THREADS, gains, si.g_ind, y);
+        for (int n = 0; n < 16; n++) s_y[n * ENT_THREADS] = sns_scale_factor(y, g, n, si.ind_lf, si.ind_hf);
     }
-
-    // scale-factor interpolation (spectral_noise_shaping.rs:85-98) evaluated per band on demand
-    auto scf_at = [&](int n) { return s_y[n * ENT_THREADS]; };
-    auto interp64 = [&](int j) -> float {
-        if (j < 2) return scf_at(0);
-        if (j >= 62) {
-            const float d = xs(scf_at(15), scf_at(14));
-            return xa(scf_at(15), xm(j == 62 ? 0.125f : 0.375f, d));
-        }
-        const int n = (j - 2) >> 2, r = (j - 2) & 3;
-        const float fn = scf_at(n), d = xs(scf_at(n + 1), fn);
-        const float w = r == 0 ? 0.125f : r == 1 ? 0.375f : r == 2 ? 0.625f : 0.875f;
-        return xa(fn, xm(w, d));
-    };
-    const int nb = c.nb, n2 = 64 - nb;
-    auto band_gain = [&](int b) -> float {                             // :100-123 incl. the nb < 64 folding
-        float s;
-        if (n2 != 0) s = b < n2 ? xd(xa(interp64(2 * b), interp64(2 * b + 1)), 2.0f) : interp64(b + n2);
-        else s = interp64(b);
-        return exp2_raw_fm(s);
-    };
+    const int nb = c.nb;
 
     // rows of one warp belong to arbitrary streams of the CTA (work sorting) and may sit in different slots
     // (a slot only flips on a good frame): every row is addressed through its own stream id and slot
@@ -862,7 +978,7 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
         float st[8] = {0, 0, 0, 0, 0, 0, 0, 0};
         float rc[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // coefficient set in use
         int ord = 0, om = 0;                     // this lane's order in use, the warp's largest
-        int tns_phase = 0, tns_next = ok ? tns_s0 : 0x7fffffff;   // next line at which this lane switches filters
+        int tns_phase = 0, tns_next = ok ? tf.s0 : 0x7fffffff;    // next line at which this lane switches filters
         int last_nz = -1000;
         int nf_state = (int)(seed_acc & 0xffffu);
         int res_used = 0;
@@ -888,48 +1004,37 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
             const int32_t e[4] = {g.x, g.y, g.z, g.w};
 #pragma unroll
             for (int j = 0; j < W; j++)
-                if (e[j] != 0 && j < bw_stop) last_nz = j;
+                if (e[j] != 0 && j < fs.bw_stop) last_nz = j;
         }
         const bool res_on = ok && !si.lsb_mode;
         const bool nf_on = ok && !is_zero_frame;
-        auto lines_fast = [&](auto omc, const int32_t (&e)[8], const float (&gl)[4], const int k4, float (&o)[4]) {
+        // The four lines of group k4.  SW: some lane changes its TNS filter inside the group, so the switch is tested at
+        // every line and the lattice runs at the warp's largest order of that line; otherwise at the compile-time depth OM.
+        auto lines = [&](auto swc, auto omc, const int32_t (&e)[8], const float (&gl)[4], const int k4, float (&o)[4]) {
+            constexpr bool SW = decltype(swc)::value;
             constexpr int OM = decltype(omc)::value;
 #pragma unroll
             for (int u = 0; u < 4; u++) {
                 const int k = k4 + u;
-                last_nz = (e[u + W] != 0 && k + W < bw_stop) ? k + W : last_nz;
+                last_nz = (e[u + W] != 0 && k + W < fs.bw_stop) ? k + W : last_nz;
                 const int32_t xi = e[u];
                 float v = (float)xi;
-                {   // residual bit (as below)
+                {   // one tail bit per non-zero line while the budget lasts (it cannot run past the frame here, see
+                    // DESIGN.md); read straight from the staged row, no window to refill
                     const bool take = res_on && xi != 0 && res_used < nres;
                     const int bidx = max(rd.len - 1 - (rd.tail >> 3), 0);
                     const uint32_t bit = ((uint32_t)rd.buf[bidx] >> (rd.tail & 7)) & 1u;
-                    const float up = xi > 0 ? 0.3125f : 0.1875f, down = xi > 0 ? -0.1875f : -0.3125f;
-                    v = take ? xa(v, bit ? up : down) : v;
+                    v = take ? residual_refine(v, xi, bit) : v;
                     rd.tail += take ? 1 : 0;
                     res_used += take ? 1 : 0;
                 }
-                {   // noise filling (as below)
-                    const bool fill = nf_on && k >= nf_start && k < bw_stop && last_nz < k - W;
-                    const int nxt = (13849 + nf_state * 31821) & 0xFFFF;
-                    nf_state = fill ? nxt : nf_state;
-                    v = fill ? (nxt < 0x8000 ? nf_level : -nf_level) : v;
+                v = noise_fill(nf_on && k >= fs.nf_start && k < fs.bw_stop && last_nz < k - W, nf_state, fs.nf_level, v);
+                v = xm(v, fs.gg);
+                if constexpr (SW) {
+                    if (k == tns_next) tns_switch(tf, rc, ord, tns_phase, tns_next);
+                    om = __reduce_max_sync(0xffffffffu, ord);
                 }
-                v = xm(v, gg);
-                if constexpr (OM > 0) {                                 // stages >= the lane's order are selects that keep
-                    float t = v;
-#pragma unroll
-                    for (int j = OM - 1; j >= 0; j--) {
-                        const float t2 = xs(t, xm(rc[j], st[j]));
-                        t = j < ord ? t2 : t;
-                        if (j + 1 < 8) {
-                            const float s2 = xa(xm(rc[j], t), st[j]);
-                            st[j + 1 < 8 ? j + 1 : 7] = j + 1 < ord ? s2 : st[j + 1 < 8 ? j + 1 : 7];
-                        }
-                    }
-                    st[0] = ord > 0 ? t : st[0];
-                    v = t;
-                }
+                v = tns_lattice_line(v, rc, st, ord, SW ? om : OM);
                 o[u] = ok ? xm(v, gl[u]) : v;
             }
         };
@@ -943,7 +1048,7 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
             float gl[4] = {gband, gband, gband, gband};
             while (k_end < k4 + 4) {
                 band++;
-                gband = ok ? band_gain(band) : 0.0f;
+                gband = ok ? sns_band_gain<ENT_THREADS>(s_y, band, nb) : 0.0f;
                 const int first = k_end - k4;
                 k_end = band + 1 < nb ? s_band[band + 1] : ne;
 #pragma unroll
@@ -957,75 +1062,11 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
                 // lines are ONE basic block - selects only, the lattice at a compile-time depth that covers the warp's
                 // largest order - so the scheduler overlaps the lines' chains: stage j of a line needs the state stage
                 // j - 1 of the previous line left, i.e. consecutive lines run two lattice stages apart, not eight.
-                if (om == 0) lines_fast(std::integral_constant<int, 0>{}, e, gl, k4, o);
-                else if (om <= 4) lines_fast(std::integral_constant<int, 4>{}, e, gl, k4, o);
-                else lines_fast(std::integral_constant<int, 8>{}, e, gl, k4, o);
+                if (om == 0) lines(std::false_type{}, std::integral_constant<int, 0>{}, e, gl, k4, o);
+                else if (om <= 4) lines(std::false_type{}, std::integral_constant<int, 4>{}, e, gl, k4, o);
+                else lines(std::false_type{}, std::integral_constant<int, 8>{}, e, gl, k4, o);
             } else {
-#pragma unroll
-            for (int u = 0; u < 4; u++) {
-                const int k = k4 + u;
-                if (e[u + W] != 0 && k + W < bw_stop) last_nz = k + W;
-                const int32_t xi = e[u];
-                float v = (float)xi;
-                {   // residual_spectrum.rs:13-39: one tail bit per non-zero line while the budget lasts (it cannot run past
-                    // the frame here, see DESIGN.md); read straight from the staged row, no window to refill
-                    const bool take = ok && !si.lsb_mode && xi != 0 && res_used < nres;
-                    const int bidx = max(rd.len - 1 - (rd.tail >> 3), 0);
-                    const uint32_t bit = take ? ((uint32_t)rd.buf[bidx] >> (rd.tail & 7)) & 1u : 0u;
-                    const float up = xi > 0 ? 0.3125f : 0.1875f, down = xi > 0 ? -0.1875f : -0.3125f;
-                    v = take ? xa(v, bit ? up : down) : v;
-                    rd.tail += take ? 1 : 0;
-                    res_used += take ? 1 : 0;
-                }
-                {   // noise_filling.rs:37-55
-                    const bool fill = ok && !is_zero_frame && k >= nf_start && k < bw_stop && last_nz < k - W;
-                    const int nxt = (13849 + nf_state * 31821) & 0xFFFF;
-                    nf_state = fill ? nxt : nf_state;
-                    v = fill ? (nxt < 0x8000 ? nf_level : -nf_level) : v;
-                }
-                v = xm(v, gg);
-                // temporal_noise_shaping.rs:24-74.  Lanes sit in different filters (band edges depend on the bandwidth)
-                // with different orders; the coefficient set in use is switched per lane at its band edges, and the
-                // lattice runs the warp's largest order with per-lane selects, so the warp never splits over it.
-                {
-                    if (k == tns_next) {
-                        if (tns_phase == 0) {
-#pragma unroll
-                            for (int i = 0; i < 8; i++) rc[i] = rc0[i];
-                            ord = rc_order0;
-                            tns_phase = 1;
-                            tns_next = tns_e0;
-                        } else if (tns_phase == 1 && tns_e0 < tns_e1) {
-#pragma unroll
-                            for (int i = 0; i < 8; i++) rc[i] = rc1[i];
-                            ord = si.num_tns == 2 ? rc_order1 : 0;
-                            tns_phase = 2;
-                            tns_next = tns_e1;
-                        } else {
-                            ord = 0;
-                            tns_next = 0x7fffffff;
-                        }
-                    }
-                    om = __reduce_max_sync(0xffffffffu, ord);
-                }
-                if (om > 0) {                                           // QUIRK: lattice state carries across filters
-                    float t = v;
-#pragma unroll
-                    for (int j = 7; j >= 0; j--) {
-                        if (j < om) {                                   // warp-uniform
-                            const float t2 = xs(t, xm(rc[j], st[j]));
-                            t = j < ord ? t2 : t;
-                            if (j + 1 < 8) {
-                                const float s2 = xa(xm(rc[j], t), st[j]);
-                                st[j + 1 < 8 ? j + 1 : 7] = j + 1 < ord ? s2 : st[j + 1 < 8 ? j + 1 : 7];
-                            }
-                        }
-                    }
-                    st[0] = ord > 0 ? t : st[0];
-                    v = t;
-                }
-                o[u] = ok ? xm(v, gl[u]) : v;
-            }
+                lines(std::true_type{}, std::integral_constant<int, 8>{}, e, gl, k4, o);
             }
             // four finished lines leave as one 16-byte store into the thread's own stream-major row (the two halves of
             // a 32-byte sector are written four lines apart and meet in L2)
@@ -1037,16 +1078,7 @@ __device__ __forceinline__ void dequant_body(const EntropyParams& p, const int b
         }
     }
 
-    // ---- hand-off record for the synthesis kernel, slot flip
-    if (live) {
-        int32_t* sd = p.side + (size_t)srow * SIDE_WORDS;
-        sd[SD_OK] = ok;
-        sd[SD_LTPF_ACTIVE] = ok ? si.ltpf_active : 0;
-        sd[SD_PITCH_INDEX] = ok ? si.pitch_index : 0;
-        sd[SD_NBITS] = nbits;
-        sd[SD_SLOT] = ok ? new_slot : slot;
-        if (ok && p.fixed_slot < 0) p.sstate[(size_t)srow * SS_WORDS + SS_SLOT] = new_slot;
-    }
+    if (live) write_side(p, srow, ok, si.ltpf_active, si.pitch_index, nbits, slot, new_slot);
 }
 
 // 5 CTAs per SM (96 registers): measured against 4 (119 registers, 0.80 ms), 6 (80, 0.74 ms) and 7 (72, spills, 0.82 ms): 0.667 ms
@@ -1059,7 +1091,7 @@ template <int W>
 __global__ void __launch_bounds__(ENT_THREADS, 5) dequant_mixed_kernel(const __grid_constant__ MixedParams m) {
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
-    mixed_select(m, &s_p, &s_block);
+    mixed_select(m, &s_p, &s_block, 1);
     dequant_body<W, false>(s_p, s_block);
 }
 
@@ -1077,23 +1109,12 @@ __global__ void __launch_bounds__(ENT_THREADS, 5) dequant_mixed_kernel(const __g
 //     * frames without TNS leave finished; a frame with an active TNS filter leaves its gain-scaled lines and its 64
 //       band gains, and appends itself to a list;
 //   tns_list_kernel (one THREAD per listed frame): the TNS lattice - a true recurrence over lines - then the SNS gains,
-//     in place on the frame's spectrum row, with dequant_kernel's select-based lattice so the warp never splits.
-// Every f32 operation per line is dequant_kernel's, in its order: the spectrum is bit-identical (tested).
+//     in place on the frame's spectrum row, with the select-based lattice so the warp never splits.
+// The three kernels share one definition of each reference step (above dequant_body), so the f32 operations per line are
+// the same in the same order: the spectrum is bit-identical (tested).
 constexpr int DQW_WARPS = 8;
 __host__ __device__ inline size_t dequant_warp_smem_bytes() {
     return sizeof(float) * DQW_WARPS * (64 + 16 + 16) + MAX_NE;
-}
-
-__device__ __forceinline__ float sns_interp64(const float* scf, int j) {             // spectral_noise_shaping.rs:85-98
-    if (j < 2) return scf[0];
-    if (j >= 62) {
-        const float d = xs(scf[15], scf[14]);
-        return xa(scf[15], xm(j == 62 ? 0.125f : 0.375f, d));
-    }
-    const int n = (j - 2) >> 2, r = (j - 2) & 3;
-    const float fn = scf[n], d = xs(scf[n + 1], fn);
-    const float w = r == 0 ? 0.125f : r == 1 ? 0.375f : r == 2 ? 0.625f : 0.875f;
-    return xa(fn, xm(w, d));
 }
 
 template <bool IDS>
@@ -1150,19 +1171,10 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
     const int new_slot = p.fixed_slot >= 0 ? p.fixed_slot : slot_cur ^ 1;
     constexpr int NR = (MAX_NE + 31) / 32;                             // rows of 32 lines
     if (ok) {                                                          // warp-uniform
-        const bool d10 = c.n_ms == LC3B_10MS;
-        const int bw_stop = d10 ? 80 * (bw + 1) : 60 * (bw + 1);
-        const int nf_start = d10 ? 24 : 18;
+        const FrameScalars fs = frame_scalars(c, nbits, gg_ind, noise_factor, bw);
         // does any TNS filter of this frame do anything?  (phase 2 exists only for bw >= 3, temporal_noise_shaping.rs:83-138)
         const bool has_tns = rc_order0 > 0 || (bw >= 3 && num_tns == 2 && rc_order1 > 0);
-        float gg;
-        {                                                              // global_gain.rs:15-25
-            const int fs = c.fs_ind + 1;
-            const int gg_off = -min(nbits / (10 * fs), 115) - 105 - 5 * fs;
-            gg = c.gg_table[gg_ind + gg_off + 245];
-        }
-        const float nf_level = xd(xs(8.0f, (float)noise_factor), 16.0f);
-        // ---- SNS scale factors (spectral_noise_shaping.rs:21-98) -> 64 band gains
+        // ---- SNS scale factors -> 64 band gains
         float* scf = s_scf + wid * 16;
         float* yv = s_y + wid * 16;
         float* gband = s_gband + wid * 64;
@@ -1171,7 +1183,7 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
             const int submode_lsb = field(HO_SUBMODE_LSB), g_ind = field(HO_G_IND), ls_inda = field(HO_LS_INDA);
             const int ls_indb = field(HO_LS_INDB), idx_a = field(HO_IDX_A), idx_b = field(HO_IDX_B);
             const int shape_j = (submode_msb << 1) + submode_lsb;
-            if (lane == 0) {
+            if (lane == 0) {                                            // the thread kernel's switch, see there
                 switch (shape_j) {
                     case 0:
                         mpvq_deenum(10, 10, ls_inda, (uint32_t)idx_a, yv, 1);
@@ -1190,28 +1202,13 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
                 const float* gains = shape_j == 0 ? LC3T_SNS_VQ_REG_ADJ_GAINS : shape_j == 1 ? LC3T_SNS_VQ_REG_LF_ADJ_GAINS
                                      : shape_j == 2 ? LC3T_SNS_VQ_NEAR_ADJ_GAINS : LC3T_SNS_VQ_FAR_ADJ_GAINS;
                 float y[16];
-                float sum = 0.0f;
-#pragma unroll
-                for (int i = 0; i < 16; i++) { y[i] = yv[i]; sum = xa(sum, xm(y[i], y[i])); }
-                const float y_norm = sqrtf(sum);
-                float g = gains[g_ind];
-                if (y_norm != 0.0f) g = xd(g, y_norm);
-                float factor = 0.0f;
-#pragma unroll
-                for (int col = 0; col < 16; col++) factor = xa(factor, xm(y[col], LC3T_D[lane][col]));
-                const float st1 = lane < 8 ? LC3T_LFCB[ind_lf][lane] : LC3T_HFCB[ind_hf][lane - 8];
-                scf[lane] = xa(st1, xm(g, factor));
+                const float g = sns_norm_gain(yv, 1, gains, g_ind, y);
+                scf[lane] = sns_scale_factor(y, g, lane, ind_lf, ind_hf);
             }
             __syncwarp();
-            const int n2 = 64 - nb;
-            for (int b0 = 0; b0 < 64; b0 += 32) {                      // :100-123 incl. the nb < 64 folding
+            for (int b0 = 0; b0 < 64; b0 += 32) {
                 const int b = b0 + lane;
-                if (b < nb) {
-                    float sc;
-                    if (n2 != 0) sc = b < n2 ? xd(xa(sns_interp64(scf, 2 * b), sns_interp64(scf, 2 * b + 1)), 2.0f) : sns_interp64(scf, b + n2);
-                    else sc = sns_interp64(scf, b);
-                    gband[b] = exp2_raw_fm(sc);
-                }
+                if (b < nb) gband[b] = sns_band_gain<1>(scf, b, nb);
             }
             __syncwarp();
         }
@@ -1223,7 +1220,7 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
         for (int j = 0; j < NR; j++) {
             const int k = 32 * j + lane;
             x[j] = (32 * j < ne && k < lastnz) ? xq[xq_off(k)] : 0;    // lastnz <= ne
-            nzb[j] = __ballot_sync(0xffffffffu, x[j] != 0 && k < bw_stop);
+            nzb[j] = __ballot_sync(0xffffffffu, x[j] != 0 && k < fs.bw_stop);
         }
         const bool is_zero_frame = lastnz == 2 && (__ballot_sync(0xffffffffu, x[0] != 0) & 3u) == 0 && gg_ind == 0;
         const uint8_t* fr = p.frames + (size_t)stream * p.frame_stride;
@@ -1243,23 +1240,22 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
                     const int pos = tail + rank;
                     const int bidx = max(len - 1 - (pos >> 3), 0);
                     const uint32_t bit = take ? ((uint32_t)fr[bidx] >> (pos & 7)) & 1u : 0u;
-                    const float up = xi > 0 ? 0.3125f : 0.1875f, down = xi > 0 ? -0.1875f : -0.3125f;
-                    v = take ? xa(v, bit ? up : down) : v;
+                    v = take ? residual_refine(v, xi, bit) : v;
                 }
                 {   // noise_filling.rs:37-55: lines whose +-W neighbourhood holds no non-zero integer
                     const uint32_t lo = j > 0 ? nzb[j > 0 ? j - 1 : 0] : 0u, mid = nzb[j], hi = j + 1 < NR ? nzb[j + 1 < NR ? j + 1 : j] : 0u;
                     const uint64_t a = ((uint64_t)mid << 32) | lo, b = ((uint64_t)hi << 32) | mid;
                     const uint32_t wm = (1u << (W + 1)) - 1u;
                     const uint32_t near = ((uint32_t)(a >> (32 + lane - W)) | (uint32_t)(b >> lane)) & wm;
-                    const bool fill = !is_zero_frame && k >= nf_start && k < bw_stop && near == 0;
+                    const bool fill = !is_zero_frame && k >= fs.nf_start && k < fs.bw_stop && near == 0;
                     const uint32_t fm = __ballot_sync(0xffffffffu, fill);
                     const int n = fill_base + __popc(fm & lt_mask) + 1;     // this line takes the LCG's n-th output
                     fill_base += __popc(fm);
                     const uint32_t ac = c.nf_lcg[fill ? n : 0];
                     const uint32_t st = ((ac >> 16) * seed0 + (ac & 0xffffu)) & 0xffffu;
-                    v = fill ? (st < 0x8000u ? nf_level : -nf_level) : v;
+                    v = fill ? nf_fill_level(st, fs.nf_level) : v;
                 }
-                v = xm(v, gg);
+                v = xm(v, fs.gg);
                 if (k < ne) dst[k] = has_tns ? v : xm(v, gband[s_band_of[k]]);   // coalesced row
             }
         }
@@ -1270,15 +1266,7 @@ __device__ __forceinline__ void dequant_warp_body(const EntropyParams& p, const 
             if (lane == 0) p.tns_list[2 + atomicAdd(p.tns_list, 1)] = slot;
         }
     }
-    if (live && lane == 0) {
-        int32_t* sd = p.side + (size_t)srow * SIDE_WORDS;
-        sd[SD_OK] = ok;
-        sd[SD_LTPF_ACTIVE] = ok ? ltpf_active : 0;
-        sd[SD_PITCH_INDEX] = ok ? pitch_index : 0;
-        sd[SD_NBITS] = nbits;
-        sd[SD_SLOT] = ok ? new_slot : slot_cur;
-        if (ok && p.fixed_slot < 0) p.sstate[(size_t)srow * SS_WORDS + SS_SLOT] = new_slot;
-    }
+    if (live && lane == 0) write_side(p, srow, ok, ltpf_active, pitch_index, nbits, slot_cur, new_slot);
 }
 
 // The listed frames' lattices, one thread each: temporal_noise_shaping.rs:24-74 then the SNS gains, four lines at a time
@@ -1317,31 +1305,17 @@ __device__ __forceinline__ void tns_list_body(const EntropyParams& p, const int 
             s_g[(4 * q + 3) * ENT_THREADS + tid] = g4.w;
         }
     }
-    int ord0 = 0, ord1 = 0, s0 = 0x7fffffff, e0 = 0, e1 = 0;
-    float rc0[8] = {0, 0, 0, 0, 0, 0, 0, 0}, rc1[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    TnsPlan tf{};
     float* row = p.spec;
     if (mine) {
         const int stream = state_row<IDS>(p.ids, (slot / ENT_THREADS) * ENT_THREADS + ho[HO_FID]);   // listed frames are live
-        const int bw = ho[HO_BW];
-        const bool d10 = c.n_ms == LC3B_10MS;
-        const int bw_stop = d10 ? 80 * (bw + 1) : 60 * (bw + 1);
-        s0 = d10 ? 12 : 9;
-        if (bw < 3) { e0 = bw_stop; e1 = bw_stop; }
-        else { e0 = bw_stop / 2; e1 = bw_stop; }
-        ord0 = ho[HO_RC_ORDER0];
-        ord1 = ho[HO_NUM_TNS] == 2 ? ho[HO_RC_ORDER1] : 0;
-#pragma unroll
-        for (int j = 0; j < 8; j++) {                                  // QUIRK: index 0 -> rc = 0.0
-            const int a = ho[HO_RC_I + j], b = ho[HO_RC_I + 8 + j];
-            rc0[j] = a != 0 ? c.tns_sin[a] : 0.0f;
-            rc1[j] = b != 0 ? c.tns_sin[b] : 0.0f;
-        }
+        tns_plan(tf, c, ho[HO_BW], ho[HO_NUM_TNS], ho[HO_RC_ORDER0], ho[HO_RC_ORDER1], ho + HO_RC_I);
         const int cur = p.fixed_slot >= 0 ? p.fixed_slot : p.sstate[(size_t)stream * SS_WORDS + SS_SLOT];
         row = p.spec + ((size_t)cur * p.slot_streams + stream) * ne;
     }
     __syncthreads();
     float st[8] = {0, 0, 0, 0, 0, 0, 0, 0}, rc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    int ord = 0, om = 0, phase = 0, next = s0;
+    int ord = 0, om = 0, phase = 0, next = mine ? tf.s0 : 0x7fffffff;
     int band = 0, band_end = mine ? s_edge[1] : 0x7fffffff;
     float gcur = mine ? s_g[tid] : 0.0f;
     const int n4 = ne >> 2;                                            // ne is a multiple of 4 in every configuration
@@ -1357,35 +1331,10 @@ __device__ __forceinline__ void tns_list_body(const EntropyParams& p, const int 
             float v = vv[e];
             const bool sw = k == next;
             if (__any_sync(0xffffffffu, sw)) {
-                if (sw) {
-                    if (phase == 0) {
-#pragma unroll
-                        for (int j = 0; j < 8; j++) rc[j] = rc0[j];
-                        ord = ord0; phase = 1; next = e0;
-                    } else if (phase == 1 && e0 < e1) {
-#pragma unroll
-                        for (int j = 0; j < 8; j++) rc[j] = rc1[j];
-                        ord = ord1; phase = 2; next = e1;
-                    } else { ord = 0; next = 0x7fffffff; }
-                }
+                if (sw) tns_switch(tf, rc, ord, phase, next);
                 om = __reduce_max_sync(0xffffffffu, ord);
             }
-            if (om > 0) {                                              // QUIRK: lattice state carries across filters
-                float t = v;
-#pragma unroll
-                for (int j = 7; j >= 0; j--) {
-                    if (j < om) {                                      // warp-uniform
-                        const float t2 = xs(t, xm(rc[j], st[j]));
-                        t = j < ord ? t2 : t;
-                        if (j + 1 < 8) {
-                            const float s2 = xa(xm(rc[j], t), st[j]);
-                            st[j + 1 < 8 ? j + 1 : 7] = j + 1 < ord ? s2 : st[j + 1 < 8 ? j + 1 : 7];
-                        }
-                    }
-                }
-                st[0] = ord > 0 ? t : st[0];
-                v = t;
-            }
+            v = tns_lattice_line(v, rc, st, ord, om);
             while (k >= band_end) {                                    // next band; zero-width bands are skipped
                 band++;
                 band_end = s_edge[band + 1 < 64 ? band + 1 : 64];
@@ -1409,35 +1358,17 @@ __global__ void __launch_bounds__(ENT_THREADS) tns_list_kernel(const __grid_cons
     tns_list_body<IDS>(p, blockIdx.x);
 }
 
-// mixed-rate variants.  per_cta_slots: thread slots one CTA covers (DQW_WARPS for the warp kernel, ENT_THREADS for the list
-// kernel); a bucket's first_cta counts entropy CTAs of ENT_THREADS slots.
-__device__ __forceinline__ void mixed_select_scaled(const MixedParams& m, EntropyParams* s_p, int* s_block, int per_entropy_cta) {
-    if (threadIdx.x == 0) {
-        int b = 0;
-        while (b + 1 < m.n_buckets && (int)blockIdx.x >= m.buckets[b + 1].first_cta * per_entropy_cta) b++;
-        const MixedBucket& bk = m.buckets[b];
-        EntropyParams q = bk.ep;
-        q.frames = m.frames + (size_t)bk.first_row * m.frame_stride;
-        q.frame_nbytes = m.frame_nbytes ? m.frame_nbytes + bk.first_row : nullptr;
-        q.nbytes = m.nbytes;
-        q.frame_stride = m.frame_stride;
-        q.status_out = m.status_out ? m.status_out + bk.first_row : nullptr;
-        q.row_pitch = m.row_pitch;
-        *s_p = q;
-        *s_block = (int)blockIdx.x - bk.first_cta * per_entropy_cta;
-    }
-    __syncthreads();
-}
+// mixed-rate variants
 __global__ void __launch_bounds__(DQW_WARPS * 32) dequant_warp_mixed_kernel(const __grid_constant__ MixedParams m) {
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
-    mixed_select_scaled(m, &s_p, &s_block, ENT_THREADS / DQW_WARPS);
+    mixed_select(m, &s_p, &s_block, ENT_THREADS / DQW_WARPS);
     dequant_warp_body<false>(s_p, s_block);
 }
 __global__ void __launch_bounds__(ENT_THREADS) tns_list_mixed_kernel(const __grid_constant__ MixedParams m) {
     __shared__ EntropyParams s_p;
     __shared__ int s_block;
-    mixed_select_scaled(m, &s_p, &s_block, 1);
+    mixed_select(m, &s_p, &s_block, 1);
     tns_list_body<false>(s_p, s_block);
 }
 
