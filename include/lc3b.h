@@ -125,6 +125,31 @@ int lc3b_decode_stream_frames(lc3b_decoder* h, int bits_per_sample, const uint8_
                               int nbytes, size_t frame_stride, int n_frames, int16_t* pcm_out, int32_t* status_out,
                               void* scratch, size_t scratch_bytes, void* cuda_stream);
 
+/* Time-parallel decode of a chosen subset of streams, each with its own number of frames: a batch of files of different
+ * lengths in one handle, or per-stream jitter buffers of different depths, in one call.  Row i of the call advances
+ * stream stream_ids[i] by frame_counts[i] frames and equals that many lc3b_decode_frames calls on it (same PCM, status
+ * and per-stream state afterwards); streams not listed, and rows with count 0, are untouched.
+ *   stream_ids, frame_counts  HOST int32[n_rows], only read during the call.  Ids as in lc3b_decode_frames_subset (any
+ *               order, each in [0, n_streams) and at most once); counts >= 0.
+ *   units       let off_i be the sum of frame_counts[0 .. i-1] (the caller's row order): frame f of row i is unit off_i + f,
+ *               so each row's frames and audio are contiguous and rows follow each other in the caller's order
+ *   frames      device; unit v at frames + v*frame_stride
+ *   frame_nbytes, status_out  device int32[total] or NULL, one per unit (as in lc3b_decode_stream_frames)
+ *   pcm_out     device int16; unit v at pcm_out + v*nf
+ *   scratch     device, at least lc3b_decoder_multi_subset_scratch_bytes(h, n_rows, total) bytes, 256-byte aligned;
+ *               caller-owned, only used during the call
+ * total = sum of the counts.  Returns LC3B_OK and enqueues nothing when n_rows or total is 0; LC3B_ERR_INVALID_ARG for a
+ * bad or duplicate id, a negative count, a total beyond 0x7fffffff / 512 and the argument errors of
+ * lc3b_decode_stream_frames; LC3B_ERR_WORKSPACE for scratch that is too small or misaligned; LC3B_ERR_BITS_PER_SAMPLE
+ * when bits_per_sample != 16.  Nothing is enqueued on an error.  The row table is copied to the front of the scratch with
+ * one cudaMemcpyAsync on `cuda_stream`.  lc3b_decoder_set_split and set_dequant_mode apply as to
+ * lc3b_decode_stream_frames, by the total. */
+int lc3b_decoder_multi_subset_scratch_bytes(const lc3b_decoder* h, int n_rows, long long total_frames, size_t* device_bytes);
+int lc3b_decode_stream_frames_subset(lc3b_decoder* h, int bits_per_sample, const int32_t* stream_ids, const int32_t* frame_counts,
+                                     int n_rows, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
+                                     size_t frame_stride, int16_t* pcm_out, int32_t* status_out, void* scratch,
+                                     size_t scratch_bytes, void* cuda_stream);
+
 /* Inspection (parity gate i, SURVEY.md 8d): when set, every decode also writes, per stream, a record of
  * LC3B_TRACE_WORDS int32 (layout below) and the entropy-decoded integer spectrum x[0..ne).  Device pointers,
  * NULL to disable.  trace: [n_streams][LC3B_TRACE_WORDS], x: [n_streams][ne].  lc3b_decode_frames_subset writes
@@ -271,6 +296,21 @@ int lc3b_encoder_set_host_pipelining(lc3b_encoder* h, int on);
 int lc3b_encoder_multi_scratch_bytes(const lc3b_encoder* h, int n_frames, size_t* device_bytes);
 int lc3b_encode_stream_frames(lc3b_encoder* h, const int16_t* pcm_in, int n_frames, uint8_t* frames_out, int nbytes,
                               size_t frame_stride, void* scratch, size_t scratch_bytes, void* cuda_stream);
+/* Time-parallel encode of a chosen subset of streams, each with its own number of frames (the encoder twin of
+ * lc3b_decode_stream_frames_subset, same ids, counts and unit layout).  Row i equals frame_counts[i] calls of
+ * lc3b_encode_frames on stream stream_ids[i] with the same `nbytes` (same bytes and per-stream state afterwards); streams
+ * not listed, and rows with count 0, are untouched.
+ *   pcm_in      device int16; unit v at pcm_in + v*nf
+ *   frames_out  device; unit v at frames_out + v*frame_stride, `nbytes` bytes each
+ *   scratch     device, at least lc3b_encoder_multi_subset_scratch_bytes(h, n_rows, total) bytes, 256-byte aligned
+ * Returns LC3B_OK and enqueues nothing when n_rows or total is 0; LC3B_ERR_INVALID_ARG for a bad or duplicate id, a
+ * negative count, a total beyond INT32_MAX and the argument errors of lc3b_encode_stream_frames; LC3B_ERR_WORKSPACE for
+ * scratch that is too small or misaligned.  Nothing is enqueued on an error.  Follows lc3b_encoder_set_graph_mode like
+ * lc3b_encode_stream_frames; the row table goes to the front of the scratch with one cudaMemcpyAsync on `cuda_stream`. */
+int lc3b_encoder_multi_subset_scratch_bytes(const lc3b_encoder* h, int n_rows, long long total_frames, size_t* device_bytes);
+int lc3b_encode_stream_frames_subset(lc3b_encoder* h, const int32_t* stream_ids, const int32_t* frame_counts, int n_rows,
+                                     const int16_t* pcm_in, uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch,
+                                     size_t scratch_bytes, void* cuda_stream);
 int lc3b_encoder_set_graph_mode(lc3b_encoder* h, int mode);   /* as lc3b_decoder_set_graph_mode */
 /* Test hook: device copies of the last encode's intermediates (any pointer may be NULL): xf [S][ne] f32 (quantiser
  * input, after SNS and TNS), e_b [S][64] f32, hand [S][8] i32 (near_nyquist, attack, pitch_index, pitch_present,

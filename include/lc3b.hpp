@@ -129,6 +129,26 @@ class Lc3BatchDecoder {
         detail::check(rc, "lc3b_decode_stream_frames");
         return std::nullopt;
     }
+    // Ragged time-parallel decode: frame_counts[i] consecutive frames of stream stream_ids[i] (host arrays of n_rows, ids
+    // as in decode_frames_subset, counts >= 0); equivalent to that many decode_frames calls on each listed stream.  Units are
+    // packed row after row in the caller's order: device frames [total][nbytes], samples_out [total * nf], frame_nbytes /
+    // status_out [total]; scratch >= multi_subset_scratch_bytes(n_rows, total) bytes (caller-owned).
+    size_t multi_subset_scratch_bytes(size_t n_rows, long long total_frames) const {
+        size_t n = 0;
+        detail::check(lc3b_decoder_multi_subset_scratch_bytes(h_, (int)n_rows, total_frames, &n), "lc3b_decoder_multi_subset_scratch_bytes");
+        return n;
+    }
+    Result<Lc3DecoderError> decode_stream_frames_subset(size_t num_bits_per_audio_sample, const int32_t* stream_ids,
+                                                        const int32_t* frame_counts, size_t n_rows, const uint8_t* frames,
+                                                        size_t nbytes, int16_t* samples_out, void* scratch, size_t scratch_bytes,
+                                                        const int32_t* frame_nbytes = nullptr, int32_t* status_out = nullptr) {
+        const int rc = lc3b_decode_stream_frames_subset(h_, (int)num_bits_per_audio_sample, stream_ids, frame_counts, (int)n_rows,
+                                                        frames, frame_nbytes, (int)nbytes, nbytes, samples_out, status_out, scratch,
+                                                        scratch_bytes, stream_);
+        if (rc == LC3B_ERR_BITS_PER_SAMPLE) return Lc3DecoderError::Only16BitsPerAudioSampleSupported;
+        detail::check(rc, "lc3b_decode_stream_frames_subset");
+        return std::nullopt;
+    }
     // extension: issue every call as one cached CUDA graph (true) or one launch per kernel (false); same results
     void set_graph_mode(bool on) { detail::check(lc3b_decoder_set_graph_mode(h_, on ? 1 : 0), "lc3b_decoder_set_graph_mode"); }
     // extension: cut every call into k independent sub-batches whose kernels overlap (0 = by batch size, 1, 2, 4); same results
@@ -200,6 +220,22 @@ class Lc3BatchEncoder {
         detail::check(lc3b_encode_stream_frames(h_, samples_in, (int)n_frames, buf_out, (int)nbytes, frame_stride, scratch,
                                                 scratch_bytes, stream_),
                       "lc3b_encode_stream_frames");
+        return std::nullopt;
+    }
+    // Ragged time-parallel encode: frame_counts[i] consecutive frames of stream stream_ids[i] (host arrays of n_rows);
+    // equivalent to that many encode_frames calls on each listed stream.  Units packed row after row in the caller's
+    // order: samples_in [total * nf], buf_out unit v at v * frame_stride; scratch >= multi_subset_scratch_bytes(n_rows, total).
+    size_t multi_subset_scratch_bytes(size_t n_rows, long long total_frames) const {
+        size_t n = 0;
+        detail::check(lc3b_encoder_multi_subset_scratch_bytes(h_, (int)n_rows, total_frames, &n), "lc3b_encoder_multi_subset_scratch_bytes");
+        return n;
+    }
+    Result<Lc3EncoderError> encode_stream_frames_subset(const int32_t* stream_ids, const int32_t* frame_counts, size_t n_rows,
+                                                        const int16_t* samples_in, uint8_t* buf_out, size_t nbytes, size_t frame_stride,
+                                                        void* scratch, size_t scratch_bytes) {
+        detail::check(lc3b_encode_stream_frames_subset(h_, stream_ids, frame_counts, (int)n_rows, samples_in, buf_out, (int)nbytes,
+                                                       frame_stride, scratch, scratch_bytes, stream_),
+                      "lc3b_encode_stream_frames_subset");
         return std::nullopt;
     }
     void set_host_pipelining(bool on) { detail::check(lc3b_encoder_set_host_pipelining(h_, on ? 1 : 0), "lc3b_encoder_set_host_pipelining"); }

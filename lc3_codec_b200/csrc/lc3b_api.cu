@@ -493,6 +493,35 @@ int lc3b_decode_stream_frames(lc3b_decoder* h, int bits_per_sample, const uint8_
     return LC3B_OK;
 }
 
+static constexpr long long MULTI_MAX_UNITS = 0x7fffffffLL / 512;          // 32-bit unit indices
+
+int lc3b_decoder_multi_subset_scratch_bytes(const lc3b_decoder* h, int n_rows, long long total_frames, size_t* device_bytes) {
+    if (!h || !device_bytes || n_rows < 0 || n_rows > h->st.n_streams || total_frames < 0 || total_frames > MULTI_MAX_UNITS)
+        return LC3B_ERR_INVALID_ARG;
+    *device_bytes = multi_rows_scratch_bytes(h->st, n_rows, total_frames);
+    return LC3B_OK;
+}
+
+int lc3b_decode_stream_frames_subset(lc3b_decoder* h, int bits_per_sample, const int32_t* stream_ids, const int32_t* frame_counts,
+                                     int n_rows, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
+                                     size_t frame_stride, int16_t* pcm_out, int32_t* status_out, void* scratch,
+                                     size_t scratch_bytes, void* cuda_stream) {
+    if (!h || !stream_ids || !frame_counts) return LC3B_ERR_INVALID_ARG;
+    if (bits_per_sample != 16) return LC3B_ERR_BITS_PER_SAMPLE;             // lc3_decoder.rs:80
+    const DecoderState& st = h->st;
+    if (nbytes <= 0 || nbytes > st.max_nbytes || frame_stride < (size_t)nbytes) return LC3B_ERR_INVALID_ARG;
+    RowTable& rt = h->row_table;
+    if (!rt.take(h->id_list, stream_ids, frame_counts, n_rows, st.n_streams, MULTI_MAX_UNITS)) return LC3B_ERR_INVALID_ARG;
+    if (rt.total == 0) return LC3B_OK;
+    if (!frames || !pcm_out || !scratch) return LC3B_ERR_INVALID_ARG;
+    if (scratch_bytes < multi_rows_scratch_bytes(st, n_rows, rt.total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    CU(rt.send(scratch, stream));
+    CU(launch_decode_multi_rows(st, frames, frame_nbytes, nbytes, frame_stride, n_rows, rt.n_live, rt.total, pcm_out, status_out,
+                                scratch, stream, h->split == 1 ? nullptr : &h->lanes));
+    return LC3B_OK;
+}
+
 int lc3b_decoder_set_trace(lc3b_decoder* h, int32_t* trace, int32_t* x) {
     if (!h) return LC3B_ERR_INVALID_ARG;
     h->st.trace = trace;

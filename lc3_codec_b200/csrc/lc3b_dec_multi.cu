@@ -17,6 +17,10 @@
 //                           overwriting those frames' PCM; then leaves the handle's per-stream state (overlap memory,
 //                           LTPF ring, last good spectrum) exactly as F frame-by-frame calls would have
 // Arithmetic is the frame-by-frame path's, operation for operation, so both paths produce identical PCM.
+//
+// A ragged call (lc3b_decode_stream_frames_subset, the RAGGED instantiations) lists rows of any frame counts: stages 1, 3
+// and 4 run over its units unchanged, stages 2 and 5 run a warp per row of the row table (lc3b_common.cuh) and address the
+// handle's state by the row's state row.  Stages 3 and 4 find a unit's row in unit_row[], written by unit_rows_kernel.
 #include "lc3b_common.cuh"
 #include "lc3b_imdct.cuh"
 #include "lc3b_plan.cuh"
@@ -25,13 +29,14 @@
 
 namespace lc3b {
 
-struct MultiLayout { size_t spec, xq, handoff, gband, tns_list, side, head, tail, xhat, last_good, total; };
+struct MultiLayout { size_t rows, spec, xq, handoff, gband, tns_list, side, head, tail, xhat, last_good, unit_row, total; };
 
-static MultiLayout multi_layout(const lc3b_config& c, int S, int F) {
+// V units of S rows; ragged: the row table at the front (where RowTable::send puts it) and unit_row[V] at the end
+static MultiLayout multi_layout(const lc3b_config& c, int S, size_t V, bool ragged) {
     MultiLayout L;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~(size_t)255; return o; };
-    const size_t V = (size_t)S * F;
+    L.rows = take(ragged ? sizeof(int32_t) * RT_WORDS * S : 0);
     const size_t nblk = ((V + 127) / 128) * 4;                    // 32-stream blocks, whole entropy CTAs
     L.spec = take(sizeof(float) * V * c.ne);
     L.xq = take(sizeof(int32_t) * nblk * c.ne * 32);
@@ -43,25 +48,34 @@ static MultiLayout multi_layout(const lc3b_config& c, int S, int F) {
     L.tail = take(sizeof(float) * V * (c.nf - c.z));
     L.xhat = take(sizeof(float) * V * c.nf);
     L.last_good = take(sizeof(int32_t) * S);
+    L.unit_row = take(ragged ? sizeof(int32_t) * V : 0);
     L.total = off;
     return L;
 }
 
-size_t multi_scratch_bytes(const DecoderState& st, int n_frames) { return multi_layout(st.cfg, st.n_streams, n_frames).total; }
+size_t multi_scratch_bytes(const DecoderState& st, int n_frames) {
+    return multi_layout(st.cfg, st.n_streams, (size_t)st.n_streams * n_frames, false).total;
+}
+size_t multi_rows_scratch_bytes(const DecoderState& st, int n_rows, long long total) {
+    return multi_layout(st.cfg, n_rows, (size_t)total, true).total;
+}
 
 struct MultiParams {
     const DevConfig* cfg;
     const float* win;
     const float2* dtw;
     const float2* ftw;
-    int S, F;
+    int S, F;             // the handle's streams; frames per row of a dense call
+    int n_rows, V;        // ragged call: rows of the row table, units
+    const int32_t* rows;  // ragged call: row table (lc3b_common.cuh)
+    int32_t* unit_row;    // ragged call: [V] the state row of each unit's row, ~row for a row's first unit
     // per-unit scratch
     const float* spec_v;
     int32_t* side_v;
     float* head;
     float* tail;
     float* xhat;
-    int32_t* last_good;
+    int32_t* last_good;   // [rows]
     // the handle's per-stream state
     float* spec;
     float* ola;
@@ -78,10 +92,13 @@ constexpr int MW = 4;     // warps per CTA in the warp-per-unit kernels
 // ---------------------------------------------------------------- 2. concealment bookkeeping along time
 // One warp per stream; the ok flags are fetched 32 frames at a time so that the walk along time is not one dependent
 // global load per frame.  Every lane tracks the same running state; lane j writes frame j's record.
+template <bool RAGGED>
 __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int s = blockIdx.x * MW + wid;
-    if (s >= p.S) return;
+    const int r = blockIdx.x * MW + wid;
+    if (r >= (RAGGED ? p.n_rows : p.S)) return;
+    const RowSpan rs = row_span<RAGGED>(p.rows, r, p.F);
+    const int s = rs.row, F = rs.count, v0 = rs.off;
     const int ne = p.cfg->ne;
     int32_t* ss = p.sstate + (size_t)s * SS_WORDS;
     int lost = ss[SS_PLC_LOST];
@@ -90,18 +107,18 @@ __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
     __syncwarp();
     const PlcJump jump = plc_lcg_jump(ne);                         // a concealed frame takes ne steps of the LCG
     int last = -1;
-    for (int f0 = 0; f0 < p.F; f0 += 32) {
+    for (int f0 = 0; f0 < F; f0 += 32) {
         const int f = f0 + lane;
-        const int v = s * p.F + f;
+        const int v = v0 + f;
         int32_t* sd = p.side_v + (size_t)v * SIDE_WORDS;
-        const bool in = f < p.F;
+        const bool in = f < F;
         const bool ok = in && sd[SD_OK] != 0;
         const uint32_t okm = __ballot_sync(0xffffffffu, ok), inm = __ballot_sync(0xffffffffu, in);
         if (okm == inm) {                                          // the usual chunk: every frame decoded
             if (in) sd[SD_SRC] = -2;
             lost = 0;
             alpha = 1.0f;
-            last = s * p.F + f0 + (31 - __clz(inm));
+            last = v0 + f0 + (31 - __clz(inm));
             continue;
         }
         const int cnt = __popc(inm);
@@ -109,7 +126,7 @@ __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
             if ((okm >> j) & 1u) {
                 lost = 0;
                 alpha = 1.0f;
-                last = s * p.F + f0 + j;
+                last = v0 + f0 + j;
                 if (lane == j) sd[SD_SRC] = -2;
             } else {
                 alpha = plc_fade(alpha, lost);
@@ -127,20 +144,20 @@ __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
         ss[SS_PLC_LOST] = lost;
         ss[SS_PLC_ALPHA] = (int32_t)f2u(alpha);
         ss[SS_PLC_SEED] = (int32_t)seed;
-        p.last_good[s] = last;
+        p.last_good[r] = last;
     }
 }
 
 // ---------------------------------------------------------------- 3. spectrum -> windowed time signal, per unit
-template <int NF, bool MS10>
+template <int NF, bool MS10, bool RAGGED>
 __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
     using G = FrameGeo<NF, MS10>;
     constexpr int NE = G::NE, Z = G::Z, NP = G::NP, NPT = G::NPT;
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const long long v = (long long)blockIdx.x * MW + wid;
-    if (v >= (long long)p.S * p.F) return;
-    const int s = (int)(v / p.F);
+    if (v >= (RAGGED ? (long long)p.V : (long long)p.S * p.F)) return;
+    const int s = RAGGED ? 0 : (int)(v / p.F);
     float* P = (float*)smem + (size_t)wid * 2 * NF;
     float* Q = P + NF;
 
@@ -149,7 +166,10 @@ __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
     const float* sp;
     if (src == -2) sp = p.spec_v + (size_t)v * NE;
     else if (src >= 0) sp = p.spec_v + (size_t)src * NE;
-    else sp = p.spec + ((size_t)p.sstate[(size_t)s * SS_WORDS + SS_SLOT] * p.S + s) * NE;   // last good of earlier calls
+    else {                                                        // last good of earlier calls
+        const int sr = RAGGED ? unit_state_row(p.unit_row[v]) : s;
+        sp = p.spec + ((size_t)p.sstate[(size_t)sr * SS_WORDS + SS_SLOT] * p.S + sr) * NE;
+    }
     if (src == -2) {
 #pragma unroll
         for (int k0 = 0; k0 < NF / 4; k0 += 32) {
@@ -175,15 +195,25 @@ __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
 }
 
 // ---------------------------------------------------------------- 4. overlap-add across units, PCM
+template <bool RAGGED>
 __global__ void __launch_bounds__(MW * 32) ola_multi_kernel(MultiParams p) {
     const DevConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const long long v = (long long)blockIdx.x * MW + wid;
-    if (v >= (long long)p.S * p.F) return;
+    if (v >= (RAGGED ? (long long)p.V : (long long)p.S * p.F)) return;
     const int nf = c.nf, z = c.z;
-    const int s = (int)(v / p.F), f = (int)(v - (long long)s * p.F);
+    int s;
+    bool cont;                                                     // not the first frame of its row: the previous unit's tail
+    if constexpr (RAGGED) {
+        const int u = p.unit_row[v];
+        s = unit_state_row(u);
+        cont = u >= 0;
+    } else {
+        s = (int)(v / p.F);
+        cont = (int)(v - (long long)s * p.F) > 0;
+    }
     const float* head = p.head + (size_t)v * nf;
-    const float* prev = f > 0 ? p.tail + (size_t)(v - 1) * (nf - z) : p.ola + (size_t)s * (nf - z);
+    const float* prev = cont ? p.tail + (size_t)(v - 1) * (nf - z) : p.ola + (size_t)s * (nf - z);
     float* xhat = p.xhat + (size_t)v * nf;
     int16_t* out = p.pcm_out + (size_t)v * nf;                     // [S][F * nf]
     for (int n = lane; n < nf; n += 32) {
@@ -195,14 +225,19 @@ __global__ void __launch_bounds__(MW * 32) ola_multi_kernel(MultiParams p) {
 }
 
 // ---------------------------------------------------------------- 5. LTPF over its active spans + state hand-back
+// The dense instantiation keeps the stream, frame count and first unit as it computed them before the row table existed:
+// taken from a RowSpan they cost it spills.
+template <bool RAGGED>
 __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const DevConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int s = blockIdx.x * MW + wid;
-    if (s >= p.S) return;
+    const int r = blockIdx.x * MW + wid;
+    if (r >= (RAGGED ? p.n_rows : p.S)) return;
+    const RowSpan rs = row_span<RAGGED>(p.rows, r, p.F);
+    const int s = RAGGED ? rs.row : r;
     const LtpfGeo g = ltpf_geo(c, p.hist_len);
-    const int nf = g.nf, ne = c.ne, z = c.z, F = p.F, blocks = g.blocks;
+    const int nf = g.nf, ne = c.ne, z = c.z, F = RAGGED ? rs.count : p.F, blocks = g.blocks;
     float* Y = (float*)(smem + (size_t)wid * p.smem_per_warp);     // per-warp buffer, see ltpf_warp_bytes
     float* X = Y + p.hist_len;
     float* xt = X + nf;
@@ -217,7 +252,7 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
     for (int n = lane; n < p.hist_len; n += 32) Y[n] = yhist[n];
     __syncwarp();
     bool span1 = false, span2 = false, span3 = false;              // were frames f-1 / f-2 / f-3 filtered by this kernel
-    const size_t v0 = (size_t)s * F;
+    const size_t v0 = RAGGED ? (size_t)rs.off : (size_t)s * F;
     uint32_t actm = 0;                                             // LTPF-active flags of the current 32-frame chunk
     for (int f = 0; f < F; f++) {
         if ((f & 31) == 0) {                                       // fetch 32 frames' flags at once; skip idle chunks
@@ -276,7 +311,7 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
         float* ola = p.ola + (size_t)s * (nf - z);
         for (int n = lane; n < nf - z; n += 32) ola[n] = t[n];
     }
-    const int lg = p.last_good[s];
+    const int lg = p.last_good[r];
     if (lg >= 0) {                                                 // PacketLossConcealment::save of the last good frame
         const float* src = p.spec_v + (size_t)lg * ne;
         float* dst = p.spec + ((size_t)(slot ^ 1) * p.S + s) * ne;
@@ -289,24 +324,46 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
     }
 }
 
+// ---------------------------------------------------------------- ragged calls: each unit's row, for stages 3 and 4
+__global__ void __launch_bounds__(MW * 32) unit_rows_kernel(MultiParams p) {
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int r = blockIdx.x * MW + wid;
+    if (r >= p.n_rows) return;
+    const RowSpan rs = row_span<true>(p.rows, r, 0);
+    for (int f = lane; f < rs.count; f += 32) p.unit_row[(size_t)rs.off + f] = f ? rs.row : ~rs.row;
+}
+
+void plan_unit_rows(LaunchPlan& plan, const int32_t* rows, int n_live, int32_t* unit_row) {
+    MultiParams p;
+    memset(&p, 0, sizeof(p));
+    p.rows = rows;
+    p.unit_row = unit_row;
+    p.n_rows = n_live;
+    plan.add(unit_rows_kernel, (unsigned)((n_live + MW - 1) / MW), MW * 32, 0, p);
+}
+
 namespace {
 struct PrepareImdct {
     cudaError_t e = cudaSuccess;
     template <int NF, bool MS10> void operator()() {
-        e = cudaFuncSetAttribute(imdct_multi_kernel<NF, MS10>, cudaFuncAttributeMaxDynamicSharedMemorySize, MW * 2 * NF * 4);
+        e = cudaFuncSetAttribute(imdct_multi_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MW * 2 * NF * 4);
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(imdct_multi_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MW * 2 * NF * 4);
     }
 };
+template <bool RAGGED>
 struct PlanImdct {
     LaunchPlan& plan;
     const MultiParams& p;
     unsigned grid;
-    template <int NF, bool MS10> void operator()() { plan.add(imdct_multi_kernel<NF, MS10>, grid, MW * 32, MW * 2 * NF * 4, p); }
+    template <int NF, bool MS10> void operator()() { plan.add(imdct_multi_kernel<NF, MS10, RAGGED>, grid, MW * 32, MW * 2 * NF * 4, p); }
 };
 }  // namespace
 
 cudaError_t prepare_multi(const DecoderState& st) {
-    cudaError_t e = cudaFuncSetAttribute(ltpf_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)(ltpf_warp_bytes(st.cfg) * MW));
+    const int lb = (int)(ltpf_warp_bytes(st.cfg) * MW);
+    cudaError_t e = cudaFuncSetAttribute(ltpf_multi_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ltpf_multi_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     if (e == cudaSuccess) {
         PrepareImdct pi;
         if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
@@ -315,14 +372,14 @@ cudaError_t prepare_multi(const DecoderState& st) {
     return e;
 }
 
-cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                                size_t frame_stride, int n_frames, int16_t* pcm_out, int32_t* status_out, void* scratch,
-                                cudaStream_t stream, PlanLanes* lanes) {
-    const int S = st.n_streams, F = n_frames;
-    if (F <= 0) return cudaSuccess;
-    const MultiLayout L = multi_layout(st.cfg, S, F);
+// The dense call (rows == nullptr: S rows of F frames) and the ragged one (the n_live rows of the row table at the front of
+// the scratch, V units in all; the layout counts n_rows rows) share everything but the row addressing.
+static cudaError_t decode_multi(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
+                                size_t frame_stride, int F, bool ragged, int n_rows, int n_live, long long V, int16_t* pcm_out,
+                                int32_t* status_out, void* scratch, cudaStream_t stream, PlanLanes* lanes) {
+    const int S = st.n_streams;
+    const MultiLayout L = multi_layout(st.cfg, n_rows, (size_t)V, ragged);
     uint8_t* base = (uint8_t*)scratch;
-    const long long V = (long long)S * F;
     // 1. entropy decode of all units with the unchanged kernel: a view of the handle with V virtual streams
     DecoderState vs = st;
     vs.n_streams = (int)V;
@@ -355,6 +412,9 @@ cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, c
     memset(&p, 0, sizeof(p));
     p.cfg = st.dcfg; p.win = st.win; p.dtw = st.dtw; p.ftw = st.ftw;
     p.S = S; p.F = F;
+    p.n_rows = n_live; p.V = (int)V;
+    p.rows = ragged ? (const int32_t*)(base + L.rows) : nullptr;
+    p.unit_row = ragged ? (int32_t*)(base + L.unit_row) : nullptr;
     p.spec_v = vs.spec; p.side_v = vs.side;
     p.head = (float*)(base + L.head); p.tail = (float*)(base + L.tail); p.xhat = (float*)(base + L.xhat);
     p.last_good = (int32_t*)(base + L.last_good);
@@ -365,13 +425,40 @@ cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, c
     // 2-5. a second plan on the caller's stream: plan_launch_direct joins the entropy plan's lanes back into the caller's
     // stream only at the end of that plan, so lane-0 nodes added to it would not wait for lanes 1-3
     LaunchPlan tail;
-    const unsigned grid_s = (unsigned)((S + MW - 1) / MW), grid_v = (unsigned)((V + MW - 1) / MW);
-    tail.add(plc_scan_kernel, grid_s, MW * 32, 0, p, -1);
-    PlanImdct pi{tail, p, grid_v};
-    if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
-    tail.add(ola_multi_kernel, grid_v, MW * 32, 0, p);
-    tail.add(ltpf_multi_kernel, grid_s, MW * 32, (size_t)p.smem_per_warp * MW, p);
+    const int rows = ragged ? n_live : S;
+    const unsigned grid_s = (unsigned)((rows + MW - 1) / MW), grid_v = (unsigned)((V + MW - 1) / MW);
+    const size_t ltpf_smem = (size_t)p.smem_per_warp * MW;
+    if (ragged) {
+        plan_unit_rows(tail, p.rows, n_live, p.unit_row);
+        tail.add(plc_scan_kernel<true>, grid_s, MW * 32, 0, p);
+        PlanImdct<true> pi{tail, p, grid_v};
+        if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
+        tail.add(ola_multi_kernel<true>, grid_v, MW * 32, 0, p);
+        tail.add(ltpf_multi_kernel<true>, grid_s, MW * 32, ltpf_smem, p);
+    } else {
+        tail.add(plc_scan_kernel<false>, grid_s, MW * 32, 0, p, -1);
+        PlanImdct<false> pi{tail, p, grid_v};
+        if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
+        tail.add(ola_multi_kernel<false>, grid_v, MW * 32, 0, p);
+        tail.add(ltpf_multi_kernel<false>, grid_s, MW * 32, ltpf_smem, p);
+    }
     return plan_launch_direct(tail, stream);
+}
+
+cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
+                                size_t frame_stride, int n_frames, int16_t* pcm_out, int32_t* status_out, void* scratch,
+                                cudaStream_t stream, PlanLanes* lanes) {
+    if (n_frames <= 0) return cudaSuccess;
+    return decode_multi(st, frames, frame_nbytes, nbytes, frame_stride, n_frames, false, st.n_streams, st.n_streams,
+                        (long long)st.n_streams * n_frames, pcm_out, status_out, scratch, stream, lanes);
+}
+
+cudaError_t launch_decode_multi_rows(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
+                                     size_t frame_stride, int n_rows, int n_live, long long total, int16_t* pcm_out,
+                                     int32_t* status_out, void* scratch, cudaStream_t stream, PlanLanes* lanes) {
+    if (total <= 0) return cudaSuccess;
+    return decode_multi(st, frames, frame_nbytes, nbytes, frame_stride, 0, true, n_rows, n_live, total, pcm_out, status_out,
+                        scratch, stream, lanes);
 }
 
 }  // namespace lc3b

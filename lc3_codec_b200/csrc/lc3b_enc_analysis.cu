@@ -41,7 +41,8 @@ struct AnalysisParams {
     float* e_b;
     int32_t* ehand;
     int smem_per_warp;
-    const int32_t* ids;   // subset call: row u is handle stream ids[u] (the IDS instantiations only)
+    const int32_t* ids;   // subset call: row u is handle stream ids[u] (the IDS instantiations only); enc_ltpf_kernel<true,
+                          // true>: the row table of a ragged call (lc3b_common.cuh), n_streams its rows
 };
 
 constexpr int ANA_WARPS = 4;
@@ -209,9 +210,10 @@ __global__ void __launch_bounds__(ANA_WARPS * 32) enc_mdct_kernel(AnalysisParams
 
 // Kernel 2, one frame: attack detector and LTPF analysis of stream `stream` (per-stream state) on the input and
 // hand-off record of unit `unit` (runs after enc_mdct_kernel, whose near-Nyquist flag it reads).  IDS: the CTA's warps hold
-// rows stream0 .. stream0 + 3 of a subset call, whose states the shared biquad reaches through the id list.
-template <bool IDS>
-__device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* smem, int stream, size_t unit) {
+// rows stream0 .. stream0 + 3 of a subset call, whose states the shared biquad reaches through the id list; RAGGED: rows of
+// a ragged call's row table.  n_live_c: warps of the CTA that have a frame now, always warps 0 .. n_live_c - 1.
+template <bool IDS, bool RAGGED>
+__device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* smem, int stream, size_t unit, int n_live_c) {
     const EncConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int nf = c.nf;
@@ -227,7 +229,6 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
 
     const int16_t* x = p.pcm + unit * p.pcm_stride;               // this frame's input samples
     int32_t* es = p.estate + (size_t)stream * ES_WORDS;
-    const int n_live_c = min(ANA_WARPS, p.n_streams - (int)blockIdx.x * ANA_WARPS);   // warps of this CTA that have a frame
     const int near_nyquist = p.ehand[unit * EH_WORDS + EH_NEAR_NYQUIST];
     const int up = c.up, ns_keep = 240 / up;
     {   // x_s_extended (long_term_post_filter.rs:217-224): last 240/up samples of the previous frame, then this frame
@@ -377,13 +378,13 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
         const float m1_0 = __uint_as_float((uint32_t)es[ES_H50_M1]), m2_0 = __uint_as_float((uint32_t)es[ES_H50_M2]);
         float* h50s = wk;                            // len12 <= 128 floats (attack scratch is dead by now)
         const int stream0 = blockIdx.x * ANA_WARPS;
-        const int n_live = min(ANA_WARPS, p.n_streams - stream0);   // warps of this CTA that have a frame (the others returned)
-        asm volatile("bar.sync 1, %0;" ::"r"(n_live * 32) : "memory");
-        if (wid == 0 && lane < n_live) {
+        asm volatile("bar.sync 1, %0;" ::"r"(n_live_c * 32) : "memory");
+        if (wid == 0 && lane < n_live_c) {
             uint8_t* ob = smem + (size_t)lane * p.smem_per_warp;      // warp `lane`'s slice: same carve-up as above
             float* o_wk = (float*)ob;
             const float* o_x12n = o_wk + 320 + 98 + 98 + 236 + c.delay + NMEM;
-            int32_t* o_es = p.estate + (size_t)state_row<IDS>(p.ids, stream0 + lane) * ES_WORDS;
+            const int o_row = RAGGED ? row_span<true>(p.ids, stream0 + lane, 0).row : state_row<IDS>(p.ids, stream0 + lane);
+            int32_t* o_es = p.estate + (size_t)o_row * ES_WORDS;
             float m1 = __uint_as_float((uint32_t)o_es[ES_H50_M1]), m2 = __uint_as_float((uint32_t)o_es[ES_H50_M2]);
             for (int n = 0; n < len12; n++) {
                 const float h50 = o_x12n[n] - -1.9652933726226904f * m1 - 0.9658854605688177f * m2;
@@ -394,7 +395,7 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
             o_es[ES_H50_M1] = (int32_t)__float_as_uint(m1);
             o_es[ES_H50_M2] = (int32_t)__float_as_uint(m2);
         }
-        asm volatile("bar.sync 1, %0;" ::"r"(n_live * 32) : "memory");
+        asm volatile("bar.sync 1, %0;" ::"r"(n_live_c * 32) : "memory");
         WARP_STRIDE(n, len12) {
             const float h50 = h50s[n];
             const float m1 = n >= 1 ? h50s[n - 1] : m1_0;
@@ -618,15 +619,31 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
 // separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a CTA walks the same count, so
 // the named barriers inside a frame stay matched.  The __syncwarp orders the state lane 0 (and warp 0, for the biquad)
 // wrote in frame f before the lanes read it in frame f + 1.
+// WALK and IDS: a ragged call, a warp per row of the row table walking the row's own count.  The table is sorted by count,
+// descending, so the warps of a CTA that still have frame f are warps 0 .. n_live - 1, n_live the number of the CTA's rows
+// with count > f: the named barriers count exactly them, a warp leaves when its row is done, and warp 0 (the CTA's longest
+// row) is there for every frame to do the ordered sums of lanes < n_live.
 template <bool WALK, bool IDS>
 __global__ void __launch_bounds__(ANA_WARPS * 32) enc_ltpf_kernel(AnalysisParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const int stream = blockIdx.x * ANA_WARPS + (threadIdx.x >> 5);
     if (stream >= p.n_streams) return;
-    const int F = WALK ? p.n_frames : 1;
-    for (int f = 0; f < F; f++) {
-        ltpf_frame<IDS>(p, smem, state_row<IDS>(p.ids, stream), (size_t)stream * F + f);
-        if (WALK) __syncwarp();
+    if constexpr (WALK && IDS) {
+        const int lane = threadIdx.x & 31;
+        const int n_live = min(ANA_WARPS, p.n_streams - (int)blockIdx.x * ANA_WARPS);   // the CTA's rows
+        const RowSpan rs = row_span<true>(p.ids, stream, 0);
+        const int cnt = lane < n_live ? row_span<true>(p.ids, blockIdx.x * ANA_WARPS + lane, 0).count : 0;   // lane j: warp j's
+        for (int f = 0; f < rs.count; f++) {
+            ltpf_frame<true, true>(p, smem, rs.row, (size_t)rs.off + f, __popc(__ballot_sync(0xffffffffu, cnt > f)));
+            __syncwarp();
+        }
+    } else {
+        const int F = WALK ? p.n_frames : 1;
+        for (int f = 0; f < F; f++) {
+            ltpf_frame<IDS, false>(p, smem, state_row<IDS>(p.ids, stream), (size_t)stream * F + f,
+                                   min(ANA_WARPS, p.n_streams - (int)blockIdx.x * ANA_WARPS));   // warps of this CTA that have a frame
+            if (WALK) __syncwarp();
+        }
     }
 }
 
@@ -650,11 +667,12 @@ cudaError_t prepare_enc_analysis(const EncoderState& st) {
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     return e;
 }
 
 void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
-                       int n_frames, const int32_t* ids) {
+                       int n_frames, const int32_t* ids, const int32_t* rows, int n_rows) {
     AnalysisParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
@@ -685,9 +703,10 @@ void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     if (stages & 2) {
         const size_t per_warp = ltpf_warp_bytes(st.cfg);
         p.smem_per_warp = (int)per_warp;
-        p.n_streams = st.n_streams / n_frames;                   // one warp per stream, walking its frames
+        p.n_streams = rows ? n_rows : st.n_streams / n_frames;  // one warp per stream (or row), walking its frames
         p.n_frames = n_frames;
-        plan.add(n_frames > 1 ? enc_ltpf_kernel<true, false> : ids ? enc_ltpf_kernel<false, true> : enc_ltpf_kernel<false, false>,
+        if (rows) p.ids = rows;
+        plan.add(rows ? enc_ltpf_kernel<true, true> : n_frames > 1 ? enc_ltpf_kernel<true, false> : ids ? enc_ltpf_kernel<false, true> : enc_ltpf_kernel<false, false>,
                  (unsigned)((p.n_streams + ANA_WARPS - 1) / ANA_WARPS), ANA_WARPS * 32, per_warp * ANA_WARPS, p);
     }
 }

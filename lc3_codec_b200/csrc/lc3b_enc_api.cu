@@ -193,6 +193,7 @@ struct lc3b_encoder {
     int graph_mode = 0;                 // 0 = one launch per kernel, 1 = one cached CUDA graph per call (lc3b_plan.cuh)
     GraphCache graphs;
     IdList id_list;                     // subset calls and resets (lc3b_encode_frames_subset, lc3b_encoder_reset_streams)
+    RowTable row_table;                 // ragged time-parallel calls (lc3b_encode_stream_frames_subset)
     // optional pipelining of the host entry point: PCM arrives on an internal copy stream into a double-buffered
     // staging area, so the upload of call i+1 overlaps the kernels of call i
     int pipelined = 0, buf = 0;
@@ -367,6 +368,32 @@ int lc3b_encode_stream_frames(lc3b_encoder* h, const int16_t* pcm_in, int n_fram
     LaunchPlan plan;                                      // the whole call is one plan: one graph launch in graph mode
     plan_enc_multi(plan, st, pcm_in, n_frames, frames_out, nbytes, frame_stride, scratch);
     cudaStream_t stream = (cudaStream_t)cuda_stream;
+    CU(h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream));
+    return LC3B_OK;
+}
+
+int lc3b_encoder_multi_subset_scratch_bytes(const lc3b_encoder* h, int n_rows, long long total_frames, size_t* device_bytes) {
+    if (!h || !device_bytes || n_rows < 0 || n_rows > h->st.n_streams || total_frames < 0 || total_frames > (long long)INT32_MAX)
+        return LC3B_ERR_INVALID_ARG;
+    *device_bytes = enc_multi_rows_scratch_bytes(h->st, n_rows, total_frames);
+    return LC3B_OK;
+}
+
+int lc3b_encode_stream_frames_subset(lc3b_encoder* h, const int32_t* stream_ids, const int32_t* frame_counts, int n_rows,
+                                     const int16_t* pcm_in, uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch,
+                                     size_t scratch_bytes, void* cuda_stream) {
+    if (!h || !stream_ids || !frame_counts) return LC3B_ERR_INVALID_ARG;
+    const EncoderState& st = h->st;
+    if (nbytes < 20 || nbytes > st.max_nbytes || (size_t)nbytes > frame_stride) return LC3B_ERR_INVALID_ARG;
+    RowTable& rt = h->row_table;
+    if (!rt.take(h->id_list, stream_ids, frame_counts, n_rows, st.n_streams, (long long)INT32_MAX)) return LC3B_ERR_INVALID_ARG;
+    if (rt.total == 0) return LC3B_OK;
+    if (!pcm_in || !frames_out || !scratch) return LC3B_ERR_INVALID_ARG;
+    if (scratch_bytes < enc_multi_rows_scratch_bytes(st, n_rows, rt.total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
+    LaunchPlan plan;                                      // the whole call is one plan: one graph launch in graph mode
+    plan_enc_multi_rows(plan, st, pcm_in, n_rows, rt.n_live, rt.total, frames_out, nbytes, frame_stride, scratch);
+    cudaStream_t stream = (cudaStream_t)cuda_stream;
+    CU(rt.send(scratch, stream));
     CU(h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream));
     return LC3B_OK;
 }

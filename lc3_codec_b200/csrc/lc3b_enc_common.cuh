@@ -81,14 +81,20 @@ cudaError_t launch_enc_quant(const EncoderState& st, uint8_t* frames_out, int nb
 // quantise kernel then run a warp per stream that walks the stream's frames in order; every other kernel runs per unit.
 // ids (n_frames == 1 only): a subset call, `st` a view whose st.n_streams is the call's row count; row u's persistent state
 // (thist, xs_hist, x12, x6, estate) is that of handle stream ids[u] (device memory), every other buffer has a row per call row.
+// rows: a ragged call, `st` a view of st.n_streams units as with n_frames > 1; the attack / LTPF kernel and the quantise
+// kernel run a warp per row of the device row table (n_rows rows with frames, lc3b_common.cuh), walking the row's units.
 struct LaunchPlan;
 void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
-                       int n_frames = 1, const int32_t* ids = nullptr);
+                       int n_frames = 1, const int32_t* ids = nullptr, const int32_t* rows = nullptr, int n_rows = 0);
 void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
-                    int n_frames = 1, const int32_t* ids = nullptr);
+                    int n_frames = 1, const int32_t* ids = nullptr, const int32_t* rows = nullptr, int n_rows = 0);
 // time-parallel encode (lc3b_enc_multi.cu): n_frames consecutive frames of every stream as one plan
 size_t enc_multi_scratch_bytes(const EncoderState& st, int n_frames);
 void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_frames, uint8_t* frames_out, int nbytes,
                     size_t frame_stride, void* scratch);
+// ragged time-parallel encode: n_rows listed rows, `total` units, the row table (n_live rows) at the front of the scratch
+size_t enc_multi_rows_scratch_bytes(const EncoderState& st, int n_rows, long long total);
+void plan_enc_multi_rows(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_rows, int n_live, long long total,
+                         uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch);
 
 }  // namespace lc3b

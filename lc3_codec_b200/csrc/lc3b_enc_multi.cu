@@ -15,19 +15,24 @@
 //   7. bitstream prepare / range coder / finish over the units; unit s*F + f writes frames_out + (s*F + f)*frame_stride
 // The per-frame buffers of the units live in the caller's scratch; the handle's own per-frame buffers (what
 // lc3b_encoder_debug_read reports) are not touched.  Arithmetic is the frame-by-frame path's, so the bytes are identical.
+//
+// A ragged call (lc3b_encode_stream_frames_subset) lists rows of any frame counts: kernels 1 and 3 find a unit's row in
+// unit_row[] (plan_unit_rows, lc3b_dec_multi.cu), kernels 4 and 6 walk the rows of the row table (lc3b_common.cuh), the
+// rest runs over the units unchanged.
 #include "lc3b_enc_common.cuh"
 #include "lc3b_plan.cuh"
 
 namespace lc3b {
 
-struct EncMultiLayout { size_t thist, xf, e_b, ehand, xq, qhand, lsbs, bs_scratch, total; };
+struct EncMultiLayout { size_t rows, thist, xf, e_b, ehand, xq, qhand, lsbs, bs_scratch, unit_row, total; };
 
-static EncMultiLayout enc_multi_layout(const EncoderState& st, int F) {
+// V units of n_rows rows; ragged: the row table at the front (where RowTable::send puts it) and unit_row[V] at the end
+static EncMultiLayout enc_multi_layout(const EncoderState& st, int n_rows, size_t V, bool ragged) {
     EncMultiLayout L;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~(size_t)255; return o; };
     const lc3b_config& c = st.cfg;
-    const size_t V = (size_t)st.n_streams * (size_t)F;
+    L.rows = take(ragged ? sizeof(int32_t) * RT_WORDS * n_rows : 0);
     L.thist = take(sizeof(int16_t) * V * (c.nf - c.z));
     L.xf = take(sizeof(float) * V * c.ne);
     L.e_b = take(sizeof(float) * V * 64);
@@ -36,38 +41,61 @@ static EncMultiLayout enc_multi_layout(const EncoderState& st, int F) {
     L.qhand = take(sizeof(int32_t) * V * QH_WORDS);
     L.lsbs = take(V * 2 * c.ne);
     L.bs_scratch = take(sizeof(uint32_t) * V * (size_t)st.bs_words);
+    L.unit_row = take(ragged ? sizeof(int32_t) * V : 0);
     L.total = off;
     return L;
 }
 
-size_t enc_multi_scratch_bytes(const EncoderState& st, int n_frames) { return enc_multi_layout(st, n_frames).total; }
+size_t enc_multi_scratch_bytes(const EncoderState& st, int n_frames) {
+    return enc_multi_layout(st, st.n_streams, (size_t)st.n_streams * (size_t)n_frames, false).total;
+}
+size_t enc_multi_rows_scratch_bytes(const EncoderState& st, int n_rows, long long total) {
+    return enc_multi_layout(st, n_rows, (size_t)total, true).total;
+}
 
 struct ThistParams {
     const int16_t* pcm;      // [S][F * nf]
     int16_t* hist;           // the handle's [S][nf - z]
     int16_t* thist_v;        // [S * F][nf - z]
     int S, F, nf, z;
+    // ragged call: S = rows of the row table, V units; unit_row[v] the state row of unit v's row, ~row for its first unit
+    const int32_t* rows;
+    const int32_t* unit_row;
+    size_t V;
 };
 
 // update_time_buffer (modified_dct.rs:126-138) keeps the last nf - z input samples: for unit (s, f > 0) those are
 // pcm[s][(f - 1) nf + z, f nf), known before any kernel runs
+template <bool RAGGED>
 __global__ void __launch_bounds__(256) enc_thist_prefill_kernel(ThistParams p) {
     const int L = p.nf - p.z;
-    const size_t n_all = (size_t)p.S * p.F * L;
+    const size_t n_all = (RAGGED ? p.V : (size_t)p.S * p.F) * L;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_all; i += (size_t)gridDim.x * blockDim.x) {
         const size_t v = i / L;
         const int n = (int)(i - v * L);
-        const int f = (int)(v % p.F);
-        p.thist_v[i] = f ? p.pcm[(v - 1) * p.nf + p.z + n] : p.hist[(v / p.F) * L + n];
+        if constexpr (RAGGED) {
+            const int u = p.unit_row[v];
+            p.thist_v[i] = u >= 0 ? p.pcm[(v - 1) * p.nf + p.z + n] : p.hist[(size_t)~u * L + n];
+        } else {
+            const int f = (int)(v % p.F);
+            p.thist_v[i] = f ? p.pcm[(v - 1) * p.nf + p.z + n] : p.hist[(v / p.F) * L + n];
+        }
     }
 }
 
+// the history of each row's last unit back to its state row
+template <bool RAGGED>
 __global__ void __launch_bounds__(256) enc_thist_handback_kernel(ThistParams p) {
     const int L = p.nf - p.z;
     const size_t n_all = (size_t)p.S * L;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_all; i += (size_t)gridDim.x * blockDim.x) {
         const size_t s = i / L;
-        p.hist[i] = p.thist_v[((s + 1) * p.F - 1) * L + (i - s * L)];
+        if constexpr (RAGGED) {
+            const RowSpan rs = row_span<true>(p.rows, (int)s, 0);
+            p.hist[(size_t)rs.row * L + (i - s * L)] = p.thist_v[((size_t)rs.off + rs.count - 1) * L + (i - s * L)];
+        } else {
+            p.hist[i] = p.thist_v[((s + 1) * p.F - 1) * L + (i - s * L)];
+        }
     }
 }
 
@@ -76,14 +104,16 @@ static unsigned copy_grid(size_t n) {
     return (unsigned)(g < 4096 ? g : 4096);
 }
 
-void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_frames, uint8_t* frames_out, int nbytes,
-                    size_t frame_stride, void* scratch) {
-    const int S = st.n_streams, F = n_frames;
-    const EncMultiLayout L = enc_multi_layout(st, F);
+// The dense call (rows == nullptr: S rows of F frames) and the ragged one (the n_live rows of the row table at the front
+// of the scratch, V units in all; the layout counts n_rows rows) share everything but the row addressing.
+static void plan_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int F, bool ragged, int n_rows, int n_live,
+                       size_t V, uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch) {
+    const int S = st.n_streams;
+    const EncMultiLayout L = enc_multi_layout(st, n_rows, V, ragged);
     uint8_t* base = (uint8_t*)scratch;
-    // a view of the handle with S*F units: per-frame buffers in the scratch, per-stream state the handle's
+    // a view of the handle with V units: per-frame buffers in the scratch, per-stream state the handle's
     EncoderState vs = st;
-    vs.n_streams = S * F;
+    vs.n_streams = (int)V;
     vs.thist = (int16_t*)(base + L.thist);
     vs.xf = (float*)(base + L.xf);
     vs.e_b = (float*)(base + L.e_b);
@@ -92,14 +122,37 @@ void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm
     vs.qhand = (int32_t*)(base + L.qhand);
     vs.lsbs = base + L.lsbs;
     vs.bs_scratch = (uint32_t*)(base + L.bs_scratch);
-    const ThistParams tp{pcm, st.thist, vs.thist, S, F, st.cfg.nf, st.cfg.z};
     const size_t hist_len = (size_t)(st.cfg.nf - st.cfg.z);
     const size_t nf = (size_t)st.cfg.nf;
-    plan.add(enc_thist_prefill_kernel, copy_grid((size_t)S * F * hist_len), 256, 0, tp);
-    plan_enc_analysis(plan, vs, pcm, nf, nbytes, 1, F);
-    plan.add(enc_thist_handback_kernel, copy_grid((size_t)S * hist_len), 256, 0, tp);
-    plan_enc_analysis(plan, vs, pcm, nf, nbytes, 2, F);
-    plan_enc_quant(plan, vs, frames_out, nbytes, frame_stride, 15, F);
+    if (!ragged) {
+        const ThistParams tp{pcm, st.thist, vs.thist, S, F, st.cfg.nf, st.cfg.z, nullptr, nullptr, 0};
+        plan.add(enc_thist_prefill_kernel<false>, copy_grid((size_t)S * F * hist_len), 256, 0, tp);
+        plan_enc_analysis(plan, vs, pcm, nf, nbytes, 1, F);
+        plan.add(enc_thist_handback_kernel<false>, copy_grid((size_t)S * hist_len), 256, 0, tp);
+        plan_enc_analysis(plan, vs, pcm, nf, nbytes, 2, F);
+        plan_enc_quant(plan, vs, frames_out, nbytes, frame_stride, 15, F);
+        return;
+    }
+    const int32_t* rows = (const int32_t*)(base + L.rows);
+    int32_t* unit_row = (int32_t*)(base + L.unit_row);
+    const ThistParams tp{pcm, st.thist, vs.thist, n_live, 0, st.cfg.nf, st.cfg.z, rows, unit_row, V};
+    plan_unit_rows(plan, rows, n_live, unit_row);
+    plan.add(enc_thist_prefill_kernel<true>, copy_grid(V * hist_len), 256, 0, tp);
+    plan_enc_analysis(plan, vs, pcm, nf, nbytes, 1);
+    plan.add(enc_thist_handback_kernel<true>, copy_grid((size_t)n_live * hist_len), 256, 0, tp);
+    plan_enc_analysis(plan, vs, pcm, nf, nbytes, 2, 1, nullptr, rows, n_live);
+    plan_enc_quant(plan, vs, frames_out, nbytes, frame_stride, 15, 1, nullptr, rows, n_live);
+}
+
+void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_frames, uint8_t* frames_out, int nbytes,
+                    size_t frame_stride, void* scratch) {
+    plan_multi(plan, st, pcm, n_frames, false, st.n_streams, st.n_streams, (size_t)st.n_streams * n_frames, frames_out, nbytes,
+               frame_stride, scratch);
+}
+
+void plan_enc_multi_rows(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_rows, int n_live, long long total,
+                         uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch) {
+    plan_multi(plan, st, pcm, 0, true, n_rows, n_live, (size_t)total, frames_out, nbytes, frame_stride, scratch);
 }
 
 }  // namespace lc3b

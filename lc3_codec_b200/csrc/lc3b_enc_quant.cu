@@ -1512,6 +1512,10 @@ __global__ void __launch_bounds__(QNT_THREADS, 4) enc_tns_kernel(QuantParams p) 
 // walks p.n_frames frames in order, the rate loop's offsets (ES_Q_*) carrying from one frame to the next; otherwise one
 // frame (lc3b_encode_frames: a separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a
 // CTA walks the same count, so the named barriers inside a frame stay matched.
+// WALK and IDS: a ragged call, p.ids its row table, a warp per row walking the row's own count.  As in enc_ltpf_kernel the
+// table is sorted by count, descending: the warps that still have frame f are warps 0 .. n_live - 1 (n_live = the CTA's
+// rows with count > f, recounted every frame), the barriers count exactly them and warp 0 does the ordered sums of
+// lanes < n_live.
 template <bool WALK, bool IDS>
 __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
@@ -1525,11 +1529,15 @@ __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p
     float* e4 = xf + NE_MAX;                                      // [100]
     float* T = e4 + 100;                                          // [224]
     int16_t* xq = (int16_t*)(T + 224);                            // [NE_MAX]
-    int32_t* es = p.estate + (size_t)state_row<IDS>(p.ids, stream) * ES_WORDS;
-    const int n_live = min(QW, p.n_streams - blockIdx.x * QW);    // warps of this CTA that have a frame
-    const int F = WALK ? p.n_frames : 1;
+    constexpr bool RAGGED = WALK && IDS;
+    const RowSpan rs = row_span<RAGGED>(p.ids, stream, 0);
+    int32_t* es = p.estate + (size_t)(RAGGED ? rs.row : state_row<IDS>(p.ids, stream)) * ES_WORDS;
+    const int n_cta = min(QW, p.n_streams - blockIdx.x * QW);     // warps of this CTA that have a frame
+    const int cnt = RAGGED && lane < n_cta ? row_span<RAGGED>(p.ids, blockIdx.x * QW + lane, 0).count : 0;   // lane j: warp j's
+    const int F = RAGGED ? rs.count : WALK ? p.n_frames : 1;
     for (int f = 0; f < F; f++) {
-        const size_t unit = (size_t)stream * F + f;
+        const int n_live = RAGGED ? __popc(__ballot_sync(0xffffffffu, cnt > f)) : n_cta;
+        const size_t unit = RAGGED ? (size_t)rs.off + f : (size_t)stream * F + f;
         const float4* gx = (const float4*)(p.xf + unit * ne);
         WARP_STRIDE(i, ne / 4) ((float4*)xf)[i] = gx[i];
         __syncwarp();
@@ -1728,6 +1736,7 @@ cudaError_t prepare_enc_quant(const EncoderState& st) {
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess)
         e = cudaFuncSetAttribute(enc_bs_prepare_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)(QW * bitstream_warp_bytes(st.cfg.ne, st.max_nbytes, nullptr)));
@@ -1735,7 +1744,7 @@ cudaError_t prepare_enc_quant(const EncoderState& st) {
 }
 
 void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
-                    int n_frames, const int32_t* ids) {
+                    int n_frames, const int32_t* ids, const int32_t* rows, int n_rows) {
     QuantParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
@@ -1759,11 +1768,12 @@ void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_ou
     const int grid = (p.n_streams + QW - 1) / QW;
     if (stages & 1) plan.add(enc_sns_kernel, (unsigned)((p.n_streams + SNS_WARPS - 1) / SNS_WARPS), SNS_WARPS * 32, SHAPE_SMEM / QW * SNS_WARPS, p);
     if (stages & 2) plan.add(enc_tns_kernel, (unsigned)grid, QNT_THREADS, SHAPE_SMEM, p);
-    if (stages & 4) {                                              // one warp per stream, walking its frames
+    if (stages & 4) {                                              // one warp per stream (or row), walking its frames
         QuantParams pw = p;
-        pw.n_streams = st.n_streams / n_frames;
+        pw.n_streams = rows ? n_rows : st.n_streams / n_frames;
         pw.n_frames = n_frames;
-        plan.add(n_frames > 1 ? enc_quantize_kernel<true, false> : ids ? enc_quantize_kernel<false, true> : enc_quantize_kernel<false, false>,
+        if (rows) pw.ids = rows;
+        plan.add(rows ? enc_quantize_kernel<true, true> : n_frames > 1 ? enc_quantize_kernel<true, false> : ids ? enc_quantize_kernel<false, true> : enc_quantize_kernel<false, false>,
                  (unsigned)((pw.n_streams + QW - 1) / QW), QNT_THREADS, QUANTIZE_SMEM, pw);
     }
     if (stages & 8) {

@@ -27,6 +27,54 @@ struct IdList {
         return true;
     }
 };
+
+// The host-side plan of a ragged time-parallel call (lc3b_decode_stream_frames_subset, lc3b_encode_stream_frames_subset):
+// an id list as for a subset call and a frame count per row.  Row i's frames are the call's units off_i .. off_i + count_i - 1,
+// off_i the exclusive prefix sum of the counts in the caller's order.  The rows with frames become the row table
+// (lc3b_common.cuh), sorted by count, descending, with a stable LSD radix sort: one pass per byte of the largest count,
+// so planning is O(n_rows) and never touches a unit.  Like IdList the table is a pageable copy that one cudaMemcpyAsync
+// sends to the front of the caller's scratch.
+struct RowTable {
+    std::vector<int32_t> words, tmp;
+    long long total = 0;
+    int n_live = 0;                       // rows with frames = rows of the table
+    // false for a bad or duplicate id, a negative count or more than max_total frames in all
+    bool take(IdList& idl, const int32_t* ids, const int32_t* counts, int n_rows, int n_streams, long long max_total) {
+        if (n_rows < 0 || n_rows > n_streams || !idl.take(ids, n_rows, n_streams)) return false;
+        words.resize((size_t)n_rows * RT_WORDS);
+        tmp.resize(words.size());
+        total = 0;
+        n_live = 0;
+        int32_t cmax = 0;
+        for (int i = 0; i < n_rows; i++) {
+            const int32_t c = counts[i];
+            if (c < 0 || total + c > max_total) return false;
+            if (c > 0) {
+                int32_t* w = &words[(size_t)n_live++ * RT_WORDS];
+                w[RT_ROW] = idl.ids[(size_t)i];
+                w[RT_OFF] = (int32_t)total;
+                w[RT_COUNT] = c;
+                if (c > cmax) cmax = c;
+            }
+            total += c;
+        }
+        for (int shift = 0; shift < 32 && (cmax >> shift) != 0; shift += 8) {
+            size_t start[257] = {0};
+            auto digit = [&](int r) { return 255 - ((words[(size_t)r * RT_WORDS + RT_COUNT] >> shift) & 255); };
+            for (int r = 0; r < n_live; r++) start[digit(r) + 1]++;
+            for (int d = 0; d < 256; d++) start[d + 1] += start[d];
+            for (int r = 0; r < n_live; r++) {
+                const size_t dst = start[digit(r)]++;
+                for (int k = 0; k < RT_WORDS; k++) tmp[dst * RT_WORDS + k] = words[(size_t)r * RT_WORDS + k];
+            }
+            words.swap(tmp);
+        }
+        return true;
+    }
+    cudaError_t send(void* scratch, cudaStream_t stream) const {
+        return cudaMemcpyAsync(scratch, words.data(), sizeof(int32_t) * RT_WORDS * (size_t)n_live, cudaMemcpyHostToDevice, stream);
+    }
+};
 }  // namespace lc3b
 
 struct lc3b_decoder {
@@ -46,6 +94,7 @@ struct lc3b_decoder {
     cudaEvent_t compute_done[2] = {nullptr, nullptr}, d2h_done[2] = {nullptr, nullptr};
     bool d2h_pending[2] = {false, false};
     lc3b::IdList id_list;                 // subset calls and resets (lc3b_decode_frames_subset, lc3b_decoder_reset_streams)
+    lc3b::RowTable row_table;             // ragged time-parallel calls (lc3b_decode_stream_frames_subset)
 };
 
 namespace lc3b {

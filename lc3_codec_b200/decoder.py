@@ -6,6 +6,7 @@ Lc3Decoder::calc_working_buffer_lengths     Lc3BatchDecoder.calc_working_buffer_
 Lc3Decoder::new(num_channels, ..bufs)       Lc3BatchDecoder(num_streams, .., workspace)  (caller-owned torch buffer)
 decode_frame(bits, channel, buf_in, out)    decode_frames(bits, frames, pcm_out, ..)     one frame for EVERY stream
   the same for some channels only           decode_frames_subset(bits, stream_ids, ..)   one frame for each listed stream
+  many frames of some channels              decode_stream_frames_subset(bits, ids, counts, ..) counts[i] frames of ids[i]
 fresh channel state (Lc3Decoder::new)       reset_streams(stream_ids)                    for the listed streams only
 Err(Only16BitsPerAudioSampleSupported)      raises Lc3DecoderError("Only16BitsPerAudioSampleSupported")
 panic on bad channel index / slice length   raises Lc3bError(LC3B_ERR_INVALID_ARG)
@@ -15,6 +16,7 @@ from __future__ import annotations
 
 import ctypes as C
 
+import numpy as np
 import torch
 
 from . import native
@@ -155,6 +157,46 @@ class Lc3BatchDecoder:
                                                         _ptr(status_out), _ptr(scratch), scratch.numel(), C.c_void_p(stream))
         if rc:
             raise Lc3bError(rc, "lc3b_decode_stream_frames")
+
+    def multi_subset_scratch_bytes(self, n_rows: int, total_frames: int) -> int:
+        """Bytes of caller-owned device scratch decode_stream_frames_subset needs for n_rows rows and total_frames frames."""
+        n = C.c_size_t(0)
+        rc = native.lib().lc3b_decoder_multi_subset_scratch_bytes(self._h, int(n_rows), int(total_frames), C.byref(n))
+        if rc:
+            raise Lc3bError(rc, "lc3b_decoder_multi_subset_scratch_bytes")
+        return int(n.value)
+
+    def decode_stream_frames_subset(self, num_bits_per_audio_sample: int, stream_ids, frame_counts, frames: torch.Tensor,
+                                    pcm_out: torch.Tensor, scratch: torch.Tensor, frame_nbytes: torch.Tensor | None = None,
+                                    status_out: torch.Tensor | None = None) -> None:
+        """frame_counts[i] consecutive frames of stream stream_ids[i] in one call, equal to that many decode_frames calls on
+        it; streams not listed are untouched (include/lc3b.h).  stream_ids, frame_counts: host sequences, numpy arrays or
+        CPU int32 tensors of one length.  The rows' frames are packed row after row in the caller's order (V = sum of the
+        counts): frames: contiguous CUDA uint8 [V, nbytes]; pcm_out: contiguous CUDA int16 with V * nf samples;
+        scratch: CUDA uint8, >= multi_subset_scratch_bytes(len(stream_ids), V); frame_nbytes / status_out: CUDA int32 [V]."""
+        if num_bits_per_audio_sample != 16:
+            raise Lc3DecoderError("Only16BitsPerAudioSampleSupported")
+        ids = native.host_ids(stream_ids)
+        counts = native.host_counts(frame_counts, ids.size)
+        V = int(counts.astype(np.int64).sum()) if counts.size else 0
+        if not (frames.is_cuda and frames.dtype == torch.uint8 and frames.dim() == 2 and frames.shape[0] == V
+                and frames.is_contiguous()):
+            raise Lc3bError(2, f"frames: want contiguous CUDA uint8 [{V}, nbytes]")
+        nb = frames.shape[1]
+        if not (pcm_out.is_cuda and pcm_out.dtype == torch.int16 and pcm_out.is_contiguous() and pcm_out.numel() == V * self.nf):
+            raise Lc3bError(2, f"pcm_out: want contiguous CUDA int16 with {V} * nf samples")
+        for t, what in ((frame_nbytes, "frame_nbytes"), (status_out, "status_out")):
+            if t is not None and not (t.is_cuda and t.dtype == torch.int32 and t.numel() == V and t.is_contiguous()):
+                raise Lc3bError(2, f"{what}: wrong device/dtype/shape")
+        if not (scratch.is_cuda and scratch.dtype == torch.uint8):
+            raise Lc3bError(2, "scratch must be a CUDA uint8 tensor")
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = native.lib().lc3b_decode_stream_frames_subset(
+                self._h, 16, C.c_void_p(ids.ctypes.data), C.c_void_p(counts.ctypes.data), ids.size, _ptr(frames),
+                _ptr(frame_nbytes), nb, nb, _ptr(pcm_out), _ptr(status_out), _ptr(scratch), scratch.numel(), C.c_void_p(stream))
+        if rc:
+            raise Lc3bError(rc, "lc3b_decode_stream_frames_subset")
 
     # ------------------------------------------------------------------ inspection (parity gate i)
     def enable_trace(self):

@@ -6,6 +6,7 @@ Lc3Encoder::calc_working_buffer_lengths     Lc3BatchEncoder.calc_working_buffer_
 Lc3Encoder::new(num_channels, ..bufs)       Lc3BatchEncoder(num_streams, .., workspace)
 encode_frame(channel, samples_in, buf_out)  encode_frames(pcm_in, frames_out)            one frame for EVERY stream
   the same for some channels only           encode_frames_subset(stream_ids, ..)         one frame for each listed stream
+  many frames of some channels              encode_stream_frames_subset(ids, counts, ..) counts[i] frames of ids[i]
 fresh channel state (Lc3Encoder::new)       reset_streams(stream_ids)                    for the listed streams only
 Result<(), Lc3EncoderError> (empty enum)    returns None; cannot fail for valid shapes
 assert_eq!(samples_in.len(), nf) panics     raises Lc3bError(LC3B_ERR_INVALID_ARG)
@@ -15,6 +16,7 @@ from __future__ import annotations
 
 import ctypes as C
 
+import numpy as np
 import torch
 
 from . import native
@@ -124,6 +126,39 @@ class Lc3BatchEncoder:
                                                         scratch.numel(), C.c_void_p(stream))
         if rc:
             raise Lc3bError(rc, "lc3b_encode_stream_frames")
+
+    def multi_subset_scratch_bytes(self, n_rows: int, total_frames: int) -> int:
+        """Bytes of caller-owned device scratch encode_stream_frames_subset needs for n_rows rows and total_frames frames."""
+        n = C.c_size_t(0)
+        rc = native.lib().lc3b_encoder_multi_subset_scratch_bytes(self._h, int(n_rows), int(total_frames), C.byref(n))
+        if rc:
+            raise Lc3bError(rc, "lc3b_encoder_multi_subset_scratch_bytes")
+        return int(n.value)
+
+    def encode_stream_frames_subset(self, stream_ids, frame_counts, pcm_in: torch.Tensor, frames_out: torch.Tensor,
+                                    scratch: torch.Tensor) -> None:
+        """frame_counts[i] consecutive frames of stream stream_ids[i] in one call, equal to that many encode_frames calls on
+        it; streams not listed are untouched (include/lc3b.h).  Frames are packed row after row in the caller's order
+        (V = sum of the counts): pcm_in: contiguous CUDA int16 with V * nf samples; frames_out: contiguous CUDA uint8
+        [V, nbytes]; scratch: CUDA uint8, >= multi_subset_scratch_bytes(len(stream_ids), V)."""
+        ids = native.host_ids(stream_ids)
+        counts = native.host_counts(frame_counts, ids.size)
+        V = int(counts.astype(np.int64).sum()) if counts.size else 0
+        if not (frames_out.is_cuda and frames_out.dtype == torch.uint8 and frames_out.dim() == 2 and frames_out.shape[0] == V
+                and frames_out.is_contiguous()):
+            raise Lc3bError(2, f"frames_out: want contiguous CUDA uint8 [{V}, nbytes]")
+        nb = frames_out.shape[1]
+        if not (pcm_in.is_cuda and pcm_in.dtype == torch.int16 and pcm_in.is_contiguous() and pcm_in.numel() == V * self.nf):
+            raise Lc3bError(2, f"pcm_in: want contiguous CUDA int16 with {V} * nf samples")
+        if not (scratch.is_cuda and scratch.dtype == torch.uint8):
+            raise Lc3bError(2, "scratch must be a CUDA uint8 tensor")
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        with torch.cuda.device(self.device):
+            rc = native.lib().lc3b_encode_stream_frames_subset(
+                self._h, C.c_void_p(ids.ctypes.data), C.c_void_p(counts.ctypes.data), ids.size, _ptr(pcm_in), _ptr(frames_out),
+                nb, nb, _ptr(scratch), scratch.numel(), C.c_void_p(stream))
+        if rc:
+            raise Lc3bError(rc, "lc3b_encode_stream_frames_subset")
 
     def set_host_pipelining(self, on: bool) -> None:
         """Let the PCM upload of encode_frames_host call i+1 overlap the kernels of call i (include/lc3b.h)."""

@@ -68,7 +68,9 @@ EXPORTS = ["lc3b_config_new", "lc3b_last_cuda_error", "lc3b_version", "lc3b_deco
            "lc3b_sharded_encoder_create", "lc3b_sharded_encoder_n_shards", "lc3b_sharded_encoder_shard",
            "lc3b_sharded_encode_frames_host", "lc3b_sharded_encoder_wait", "lc3b_sharded_encoder_destroy",
            "lc3b_host_alloc", "lc3b_host_free",
-           "lc3b_decode_frames_subset", "lc3b_decoder_reset_streams", "lc3b_encode_frames_subset", "lc3b_encoder_reset_streams"]
+           "lc3b_decode_frames_subset", "lc3b_decoder_reset_streams", "lc3b_encode_frames_subset", "lc3b_encoder_reset_streams",
+           "lc3b_decoder_multi_subset_scratch_bytes", "lc3b_decode_stream_frames_subset",
+           "lc3b_encoder_multi_subset_scratch_bytes", "lc3b_encode_stream_frames_subset"]
 
 
 class MixedBucket(C.Structure):             # lc3b_mixed_bucket
@@ -105,6 +107,8 @@ def lib() -> C.CDLL:
         L.lc3b_decode_stream_frames.argtypes = [vp, i32, vp, vp, i32, sz, i32, vp, vp, vp, sz, vp]
         L.lc3b_decode_frames_subset.argtypes = [vp, i32, vp, i32, vp, vp, i32, sz, vp, sz, vp, vp]
         L.lc3b_decoder_reset_streams.argtypes = [vp, vp, i32, vp]
+        L.lc3b_decoder_multi_subset_scratch_bytes.argtypes = [vp, i32, C.c_longlong, C.POINTER(sz)]
+        L.lc3b_decode_stream_frames_subset.argtypes = [vp, i32, vp, vp, i32, vp, vp, i32, sz, vp, vp, vp, sz, vp]
         L.lc3b_decoder_destroy.argtypes = [vp]
         L.lc3b_decoder_destroy.restype = None
         L.lc3b_encoder_workspace_bytes.argtypes = [i32, i32, i32, i32, C.POINTER(sz)]
@@ -115,6 +119,8 @@ def lib() -> C.CDLL:
         L.lc3b_encode_stream_frames.argtypes = [vp, vp, i32, vp, i32, sz, vp, sz, vp]
         L.lc3b_encode_frames_subset.argtypes = [vp, vp, i32, vp, sz, vp, i32, sz, vp]
         L.lc3b_encoder_reset_streams.argtypes = [vp, vp, i32, vp]
+        L.lc3b_encoder_multi_subset_scratch_bytes.argtypes = [vp, i32, C.c_longlong, C.POINTER(sz)]
+        L.lc3b_encode_stream_frames_subset.argtypes = [vp, vp, vp, i32, vp, vp, i32, sz, vp, sz, vp]
         L.lc3b_encoder_debug_read.argtypes = [vp, vp, vp, vp, vp, vp]
         L.lc3b_encoder_set_stage_mask.argtypes = [vp, i32]
         L.lc3b_encoder_set_host_pipelining.argtypes = [vp, i32]
@@ -170,6 +176,23 @@ def host_ids(stream_ids) -> np.ndarray:
         raise Lc3bError(2, "stream_ids: want a 1-D sequence of integers")
     if a.size and (int(a.min()) < -2**31 or int(a.max()) >= 2**31):
         raise Lc3bError(2, "stream_ids: ids beyond int32")
+    return np.ascontiguousarray(a, dtype=np.int32)
+
+
+def host_counts(frame_counts, n_rows: int) -> np.ndarray:
+    """A ragged call's frame counts (a sequence, a numpy array or a CPU int32 tensor), one per row of its id list, as a
+    contiguous host int32 array.  Signs and the total are checked by the library."""
+    if hasattr(frame_counts, "is_cuda"):               # a torch tensor
+        if frame_counts.is_cuda or str(frame_counts.dtype) != "torch.int32" or frame_counts.dim() != 1:
+            raise Lc3bError(2, "frame_counts: want a 1-D CPU int32 tensor")
+        frame_counts = frame_counts.contiguous().numpy()
+    a = np.asarray(frame_counts)
+    if a.ndim != 1 or (a.size and a.dtype.kind not in "iu"):
+        raise Lc3bError(2, "frame_counts: want a 1-D sequence of integers")
+    if a.size != n_rows:
+        raise Lc3bError(2, f"frame_counts: {a.size} counts for {n_rows} stream ids")
+    if a.size and (int(a.min()) < -2**31 or int(a.max()) >= 2**31):
+        raise Lc3bError(2, "frame_counts: counts beyond int32")
     return np.ascontiguousarray(a, dtype=np.int32)
 
 

@@ -95,6 +95,15 @@ extern "C" {
                                      nbytes: c_int, frame_stride: usize, n_frames: c_int, pcm_out: *mut i16,
                                      status_out: *mut i32, scratch: *mut c_void, scratch_bytes: usize,
                                      cuda_stream: *mut c_void) -> c_int;
+    /// ragged time-parallel decode: `frame_counts[i]` frames of stream `stream_ids[i]` (host arrays of `n_rows`), units
+    /// packed row after row in the caller's order
+    pub fn lc3b_decoder_multi_subset_scratch_bytes(h: *const lc3b_decoder, n_rows: c_int, total_frames: i64,
+                                                   device_bytes: *mut usize) -> c_int;
+    pub fn lc3b_decode_stream_frames_subset(h: *mut lc3b_decoder, bits_per_sample: c_int, stream_ids: *const i32,
+                                            frame_counts: *const i32, n_rows: c_int, frames: *const u8,
+                                            frame_nbytes: *const i32, nbytes: c_int, frame_stride: usize, pcm_out: *mut i16,
+                                            status_out: *mut i32, scratch: *mut c_void, scratch_bytes: usize,
+                                            cuda_stream: *mut c_void) -> c_int;
     /// 0 = one launch per kernel, 1 = one cached CUDA graph per call
     pub fn lc3b_decoder_set_graph_mode(h: *mut lc3b_decoder, mode: c_int) -> c_int;
     pub fn lc3b_decoder_set_split(h: *mut lc3b_decoder, k: c_int) -> c_int;
@@ -183,6 +192,13 @@ extern "C" {
     pub fn lc3b_encode_stream_frames(h: *mut lc3b_encoder, pcm_in: *const i16, n_frames: c_int, frames_out: *mut u8,
                                      nbytes: c_int, frame_stride: usize, scratch: *mut c_void, scratch_bytes: usize,
                                      cuda_stream: *mut c_void) -> c_int;
+    /// ragged time-parallel encode: `frame_counts[i]` frames of stream `stream_ids[i]` (host arrays of `n_rows`)
+    pub fn lc3b_encoder_multi_subset_scratch_bytes(h: *const lc3b_encoder, n_rows: c_int, total_frames: i64,
+                                                   device_bytes: *mut usize) -> c_int;
+    pub fn lc3b_encode_stream_frames_subset(h: *mut lc3b_encoder, stream_ids: *const i32, frame_counts: *const i32,
+                                            n_rows: c_int, pcm_in: *const i16, frames_out: *mut u8, nbytes: c_int,
+                                            frame_stride: usize, scratch: *mut c_void, scratch_bytes: usize,
+                                            cuda_stream: *mut c_void) -> c_int;
     pub fn lc3b_encoder_set_graph_mode(h: *mut lc3b_encoder, mode: c_int) -> c_int;
     pub fn lc3b_encoder_destroy(h: *mut lc3b_encoder);
 }

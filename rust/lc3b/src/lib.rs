@@ -180,6 +180,37 @@ impl<'a> Lc3BatchDecoder<'a> {
         }
     }
 
+    /// Bytes of caller-owned device scratch `decode_stream_frames_subset` needs for `n_rows` rows and `total_frames` frames.
+    pub fn multi_subset_scratch_bytes(&self, n_rows: usize, total_frames: usize) -> usize {
+        let mut n = 0usize;
+        check(unsafe { sys::lc3b_decoder_multi_subset_scratch_bytes(self.h, n_rows as i32, total_frames as i64, &mut n) },
+              "lc3b_decoder_multi_subset_scratch_bytes");
+        n
+    }
+
+    /// `frame_counts[i]` consecutive frames of stream `stream_ids[i]` in ONE call (files of different lengths, jitter
+    /// buffers of different depths); the same PCM and state as that many `decode_frames` calls on each listed stream,
+    /// every other stream untouched.  Device buffers hold the frames packed row after row in the caller's order
+    /// (`total` = sum of the counts): `frames` `[total][nbytes]`, `samples_out` `[total * nf]`, `frame_nbytes` /
+    /// `status_out` (nullable) `[total]`.
+    ///
+    /// # Safety
+    /// Device pointers valid for the stated extents until the stream has drained.
+    pub unsafe fn decode_stream_frames_subset(&mut self, num_bits_per_audio_sample: usize, stream_ids: &[i32],
+                                              frame_counts: &[i32], frames: *const u8, frame_nbytes: *const i32, nbytes: usize,
+                                              samples_out: *mut i16, status_out: *mut i32, scratch: DeviceBuf<'_>)
+                                              -> Result<(), Lc3DecoderError> {
+        assert_eq!(stream_ids.len(), frame_counts.len(), "one frame count per stream id");
+        match sys::lc3b_decode_stream_frames_subset(self.h, num_bits_per_audio_sample as i32, stream_ids.as_ptr(),
+                                                    frame_counts.as_ptr(), stream_ids.len() as i32, frames, frame_nbytes,
+                                                    nbytes as i32, nbytes, samples_out, status_out, scratch.ptr, scratch.bytes,
+                                                    self.stream) {
+            sys::LC3B_OK => Ok(()),
+            sys::LC3B_ERR_BITS_PER_SAMPLE => Err(Lc3DecoderError::Only16BitsPerAudioSampleSupported),
+            rc => { check(rc, "lc3b_decode_stream_frames_subset"); unreachable!() }
+        }
+    }
+
     /// Issue every call as one cached CUDA graph (`true`) or one launch per kernel (`false`); results are identical.
     pub fn set_graph_mode(&mut self, on: bool) {
         check(unsafe { sys::lc3b_decoder_set_graph_mode(self.h, on as i32) }, "lc3b_decoder_set_graph_mode");
@@ -286,6 +317,30 @@ impl<'a> Lc3BatchEncoder<'a> {
                                        stride: usize, scratch: DeviceBuf<'_>) -> Result<(), Lc3EncoderError> {
         check(sys::lc3b_encode_stream_frames(self.h, samples_in, n_frames as i32, buf_out, nbytes as i32, stride, scratch.ptr,
                                              scratch.bytes, self.stream), "lc3b_encode_stream_frames");
+        Ok(())
+    }
+
+    /// Bytes of caller-owned device scratch `encode_stream_frames_subset` needs for `n_rows` rows and `total_frames` frames.
+    pub fn multi_subset_scratch_bytes(&self, n_rows: usize, total_frames: usize) -> usize {
+        let mut n = 0usize;
+        check(unsafe { sys::lc3b_encoder_multi_subset_scratch_bytes(self.h, n_rows as i32, total_frames as i64, &mut n) },
+              "lc3b_encoder_multi_subset_scratch_bytes");
+        n
+    }
+
+    /// `frame_counts[i]` consecutive frames of stream `stream_ids[i]` in ONE call; the same bytes and state as that many
+    /// `encode_frames` calls on each listed stream, every other stream untouched.  Device buffers hold the frames packed
+    /// row after row in the caller's order: `samples_in` `[total * nf]`, unit v to `buf_out[v * stride ..][.. nbytes]`.
+    ///
+    /// # Safety
+    /// Device pointers valid for the stated extents until the stream has drained.
+    pub unsafe fn encode_stream_frames_subset(&mut self, stream_ids: &[i32], frame_counts: &[i32], samples_in: *const i16,
+                                              buf_out: *mut u8, nbytes: usize, stride: usize, scratch: DeviceBuf<'_>)
+                                              -> Result<(), Lc3EncoderError> {
+        assert_eq!(stream_ids.len(), frame_counts.len(), "one frame count per stream id");
+        check(sys::lc3b_encode_stream_frames_subset(self.h, stream_ids.as_ptr(), frame_counts.as_ptr(), stream_ids.len() as i32,
+                                                    samples_in, buf_out, nbytes as i32, stride, scratch.ptr, scratch.bytes,
+                                                    self.stream), "lc3b_encode_stream_frames_subset");
         Ok(())
     }
     pub fn num_streams(&self) -> usize { self.n_streams }
