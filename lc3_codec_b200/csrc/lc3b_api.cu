@@ -475,7 +475,7 @@ int lc3b_decoder_set_stage_mask(lc3b_decoder* h, int mask) {
 int lc3b_decoder_multi_scratch_bytes(const lc3b_decoder* h, int n_frames, size_t* device_bytes) {
     if (!h || !device_bytes || n_frames <= 0) return LC3B_ERR_INVALID_ARG;
     if ((long long)h->st.n_streams * n_frames > 0x7fffffffLL / 512) return LC3B_ERR_INVALID_ARG;   // 32-bit unit indices
-    *device_bytes = multi_scratch_bytes(h->st, n_frames);
+    *device_bytes = multi_scratch_bytes(h->st, h->st.n_streams, (long long)h->st.n_streams * n_frames);
     return LC3B_OK;
 }
 
@@ -487,9 +487,10 @@ int lc3b_decode_stream_frames(lc3b_decoder* h, int bits_per_sample, const uint8_
     const DecoderState& st = h->st;
     if (n_frames <= 0 || nbytes <= 0 || nbytes > st.max_nbytes || frame_stride < (size_t)nbytes) return LC3B_ERR_INVALID_ARG;
     if ((long long)st.n_streams * n_frames > 0x7fffffffLL / 512) return LC3B_ERR_INVALID_ARG;
-    if (scratch_bytes < multi_scratch_bytes(st, n_frames) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
-    CU(launch_decode_multi(st, frames, frame_nbytes, nbytes, frame_stride, n_frames, pcm_out, status_out, scratch,
-                           (cudaStream_t)cuda_stream, h->split == 1 ? nullptr : &h->lanes));
+    const long long total = (long long)st.n_streams * n_frames;
+    if (scratch_bytes < multi_scratch_bytes(st, st.n_streams, total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
+    CU(launch_decode_multi(st, frames, frame_nbytes, nbytes, frame_stride, st.n_streams, st.n_streams, total, n_frames, pcm_out,
+                           status_out, scratch, (cudaStream_t)cuda_stream, h->split == 1 ? nullptr : &h->lanes));
     return LC3B_OK;
 }
 
@@ -498,7 +499,7 @@ static constexpr long long MULTI_MAX_UNITS = 0x7fffffffLL / 512;          // 32-
 int lc3b_decoder_multi_subset_scratch_bytes(const lc3b_decoder* h, int n_rows, long long total_frames, size_t* device_bytes) {
     if (!h || !device_bytes || n_rows < 0 || n_rows > h->st.n_streams || total_frames < 0 || total_frames > MULTI_MAX_UNITS)
         return LC3B_ERR_INVALID_ARG;
-    *device_bytes = multi_rows_scratch_bytes(h->st, n_rows, total_frames);
+    *device_bytes = multi_scratch_bytes(h->st, n_rows, total_frames);
     return LC3B_OK;
 }
 
@@ -514,11 +515,11 @@ int lc3b_decode_stream_frames_subset(lc3b_decoder* h, int bits_per_sample, const
     if (!rt.take(h->id_list, stream_ids, frame_counts, n_rows, st.n_streams, MULTI_MAX_UNITS)) return LC3B_ERR_INVALID_ARG;
     if (rt.total == 0) return LC3B_OK;
     if (!frames || !pcm_out || !scratch) return LC3B_ERR_INVALID_ARG;
-    if (scratch_bytes < multi_rows_scratch_bytes(st, n_rows, rt.total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
+    if (scratch_bytes < multi_scratch_bytes(st, n_rows, rt.total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     CU(rt.send(scratch, stream));
-    CU(launch_decode_multi_rows(st, frames, frame_nbytes, nbytes, frame_stride, n_rows, rt.n_live, rt.total, pcm_out, status_out,
-                                scratch, stream, h->split == 1 ? nullptr : &h->lanes));
+    CU(launch_decode_multi(st, frames, frame_nbytes, nbytes, frame_stride, n_rows, rt.n_live, rt.total, 0, pcm_out, status_out,
+                           scratch, stream, h->split == 1 ? nullptr : &h->lanes));
     return LC3B_OK;
 }
 

@@ -53,21 +53,18 @@ __device__ __forceinline__ int state_row(const int32_t* ids, int u) {
     else return u;
 }
 
-// Ragged time-parallel calls (lc3b_decode_stream_frames_subset, lc3b_encode_stream_frames_subset) list their rows in a
+// Time-parallel calls (lc3b_decode_stream_frames, lc3b_encode_stream_frames and their _subset forms) list their rows in a
 // device ROW TABLE of RT_WORDS int32 per row: the state row (handle stream) the row advances, its first unit and its frame
 // count.  A row's units are consecutive; the table holds only rows with frames, sorted by count, descending (RowTable in
-// lc3b_handles.cuh), so the rows of a CTA that still have frame f are always the CTA's first rows.
+// lc3b_handles.cuh), so the rows of a CTA that still have frame f are always the CTA's first rows.  A dense call's table
+// is the identity {r, r * F, F}, which unit_rows_kernel writes on the device (already in that order).
 constexpr int RT_WORDS = 3;
 enum { RT_ROW = 0, RT_OFF, RT_COUNT };
 struct RowSpan { int row, off, count; };
-// Row r of a time-parallel call: dense (RAGGED = false) row r is stream r with F frames from unit r * F.
-template <bool RAGGED>
-__device__ __forceinline__ RowSpan row_span(const int32_t* rows, int r, int F) {
-    if constexpr (RAGGED) return RowSpan{__ldg(rows + RT_WORDS * r + RT_ROW), __ldg(rows + RT_WORDS * r + RT_OFF),
-                                         __ldg(rows + RT_WORDS * r + RT_COUNT)};
-    else return RowSpan{r, r * F, F};
+__device__ __forceinline__ RowSpan row_span(const int32_t* rows, int r) {
+    return RowSpan{__ldg(rows + RT_WORDS * r + RT_ROW), __ldg(rows + RT_WORDS * r + RT_OFF), __ldg(rows + RT_WORDS * r + RT_COUNT)};
 }
-// unit_row[v] of a ragged call (plan_unit_rows): the state row of unit v's row, bit-inverted for the row's first unit
+// unit_row[v] of a time-parallel call (plan_unit_rows): the state row of unit v's row, bit-inverted for the row's first unit
 __device__ __forceinline__ int unit_state_row(int u) { return u < 0 ? ~u : u; }
 
 // Everything a kernel needs to know about the (fs, duration) configuration; lives in the workspace.
@@ -214,20 +211,17 @@ cudaError_t prepare_entropy(const DecoderState& st);   // shared-memory limits o
 cudaError_t prepare_synth(const DecoderState& st);
 cudaError_t launch_init_state(const DecoderState& st, cudaStream_t stream);
 
-// time-parallel decode (SURVEY.md 8f-1), lc3b_dec_multi.cu
-size_t multi_scratch_bytes(const DecoderState& st, int n_frames);
+// time-parallel decode (SURVEY.md 8f-1), lc3b_dec_multi.cu: n_rows listed rows, `total` units.  dense_frames > 0: a dense
+// call, n_rows = n_live = the handle's streams of dense_frames frames each, whose row table the call writes itself;
+// otherwise the row table (n_live rows with frames) is at the front of the scratch already (RowTable::send).
+int decode_split_min_streams();    // from this many streams (or units) a decode call is cut into sub-batches
+size_t multi_scratch_bytes(const DecoderState& st, int n_rows, long long total);
 cudaError_t prepare_multi(const DecoderState& st);
 cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                                size_t frame_stride, int n_frames, int16_t* pcm_out, int32_t* status_out, void* scratch,
-                                cudaStream_t stream, struct PlanLanes* lanes = nullptr);
-int decode_split_min_streams();    // from this many streams (or units) a decode call is cut into sub-batches
-// ragged time-parallel decode: n_rows listed rows, `total` units; the row table (n_live rows with frames) is at the front
-// of the scratch already (RowTable::send)
-size_t multi_rows_scratch_bytes(const DecoderState& st, int n_rows, long long total);
-cudaError_t launch_decode_multi_rows(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                                     size_t frame_stride, int n_rows, int n_live, long long total, int16_t* pcm_out,
-                                     int32_t* status_out, void* scratch, cudaStream_t stream, struct PlanLanes* lanes);
-// one kernel writing unit_row[v] for the `total` units of the n_live rows of a device row table (shared with the encoder)
-void plan_unit_rows(struct LaunchPlan& plan, const int32_t* rows, int n_live, int32_t* unit_row);
+                                size_t frame_stride, int n_rows, int n_live, long long total, int dense_frames, int16_t* pcm_out,
+                                int32_t* status_out, void* scratch, cudaStream_t stream, struct PlanLanes* lanes);
+// one kernel writing unit_row[v] for the units of the n_live rows of a device row table (shared with the encoder); with
+// dense_frames > 0 it first writes the identity table of n_live rows of dense_frames frames
+void plan_unit_rows(struct LaunchPlan& plan, int32_t* rows, int n_live, int dense_frames, int32_t* unit_row);
 
 }  // namespace lc3b

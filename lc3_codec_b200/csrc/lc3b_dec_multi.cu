@@ -1,4 +1,4 @@
-// lc3b engine: time-parallel decode - many consecutive frames of every stream in ONE call (SURVEY.md 8f-1).
+// lc3b engine: time-parallel decode - many consecutive frames of many streams in ONE call (SURVEY.md 8f-1).
 //
 // The reference decodes a file frame by frame (examples/decode.rs:85-123); with few channels that leaves a GPU idle.
 // Of the decoder's state only three things really run along time:
@@ -6,21 +6,20 @@
 //   * concealment needs the last good spectrum, a fading factor and an LCG seed (packet_loss_concealment.rs:63-85)
 //                                                                     -> a scan over the frames' ok flags
 //   * the LTPF is an IIR across frame boundaries, but only while it is active (long_term_post_filter.rs:252)
-// so a call with F frames of S streams runs as S*F independent "units" through the expensive stages and touches the
-// time axis only where it must:
-//   1. entropy_kernel + dequant_kernel over the S*F units (the unchanged kernels; spectrum to a per-unit slot)
-//   2. plc_scan_kernel      thread per stream: walks the ok flags, assigns each concealed unit its source spectrum,
+// A call lists rows in a row table (lc3b_common.cuh): row i advances handle stream row_i by count_i consecutive frames,
+// units off_i .. off_i + count_i - 1.  lc3b_decode_stream_frames_subset sends its table; lc3b_decode_stream_frames is the
+// identity table of S rows of F frames, which unit_rows_kernel writes on the device.  The units run independently through
+// the expensive stages and the time axis is touched only where it must be:
+//   1. entropy_kernel + dequant_kernel over the units (the unchanged kernels; spectrum to a per-unit slot)
+//   2. unit_rows_kernel     warp per row: unit_row[v], the state row of each unit's row (stages 3 and 4 read it)
+//      plc_scan_kernel      warp per row: walks the ok flags, assigns each concealed unit its source spectrum,
 //                           alpha and seed (the LCG is jumped ne steps at a time), updates the handle's PLC scalars
 //   3. imdct_multi_kernel   warp per unit: concealment scramble, DCT-IV (same FFT as kernel 2), window -> head / tail
 //   4. ola_multi_kernel     warp per unit: x_hat = head + previous unit's tail, PCM of every frame
-//   5. ltpf_multi_kernel    warp per stream: replays the post filter over the spans where it is (or just was) active,
+//   5. ltpf_multi_kernel    warp per row: replays the post filter over the spans where it is (or just was) active,
 //                           overwriting those frames' PCM; then leaves the handle's per-stream state (overlap memory,
-//                           LTPF ring, last good spectrum) exactly as F frame-by-frame calls would have
+//                           LTPF ring, last good spectrum) exactly as count_i frame-by-frame calls would have
 // Arithmetic is the frame-by-frame path's, operation for operation, so both paths produce identical PCM.
-//
-// A ragged call (lc3b_decode_stream_frames_subset, the RAGGED instantiations) lists rows of any frame counts: stages 1, 3
-// and 4 run over its units unchanged, stages 2 and 5 run a warp per row of the row table (lc3b_common.cuh) and address the
-// handle's state by the row's state row.  Stages 3 and 4 find a unit's row in unit_row[], written by unit_rows_kernel.
 #include "lc3b_common.cuh"
 #include "lc3b_imdct.cuh"
 #include "lc3b_plan.cuh"
@@ -31,12 +30,12 @@ namespace lc3b {
 
 struct MultiLayout { size_t rows, spec, xq, handoff, gband, tns_list, side, head, tail, xhat, last_good, unit_row, total; };
 
-// V units of S rows; ragged: the row table at the front (where RowTable::send puts it) and unit_row[V] at the end
-static MultiLayout multi_layout(const lc3b_config& c, int S, size_t V, bool ragged) {
+// V units of S rows: the row table at the front (where RowTable::send puts it) and unit_row[V] at the end
+static MultiLayout multi_layout(const lc3b_config& c, int S, size_t V) {
     MultiLayout L;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~(size_t)255; return o; };
-    L.rows = take(ragged ? sizeof(int32_t) * RT_WORDS * S : 0);
+    L.rows = take(sizeof(int32_t) * RT_WORDS * S);
     const size_t nblk = ((V + 127) / 128) * 4;                    // 32-stream blocks, whole entropy CTAs
     L.spec = take(sizeof(float) * V * c.ne);
     L.xq = take(sizeof(int32_t) * nblk * c.ne * 32);
@@ -48,16 +47,13 @@ static MultiLayout multi_layout(const lc3b_config& c, int S, size_t V, bool ragg
     L.tail = take(sizeof(float) * V * (c.nf - c.z));
     L.xhat = take(sizeof(float) * V * c.nf);
     L.last_good = take(sizeof(int32_t) * S);
-    L.unit_row = take(ragged ? sizeof(int32_t) * V : 0);
+    L.unit_row = take(sizeof(int32_t) * V);
     L.total = off;
     return L;
 }
 
-size_t multi_scratch_bytes(const DecoderState& st, int n_frames) {
-    return multi_layout(st.cfg, st.n_streams, (size_t)st.n_streams * n_frames, false).total;
-}
-size_t multi_rows_scratch_bytes(const DecoderState& st, int n_rows, long long total) {
-    return multi_layout(st.cfg, n_rows, (size_t)total, true).total;
+size_t multi_scratch_bytes(const DecoderState& st, int n_rows, long long total) {
+    return multi_layout(st.cfg, n_rows, (size_t)total).total;
 }
 
 struct MultiParams {
@@ -65,10 +61,10 @@ struct MultiParams {
     const float* win;
     const float2* dtw;
     const float2* ftw;
-    int S, F;             // the handle's streams; frames per row of a dense call
-    int n_rows, V;        // ragged call: rows of the row table, units
-    const int32_t* rows;  // ragged call: row table (lc3b_common.cuh)
-    int32_t* unit_row;    // ragged call: [V] the state row of each unit's row, ~row for a row's first unit
+    int S;                // the handle's streams (stride between its two spectrum slots)
+    int n_rows, V;        // rows of the row table, units
+    const int32_t* rows;  // row table (lc3b_common.cuh)
+    const int32_t* unit_row;   // [V] the state row of each unit's row, ~row for a row's first unit
     // per-unit scratch
     const float* spec_v;
     int32_t* side_v;
@@ -90,14 +86,13 @@ struct MultiParams {
 constexpr int MW = 4;     // warps per CTA in the warp-per-unit kernels
 
 // ---------------------------------------------------------------- 2. concealment bookkeeping along time
-// One warp per stream; the ok flags are fetched 32 frames at a time so that the walk along time is not one dependent
+// One warp per row; the ok flags are fetched 32 frames at a time so that the walk along time is not one dependent
 // global load per frame.  Every lane tracks the same running state; lane j writes frame j's record.
-template <bool RAGGED>
 __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int r = blockIdx.x * MW + wid;
-    if (r >= (RAGGED ? p.n_rows : p.S)) return;
-    const RowSpan rs = row_span<RAGGED>(p.rows, r, p.F);
+    if (r >= p.n_rows) return;
+    const RowSpan rs = row_span(p.rows, r);
     const int s = rs.row, F = rs.count, v0 = rs.off;
     const int ne = p.cfg->ne;
     int32_t* ss = p.sstate + (size_t)s * SS_WORDS;
@@ -149,15 +144,14 @@ __global__ void __launch_bounds__(MW * 32) plc_scan_kernel(MultiParams p) {
 }
 
 // ---------------------------------------------------------------- 3. spectrum -> windowed time signal, per unit
-template <int NF, bool MS10, bool RAGGED>
+template <int NF, bool MS10>
 __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
     using G = FrameGeo<NF, MS10>;
     constexpr int NE = G::NE, Z = G::Z, NP = G::NP, NPT = G::NPT;
     extern __shared__ __align__(16) uint8_t smem[];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const long long v = (long long)blockIdx.x * MW + wid;
-    if (v >= (RAGGED ? (long long)p.V : (long long)p.S * p.F)) return;
-    const int s = RAGGED ? 0 : (int)(v / p.F);
+    if (v >= (long long)p.V) return;
     float* P = (float*)smem + (size_t)wid * 2 * NF;
     float* Q = P + NF;
 
@@ -167,7 +161,7 @@ __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
     if (src == -2) sp = p.spec_v + (size_t)v * NE;
     else if (src >= 0) sp = p.spec_v + (size_t)src * NE;
     else {                                                        // last good of earlier calls
-        const int sr = RAGGED ? unit_state_row(p.unit_row[v]) : s;
+        const int sr = unit_state_row(p.unit_row[v]);
         sp = p.spec + ((size_t)p.sstate[(size_t)sr * SS_WORDS + SS_SLOT] * p.S + sr) * NE;
     }
     if (src == -2) {
@@ -195,50 +189,42 @@ __global__ void __launch_bounds__(MW * 32) imdct_multi_kernel(MultiParams p) {
 }
 
 // ---------------------------------------------------------------- 4. overlap-add across units, PCM
-template <bool RAGGED>
 __global__ void __launch_bounds__(MW * 32) ola_multi_kernel(MultiParams p) {
     const DevConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const long long v = (long long)blockIdx.x * MW + wid;
-    if (v >= (RAGGED ? (long long)p.V : (long long)p.S * p.F)) return;
+    if (v >= (long long)p.V) return;
     const int nf = c.nf, z = c.z;
-    int s;
-    bool cont;                                                     // not the first frame of its row: the previous unit's tail
-    if constexpr (RAGGED) {
-        const int u = p.unit_row[v];
-        s = unit_state_row(u);
-        cont = u >= 0;
-    } else {
-        s = (int)(v / p.F);
-        cont = (int)(v - (long long)s * p.F) > 0;
-    }
+    const int u = __ldg(p.unit_row + v);                           // >= 0: not the first frame of its row, the previous unit's tail
     const float* head = p.head + (size_t)v * nf;
-    const float* prev = cont ? p.tail + (size_t)(v - 1) * (nf - z) : p.ola + (size_t)s * (nf - z);
+    const float* prev = u >= 0 ? p.tail + (size_t)(v - 1) * (nf - z) : p.ola + (size_t)~u * (nf - z);
     float* xhat = p.xhat + (size_t)v * nf;
-    int16_t* out = p.pcm_out + (size_t)v * nf;                     // [S][F * nf]
+    int16_t* out = p.pcm_out + (size_t)v * nf;
+    // read-only loads: the compiler may then issue all of a lane's loads before its stores to xhat and out, which it would
+    // otherwise have to assume alias them (a unit's row costs this kernel one more load latency than v / F did)
     for (int n = lane; n < nf; n += 32) {
-        float o = head[n];
-        if (n < nf - z) o = xa(prev[n], o);
+        float o = __ldg(head + n);
+        if (n < nf - z) o = xa(__ldg(prev + n), o);
         xhat[n] = o;
         out[n] = (int16_t)round_pcm_i32(o);
     }
 }
 
 // ---------------------------------------------------------------- 5. LTPF over its active spans + state hand-back
-// The dense instantiation keeps the stream, frame count and first unit as it computed them before the row table existed:
-// taken from a RowSpan they cost it spills.
-template <bool RAGGED>
-__global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
+// One warp per CTA: the row is then blockIdx.x, which ptxas knows to be the same for the whole warp, and so are the
+// row's entry and the bound of the walk.  With four warps per CTA they are per-thread values to it: the walk's control
+// flow leaves the uniform datapath and the kernel ran 5 % slower on bench.py --workload file16.  The minimum of 32 CTAs
+// per SM holds it to 64 registers (and 32 warps per SM); without it ptxas takes 72 and still spills a little.
+__global__ void __launch_bounds__(32, 32) ltpf_multi_kernel(MultiParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
     const DevConfig& c = *p.cfg;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int r = blockIdx.x * MW + wid;
-    if (r >= (RAGGED ? p.n_rows : p.S)) return;
-    const RowSpan rs = row_span<RAGGED>(p.rows, r, p.F);
-    const int s = RAGGED ? rs.row : r;
+    const int lane = threadIdx.x;
+    const int r = blockIdx.x;
+    const RowSpan rs = row_span(p.rows, r);
+    const int s = rs.row;
     const LtpfGeo g = ltpf_geo(c, p.hist_len);
-    const int nf = g.nf, ne = c.ne, z = c.z, F = RAGGED ? rs.count : p.F, blocks = g.blocks;
-    float* Y = (float*)(smem + (size_t)wid * p.smem_per_warp);     // per-warp buffer, see ltpf_warp_bytes
+    const int nf = g.nf, ne = c.ne, z = c.z, F = rs.count, blocks = g.blocks;
+    float* Y = (float*)smem;                                       // see ltpf_warp_bytes
     float* X = Y + p.hist_len;
     float* xt = X + nf;
     float* scratch = xt + 16;
@@ -252,7 +238,7 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
     for (int n = lane; n < p.hist_len; n += 32) Y[n] = yhist[n];
     __syncwarp();
     bool span1 = false, span2 = false, span3 = false;              // were frames f-1 / f-2 / f-3 filtered by this kernel
-    const size_t v0 = RAGGED ? (size_t)rs.off : (size_t)s * F;
+    const size_t v0 = (size_t)rs.off;
     uint32_t actm = 0;                                             // LTPF-active flags of the current 32-frame chunk
     for (int f = 0; f < F; f++) {
         if ((f & 31) == 0) {                                       // fetch 32 frames' flags at once; skip idle chunks
@@ -324,46 +310,57 @@ __global__ void __launch_bounds__(MW * 32) ltpf_multi_kernel(MultiParams p) {
     }
 }
 
-// ---------------------------------------------------------------- ragged calls: each unit's row, for stages 3 and 4
-__global__ void __launch_bounds__(MW * 32) unit_rows_kernel(MultiParams p) {
+// ---------------------------------------------------------------- each unit's row, for stages 3 and 4
+constexpr int UR_WARPS = 8;   // warps per CTA of unit_rows_kernel: a dense call of many short rows is thousands of CTAs
+
+struct UnitRowsParams {
+    int32_t* rows;        // row table; written here for a dense call
+    int32_t* unit_row;
+    int n_rows;
+    int dense_frames;     // > 0: a dense call, row r is stream r with dense_frames frames from unit r * dense_frames
+};
+
+__global__ void __launch_bounds__(UR_WARPS * 32) unit_rows_kernel(UnitRowsParams p) {
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    const int r = blockIdx.x * MW + wid;
+    const int r = blockIdx.x * UR_WARPS + wid;
     if (r >= p.n_rows) return;
-    const RowSpan rs = row_span<true>(p.rows, r, 0);
+    RowSpan rs;
+    if (p.dense_frames > 0) {
+        rs = RowSpan{r, r * p.dense_frames, p.dense_frames};
+        if (lane == 0) {
+            int32_t* w = p.rows + RT_WORDS * r;
+            w[RT_ROW] = rs.row;
+            w[RT_OFF] = rs.off;
+            w[RT_COUNT] = rs.count;
+        }
+    } else {
+        rs = row_span(p.rows, r);
+    }
     for (int f = lane; f < rs.count; f += 32) p.unit_row[(size_t)rs.off + f] = f ? rs.row : ~rs.row;
 }
 
-void plan_unit_rows(LaunchPlan& plan, const int32_t* rows, int n_live, int32_t* unit_row) {
-    MultiParams p;
-    memset(&p, 0, sizeof(p));
-    p.rows = rows;
-    p.unit_row = unit_row;
-    p.n_rows = n_live;
-    plan.add(unit_rows_kernel, (unsigned)((n_live + MW - 1) / MW), MW * 32, 0, p);
+void plan_unit_rows(LaunchPlan& plan, int32_t* rows, int n_live, int dense_frames, int32_t* unit_row) {
+    const UnitRowsParams p{rows, unit_row, n_live, dense_frames};
+    plan.add(unit_rows_kernel, (unsigned)((n_live + UR_WARPS - 1) / UR_WARPS), UR_WARPS * 32, 0, p);
 }
 
 namespace {
 struct PrepareImdct {
     cudaError_t e = cudaSuccess;
     template <int NF, bool MS10> void operator()() {
-        e = cudaFuncSetAttribute(imdct_multi_kernel<NF, MS10, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, MW * 2 * NF * 4);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(imdct_multi_kernel<NF, MS10, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, MW * 2 * NF * 4);
+        e = cudaFuncSetAttribute(imdct_multi_kernel<NF, MS10>, cudaFuncAttributeMaxDynamicSharedMemorySize, MW * 2 * NF * 4);
     }
 };
-template <bool RAGGED>
 struct PlanImdct {
     LaunchPlan& plan;
     const MultiParams& p;
     unsigned grid;
-    template <int NF, bool MS10> void operator()() { plan.add(imdct_multi_kernel<NF, MS10, RAGGED>, grid, MW * 32, MW * 2 * NF * 4, p); }
+    template <int NF, bool MS10> void operator()() { plan.add(imdct_multi_kernel<NF, MS10>, grid, MW * 32, MW * 2 * NF * 4, p); }
 };
 }  // namespace
 
 cudaError_t prepare_multi(const DecoderState& st) {
-    const int lb = (int)(ltpf_warp_bytes(st.cfg) * MW);
-    cudaError_t e = cudaFuncSetAttribute(ltpf_multi_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(ltpf_multi_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
+    cudaError_t e = cudaFuncSetAttribute(ltpf_multi_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ltpf_warp_bytes(st.cfg));
     if (e == cudaSuccess) {
         PrepareImdct pi;
         if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
@@ -372,13 +369,11 @@ cudaError_t prepare_multi(const DecoderState& st) {
     return e;
 }
 
-// The dense call (rows == nullptr: S rows of F frames) and the ragged one (the n_live rows of the row table at the front of
-// the scratch, V units in all; the layout counts n_rows rows) share everything but the row addressing.
-static cudaError_t decode_multi(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                                size_t frame_stride, int F, bool ragged, int n_rows, int n_live, long long V, int16_t* pcm_out,
+cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
+                                size_t frame_stride, int n_rows, int n_live, long long V, int dense_frames, int16_t* pcm_out,
                                 int32_t* status_out, void* scratch, cudaStream_t stream, PlanLanes* lanes) {
-    const int S = st.n_streams;
-    const MultiLayout L = multi_layout(st.cfg, n_rows, (size_t)V, ragged);
+    if (V <= 0) return cudaSuccess;
+    const MultiLayout L = multi_layout(st.cfg, n_rows, (size_t)V);
     uint8_t* base = (uint8_t*)scratch;
     // 1. entropy decode of all units with the unchanged kernel: a view of the handle with V virtual streams
     DecoderState vs = st;
@@ -408,13 +403,15 @@ static cudaError_t decode_multi(const DecoderState& st, const uint8_t* frames, c
         e = plan_launch_direct(plan, stream, lanes);
     }
     if (e != cudaSuccess) return e;
+    int32_t* rows = (int32_t*)(base + L.rows);
+    int32_t* unit_row = (int32_t*)(base + L.unit_row);
     MultiParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.dcfg; p.win = st.win; p.dtw = st.dtw; p.ftw = st.ftw;
-    p.S = S; p.F = F;
+    p.S = st.n_streams;
     p.n_rows = n_live; p.V = (int)V;
-    p.rows = ragged ? (const int32_t*)(base + L.rows) : nullptr;
-    p.unit_row = ragged ? (int32_t*)(base + L.unit_row) : nullptr;
+    p.rows = rows;
+    p.unit_row = unit_row;
     p.spec_v = vs.spec; p.side_v = vs.side;
     p.head = (float*)(base + L.head); p.tail = (float*)(base + L.tail); p.xhat = (float*)(base + L.xhat);
     p.last_good = (int32_t*)(base + L.last_good);
@@ -425,40 +422,14 @@ static cudaError_t decode_multi(const DecoderState& st, const uint8_t* frames, c
     // 2-5. a second plan on the caller's stream: plan_launch_direct joins the entropy plan's lanes back into the caller's
     // stream only at the end of that plan, so lane-0 nodes added to it would not wait for lanes 1-3
     LaunchPlan tail;
-    const int rows = ragged ? n_live : S;
-    const unsigned grid_s = (unsigned)((rows + MW - 1) / MW), grid_v = (unsigned)((V + MW - 1) / MW);
-    const size_t ltpf_smem = (size_t)p.smem_per_warp * MW;
-    if (ragged) {
-        plan_unit_rows(tail, p.rows, n_live, p.unit_row);
-        tail.add(plc_scan_kernel<true>, grid_s, MW * 32, 0, p);
-        PlanImdct<true> pi{tail, p, grid_v};
-        if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
-        tail.add(ola_multi_kernel<true>, grid_v, MW * 32, 0, p);
-        tail.add(ltpf_multi_kernel<true>, grid_s, MW * 32, ltpf_smem, p);
-    } else {
-        tail.add(plc_scan_kernel<false>, grid_s, MW * 32, 0, p, -1);
-        PlanImdct<false> pi{tail, p, grid_v};
-        if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
-        tail.add(ola_multi_kernel<false>, grid_v, MW * 32, 0, p);
-        tail.add(ltpf_multi_kernel<false>, grid_s, MW * 32, ltpf_smem, p);
-    }
+    const unsigned grid_s = (unsigned)((n_live + MW - 1) / MW), grid_v = (unsigned)((V + MW - 1) / MW);
+    plan_unit_rows(tail, rows, n_live, dense_frames, unit_row);
+    tail.add(plc_scan_kernel, grid_s, MW * 32, 0, p);
+    PlanImdct pi{tail, p, grid_v};
+    if (!dispatch_frame_geo(st.cfg.nf, st.cfg.n_ms == LC3B_10MS, pi)) return cudaErrorInvalidValue;
+    tail.add(ola_multi_kernel, grid_v, MW * 32, 0, p);
+    tail.add(ltpf_multi_kernel, (unsigned)n_live, 32, (size_t)p.smem_per_warp, p);
     return plan_launch_direct(tail, stream);
-}
-
-cudaError_t launch_decode_multi(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                                size_t frame_stride, int n_frames, int16_t* pcm_out, int32_t* status_out, void* scratch,
-                                cudaStream_t stream, PlanLanes* lanes) {
-    if (n_frames <= 0) return cudaSuccess;
-    return decode_multi(st, frames, frame_nbytes, nbytes, frame_stride, n_frames, false, st.n_streams, st.n_streams,
-                        (long long)st.n_streams * n_frames, pcm_out, status_out, scratch, stream, lanes);
-}
-
-cudaError_t launch_decode_multi_rows(const DecoderState& st, const uint8_t* frames, const int32_t* frame_nbytes, int nbytes,
-                                     size_t frame_stride, int n_rows, int n_live, long long total, int16_t* pcm_out,
-                                     int32_t* status_out, void* scratch, cudaStream_t stream, PlanLanes* lanes) {
-    if (total <= 0) return cudaSuccess;
-    return decode_multi(st, frames, frame_nbytes, nbytes, frame_stride, 0, true, n_rows, n_live, total, pcm_out, status_out,
-                        scratch, stream, lanes);
 }
 
 }  // namespace lc3b

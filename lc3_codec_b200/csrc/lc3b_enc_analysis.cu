@@ -31,7 +31,6 @@ struct AnalysisParams {
     size_t pcm_stride;
     int nbytes;
     int n_streams;
-    int n_frames;         // enc_ltpf_kernel: consecutive frames each warp walks; its frame f is unit s * n_frames + f
     int16_t* thist;
     int16_t* xs_hist;
     float* x12;
@@ -41,8 +40,8 @@ struct AnalysisParams {
     float* e_b;
     int32_t* ehand;
     int smem_per_warp;
-    const int32_t* ids;   // subset call: row u is handle stream ids[u] (the IDS instantiations only); enc_ltpf_kernel<true,
-                          // true>: the row table of a ragged call (lc3b_common.cuh), n_streams its rows
+    const int32_t* ids;   // subset call: row u is handle stream ids[u] (the one-frame IDS instantiations only)
+    const int32_t* rows;  // time-parallel call: the row table (lc3b_common.cuh), n_streams its rows (enc_ltpf_kernel<true, true>)
 };
 
 constexpr int ANA_WARPS = 4;
@@ -210,9 +209,9 @@ __global__ void __launch_bounds__(ANA_WARPS * 32) enc_mdct_kernel(AnalysisParams
 
 // Kernel 2, one frame: attack detector and LTPF analysis of stream `stream` (per-stream state) on the input and
 // hand-off record of unit `unit` (runs after enc_mdct_kernel, whose near-Nyquist flag it reads).  IDS: the CTA's warps hold
-// rows stream0 .. stream0 + 3 of a subset call, whose states the shared biquad reaches through the id list; RAGGED: rows of
-// a ragged call's row table.  n_live_c: warps of the CTA that have a frame now, always warps 0 .. n_live_c - 1.
-template <bool IDS, bool RAGGED>
+// rows stream0 .. stream0 + 3 of a subset call, whose states the shared biquad reaches through the id list; WALK: rows of
+// a time-parallel call's row table.  n_live_c: warps of the CTA that have a frame now, always warps 0 .. n_live_c - 1.
+template <bool IDS, bool WALK>
 __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* smem, int stream, size_t unit, int n_live_c) {
     const EncConfig& c = *p.cfg;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
@@ -383,7 +382,7 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
             uint8_t* ob = smem + (size_t)lane * p.smem_per_warp;      // warp `lane`'s slice: same carve-up as above
             float* o_wk = (float*)ob;
             const float* o_x12n = o_wk + 320 + 98 + 98 + 236 + c.delay + NMEM;
-            const int o_row = RAGGED ? row_span<true>(p.ids, stream0 + lane, 0).row : state_row<IDS>(p.ids, stream0 + lane);
+            const int o_row = WALK ? row_span(p.rows, stream0 + lane).row : state_row<IDS>(p.ids, stream0 + lane);
             int32_t* o_es = p.estate + (size_t)o_row * ES_WORDS;
             float m1 = __uint_as_float((uint32_t)o_es[ES_H50_M1]), m2 = __uint_as_float((uint32_t)o_es[ES_H50_M2]);
             for (int n = 0; n < len12; n++) {
@@ -615,35 +614,33 @@ __device__ __forceinline__ void ltpf_frame(const AnalysisParams& p, uint8_t* sme
     }
 }
 
-// Kernel 2: a warp per stream walks p.n_frames frames in order (WALK), or encodes one frame (lc3b_encode_frames: a
-// separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a CTA walks the same count, so
-// the named barriers inside a frame stay matched.  The __syncwarp orders the state lane 0 (and warp 0, for the biquad)
-// wrote in frame f before the lanes read it in frame f + 1.
-// WALK and IDS: a ragged call, a warp per row of the row table walking the row's own count.  The table is sorted by count,
-// descending, so the warps of a CTA that still have frame f are warps 0 .. n_live - 1, n_live the number of the CTA's rows
-// with count > f: the named barriers count exactly them, a warp leaves when its row is done, and warp 0 (the CTA's longest
-// row) is there for every frame to do the ordered sums of lanes < n_live.
+// Kernel 2: one frame per warp (lc3b_encode_frames; IDS: lc3b_encode_frames_subset), or, WALK (always with IDS: a row's
+// state row comes from the row table), a warp per row of a time-parallel call's row table walking the row's frames in
+// order.  The walk is a separate instantiation, so the frame-by-frame path keeps its registers.  The __syncwarp orders
+// the state lane 0 (and warp 0, for the biquad) wrote in frame f before the lanes read it in frame f + 1.  The table is
+// sorted by count, descending, so the warps of a CTA that still have frame f are warps 0 .. n_live - 1, n_live the number
+// of the CTA's rows with count > f: the named barriers count exactly them, a warp leaves when its row is done, and warp 0
+// (the CTA's longest row) is there for every frame to do the ordered sums of lanes < n_live.
 template <bool WALK, bool IDS>
 __global__ void __launch_bounds__(ANA_WARPS * 32) enc_ltpf_kernel(AnalysisParams p) {
+    static_assert(!WALK || IDS, "the row walk addresses state through the row table");
     extern __shared__ __align__(16) uint8_t smem[];
     const int stream = blockIdx.x * ANA_WARPS + (threadIdx.x >> 5);
     if (stream >= p.n_streams) return;
-    if constexpr (WALK && IDS) {
+    const int n_cta = min(ANA_WARPS, p.n_streams - (int)blockIdx.x * ANA_WARPS);   // the CTA's rows
+    if constexpr (WALK) {
         const int lane = threadIdx.x & 31;
-        const int n_live = min(ANA_WARPS, p.n_streams - (int)blockIdx.x * ANA_WARPS);   // the CTA's rows
-        const RowSpan rs = row_span<true>(p.ids, stream, 0);
-        const int cnt = lane < n_live ? row_span<true>(p.ids, blockIdx.x * ANA_WARPS + lane, 0).count : 0;   // lane j: warp j's
-        for (int f = 0; f < rs.count; f++) {
-            ltpf_frame<true, true>(p, smem, rs.row, (size_t)rs.off + f, __popc(__ballot_sync(0xffffffffu, cnt > f)));
+        const RowSpan rs = row_span(p.rows, stream);
+        const int cnt = lane < n_cta ? row_span(p.rows, blockIdx.x * ANA_WARPS + lane).count : 0;   // lane j: warp j's
+        // the count and the live warps as warp reductions: their results are uniform registers, so the walk's control flow
+        // stays on the uniform datapath (as with a frame count in a kernel parameter; as per-lane values it ran 4-5 % slower)
+        const int F = __reduce_max_sync(0xffffffffu, rs.count);
+        for (int f = 0; f < F; f++) {
+            ltpf_frame<true, true>(p, smem, rs.row, (size_t)rs.off + f, __reduce_add_sync(0xffffffffu, cnt > f ? 1u : 0u));
             __syncwarp();
         }
     } else {
-        const int F = WALK ? p.n_frames : 1;
-        for (int f = 0; f < F; f++) {
-            ltpf_frame<IDS, false>(p, smem, state_row<IDS>(p.ids, stream), (size_t)stream * F + f,
-                                   min(ANA_WARPS, p.n_streams - (int)blockIdx.x * ANA_WARPS));   // warps of this CTA that have a frame
-            if (WALK) __syncwarp();
-        }
+        ltpf_frame<IDS, false>(p, smem, state_row<IDS>(p.ids, stream), (size_t)stream, n_cta);
     }
 }
 
@@ -666,13 +663,12 @@ cudaError_t prepare_enc_analysis(const EncoderState& st) {
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_mdct_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mb);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_ltpf_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lb);
     return e;
 }
 
 void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
-                       int n_frames, const int32_t* ids, const int32_t* rows, int n_rows) {
+                       const int32_t* ids, const int32_t* rows, int n_rows) {
     AnalysisParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
@@ -684,7 +680,6 @@ void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     p.pcm_stride = pcm_stride;
     p.nbytes = nbytes;
     p.n_streams = st.n_streams;
-    p.n_frames = 1;
     p.thist = st.thist;
     p.xs_hist = st.xs_hist;
     p.x12 = st.x12;
@@ -694,6 +689,7 @@ void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     p.e_b = st.e_b;
     p.ehand = st.ehand;
     p.ids = ids;
+    p.rows = rows;
     if (stages & 1) {
         const size_t per_warp = mdct_warp_bytes(st.cfg.nf);
         p.smem_per_warp = (int)per_warp;
@@ -703,18 +699,10 @@ void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     if (stages & 2) {
         const size_t per_warp = ltpf_warp_bytes(st.cfg);
         p.smem_per_warp = (int)per_warp;
-        p.n_streams = rows ? n_rows : st.n_streams / n_frames;  // one warp per stream (or row), walking its frames
-        p.n_frames = n_frames;
-        if (rows) p.ids = rows;
-        plan.add(rows ? enc_ltpf_kernel<true, true> : n_frames > 1 ? enc_ltpf_kernel<true, false> : ids ? enc_ltpf_kernel<false, true> : enc_ltpf_kernel<false, false>,
+        if (rows) p.n_streams = n_rows;                         // one warp per row, walking its frames
+        plan.add(rows ? enc_ltpf_kernel<true, true> : ids ? enc_ltpf_kernel<false, true> : enc_ltpf_kernel<false, false>,
                  (unsigned)((p.n_streams + ANA_WARPS - 1) / ANA_WARPS), ANA_WARPS * 32, per_warp * ANA_WARPS, p);
     }
-}
-
-cudaError_t launch_enc_analysis(const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages, cudaStream_t stream) {
-    LaunchPlan plan;
-    plan_enc_analysis(plan, st, pcm, pcm_stride, nbytes, stages);
-    return plan_launch_direct(plan, stream);
 }
 
 }  // namespace lc3b

@@ -209,8 +209,8 @@ static cudaError_t run_encode(lc3b_encoder* h, const int16_t* pcm, size_t pcm_st
     LaunchPlan plan;
     EncoderState v = h->st;                                 // a subset call: a view of n rows
     if (ids) v.n_streams = n;
-    if (mask & 3) plan_enc_analysis(plan, v, pcm, pcm_stride, nbytes, mask & 3, 1, ids);
-    if (mask & 60) plan_enc_quant(plan, v, frames_out, nbytes, frame_stride, mask >> 2, 1, ids);
+    if (mask & 3) plan_enc_analysis(plan, v, pcm, pcm_stride, nbytes, mask & 3, ids);
+    if (mask & 60) plan_enc_quant(plan, v, frames_out, nbytes, frame_stride, mask >> 2, ids);
     return h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream);
 }
 
@@ -353,7 +353,7 @@ int lc3b_encoder_reset_streams(lc3b_encoder* h, const int32_t* stream_ids, int n
 int lc3b_encoder_multi_scratch_bytes(const lc3b_encoder* h, int n_frames, size_t* device_bytes) {
     if (!h || !device_bytes || n_frames < 1 || (size_t)h->st.n_streams * (size_t)n_frames > (size_t)INT32_MAX)
         return LC3B_ERR_INVALID_ARG;
-    *device_bytes = enc_multi_scratch_bytes(h->st, n_frames);
+    *device_bytes = enc_multi_scratch_bytes(h->st, h->st.n_streams, (long long)h->st.n_streams * n_frames);
     return LC3B_OK;
 }
 
@@ -364,9 +364,10 @@ int lc3b_encode_stream_frames(lc3b_encoder* h, const int16_t* pcm_in, int n_fram
     if (nbytes < 20 || nbytes > st.max_nbytes || (size_t)nbytes > frame_stride || n_frames < 1 ||
         (size_t)st.n_streams * (size_t)n_frames > (size_t)INT32_MAX)
         return LC3B_ERR_INVALID_ARG;
-    if (scratch_bytes < enc_multi_scratch_bytes(st, n_frames) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
+    const long long total = (long long)st.n_streams * n_frames;
+    if (scratch_bytes < enc_multi_scratch_bytes(st, st.n_streams, total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
     LaunchPlan plan;                                      // the whole call is one plan: one graph launch in graph mode
-    plan_enc_multi(plan, st, pcm_in, n_frames, frames_out, nbytes, frame_stride, scratch);
+    plan_enc_multi(plan, st, pcm_in, st.n_streams, st.n_streams, total, n_frames, frames_out, nbytes, frame_stride, scratch);
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     CU(h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream));
     return LC3B_OK;
@@ -375,7 +376,7 @@ int lc3b_encode_stream_frames(lc3b_encoder* h, const int16_t* pcm_in, int n_fram
 int lc3b_encoder_multi_subset_scratch_bytes(const lc3b_encoder* h, int n_rows, long long total_frames, size_t* device_bytes) {
     if (!h || !device_bytes || n_rows < 0 || n_rows > h->st.n_streams || total_frames < 0 || total_frames > (long long)INT32_MAX)
         return LC3B_ERR_INVALID_ARG;
-    *device_bytes = enc_multi_rows_scratch_bytes(h->st, n_rows, total_frames);
+    *device_bytes = enc_multi_scratch_bytes(h->st, n_rows, total_frames);
     return LC3B_OK;
 }
 
@@ -389,9 +390,9 @@ int lc3b_encode_stream_frames_subset(lc3b_encoder* h, const int32_t* stream_ids,
     if (!rt.take(h->id_list, stream_ids, frame_counts, n_rows, st.n_streams, (long long)INT32_MAX)) return LC3B_ERR_INVALID_ARG;
     if (rt.total == 0) return LC3B_OK;
     if (!pcm_in || !frames_out || !scratch) return LC3B_ERR_INVALID_ARG;
-    if (scratch_bytes < enc_multi_rows_scratch_bytes(st, n_rows, rt.total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
+    if (scratch_bytes < enc_multi_scratch_bytes(st, n_rows, rt.total) || ((uintptr_t)scratch & 255) != 0) return LC3B_ERR_WORKSPACE;
     LaunchPlan plan;                                      // the whole call is one plan: one graph launch in graph mode
-    plan_enc_multi_rows(plan, st, pcm_in, n_rows, rt.n_live, rt.total, frames_out, nbytes, frame_stride, scratch);
+    plan_enc_multi(plan, st, pcm_in, n_rows, rt.n_live, rt.total, 0, frames_out, nbytes, frame_stride, scratch);
     cudaStream_t stream = (cudaStream_t)cuda_stream;
     CU(rt.send(scratch, stream));
     CU(h->graph_mode ? plan_launch_graph(h->graphs, plan, stream) : plan_launch_direct(plan, stream));

@@ -71,30 +71,25 @@ struct EncoderState {
 cudaError_t prepare_enc_analysis(const EncoderState& st);   // shared-memory limits of the kernels, once per handle
 cudaError_t prepare_enc_quant(const EncoderState& st);
 int enc_bitstream_scratch_words(int ne, int max_nbytes);   // per-stream size of EncoderState::bs_scratch
-// stages: bit 0 MDCT kernel, bit 1 attack detector + LTPF analysis kernel
-cudaError_t launch_enc_analysis(const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages, cudaStream_t stream);
-// stages: bit 0 SNS kernel (with the bandwidth detector), bit 1 TNS kernel, bit 2 quantise kernel, bit 3 bitstream kernel
-cudaError_t launch_enc_quant(const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages, cudaStream_t stream);
-// the same launches written into a plan (lc3b_plan.cuh) instead of issued.  n_frames > 1: `st` is a view whose
-// st.n_streams = S * n_frames units (unit s * n_frames + f = frame f of stream s) and whose per-frame buffers have a row
-// per unit; its per-stream state (xs_hist, x12, x6, estate) keeps a row per stream.  The attack / LTPF kernel and the
-// quantise kernel then run a warp per stream that walks the stream's frames in order; every other kernel runs per unit.
-// ids (n_frames == 1 only): a subset call, `st` a view whose st.n_streams is the call's row count; row u's persistent state
-// (thist, xs_hist, x12, x6, estate) is that of handle stream ids[u] (device memory), every other buffer has a row per call row.
-// rows: a ragged call, `st` a view of st.n_streams units as with n_frames > 1; the attack / LTPF kernel and the quantise
-// kernel run a warp per row of the device row table (n_rows rows with frames, lc3b_common.cuh), walking the row's units.
+// The encoder's launches, written into a plan (lc3b_plan.cuh).
+// stages of plan_enc_analysis: bit 0 MDCT kernel, bit 1 attack detector + LTPF analysis kernel; of plan_enc_quant: bit 0
+// SNS kernel (with the bandwidth detector), bit 1 TNS kernel, bit 2 quantise kernel, bit 3 bitstream kernels.
+// ids: a subset call, `st` a view whose st.n_streams is the call's row count; row u's persistent state (thist, xs_hist,
+// x12, x6, estate) is that of handle stream ids[u] (device memory), every other buffer has a row per call row.
+// rows: a time-parallel call, `st` a view whose st.n_streams is the call's unit count and whose per-frame buffers have a
+// row per unit; its per-stream state (xs_hist, x12, x6, estate) keeps a row per stream.  The attack / LTPF kernel and
+// the quantise kernel run a warp per row of the device row table (n_rows rows with frames, lc3b_common.cuh), walking the
+// row's units in order; every other kernel runs per unit.
 struct LaunchPlan;
 void plan_enc_analysis(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, size_t pcm_stride, int nbytes, int stages,
-                       int n_frames = 1, const int32_t* ids = nullptr, const int32_t* rows = nullptr, int n_rows = 0);
+                       const int32_t* ids = nullptr, const int32_t* rows = nullptr, int n_rows = 0);
 void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
-                    int n_frames = 1, const int32_t* ids = nullptr, const int32_t* rows = nullptr, int n_rows = 0);
-// time-parallel encode (lc3b_enc_multi.cu): n_frames consecutive frames of every stream as one plan
-size_t enc_multi_scratch_bytes(const EncoderState& st, int n_frames);
-void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_frames, uint8_t* frames_out, int nbytes,
-                    size_t frame_stride, void* scratch);
-// ragged time-parallel encode: n_rows listed rows, `total` units, the row table (n_live rows) at the front of the scratch
-size_t enc_multi_rows_scratch_bytes(const EncoderState& st, int n_rows, long long total);
-void plan_enc_multi_rows(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_rows, int n_live, long long total,
-                         uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch);
+                    const int32_t* ids = nullptr, const int32_t* rows = nullptr, int n_rows = 0);
+// time-parallel encode (lc3b_enc_multi.cu) as one plan: n_rows listed rows, `total` units.  dense_frames > 0: a dense
+// call, n_rows = n_live = the handle's streams of dense_frames frames each, whose row table the plan writes itself;
+// otherwise the row table (n_live rows with frames) is at the front of the scratch (RowTable::send).
+size_t enc_multi_scratch_bytes(const EncoderState& st, int n_rows, long long total);
+void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_rows, int n_live, long long total,
+                    int dense_frames, uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch);
 
 }  // namespace lc3b

@@ -1,24 +1,25 @@
-// lc3b engine: time-parallel encode - many consecutive frames of every stream in ONE call (lc3b_encode_stream_frames).
+// lc3b engine: time-parallel encode - many consecutive frames of many streams in ONE call (lc3b_encode_stream_frames and
+// lc3b_encode_stream_frames_subset).
 //
 // Of the encoder's per-stream state (EncoderState) only three groups really run along time:
 //   * the attack envelope, the 50 Hz biquad of the LTPF analysis and its pitch / activation memory (enc_ltpf_kernel)
 //   * the rate loop's offsets (ES_Q_*, enc_quantize_kernel)
 // The MDCT time-buffer history of frame f is the tail of frame f - 1's own input, and everything else is a per-frame
-// hand-off record between kernels.  So a call with F frames of S streams runs as S*F independent "units" through the
-// unchanged kernels and touches the time axis only where it must:
-//   1. enc_thist_prefill_kernel  each unit's MDCT history: the handle's for f = 0, else the previous frame's last nf - z samples
-//   2. enc_mdct_kernel           over the S*F units (pcm row of unit s*F + f = frame f of stream s)
-//   3. enc_thist_handback_kernel the last unit's history back into the handle
-//   4. enc_ltpf_kernel           a warp per stream walks its F frames (per-stream state stays in the handle)
+// hand-off record between kernels.  A call lists rows in a row table (lc3b_common.cuh): row i advances handle stream row_i
+// by count_i consecutive frames, units off_i .. off_i + count_i - 1.  The subset call sends its table; the dense call is
+// the identity table of S rows of F frames, which unit_rows_kernel writes on the device.  The units run independently
+// through the unchanged kernels and the time axis is touched only where it must be:
+//   0. unit_rows_kernel          unit_row[v], the state row of each unit's row (plan_unit_rows, lc3b_dec_multi.cu)
+//   1. enc_thist_prefill_kernel  each unit's MDCT history: the handle's for a row's first unit, else the previous frame's
+//                                last nf - z samples
+//   2. enc_mdct_kernel           over the units (pcm row v = unit v)
+//   3. enc_thist_handback_kernel each row's last unit's history back into the handle
+//   4. enc_ltpf_kernel           a warp per row walks its frames (per-stream state stays in the handle)
 //   5. enc_sns_kernel, enc_tns_kernel over the units
-//   6. enc_quantize_kernel       a warp per stream walks its F frames
-//   7. bitstream prepare / range coder / finish over the units; unit s*F + f writes frames_out + (s*F + f)*frame_stride
+//   6. enc_quantize_kernel       a warp per row walks its frames
+//   7. bitstream prepare / range coder / finish over the units; unit v writes frames_out + v * frame_stride
 // The per-frame buffers of the units live in the caller's scratch; the handle's own per-frame buffers (what
 // lc3b_encoder_debug_read reports) are not touched.  Arithmetic is the frame-by-frame path's, so the bytes are identical.
-//
-// A ragged call (lc3b_encode_stream_frames_subset) lists rows of any frame counts: kernels 1 and 3 find a unit's row in
-// unit_row[] (plan_unit_rows, lc3b_dec_multi.cu), kernels 4 and 6 walk the rows of the row table (lc3b_common.cuh), the
-// rest runs over the units unchanged.
 #include "lc3b_enc_common.cuh"
 #include "lc3b_plan.cuh"
 
@@ -26,13 +27,13 @@ namespace lc3b {
 
 struct EncMultiLayout { size_t rows, thist, xf, e_b, ehand, xq, qhand, lsbs, bs_scratch, unit_row, total; };
 
-// V units of n_rows rows; ragged: the row table at the front (where RowTable::send puts it) and unit_row[V] at the end
-static EncMultiLayout enc_multi_layout(const EncoderState& st, int n_rows, size_t V, bool ragged) {
+// V units of n_rows rows: the row table at the front (where RowTable::send puts it) and unit_row[V] at the end
+static EncMultiLayout enc_multi_layout(const EncoderState& st, int n_rows, size_t V) {
     EncMultiLayout L;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off = (off + bytes + 255) & ~(size_t)255; return o; };
     const lc3b_config& c = st.cfg;
-    L.rows = take(ragged ? sizeof(int32_t) * RT_WORDS * n_rows : 0);
+    L.rows = take(sizeof(int32_t) * RT_WORDS * n_rows);
     L.thist = take(sizeof(int16_t) * V * (c.nf - c.z));
     L.xf = take(sizeof(float) * V * c.ne);
     L.e_b = take(sizeof(float) * V * 64);
@@ -41,61 +42,46 @@ static EncMultiLayout enc_multi_layout(const EncoderState& st, int n_rows, size_
     L.qhand = take(sizeof(int32_t) * V * QH_WORDS);
     L.lsbs = take(V * 2 * c.ne);
     L.bs_scratch = take(sizeof(uint32_t) * V * (size_t)st.bs_words);
-    L.unit_row = take(ragged ? sizeof(int32_t) * V : 0);
+    L.unit_row = take(sizeof(int32_t) * V);
     L.total = off;
     return L;
 }
 
-size_t enc_multi_scratch_bytes(const EncoderState& st, int n_frames) {
-    return enc_multi_layout(st, st.n_streams, (size_t)st.n_streams * (size_t)n_frames, false).total;
-}
-size_t enc_multi_rows_scratch_bytes(const EncoderState& st, int n_rows, long long total) {
-    return enc_multi_layout(st, n_rows, (size_t)total, true).total;
+size_t enc_multi_scratch_bytes(const EncoderState& st, int n_rows, long long total) {
+    return enc_multi_layout(st, n_rows, (size_t)total).total;
 }
 
 struct ThistParams {
-    const int16_t* pcm;      // [S][F * nf]
+    const int16_t* pcm;      // [V][nf]
     int16_t* hist;           // the handle's [S][nf - z]
-    int16_t* thist_v;        // [S * F][nf - z]
-    int S, F, nf, z;
-    // ragged call: S = rows of the row table, V units; unit_row[v] the state row of unit v's row, ~row for its first unit
+    int16_t* thist_v;        // [V][nf - z]
+    int n_rows, nf, z;       // rows of the row table
     const int32_t* rows;
-    const int32_t* unit_row;
+    const int32_t* unit_row; // [V] the state row of unit v's row, ~row for its first unit
     size_t V;
 };
 
-// update_time_buffer (modified_dct.rs:126-138) keeps the last nf - z input samples: for unit (s, f > 0) those are
-// pcm[s][(f - 1) nf + z, f nf), known before any kernel runs
-template <bool RAGGED>
+// update_time_buffer (modified_dct.rs:126-138) keeps the last nf - z input samples: for a unit v that is not its row's
+// first, those are pcm[(v - 1) nf + z, v nf), known before any kernel runs
 __global__ void __launch_bounds__(256) enc_thist_prefill_kernel(ThistParams p) {
     const int L = p.nf - p.z;
-    const size_t n_all = (RAGGED ? p.V : (size_t)p.S * p.F) * L;
+    const size_t n_all = p.V * L;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_all; i += (size_t)gridDim.x * blockDim.x) {
         const size_t v = i / L;
         const int n = (int)(i - v * L);
-        if constexpr (RAGGED) {
-            const int u = p.unit_row[v];
-            p.thist_v[i] = u >= 0 ? p.pcm[(v - 1) * p.nf + p.z + n] : p.hist[(size_t)~u * L + n];
-        } else {
-            const int f = (int)(v % p.F);
-            p.thist_v[i] = f ? p.pcm[(v - 1) * p.nf + p.z + n] : p.hist[(v / p.F) * L + n];
-        }
+        const int u = p.unit_row[v];
+        p.thist_v[i] = u >= 0 ? p.pcm[(v - 1) * p.nf + p.z + n] : p.hist[(size_t)~u * L + n];
     }
 }
 
 // the history of each row's last unit back to its state row
-template <bool RAGGED>
 __global__ void __launch_bounds__(256) enc_thist_handback_kernel(ThistParams p) {
     const int L = p.nf - p.z;
-    const size_t n_all = (size_t)p.S * L;
+    const size_t n_all = (size_t)p.n_rows * L;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_all; i += (size_t)gridDim.x * blockDim.x) {
         const size_t s = i / L;
-        if constexpr (RAGGED) {
-            const RowSpan rs = row_span<true>(p.rows, (int)s, 0);
-            p.hist[(size_t)rs.row * L + (i - s * L)] = p.thist_v[((size_t)rs.off + rs.count - 1) * L + (i - s * L)];
-        } else {
-            p.hist[i] = p.thist_v[((s + 1) * p.F - 1) * L + (i - s * L)];
-        }
+        const RowSpan rs = row_span(p.rows, (int)s);
+        p.hist[(size_t)rs.row * L + (i - s * L)] = p.thist_v[((size_t)rs.off + rs.count - 1) * L + (i - s * L)];
     }
 }
 
@@ -104,12 +90,10 @@ static unsigned copy_grid(size_t n) {
     return (unsigned)(g < 4096 ? g : 4096);
 }
 
-// The dense call (rows == nullptr: S rows of F frames) and the ragged one (the n_live rows of the row table at the front
-// of the scratch, V units in all; the layout counts n_rows rows) share everything but the row addressing.
-static void plan_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int F, bool ragged, int n_rows, int n_live,
-                       size_t V, uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch) {
-    const int S = st.n_streams;
-    const EncMultiLayout L = enc_multi_layout(st, n_rows, V, ragged);
+void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_rows, int n_live, long long total,
+                    int dense_frames, uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch) {
+    const size_t V = (size_t)total;
+    const EncMultiLayout L = enc_multi_layout(st, n_rows, V);
     uint8_t* base = (uint8_t*)scratch;
     // a view of the handle with V units: per-frame buffers in the scratch, per-stream state the handle's
     EncoderState vs = st;
@@ -124,35 +108,15 @@ static void plan_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* 
     vs.bs_scratch = (uint32_t*)(base + L.bs_scratch);
     const size_t hist_len = (size_t)(st.cfg.nf - st.cfg.z);
     const size_t nf = (size_t)st.cfg.nf;
-    if (!ragged) {
-        const ThistParams tp{pcm, st.thist, vs.thist, S, F, st.cfg.nf, st.cfg.z, nullptr, nullptr, 0};
-        plan.add(enc_thist_prefill_kernel<false>, copy_grid((size_t)S * F * hist_len), 256, 0, tp);
-        plan_enc_analysis(plan, vs, pcm, nf, nbytes, 1, F);
-        plan.add(enc_thist_handback_kernel<false>, copy_grid((size_t)S * hist_len), 256, 0, tp);
-        plan_enc_analysis(plan, vs, pcm, nf, nbytes, 2, F);
-        plan_enc_quant(plan, vs, frames_out, nbytes, frame_stride, 15, F);
-        return;
-    }
-    const int32_t* rows = (const int32_t*)(base + L.rows);
+    int32_t* rows = (int32_t*)(base + L.rows);
     int32_t* unit_row = (int32_t*)(base + L.unit_row);
-    const ThistParams tp{pcm, st.thist, vs.thist, n_live, 0, st.cfg.nf, st.cfg.z, rows, unit_row, V};
-    plan_unit_rows(plan, rows, n_live, unit_row);
-    plan.add(enc_thist_prefill_kernel<true>, copy_grid(V * hist_len), 256, 0, tp);
+    const ThistParams tp{pcm, st.thist, vs.thist, n_live, st.cfg.nf, st.cfg.z, rows, unit_row, V};
+    plan_unit_rows(plan, rows, n_live, dense_frames, unit_row);
+    plan.add(enc_thist_prefill_kernel, copy_grid(V * hist_len), 256, 0, tp);
     plan_enc_analysis(plan, vs, pcm, nf, nbytes, 1);
-    plan.add(enc_thist_handback_kernel<true>, copy_grid((size_t)n_live * hist_len), 256, 0, tp);
-    plan_enc_analysis(plan, vs, pcm, nf, nbytes, 2, 1, nullptr, rows, n_live);
-    plan_enc_quant(plan, vs, frames_out, nbytes, frame_stride, 15, 1, nullptr, rows, n_live);
-}
-
-void plan_enc_multi(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_frames, uint8_t* frames_out, int nbytes,
-                    size_t frame_stride, void* scratch) {
-    plan_multi(plan, st, pcm, n_frames, false, st.n_streams, st.n_streams, (size_t)st.n_streams * n_frames, frames_out, nbytes,
-               frame_stride, scratch);
-}
-
-void plan_enc_multi_rows(LaunchPlan& plan, const EncoderState& st, const int16_t* pcm, int n_rows, int n_live, long long total,
-                         uint8_t* frames_out, int nbytes, size_t frame_stride, void* scratch) {
-    plan_multi(plan, st, pcm, 0, true, n_rows, n_live, (size_t)total, frames_out, nbytes, frame_stride, scratch);
+    plan.add(enc_thist_handback_kernel, copy_grid((size_t)n_live * hist_len), 256, 0, tp);
+    plan_enc_analysis(plan, vs, pcm, nf, nbytes, 2, nullptr, rows, n_live);
+    plan_enc_quant(plan, vs, frames_out, nbytes, frame_stride, 15, nullptr, rows, n_live);
 }
 
 }  // namespace lc3b

@@ -37,7 +37,6 @@ namespace lc3b {
 struct QuantParams {
     const EncConfig* cfg;
     int n_streams, nbytes;
-    int n_frames;      // enc_quantize_kernel: consecutive frames each warp walks; its frame f is unit s * n_frames + f
     size_t frame_stride;
     float* xf;
     const float* e_b;
@@ -52,6 +51,7 @@ struct QuantParams {
     int w_bytes, w_bytes_fin, side_words, sym_cap, out_words;     // per-warp shared-memory slices (prepare / finish kernels)
     int inline_ac;     // small batches: the finish kernel runs the range coder itself (all lanes, same chain) and C2 is skipped
     const int32_t* ids;   // subset call: row u's rate-loop state is that of handle stream ids[u] (enc_quantize_kernel<false, true>)
+    const int32_t* rows;  // time-parallel call: the row table (lc3b_common.cuh), n_streams its rows (enc_quantize_kernel<true, true>)
 };
 
 constexpr int QW = 8;                       // frames (warps) per CTA
@@ -1508,14 +1508,13 @@ __global__ void __launch_bounds__(QNT_THREADS, 4) enc_tns_kernel(QuantParams p) 
     if (lane < 16) qh[QH_RC_I + lane] = tns.rc_i[lane];
 }
 
-// Kernel B: SpectralQuantization::run.  Shaped spectrum -> quantised spectrum + gain decisions.  WALK: a warp per stream
-// walks p.n_frames frames in order, the rate loop's offsets (ES_Q_*) carrying from one frame to the next; otherwise one
-// frame (lc3b_encode_frames: a separate instantiation, so the frame-by-frame path keeps its registers).  Every warp of a
-// CTA walks the same count, so the named barriers inside a frame stay matched.
-// WALK and IDS: a ragged call, p.ids its row table, a warp per row walking the row's own count.  As in enc_ltpf_kernel the
-// table is sorted by count, descending: the warps that still have frame f are warps 0 .. n_live - 1 (n_live = the CTA's
-// rows with count > f, recounted every frame), the barriers count exactly them and warp 0 does the ordered sums of
-// lanes < n_live.
+// Kernel B: SpectralQuantization::run.  Shaped spectrum -> quantised spectrum + gain decisions.  One frame per warp
+// (lc3b_encode_frames; IDS: lc3b_encode_frames_subset), or, WALK (always with IDS: a row's state row comes from the row
+// table), a warp per row of a time-parallel call's row table walking the row's frames in order, the rate loop's offsets
+// (ES_Q_*) carrying from one frame to the next.  The walk is a separate instantiation, so the frame-by-frame path keeps
+// its registers.  As in enc_ltpf_kernel the table is sorted by count, descending: the warps that still have frame f are
+// warps 0 .. n_live - 1 (n_live = the CTA's rows with count > f, recounted every frame), the barriers count exactly them
+// and warp 0 does the ordered sums of lanes < n_live.
 template <bool WALK, bool IDS>
 __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p) {
     extern __shared__ __align__(16) uint8_t smem[];
@@ -1529,15 +1528,15 @@ __global__ void __launch_bounds__(QNT_THREADS) enc_quantize_kernel(QuantParams p
     float* e4 = xf + NE_MAX;                                      // [100]
     float* T = e4 + 100;                                          // [224]
     int16_t* xq = (int16_t*)(T + 224);                            // [NE_MAX]
-    constexpr bool RAGGED = WALK && IDS;
-    const RowSpan rs = row_span<RAGGED>(p.ids, stream, 0);
-    int32_t* es = p.estate + (size_t)(RAGGED ? rs.row : state_row<IDS>(p.ids, stream)) * ES_WORDS;
+    static_assert(!WALK || IDS, "the row walk addresses state through the row table");
+    const RowSpan rs = WALK ? row_span(p.rows, stream) : RowSpan{state_row<IDS>(p.ids, stream), stream, 1};
+    int32_t* es = p.estate + (size_t)rs.row * ES_WORDS;
     const int n_cta = min(QW, p.n_streams - blockIdx.x * QW);     // warps of this CTA that have a frame
-    const int cnt = RAGGED && lane < n_cta ? row_span<RAGGED>(p.ids, blockIdx.x * QW + lane, 0).count : 0;   // lane j: warp j's
-    const int F = RAGGED ? rs.count : WALK ? p.n_frames : 1;
+    const int cnt = WALK && lane < n_cta ? row_span(p.rows, blockIdx.x * QW + lane).count : 0;   // lane j: warp j's
+    const int F = WALK ? __reduce_max_sync(0xffffffffu, rs.count) : 1;   // uniform registers, see enc_ltpf_kernel
     for (int f = 0; f < F; f++) {
-        const int n_live = RAGGED ? __popc(__ballot_sync(0xffffffffu, cnt > f)) : n_cta;
-        const size_t unit = RAGGED ? (size_t)rs.off + f : (size_t)stream * F + f;
+        const int n_live = WALK ? (int)__reduce_add_sync(0xffffffffu, cnt > f ? 1u : 0u) : n_cta;
+        const size_t unit = (size_t)rs.off + f;
         const float4* gx = (const float4*)(p.xf + unit * ne);
         WARP_STRIDE(i, ne / 4) ((float4*)xf)[i] = gx[i];
         __syncwarp();
@@ -1735,7 +1734,6 @@ cudaError_t prepare_enc_quant(const EncoderState& st) {
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_tns_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SHAPE_SMEM);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(enc_quantize_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)QUANTIZE_SMEM);
     if (e == cudaSuccess)
         e = cudaFuncSetAttribute(enc_bs_prepare_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -1744,12 +1742,11 @@ cudaError_t prepare_enc_quant(const EncoderState& st) {
 }
 
 void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages,
-                    int n_frames, const int32_t* ids, const int32_t* rows, int n_rows) {
+                    const int32_t* ids, const int32_t* rows, int n_rows) {
     QuantParams p;
     memset(&p, 0, sizeof(p));
     p.cfg = st.ecfg;
     p.n_streams = st.n_streams;
-    p.n_frames = 1;
     p.nbytes = nbytes;
     p.frame_stride = frame_stride;
     p.xf = st.xf;
@@ -1764,16 +1761,15 @@ void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_ou
     p.inline_ac = 0;
     p.frames_out = frames_out;
     p.ids = ids;
+    p.rows = rows;
     const size_t wbytes = bitstream_warp_bytes(st.cfg.ne, nbytes, &p);
     const int grid = (p.n_streams + QW - 1) / QW;
     if (stages & 1) plan.add(enc_sns_kernel, (unsigned)((p.n_streams + SNS_WARPS - 1) / SNS_WARPS), SNS_WARPS * 32, SHAPE_SMEM / QW * SNS_WARPS, p);
     if (stages & 2) plan.add(enc_tns_kernel, (unsigned)grid, QNT_THREADS, SHAPE_SMEM, p);
-    if (stages & 4) {                                              // one warp per stream (or row), walking its frames
+    if (stages & 4) {                                              // one warp per frame, or per row walking its frames
         QuantParams pw = p;
-        pw.n_streams = rows ? n_rows : st.n_streams / n_frames;
-        pw.n_frames = n_frames;
-        if (rows) pw.ids = rows;
-        plan.add(rows ? enc_quantize_kernel<true, true> : n_frames > 1 ? enc_quantize_kernel<true, false> : ids ? enc_quantize_kernel<false, true> : enc_quantize_kernel<false, false>,
+        if (rows) pw.n_streams = n_rows;
+        plan.add(rows ? enc_quantize_kernel<true, true> : ids ? enc_quantize_kernel<false, true> : enc_quantize_kernel<false, false>,
                  (unsigned)((pw.n_streams + QW - 1) / QW), QNT_THREADS, QUANTIZE_SMEM, pw);
     }
     if (stages & 8) {
@@ -1783,12 +1779,6 @@ void plan_enc_quant(LaunchPlan& plan, const EncoderState& st, uint8_t* frames_ou
         if (!p.inline_ac) plan.add(enc_range_coder_kernel, (unsigned)((p.n_streams + 127) / 128), 128, 0, p);
         plan.add(enc_bs_finish_kernel, (unsigned)grid, QNT_THREADS, QW * (size_t)p.w_bytes_fin, p);
     }
-}
-
-cudaError_t launch_enc_quant(const EncoderState& st, uint8_t* frames_out, int nbytes, size_t frame_stride, int stages, cudaStream_t stream) {
-    LaunchPlan plan;
-    plan_enc_quant(plan, st, frames_out, nbytes, frame_stride, stages);
-    return plan_launch_direct(plan, stream);
 }
 
 }  // namespace lc3b
